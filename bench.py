@@ -60,7 +60,41 @@ def parse():
     p.add_argument("--no-ref-python", action="store_true", help="skip timing the unmodified reference package (baseline/_ref)")
     p.add_argument("--ref-python-its", type=int, default=10001, help="iterations per reference chain (one chain per host core)")
     p.add_argument("--no-other-configs", action="store_true", help="skip BASELINE configs 3-5 / strong scaling (other_configs)")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float32 / float64, "
+                        f"at most {DUMP_BYTES >> 20} MB in all; an array over its share keeps a fixed, seeded sample of its "
+                        "chains); rank 0 only")
+    a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        p.error("--dump-outputs: the reference arm sizes its sample by the host's speed, so its outputs differ from run to run")
+    return a
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """arrays: name -> (tensor, chain axis or None).  Writes out_dir/<name>.npy.  Each array gets an equal share of
+    DUMP_BYTES; a larger one keeps the chains of a fixed permutation's head (sorted), so the same arguments dump the same
+    chains in every run and the smaller samples are subsets of the larger ones."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // len(arrays)
+    for name, (t, axis) in arrays.items():
+        t = t.detach()
+        if t.dtype not in (torch.float32, torch.float64):
+            t = t.float()
+        if axis is not None and t.numel() * t.element_size() > share:
+            n = t.shape[axis]
+            keep = share // (t.numel() // n * t.element_size())
+            if keep < 1:
+                raise ValueError(f"--dump-outputs: one chain of '{name}' {tuple(t.shape)} is larger than {share} bytes")
+            idx = np.sort(np.random.default_rng(0).permutation(n)[:keep])
+            t = t.index_select(axis, torch.from_numpy(idx).to(t.device))
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
 
 
 class ClockSampler:
@@ -229,7 +263,7 @@ def bench_kde(a, rank, world, local_rank):
 
     def one_step():
         weights, bw = eng.kde_fit(X, w)
-        return eng.kde_log_prob(X, weights, bw, x)
+        return weights, bw, eng.kde_log_prob(X, weights, bw, x)
 
     def barrier():
         if world > 1:
@@ -245,9 +279,11 @@ def bench_kde(a, rank, world, local_rank):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(a.steps):
-        out = one_step()
+        fit_w, fit_bw, out = one_step()
     e1.record()
     barrier()
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, {"weights": (fit_w, 0), "bandwidth": (fit_bw, None), "log_prob": (out, 0)})
     sampler.rows = sampler.rows[max(0, n_idle - 1):]
     clocks = sampler.stop()
     ms = torch.tensor([e0.elapsed_time(e1)], device="cuda", dtype=torch.float64)
@@ -388,6 +424,8 @@ def bench_shared(a, rank, world, local_rank):
         _, st = call(z_dev, a.warmup + s)
     e1.record()
     barrier()
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, {"stats": (st.raw, 0)})
     n_launch_calls = eng.ctx.n_calls - calls0    # every one launches at least one kernel of libglabc.so (3 binds per call aside)
     sampler.rows = sampler.rows[max(0, n_idle - 1):]
     clocks = sampler.stop()
@@ -921,6 +959,16 @@ def _main():
     last_seed = a.warmup + a.steps - 1
     first64 = trace[:64].clone() if (layout == abi.TRACE_CHAIN_MAJOR and entry == "global" and C >= 64) else None
     value = steps_per_pass * a.steps / (total_ms * 1e-3)
+    if a.dump_outputs and rank == 0:
+        # before the kernel-only timings below overwrite the state, stats and trace
+        outs = {"theta": (theta, 0), "y": (y, 0), "stats": (stats, 0), "summary": (summary, None)}
+        if trace is not None:
+            outs["trace"] = (trace, 0 if layout == abi.TRACE_CHAIN_MAJOR else 1)
+        if aux is not None:
+            outs["aux"] = (aux, 0)
+        if s64 is not None:
+            outs["state64"] = (s64, 0)
+        dump_outputs(a.dump_outputs, outs)
 
     # the step kernel alone (no state reset / summary kernels around it)
     for s in range(min(a.steps, 20)):

@@ -226,7 +226,7 @@ def test_public_api_glmcmc(eng, tmp_path):
     assert np.allclose(g.esjd(out), st.esjd().cpu().numpy(), rtol=1e-4, atol=1e-7)
 
 
-def test_esjd_sweep(eng):
+def test_esjd_sweep(eng, tmp_path):
     """examples/Mixture_hyper.py:23-41: ESJD / time over a global_frequency grid; for the README model the global (iSIR)
     move dominates the score, so the best grid point is at the high end (the reference's own sweep picks gf >= 0.8)"""
     import glabc_b200 as g
@@ -234,7 +234,7 @@ def test_esjd_sweep(eng):
     model = g.Mixture_set(epsilon=0.05)
     lp = g.DiagGaussian(2, loc=torch.zeros(1, 2), log_scale=torch.log(torch.tensor([0.35, 0.35])))
     ip = g.DiagGaussian(2, torch.tensor([0.0, 0.0]), torch.tensor([0.0, 0.0]))
-    runner = g.MCMCRunner(model, output_dir="/tmp")
+    runner = g.MCMCRunner(model, output_dir=str(tmp_path))
     best, table = esjd_sweep(lambda gf, **kw: runner.run_glmcmc(1000, torch.zeros(2), None, gf, lp, ip, 5, output_file=None, **kw),
                              grid=[0.0, 0.5, 0.9, 1.0], num_chains=4096)
     assert table.shape == (4, 4) and best >= 0.5
