@@ -1,8 +1,6 @@
-// Host launchers of K4 (RealNVP flow on tcgen05 tensor cores, flow.cuh).
+// Host launchers of K4 (RealNVP flow on tcgen05 tensor cores: flow.cuh, flow_pipe.cuh).
 #include "flow.cuh"
 #include "flow_pipe.cuh"
-
-#include <cstdlib>
 
 namespace glabc {
 
@@ -22,88 +20,47 @@ cudaError_t launch_flow_pack_aux(const float* w1, const float* b1, const float* 
     return cudaGetLastError();
 }
 
-// GLABC_FLOW_FAST: the warp-specialised pipeline (flow_pipe.cuh); GLABC_FLOW_PIPE=0 in the environment selects k_flow<., false>
-static bool use_pipe()
-{
-    static const bool on = [] {
-        const char* e = std::getenv("GLABC_FLOW_PIPE");
-        return !(e && e[0] == '0');
-    }();
-    return on;
-}
-
 cudaError_t launch_flow(const FlowDev& W, bool sample, bool precise, const float* in, int64_t n, float* out_theta, float* out_lq,
                         int sm_count, cudaStream_t st)
 {
     if (n <= 0) return cudaSuccess;
-    if (precise && (!kFlowF16 || W.w2p_lo == nullptr)) return cudaErrorInvalidValue;
+    if (W.aux == nullptr || (precise && W.w2p_lo == nullptr)) return cudaErrorInvalidValue;
     static bool configured = false;
     if (!configured) {
-        cudaError_t e = cudaFuncSetAttribute(k_flow<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFlowSmemBytes);
+        cudaError_t e = cudaFuncSetAttribute(k_flow_pipe<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPipeSmemBytes);
         if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(k_flow<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFlowSmemBytes);
+        e = cudaFuncSetAttribute(k_flow_pipe<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPipeSmemBytes);
         if (e != cudaSuccess) return e;
-        if constexpr (kFlowF16) {
-            e = cudaFuncSetAttribute(k_flow<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFlowSmemBytesPrecise);
-            if (e != cudaSuccess) return e;
-            e = cudaFuncSetAttribute(k_flow<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFlowSmemBytesPrecise);
-            if (e != cudaSuccess) return e;
-        }
-        if constexpr (kFlowF16) {
-            e = cudaFuncSetAttribute(k_flow_pipe<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPipeSmemBytes);
-            if (e != cudaSuccess) return e;
-            e = cudaFuncSetAttribute(k_flow_pipe<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPipeSmemBytes);
-            if (e != cudaSuccess) return e;
-            e = cudaFuncSetAttribute(k_flow_pipe_precise<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPipePSmemBytes);
-            if (e != cudaSuccess) return e;
-            e = cudaFuncSetAttribute(k_flow_pipe_precise<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPipePSmemBytes);
-            if (e != cudaSuccess) return e;
-        }
+        e = cudaFuncSetAttribute(k_flow_pipe_precise<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPipePSmemBytes);
+        if (e != cudaSuccess) return e;
+        e = cudaFuncSetAttribute(k_flow_pipe_precise<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPipePSmemBytes);
+        if (e != cudaSuccess) return e;
         configured = true;
     }
-    // tiles per chunk: at most what the shared-memory state holds, sized so that the chunks divide evenly over the SMs (an
-    // even number: one tile per group at least)
+    // tiles per chunk: at most what the shared-memory state holds, sized so that the chunks divide evenly over the SMs, rounded
+    // up to an even count (the pipelines' measured throughput was taken with this geometry)
     const int64_t tiles = (n + kFlowTile - 1) / kFlowTile;
     const int64_t waves = (tiles + int64_t(sm_count) * kFlowTilesPerCta - 1) / (int64_t(sm_count) * kFlowTilesPerCta);
     int64_t tpc = (tiles + sm_count * waves - 1) / (sm_count * waves);   // every SM gets `waves` chunks of (almost) equal size
     tpc = (tpc + 1) / 2 * 2;
     if (tpc < 2) tpc = 2;
     if (tpc > kFlowTilesPerCta) tpc = kFlowTilesPerCta;
-    const bool pipe = kFlowF16 && W.aux != nullptr && use_pipe();
-    if (pipe && tpc < kPipeMinTiles) tpc = kPipeMinTiles;   // the update runs kPipeLag tiles behind layer 1
+    if (tpc < kPipeMinTiles) tpc = kPipeMinTiles;   // the pipelines' smallest chunk (flow_pipe.cuh)
     const int64_t chunks = (tiles + tpc - 1) / tpc;
     const unsigned grid = static_cast<unsigned>(chunks < sm_count ? chunks : sm_count);  // persistent: one CTA per SM
-    if constexpr (kFlowF16) {
-        if (pipe && precise) {
-            if (sample) k_flow_pipe_precise<true><<<grid, 18 * 32, kPipePSmemBytes, st>>>(W, in, n, out_theta, out_lq, static_cast<int>(tpc));
-            else k_flow_pipe_precise<false><<<grid, 18 * 32, kPipePSmemBytes, st>>>(W, in, n, out_theta, out_lq, static_cast<int>(tpc));
-            return cudaGetLastError();
-        }
-        if (pipe) {
-            if (sample) k_flow_pipe<true><<<grid, kPipeThreads, kPipeSmemBytes, st>>>(W, in, n, out_theta, out_lq, static_cast<int>(tpc));
-            else k_flow_pipe<false><<<grid, kPipeThreads, kPipeSmemBytes, st>>>(W, in, n, out_theta, out_lq, static_cast<int>(tpc));
-            return cudaGetLastError();
-        }
+    if (precise) {
+        if (sample) k_flow_pipe_precise<true><<<grid, 18 * 32, kPipePSmemBytes, st>>>(W, in, n, out_theta, out_lq, static_cast<int>(tpc));
+        else k_flow_pipe_precise<false><<<grid, 18 * 32, kPipePSmemBytes, st>>>(W, in, n, out_theta, out_lq, static_cast<int>(tpc));
+    } else {
+        if (sample) k_flow_pipe<true><<<grid, kPipeThreads, kPipeSmemBytes, st>>>(W, in, n, out_theta, out_lq, static_cast<int>(tpc));
+        else k_flow_pipe<false><<<grid, kPipeThreads, kPipeSmemBytes, st>>>(W, in, n, out_theta, out_lq, static_cast<int>(tpc));
     }
-    if constexpr (kFlowF16) {
-        if (precise) {
-            if (sample) k_flow<true, true><<<grid, kFlowThreads, kFlowSmemBytesPrecise, st>>>(W, in, n, out_theta, out_lq, static_cast<int>(tpc));
-            else k_flow<false, true><<<grid, kFlowThreads, kFlowSmemBytesPrecise, st>>>(W, in, n, out_theta, out_lq, static_cast<int>(tpc));
-            return cudaGetLastError();
-        }
-    }
-    if (sample) k_flow<true, false><<<grid, kFlowThreads, kFlowSmemBytes, st>>>(W, in, n, out_theta, out_lq, static_cast<int>(tpc));
-    else k_flow<false, false><<<grid, kFlowThreads, kFlowSmemBytes, st>>>(W, in, n, out_theta, out_lq, static_cast<int>(tpc));
     return cudaGetLastError();
 }
 
 }  // namespace glabc
 
 #ifdef GLABC_FLOW_TRACE
-extern "C" __attribute__((visibility("default"))) int glabc_debug_flow_trace(long long* out)
-{
-    return static_cast<int>(cudaMemcpyFromSymbol(out, glabc::g_flow_trace, sizeof(glabc::g_flow_trace)));
-}
 extern "C" __attribute__((visibility("default"))) int glabc_debug_pipe_trace(long long* out)
 {
     return static_cast<int>(cudaMemcpyFromSymbol(out, glabc::g_pipe_trace, sizeof(glabc::g_pipe_trace)));

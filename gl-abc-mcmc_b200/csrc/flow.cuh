@@ -2,24 +2,22 @@
 // pieces restated in SURVEY.md Appendix C): 32 x [AffineCouplingBlock(MLP([1,128,128,2])), Permute(swap)] over a
 // trainable DiagGaussian(2) base.  sample(n) and log_prob(x) for large batches.
 //
-// The dense piece — the 128x128 hidden layer of every coupling MLP — runs on the 5th-generation tensor cores:
-//   * a CTA holds two groups of 128 threads; a group owns tiles of 128 samples = the 128 TMEM lanes of an M=128
-//     accumulator (each group has its own A buffer, accumulator columns and mbarrier, so one group's MMA overlaps the
-//     other's CUDA-core phases);
-//   * per coupling block: thread r computes row r of A = relu(w1 * z1[r] + b1) (the 1->128 layer is a K=1 outer
-//     product: CUDA cores) straight into shared memory in the UMMA K-major core-matrix layout, one elected thread
-//     issues 16 x tcgen05.mma.kind::tf32 (M128 N128 K8, FP32 accumulate in TMEM) against W2 (pre-packed in the
-//     same layout, fetched per block with one cp.async.bulk into shared memory), tcgen05.commit -> mbarrier;
-//   * epilogue: each warp pulls its 32 lanes x 128 columns back with tcgen05.ld, adds b2, ReLU, and contracts
-//     with the two rows of W3 (N=2: CUDA cores) -> (shift, log-scale) -> affine update of z2, log-det, swap.
-//   * W2 of a block is reused for kFlowTilesPerCta tiles (2,048 samples) before the next block's weights are
-//     fetched, so weight traffic is 1 KB per sample from L2, nothing from HBM (the whole flow is 2.1 MB).
-//   * the A operand goes registers -> TMEM (tcgen05.st) and is consumed by the TS form of tcgen05.mma: at 4 bytes per
-//     TF32 element, writing and re-reading a 64 KB A tile through shared memory costs as many smem cycles as the MMA
-//     takes tensor cycles.
-// TF32 operands: sample() and log_prob() evaluate the SAME deterministic network (same kernel, same rounding), so
-// the log-density returned for a sample is the exact density of the map that produced it — importance weights stay
-// exact whatever the operand precision; only the agreement with an fp32 evaluation of the weights is ~1e-3.
+// What the flow kernels share: the sizes, the device view of the weights (FlowDev), W2's packing into the UMMA operand
+// layout (k_flow_pack), and thin wrappers over the mbarrier, bulk-copy, tcgen05 (MMA, TMEM load / store) and FP16 pack
+// instructions.  The forward kernels (sample, log_prob; FAST and PRECISE) are k_flow_pipe / k_flow_pipe_precise in
+// flow_pipe.cuh, the training step's backward sweep is k_flow_bwd in flow_train.cuh.
+//
+// The 128 x 128 hidden layer of every coupling MLP runs on the tensor cores with FP16 operands (kind::f16, FP32 accumulate):
+// FP16 and TF32 carry the same 10-bit mantissa, but kind::f16 runs at twice the tensor rate, and ReLU + saturation + rounding
+// + packing of TWO activations is ONE instruction (F2FP.SATFINITE.RELU.F16.F32.PACK_AB).  Activations beyond 65504 saturate
+// instead of overflowing.  sample() and log_prob() evaluate the SAME deterministic network (same roundings), so the
+// log-density returned for a sample is the exact density of the map that produced it — importance weights stay exact
+// whatever the operand precision; only the agreement with an fp32 evaluation of the weights is ~1e-3 (FAST mode).
+// PRECISE mode (split precision, SURVEY.md 7.3(5)): A = A_hi + A_lo and W2 = W_hi + W_lo as FP16 pairs, three MMAs per K step
+// (A_hi W_hi + A_lo W_hi + A_hi W_lo, FP32 accumulate; the dropped A_lo W_lo term is 2^-22 of the product), layers 1 and 3 and
+// every vector in FP32 on the CUDA cores.  FP16 subnormals keep the lo parts to 3e-8 absolute, so the hidden layer carries
+// ~22 significant bits and the flow's log-density agrees with a float64 evaluation to ~1e-6 (tests/test_flow_gpu.py): the
+// tolerance north_star states (1e-5) — which single FP16 operands miss by 20-600x.
 #pragma once
 #include <cstdint>
 #include <cuda_fp16.h>
@@ -33,62 +31,21 @@ constexpr int kFlowHidden = 128;
 constexpr int kFlowTile = 128;
 // capacity (shared-memory state slots) of a CTA's chunk; the launcher picks the tiles per chunk at run time (<= this) so that a
 // small batch still spreads over all SMs: 32 tiles per weight fetch measured 4 % faster than 16 on 8.4 M samples
-#ifndef GLABC_FLOW_TILES
-#define GLABC_FLOW_TILES 32
-#endif
-constexpr int kFlowTilesPerCta = GLABC_FLOW_TILES;
-// Operand precision of the 128 x 128 layer.  FP16 (default) and TF32 carry the same 10-bit mantissa — the agreement with an
-// fp32 evaluation is the same ~1e-3 — but kind::f16 runs at twice the tensor rate, halves the A operand's TMEM columns and
-// W2's shared-memory footprint, and ReLU + saturation + rounding + packing of TWO activations is ONE instruction
-// (F2FP.SATFINITE.RELU.F16.F32.PACK_AB).  Activations beyond 65504 saturate instead of overflowing.  -DGLABC_FLOW_F16=0: TF32.
-#ifndef GLABC_FLOW_F16
-#define GLABC_FLOW_F16 1
-#endif
-constexpr bool kFlowF16 = GLABC_FLOW_F16 != 0;
-// FP16 leaves room in TMEM (per group 128 accumulator + 2 x 64 A-operand columns) to double-buffer the A operand: layer 1 of
-// the group's NEXT tile is computed while the tensor cores work on the current one (-DGLABC_FLOW_OVERLAP=0: one buffer).
-#ifndef GLABC_FLOW_OVERLAP
-#define GLABC_FLOW_OVERLAP GLABC_FLOW_F16
-#endif
-constexpr bool kFlowOverlap = kFlowF16 && GLABC_FLOW_OVERLAP != 0;
-// The N = 2 output layer as a SECOND small MMA (M128 N16 K128): the epilogue then only adds b2, applies ReLU and packs the
-// activations back into the tile's (free again) A columns — no W3 reads from shared memory, no 2 x 128 FMA contraction on
-// the CUDA cores.  -DGLABC_FLOW_MMA2=0: the contraction stays on the CUDA cores.
-#ifndef GLABC_FLOW_MMA2
-#define GLABC_FLOW_MMA2 GLABC_FLOW_OVERLAP
-#endif
-constexpr bool kFlowMma2 = kFlowOverlap && GLABC_FLOW_MMA2 != 0;
-constexpr int kFlowW3Bytes = kFlowMma2 ? 16 * kFlowHidden * 2 : 0;   // W3 as a 16 x 128 FP16 B operand (rows 2..15 zero)
-constexpr int kFlowElemBytes = kFlowF16 ? 2 : 4;
-constexpr int kFlowW2Bytes = kFlowHidden * kFlowHidden * kFlowElemBytes;   // 32 KB (FP16) / 64 KB (TF32) per block
-constexpr int kFlowVecFloats = 768;                                  // w1, b1, b2 [128], w3 [2][128], b3 [2] (+pad)
-constexpr int kFlowGroups = 2;                                        // two groups, one tile in flight each
-constexpr int kFlowGroupThreads = 2 * kFlowTile;                      // two threads per sample row (half the hidden units each)
-constexpr int kFlowThreads = kFlowGroups * kFlowGroupThreads;         // 512: four warps per scheduler
-constexpr int kFlowSmemBytes = kFlowW2Bytes + kFlowW3Bytes + kFlowVecFloats * 4 + 3 * kFlowTilesPerCta * kFlowTile * 4 +
-                               kFlowGroups * 2 * kFlowTile * 8 + 64;   // W2 of the block, vectors, states, partial sums, barriers
-constexpr uint32_t kFlowTmemCols = 512;                                // per group: 128 accumulator + 128 A-operand columns
-// PRECISE mode (split precision, SURVEY.md 7.3(5)): A = A_hi + A_lo and W2 = W_hi + W_lo as FP16 pairs, three MMAs per K step
-// (A_hi W_hi + A_lo W_hi + A_hi W_lo, FP32 accumulate; the dropped A_lo W_lo term is 2^-22 of the product), layers 1 and 3 and
-// every vector in FP32 on the CUDA cores.  FP16 subnormals keep the lo parts to 3e-8 absolute, so the hidden layer carries
-// ~22 significant bits and the flow's log-density agrees with a float64 evaluation to ~1e-6 (tests/test_flow_gpu.py): the
-// tolerance north_star states (1e-5) — which FP16 / TF32 operands alone miss by 20-600x.  Shared memory: W_hi and W_lo (64 KB);
-// TMEM per group: 128 accumulator + 64 A_hi + 64 A_lo columns (no double-buffered A).
-constexpr int kFlowSmemBytesPrecise = 2 * kFlowW2Bytes + kFlowVecFloats * 4 + 3 * kFlowTilesPerCta * kFlowTile * 4 +
-                                      kFlowGroups * 2 * kFlowTile * 8 + 64;
+constexpr int kFlowTilesPerCta = 32;
+constexpr int kFlowW2Bytes = kFlowHidden * kFlowHidden * 2;   // W2 of one coupling block as FP16: 32 KB
 
-// per coupling block, the small operands pre-packed for the pipelined FAST kernel (flow_pipe.cuh: k_flow_pack_aux)
+// per coupling block, the small operands pre-packed for the flow kernels (flow_pipe.cuh: k_flow_pack_aux)
 constexpr int kFlowAuxBytes = 10880;   // FAST reads bytes [0, 8832), PRECISE bytes [4608, 10880) of a block's blob
 
 struct FlowDev {
     const float* w1;   // [L][128]
     const float* b1;   // [L][128]
-    const float* w2p;  // [L][128*128] FP16 (or TF32 bits), UMMA K-major / no-swizzle core-matrix layout (flow_pack_offset)
+    const float* w2p;  // [L][128*128] FP16, UMMA K-major / no-swizzle core-matrix layout (flow_pack_offset)
     const float* w2p_lo;  // PRECISE mode: FP16(W2 - FP16(W2)) in the same layout
     const float* b2;   // [L][128]
     const float* w3;   // [L][2][128]
     const float* b3;   // [L][2]
-    const uint8_t* aux;   // [L][kFlowAuxBytes]: W3 as a UMMA operand, w1 / b1 as FP16 pairs, b2, b3 (null: the pipelined kernel is not used)
+    const uint8_t* aux;   // [L][kFlowAuxBytes]: W3 and b2 as UMMA operands, w1 / b1 as FP16 pairs, b3, W3 / w1 / b1 in FP32 (k_flow_pack_aux)
     float base_loc[2], base_log_scale[2];
     int32_t n_blocks;
     // sample() without an eps buffer: the base normals of sample i are Box-Muller of Philox4x32-10(counter = (i, kSlotFlowEps), key = seed)
@@ -97,12 +54,11 @@ struct FlowDev {
 
 constexpr uint32_t kSlotFlowEps = 0x60000000u;
 
-// byte offset of element (row r, k) of a [128][128] fp32 operand in the K-major no-swizzle canonical layout:
-// core matrix = 8 rows x 16 bytes, core matrices contiguous along K (LBO = 128 B), 8-row groups 4 KB apart (SBO)
+// byte offset of element (row r, k) of a [128][128] FP16 operand in the K-major no-swizzle canonical layout:
+// core matrix = 8 rows x 16 bytes (8 halves), core matrices contiguous along K (LBO = 128 B), 8-row groups 2 KB apart (SBO)
 __host__ __device__ constexpr uint32_t flow_pack_offset(uint32_t r, uint32_t k)
 {
-    return kFlowF16 ? (r >> 3) * 2048u + (k >> 3) * 128u + (r & 7u) * 16u + (k & 7u) * 2u      // 8 halves per 16-byte row
-                    : (r >> 3) * 4096u + (k >> 2) * 128u + (r & 7u) * 16u + (k & 3u) * 4u;
+    return (r >> 3) * 2048u + (k >> 3) * 128u + (r & 7u) * 16u + (k & 7u) * 2u;
 }
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return static_cast<uint32_t>(__cvta_generic_to_shared(p)); }
@@ -144,18 +100,6 @@ __device__ __forceinline__ uint64_t umma_desc(uint32_t saddr, uint32_t lbo_bytes
            (static_cast<uint64_t>(sbo_bytes >> 4) << 32) | (1ull << 46);
 }
 
-// D[tmem] (+)= A[smem] * B[smem]^T, TF32 operands, FP32 accumulate, M = 128, N = 128, K = 8
-__device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate)
-{
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-        :
-        : "r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32])
 {
     asm volatile(
@@ -195,19 +139,6 @@ __device__ __forceinline__ void tmem_st32(uint32_t taddr, const uint32_t (&v)[32
           "r"(v[10]), "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15]), "r"(v[16]), "r"(v[17]), "r"(v[18]), "r"(v[19]),
           "r"(v[20]), "r"(v[21]), "r"(v[22]), "r"(v[23]), "r"(v[24]), "r"(v[25]), "r"(v[26]), "r"(v[27]), "r"(v[28]), "r"(v[29]),
           "r"(v[30]), "r"(v[31])
-        : "memory");
-}
-
-// D[tmem] (+)= A[tmem] * B[smem]^T: the A operand (row i = TMEM lane i, 8 TF32 values = 8 columns per MMA) never touches
-// shared memory — at 4 bytes per element the smem pipe (A write + A read + B read) would otherwise bound the kernel
-__device__ __forceinline__ void umma_tf32_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t accumulate)
-{
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], %2, %3, p;\n\t}"
-        :
-        : "r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate)
         : "memory");
 }
 
@@ -272,18 +203,7 @@ __device__ __forceinline__ uint32_t pack_half2(float lo, float hi)
 }
 __device__ __forceinline__ float2 unpack_half2(uint32_t v) { return __half22float2(*reinterpret_cast<const __half2*>(&v)); }
 
-__device__ __forceinline__ float to_tf32(float x)
-{
-    uint32_t r;
-    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
-    return __uint_as_float(r);
-}
-
-// round-to-nearest TF32 of a non-negative float in ONE integer add: the tensor core ignores the low 13 mantissa bits
-// (truncation), so adding half a TF32 ulp first rounds to nearest (cvt.rna.tf32 is a multi-instruction sequence)
-__device__ __forceinline__ float round_tf32_nonneg(float x) { return __uint_as_float(__float_as_uint(x) + 0x1000u); }
-
-// pack W2 [L][out=128][in=128] (torch Linear.weight) into the UMMA layout, rounded to TF32
+// pack W2 [L][out=128][in=128] (torch Linear.weight) into the UMMA layout as FP16, and (w2p_lo non-null) the FP16 remainder
 static __global__ void __launch_bounds__(256) k_flow_pack(const float* __restrict__ w2, float* __restrict__ w2p, float* __restrict__ w2p_lo,
                                                           int64_t total)
 {
@@ -292,440 +212,10 @@ static __global__ void __launch_bounds__(256) k_flow_pack(const float* __restric
     const int64_t l = g / (kFlowHidden * kFlowHidden);
     const uint32_t e = static_cast<uint32_t>(g - l * kFlowHidden * kFlowHidden);
     const uint32_t r = e / kFlowHidden, k = e % kFlowHidden;
-    if constexpr (kFlowF16) {
-        const __half hi = __float2half_rn(w2[g]);
-        reinterpret_cast<__half*>(w2p)[l * kFlowHidden * kFlowHidden + flow_pack_offset(r, k) / 2] = hi;
-        if (w2p_lo != nullptr)
-            reinterpret_cast<__half*>(w2p_lo)[l * kFlowHidden * kFlowHidden + flow_pack_offset(r, k) / 2] = __float2half_rn(w2[g] - __half2float(hi));
-    } else {
-        w2p[l * kFlowHidden * kFlowHidden + flow_pack_offset(r, k) / 4] = to_tf32(w2[g]);
-    }
-}
-
-#ifdef GLABC_FLOW_TRACE
-// phase timeline of CTA 0 (kernel experiments only; read back with glabc_debug_flow_trace): [group][thread 0 / 224][tile][stamp]
-static __device__ long long g_flow_trace[2][2][16][12];
-#define GLABC_TR(i)                                                                                         \
-    do {                                                                                                    \
-        if (blockIdx.x == 0 && li == 4 && chunk == 0 && (gtid == 0 || gtid == 224) && (t >> 1) < 16)        \
-            g_flow_trace[group][gtid != 0][t >> 1][i] = clock64();                                          \
-    } while (0)
-#else
-#define GLABC_TR(i)
-#endif
-
-__device__ __forceinline__ void group_sync(int group)
-{
-    asm volatile("bar.sync %0, %1;" ::"r"(1 + group), "r"(kFlowGroupThreads) : "memory");
-}
-
-// SAMPLE: in = eps [n][2] standard normals -> theta [n][2], log q [n]       (NormalizingFlow.sample)
-// !SAMPLE: in = theta [n][2] -> log q [n]                                     (NormalizingFlow.log_prob)
-// 512 threads = two groups of 256.  A group owns one tile of 128 samples at a time with its own A buffer, TMEM
-// accumulator (128 columns) and mbarrier, so the MMA of one group's tile overlaps the CUDA-core phases of the other's.
-// Inside a group TWO threads serve each sample row — warps w and w+4 may both read TMEM lanes 32(w%4).., so thread
-// (row, half) computes hidden units [64 half, 64 half + 64) of layer 1 and reduces the same 64 accumulator columns in
-// the epilogue; the two partial (shift, log-scale) sums meet in shared memory.  Four warps per scheduler instead of two.
-template <bool SAMPLE, bool PRECISE>
-__global__ void __launch_bounds__(kFlowThreads, 1) k_flow(const __grid_constant__ FlowDev W, const float* __restrict__ in,
-                                                          int64_t n, float* __restrict__ out_theta, float* __restrict__ out_lq, int tpc)
-{
-    static_assert(!PRECISE || kFlowF16, "the split-precision mode splits into FP16 pairs");
-    // the fast configuration's switches, all off in PRECISE mode
-    constexpr bool kOverlap = !PRECISE && kFlowOverlap;      // double-buffered A operand
-    constexpr bool kMma2 = !PRECISE && kFlowMma2;            // output layer as a second small MMA
-    constexpr bool kVecF16 = !PRECISE && kFlowF16;           // layer vectors staged as FP16 pairs
-    // tpc: tiles per chunk (<= kFlowTilesPerCta), chosen by the launcher
-    extern __shared__ __align__(1024) uint8_t smem[];
-    float* sB = reinterpret_cast<float*>(smem);
-    __half* sW3 = reinterpret_cast<__half*>(smem + kFlowW2Bytes);   // FAST: [16][128] FP16, UMMA K-major core-matrix layout (kMma2)
-    float* sVec = reinterpret_cast<float*>(smem + (PRECISE ? 2 * kFlowW2Bytes : kFlowW2Bytes + kFlowW3Bytes));   // PRECISE: W_lo follows W_hi
-    float* sState = sVec + kFlowVecFloats;  // [3][tiles][128]: z1, z2, log q
-    float2* sPart = reinterpret_cast<float2*>(sState + 3 * kFlowTilesPerCta * kFlowTile);  // [groups][128] partial sums of half 1
-    uint64_t* bars = reinterpret_cast<uint64_t*>(sPart + kFlowGroups * 2 * kFlowTile);
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 1 + kFlowGroups);
-    const int tid = threadIdx.x, warp = tid >> 5;
-    const int group = tid / kFlowGroupThreads, gtid = tid % kFlowGroupThreads;
-    const int half = gtid >> 7, row = gtid & (kFlowTile - 1), quad = (gtid >> 5) & 3;
-    float2* part_base = sPart + group * 2 * kFlowTile;   // two buffers: a tile's partial sums are read after the next tile's may start
-    const uint32_t bar_w = smem_u32(&bars[0]), bar_m = smem_u32(&bars[1 + group]);
-    constexpr int TS = kFlowTilesPerCta * kFlowTile;
-    constexpr int HK = kFlowHidden / 2;  // hidden units per thread
-
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                     "r"(kFlowTmemCols)
-                     : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    if (tid == 0) {
-        for (int i = 0; i < 1 + kFlowGroups; ++i) mbar_init(smem_u32(&bars[i]), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if constexpr (kMma2)
-        for (int i = tid; i < kFlowW3Bytes / 4; i += kFlowThreads) reinterpret_cast<uint32_t*>(sW3)[i] = 0u;
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem = *tmem_slot + static_cast<uint32_t>(group * 256);  // this group's accumulator columns
-    const uint32_t tmem_a0 = tmem + 128u;                                   // and its A-operand columns (FP16: two buffers of 64)
-    // instruction descriptor: D = F32, A = B = TF32, both K-major, N = 128, M = 128 (cute::UMMA::InstrDescriptor bit layout)
-    // (a_format / b_format: 0 = F16 for kind::f16, 2 = TF32 for kind::tf32)
-    constexpr uint32_t idesc = kFlowF16 ? (1u << 4) | ((128u >> 3) << 17) | ((128u >> 4) << 24)
-                                        : (1u << 4) | (2u << 7) | (2u << 10) | ((128u >> 3) << 17) | ((128u >> 4) << 24);
-    const uint32_t sB_addr = smem_u32(sB);
-    uint32_t ph_w = 0, ph_m = 0;
-    const float c2 = -1.8378770664093453f;  // -0.5 * 2 * log(2 pi)
-    const int L = W.n_blocks;
-    const int64_t n_chunks = (n + static_cast<int64_t>(tpc) * kFlowTile - 1) / (static_cast<int64_t>(tpc) * kFlowTile);
-
-    for (int64_t chunk = blockIdx.x; chunk < n_chunks; chunk += gridDim.x) {
-        int tiles = 0;
-        for (int t = 0; t < tpc; ++t) {
-            if ((chunk * tpc + t) * kFlowTile < n) tiles = t + 1;
-            if ((t & 1) != group || half != 0) continue;  // a tile's state is written by half 0 of its own group only
-            const int64_t idx = (chunk * tpc + t) * kFlowTile + row;
-            float a = 0.0f, b = 0.0f, lq = 0.0f;
-            if (idx < n) {
-                if (SAMPLE && in == nullptr) {   // q0's normals generated here: no eps buffer, no HBM round trip (GLMCMC_NFs.py:72,127)
-                    const RoundKeys rk = expand_key(make_uint2(W.seed_lo, W.seed_hi));
-                    const uint4 w = philox4x32_10(make_uint4(static_cast<uint32_t>(idx), static_cast<uint32_t>(idx >> 32), 0u, kSlotFlowEps), rk);
-                    box_muller(w.x, w.y, a, b);
-                } else {
-                    a = in[idx * 2];
-                    b = in[idx * 2 + 1];
-                }
-                if (SAMPLE) {  // base DiagGaussian.forward: z = loc + exp(log_scale) * eps, log p from eps
-                    lq = c2 - ((W.base_log_scale[0] + 0.5f * (a * a)) + (W.base_log_scale[1] + 0.5f * (b * b)));
-                    a = W.base_loc[0] + expf(W.base_log_scale[0]) * a;
-                    b = W.base_loc[1] + expf(W.base_log_scale[1]) * b;
-                }
-            }
-            sState[0 * TS + t * kFlowTile + row] = a;
-            sState[1 * TS + t * kFlowTile + row] = b;
-            sState[2 * TS + t * kFlowTile + row] = lq;
-        }
-        for (int li = 0; li < L; ++li) {
-            const int l = SAMPLE ? li : L - 1 - li;
-            __syncthreads();  // both groups are done with the previous block's W2 / vectors / state updates
-            if (tid == 0) {
-                mbar_expect_tx(bar_w, PRECISE ? 2 * kFlowW2Bytes : kFlowW2Bytes);
-#pragma unroll
-                for (int q = 0; q < 4; ++q)
-                    bulk_g2s(sB_addr + q * (kFlowW2Bytes / 4), reinterpret_cast<const uint8_t*>(W.w2p) +
-                             static_cast<int64_t>(l) * kFlowW2Bytes + q * (kFlowW2Bytes / 4), kFlowW2Bytes / 4, bar_w);
-                if constexpr (PRECISE) {
-#pragma unroll
-                    for (int q = 0; q < 4; ++q)
-                        bulk_g2s(sB_addr + kFlowW2Bytes + q * (kFlowW2Bytes / 4), reinterpret_cast<const uint8_t*>(W.w2p_lo) +
-                                 static_cast<int64_t>(l) * kFlowW2Bytes + q * (kFlowW2Bytes / 4), kFlowW2Bytes / 4, bar_w);
-                }
-            }
-            if constexpr (kVecF16) {
-                // The broadcast reads of these vectors are what bounds the kernel (every warp re-reads them for every tile:
-                // 1,280 B per thread and tile in fp32 = more shared-memory cycles than the tile takes), so they are staged in
-                // the narrowest form the arithmetic allows: w1 / b1 as FP16 pairs (layer 1 runs as HFMA2.RELU straight into the
-                // A operand's format), the two W3 rows interleaved as one FP16 pair per column, b2 in fp32: 768 B.
-                uint32_t* sU = reinterpret_cast<uint32_t*>(sVec);
-                if (tid < 64) sU[tid] = pack_half2(W.w1[l * kFlowHidden + 2 * tid], W.w1[l * kFlowHidden + 2 * tid + 1]);
-                else if (tid < 128) sU[tid] = pack_half2(W.b1[l * kFlowHidden + 2 * (tid - 64)], W.b1[l * kFlowHidden + 2 * (tid - 64) + 1]);
-                else if (tid < 256) sVec[128 + tid] = W.b2[l * kFlowHidden + tid - 128];                    // [256, 384)
-                else if (tid < 384) sU[128 + tid] = pack_half2(W.w3[(l * 2) * kFlowHidden + tid - 256],       // [384, 512)
-                                                               W.w3[(l * 2 + 1) * kFlowHidden + tid - 256]);
-                else if (tid < 386) sVec[640 + tid - 384] = W.b3[l * 2 + tid - 384];
-                if constexpr (kMma2) {   // element (n, k) of the 16 x 128 operand: rows 0 (shift) and 1 (log-scale)
-                    if (tid >= 256) {
-                        const int n = (tid - 256) >> 7, k = (tid - 256) & 127;
-                        sW3[((k >> 3) * 128 + (n & 7) * 16 + (k & 7) * 2) / 2] = __float2half_rn(W.w3[(l * 2 + n) * kFlowHidden + k]);
-                    }
-                }
-            } else {
-                if (tid < 128) sVec[tid] = W.w1[l * kFlowHidden + tid];
-                else if (tid < 256) sVec[tid] = W.b1[l * kFlowHidden + tid - 128];
-                else if (tid < 384) sVec[tid] = W.b2[l * kFlowHidden + tid - 256];
-                else sVec[tid] = W.w3[(l * 2) * kFlowHidden + tid - 384];  // w3 rows 0 and 1 are contiguous: [384, 640)
-                if (tid < 128) sVec[512 + tid] = W.w3[(l * 2 + 1) * kFlowHidden + tid];
-                if (tid < 2) sVec[640 + tid] = W.b3[l * 2 + tid];
-            }
-            if constexpr (kMma2) asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // sW3: generic writes -> MMA reads
-            __syncthreads();
-            mbar_wait(bar_w, ph_w);
-            ph_w ^= 1u;
-
-            // layer 1 (K = 1) of tile t on CUDA cores, written as the A operand into TMEM columns `a_cols`: this thread's 64 hidden units
-            auto layer1 = [&](int t, uint32_t tmem_a) {
-                float z1 = sState[(SAMPLE ? 0 : 1) * TS + t * kFlowTile + row];   // !SAMPLE: Permute(swap)^-1 precedes the inverse
-                if constexpr (PRECISE) {
-                    // FP32 layer 1, then the FP16 hi / lo split of every activation: 32 + 32 packed columns, two tcgen05.st
-                    uint32_t hv[32], lv[32];
-#pragma unroll
-                    for (int j = 0; j < HK / 4; ++j) {
-                        const float4 w = *reinterpret_cast<const float4*>(&sVec[half * HK + 4 * j]);
-                        const float4 bb = *reinterpret_cast<const float4*>(&sVec[128 + half * HK + 4 * j]);
-                        const float a0 = fmaxf(fmaf(w.x, z1, bb.x), 0.0f), a1 = fmaxf(fmaf(w.y, z1, bb.y), 0.0f);
-                        const float a2 = fmaxf(fmaf(w.z, z1, bb.z), 0.0f), a3 = fmaxf(fmaf(w.w, z1, bb.w), 0.0f);
-                        const uint32_t h01 = relu_pack_f16(a0, a1), h23 = relu_pack_f16(a2, a3);   // saturating round to FP16
-                        const float2 f01 = unpack_half2(h01), f23 = unpack_half2(h23);
-                        hv[2 * j] = h01;
-                        hv[2 * j + 1] = h23;
-                        lv[2 * j] = pack_half2(a0 - f01.x, a1 - f01.y);
-                        lv[2 * j + 1] = pack_half2(a2 - f23.x, a3 - f23.y);
-                    }
-                    tmem_st32(tmem_a + (static_cast<uint32_t>(quad * 32) << 16) + half * (HK / 2), hv);
-                    tmem_st32(tmem_a + 64u + (static_cast<uint32_t>(quad * 32) << 16) + half * (HK / 2), lv);
-                } else if constexpr (kFlowF16) {
-                    // this thread's 64 hidden units as 32 packed FP16 pairs = 32 TMEM columns, ONE tcgen05.st
-                    uint32_t hv[32];
-                    // z1 as an FP16 hi + lo pair: rounding the INPUT to 11 bits would perturb all 128 hidden units coherently
-                    // (the error of the block would be the network's derivative times 5e-4 |z1|); the roundings left are per-unit
-                    const float z_hi = __half2float(__float2half_rn(z1));
-                    const uint32_t zz = pack_half2(z_hi, z_hi), zl = pack_half2(z1 - z_hi, z1 - z_hi);
-                    const uint4* w1h = reinterpret_cast<const uint4*>(sVec) + half * (HK / 8);        // 8 hidden units per 16 bytes
-                    const uint4* b1h = reinterpret_cast<const uint4*>(sVec + 64) + half * (HK / 8);
-#pragma unroll
-                    for (int j = 0; j < HK / 8; ++j) {
-                        const uint4 w = w1h[j], bb = b1h[j];
-                        hv[4 * j] = hfma2_relu(w.x, zz, hfma2(w.x, zl, bb.x));
-                        hv[4 * j + 1] = hfma2_relu(w.y, zz, hfma2(w.y, zl, bb.y));
-                        hv[4 * j + 2] = hfma2_relu(w.z, zz, hfma2(w.z, zl, bb.z));
-                        hv[4 * j + 3] = hfma2_relu(w.w, zz, hfma2(w.w, zl, bb.w));
-                    }
-                    tmem_st32(tmem_a + (static_cast<uint32_t>(quad * 32) << 16) + half * (HK / 2), hv);
-                } else {
-#pragma unroll
-                    for (int cb = 0; cb < HK / 32; ++cb) {
-                        uint32_t hv[32];
-#pragma unroll
-                        for (int j = 0; j < 32; j += 4) {
-                            const float4 w = *reinterpret_cast<const float4*>(&sVec[half * HK + cb * 32 + j]);
-                            const float4 bb = *reinterpret_cast<const float4*>(&sVec[128 + half * HK + cb * 32 + j]);
-                            hv[j] = __float_as_uint(round_tf32_nonneg(fmaxf(fmaf(w.x, z1, bb.x), 0.0f)));
-                            hv[j + 1] = __float_as_uint(round_tf32_nonneg(fmaxf(fmaf(w.y, z1, bb.y), 0.0f)));
-                            hv[j + 2] = __float_as_uint(round_tf32_nonneg(fmaxf(fmaf(w.z, z1, bb.z), 0.0f)));
-                            hv[j + 3] = __float_as_uint(round_tf32_nonneg(fmaxf(fmaf(w.w, z1, bb.w), 0.0f)));
-                        }
-                        tmem_st32(tmem_a + (static_cast<uint32_t>(quad * 32) << 16) + half * HK + cb * 32, hv);
-                    }
-                }
-                asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-            };
-            uint32_t buf = 0;
-            if (kOverlap && group < tiles) {
-                layer1(group, tmem_a0);
-                tc_fence_before();
-                group_sync(group);
-            }
-            for (int t = group; t < tiles; t += kFlowGroups) {
-                const uint32_t tmem_a = tmem_a0 + (kOverlap ? buf * 64u : 0u);
-                float2* part = part_base + buf * kFlowTile;
-                if constexpr (!kOverlap) {
-                    layer1(t, tmem_a);
-                    tc_fence_before();
-                    group_sync(group);  // (also: half 0 has consumed the previous tile's partial sums)
-                }
-                GLABC_TR(0);
-                // ---- layer 2 (128 x 128 x 128) on the tensor cores ----
-                if (gtid < 32) {   // the group's first warp, converged: one elected lane issues (see elect_one)
-                  const bool lead = elect_one();
-                  if (lead) {
-                    tc_fence_after();
-                    if constexpr (PRECISE) {
-                        // A_hi W_hi, then the two cross terms, all into the same FP32 accumulator
-#pragma unroll
-                        for (int k = 0; k < kFlowHidden / 16; ++k)
-                            umma_f16_ts(tmem, tmem_a + k * 8, umma_desc(sB_addr + k * 256, 128, 2048), idesc, k > 0 ? 1u : 0u);
-#pragma unroll
-                        for (int k = 0; k < kFlowHidden / 16; ++k)
-                            umma_f16_ts(tmem, tmem_a + 64u + k * 8, umma_desc(sB_addr + k * 256, 128, 2048), idesc, 1u);
-#pragma unroll
-                        for (int k = 0; k < kFlowHidden / 16; ++k)
-                            umma_f16_ts(tmem, tmem_a + k * 8, umma_desc(sB_addr + kFlowW2Bytes + k * 256, 128, 2048), idesc, 1u);
-                    } else if constexpr (kFlowF16) {
-#pragma unroll
-                        for (int k = 0; k < kFlowHidden / 16; ++k) {   // K = 16 halves = 2 core matrices = 256 B of B, 8 columns of A
-                            const uint64_t bd = umma_desc(sB_addr + k * 256, 128, 2048);
-                            umma_f16_ts(tmem, tmem_a + k * 8, bd, idesc, k > 0 ? 1u : 0u);
-                        }
-                    } else {
-#pragma unroll
-                        for (int k = 0; k < kFlowHidden / 8; ++k) {
-                            const uint64_t bd = umma_desc(sB_addr + k * 256, 128, 4096);
-                            umma_tf32_ts(tmem, tmem_a + k * 8, bd, idesc, k > 0 ? 1u : 0u);
-                        }
-                    }
-                    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar_m) : "memory");
-                  }
-                  __syncwarp();
-                }
-                GLABC_TR(1);
-                if constexpr (kOverlap) {   // the group's next tile: its layer 1 fills the other A buffer while the MMA runs
-                    if (t + kFlowGroups < tiles) layer1(t + kFlowGroups, tmem_a0 + (buf ^ 1u) * 64u);
-                }
-                GLABC_TR(2);
-                mbar_wait(bar_m, ph_m);
-                ph_m ^= 1u;
-                tc_fence_after();
-                GLABC_TR(3);
-                float s0 = 0.0f, s1 = 0.0f;
-                float2 o = make_float2(0.0f, 0.0f);
-                if constexpr (kMma2) {
-                    // ---- bias + ReLU from TMEM, packed back as FP16 into this tile's A columns (free since its MMA completed) ----
-                    {
-                        uint32_t v[2][16], hp[32];
-                        const uint32_t trow = tmem + (static_cast<uint32_t>(quad * 32) << 16) + half * HK;
-                        tmem_ld16_async(trow, v[0]);
-#pragma unroll
-                        for (int c = 0; c < HK / 16; ++c) {
-                            tmem_ld_wait();
-                            if (c + 1 < HK / 16) tmem_ld16_async(trow + (c + 1) * 16, v[(c + 1) & 1]);
-                            const int col0 = half * HK + c * 16;
-#pragma unroll
-                            for (int j = 0; j < 16; j += 4) {
-                                const float4 b2v = *reinterpret_cast<const float4*>(&sVec[256 + col0 + j]);
-                                const uint32_t* vv = v[c & 1];
-                                hp[c * 8 + j / 2] = relu_pack_f16(__uint_as_float(vv[j]) + b2v.x, __uint_as_float(vv[j + 1]) + b2v.y);
-                                hp[c * 8 + j / 2 + 1] = relu_pack_f16(__uint_as_float(vv[j + 2]) + b2v.z, __uint_as_float(vv[j + 3]) + b2v.w);
-                            }
-                        }
-                        tmem_st32(tmem_a + (static_cast<uint32_t>(quad * 32) << 16) + half * (HK / 2), hp);
-                        asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-                    }
-                    GLABC_TR(4);
-                    tc_fence_before();
-                    group_sync(group);  // every thread has read its accumulator columns and written its activations
-                    GLABC_TR(5);
-                    // ---- layer 3 (128 x 16 x 128, rows 0 / 1 of W3) on the tensor cores, into accumulator columns 0..15 ----
-                    if (gtid < 32) {
-                      const bool lead = elect_one();
-                      if (lead) {
-                        tc_fence_after();
-                        constexpr uint32_t idesc3 = (1u << 4) | ((16u >> 3) << 17) | ((128u >> 4) << 24);
-                        const uint32_t sW3_addr = smem_u32(sW3);
-#pragma unroll
-                        for (int k = 0; k < kFlowHidden / 16; ++k) {
-                            const uint64_t bd = umma_desc(sW3_addr + k * 256, 128, 2048);
-                            umma_f16_ts(tmem, tmem_a + k * 8, bd, idesc3, k > 0 ? 1u : 0u);
-                        }
-                        asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar_m) : "memory");
-                      }
-                      __syncwarp();
-                    }
-                    GLABC_TR(6);
-                    mbar_wait(bar_m, ph_m);
-                    ph_m ^= 1u;
-                    tc_fence_after();
-                    GLABC_TR(7);
-                    if (half == 0) {   // warp-uniform: warps 0..3 of the group
-                        uint32_t r0, r1;
-                        asm volatile("tcgen05.ld.sync.aligned.32x32b.x2.b32 {%0, %1}, [%2];"
-                                     : "=r"(r0), "=r"(r1)
-                                     : "r"(tmem + (static_cast<uint32_t>(quad * 32) << 16))
-                                     : "memory");
-                        tmem_ld_wait();
-                        s0 = __uint_as_float(r0);
-                        s1 = __uint_as_float(r1);
-                    }
-                    GLABC_TR(8);
-                    tc_fence_before();
-                    group_sync(group);  // the accumulator and both A buffers' roles are free for the group's next tile
-                    GLABC_TR(9);
-                } else {
-                // ---- bias + ReLU + layer 3 (N = 2) from TMEM: this thread's 64 columns, four independent partial sums ----
-                float p0[4] = {0.0f, 0.0f, 0.0f, 0.0f}, p1[4] = {0.0f, 0.0f, 0.0f, 0.0f};
-                {
-                    // four 16-column TMEM loads, software-pipelined: chunk c + 1 is in flight while chunk c is reduced
-                    uint32_t v[2][16];
-                    const uint32_t trow = tmem + (static_cast<uint32_t>(quad * 32) << 16) + half * HK;
-                    tmem_ld16_async(trow, v[0]);
-#pragma unroll
-                    for (int c = 0; c < HK / 16; ++c) {
-                        tmem_ld_wait();
-                        if (c + 1 < HK / 16) tmem_ld16_async(trow + (c + 1) * 16, v[(c + 1) & 1]);
-                        const int col0 = half * HK + c * 16;
-#pragma unroll
-                        for (int j = 0; j < 16; j += 4) {  // broadcast LDS.128 of b2 and of the W3 pairs: 2 loads per 4 columns
-                            const float4 b2v = *reinterpret_cast<const float4*>(&sVec[256 + col0 + j]);
-                            float2 w0, w1, w2, w3;
-                            if constexpr (kVecF16) {
-                                const uint4 wq = *reinterpret_cast<const uint4*>(&sVec[384 + col0 + j]);
-                                w0 = unpack_half2(wq.x); w1 = unpack_half2(wq.y); w2 = unpack_half2(wq.z); w3 = unpack_half2(wq.w);
-                            } else {
-                                const float4 wa = *reinterpret_cast<const float4*>(&sVec[384 + col0 + j]);
-                                const float4 wb = *reinterpret_cast<const float4*>(&sVec[512 + col0 + j]);
-                                w0 = make_float2(wa.x, wb.x); w1 = make_float2(wa.y, wb.y);
-                                w2 = make_float2(wa.z, wb.z); w3 = make_float2(wa.w, wb.w);
-                            }
-                            const uint32_t* vv = v[c & 1];
-                            const float h0 = fmaxf(__uint_as_float(vv[j]) + b2v.x, 0.0f), h1 = fmaxf(__uint_as_float(vv[j + 1]) + b2v.y, 0.0f);
-                            const float h2 = fmaxf(__uint_as_float(vv[j + 2]) + b2v.z, 0.0f), h3 = fmaxf(__uint_as_float(vv[j + 3]) + b2v.w, 0.0f);
-                            p0[0] = fmaf(w0.x, h0, p0[0]); p1[0] = fmaf(w0.y, h0, p1[0]);
-                            p0[1] = fmaf(w1.x, h1, p0[1]); p1[1] = fmaf(w1.y, h1, p1[1]);
-                            p0[2] = fmaf(w2.x, h2, p0[2]); p1[2] = fmaf(w2.y, h2, p1[2]);
-                            p0[3] = fmaf(w3.x, h3, p0[3]); p1[3] = fmaf(w3.y, h3, p1[3]);
-                        }
-                    }
-                }
-                s0 = (p0[0] + p0[1]) + (p0[2] + p0[3]);
-                s1 = (p1[0] + p1[1]) + (p1[2] + p1[3]);
-                if (half == 1) part[row] = make_float2(s0, s1);
-                tc_fence_before();
-                group_sync(group);  // TMEM columns and the A buffer are free for the group's next tile; partial sums visible
-                if (half == 0) o = part[row];
-                }
-                if (half == 0) {
-                    float z1 = sState[0 * TS + t * kFlowTile + row], z2 = sState[1 * TS + t * kFlowTile + row];
-                    if (!SAMPLE) {  // Permute(swap)^-1 precedes the coupling's inverse
-                        const float tmp = z1;
-                        z1 = z2;
-                        z2 = tmp;
-                    }
-                    const float sh = (s0 + o.x) + sVec[640];  // shift     = param[:, 0::2]
-                    const float sc = (s1 + o.y) + sVec[641];  // log-scale = param[:, 1::2]
-                    float lq = sState[2 * TS + t * kFlowTile + row];
-                    if (SAMPLE) {
-                        const float z2n = fmaf(z2, expf(sc), sh);  // z2 * exp(s) + shift; log q -= log det
-                        lq -= sc;
-                        sState[0 * TS + t * kFlowTile + row] = z2n;  // Permute(swap)
-                        sState[1 * TS + t * kFlowTile + row] = z1;
-                    } else {
-                        const float z2n = (z2 - sh) * expf(-sc);     // inverse; log det = -s
-                        lq -= sc;
-                        sState[0 * TS + t * kFlowTile + row] = z1;
-                        sState[1 * TS + t * kFlowTile + row] = z2n;
-                    }
-                    sState[2 * TS + t * kFlowTile + row] = lq;
-                }
-                GLABC_TR(10);
-                buf ^= 1u;
-            }
-        }
-        __syncthreads();
-        for (int t = group; t < tiles; t += kFlowGroups) {
-            if (half != 0) continue;
-            const int64_t idx = (chunk * tpc + t) * kFlowTile + row;
-            if (idx >= n) continue;
-            const float a = sState[0 * TS + t * kFlowTile + row], b = sState[1 * TS + t * kFlowTile + row];
-            float lq = sState[2 * TS + t * kFlowTile + row];
-            if (SAMPLE) {
-                out_theta[idx * 2] = a;
-                out_theta[idx * 2 + 1] = b;
-            } else {  // + base.log_prob(z)
-                if (out_theta != nullptr) {   // the latent z = f^-1(x): where the training step's backward sweep starts (flow_train.cuh)
-                    out_theta[idx * 2] = a;
-                    out_theta[idx * 2 + 1] = b;
-                }
-                const float r0 = (a - W.base_loc[0]) / expf(W.base_log_scale[0]);
-                const float r1 = (b - W.base_loc[1]) / expf(W.base_log_scale[1]);
-                lq += c2 - ((W.base_log_scale[0] + 0.5f * (r0 * r0)) + (W.base_log_scale[1] + 0.5f * (r1 * r1)));
-            }
-            out_lq[idx] = lq;
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 0)
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(*tmem_slot), "r"(kFlowTmemCols)
-                     : "memory");
+    const __half hi = __float2half_rn(w2[g]);
+    reinterpret_cast<__half*>(w2p)[l * kFlowHidden * kFlowHidden + flow_pack_offset(r, k) / 2] = hi;
+    if (w2p_lo != nullptr)
+        reinterpret_cast<__half*>(w2p_lo)[l * kFlowHidden * kFlowHidden + flow_pack_offset(r, k) / 2] = __float2half_rn(w2[g] - __half2float(hi));
 }
 
 cudaError_t launch_flow_pack(const float* w2, float* w2p, float* w2p_lo, int n_blocks, cudaStream_t st);

@@ -1,13 +1,8 @@
-// K4, GLABC_FLOW_FAST mode: the RealNVP flow of flow.cuh as a warp-specialised pipeline.
+// K4's forward kernels: sample() and log_prob() of the RealNVP flow (flow.cuh) as warp-specialised pipelines, k_flow_pipe
+// (GLABC_FLOW_FAST) and k_flow_pipe_precise (GLABC_FLOW_PRECISE, further down).  DESIGN.md K4 has the measurements for
+// which this layout replaced round 1's kernel, whose two thread groups each walked a tile through every phase in lock-step.
 //
-// flow.cuh's k_flow gives every tile of 128 samples to one of two thread groups, and the group walks the tile through
-// layer 1 -> MMA -> epilogue -> output-layer MMA -> state update on its own.  A phase timeline of that kernel
-// (profiles/micro/k4_trace.py, profiles/r2_k4_timeline.md) shows the two groups in lock-step: both issue their MMAs at the
-// same moment, then both run their CUDA-core phases while the tensor pipe idles — 3,700 cycles per pair of tiles, the
-// tensor pipe busy for a third of them.
-//
-// Here the PHASES own the warps and the tiles flow past them (same arithmetic and roundings as k_flow's FAST path, except
-// that b2 is added inside the accumulator and the output layer is summed from four partial accumulators):
+// The PHASES own the warps and the tiles of 128 samples flow past them:
 //   * warps 16, 17        M1: wait on mbarriers and issue the hidden layer's tcgen05.mma for alternate tiles (one warp gets
 //                            through its waits while the other's MMAs are in the tensor pipe's queue), commit to mbarriers,
 //                            and prefetch the next coupling block's operands (W2 32 KB + a pre-packed 9 KB blob of w1 / b1 /
@@ -196,7 +191,6 @@ template <bool SAMPLE>
 __global__ void __launch_bounds__(kPipeThreads, 1) k_flow_pipe(const __grid_constant__ FlowDev W, const float* __restrict__ in, int64_t n,
                                                                float* __restrict__ out_theta, float* __restrict__ out_lq, int tpc)
 {
-    static_assert(kFlowF16, "the pipeline is written for FP16 operands");
     extern __shared__ __align__(1024) uint8_t smem[];
     uint8_t* sAux = smem + 2 * kFlowW2Bytes;
     uint8_t* sOnes = sAux + 2 * kAuxFastBytes;
@@ -500,7 +494,8 @@ __global__ void __launch_bounds__(kPipeThreads, 1) k_flow_pipe(const __grid_cons
                     if (gb != gb0) mbar_wait(bar(kBarStateFull + t), (gb - 1) & 1);   // U has updated this tile in the previous coupling block
                     // the arithmetic needs no TMEM: it runs BEFORE the wait for the operand buffer, which leaves only the store behind it
                     const float z1 = lds_f32(sState_addr + static_cast<uint32_t>(((SAMPLE ? 0 : 1) * TS + t * kFlowTile + row) * 4));   // !SAMPLE: Permute(swap)^-1 precedes the inverse
-                    // z1 as an FP16 hi + lo pair (flow.cuh: rounding the INPUT would perturb all hidden units coherently)
+                    // z1 as an FP16 hi + lo pair: rounding the INPUT to 11 bits would perturb all 128 hidden units coherently (the
+                    // error of the block would be the network's derivative times 5e-4 |z1|); the roundings left are per-unit
                     const float z_hi = __half2float(__float2half_rn(z1));
                     const uint32_t zz = pack_half2(z_hi, z_hi), zl = pack_half2(z1 - z_hi, z1 - z_hi);
                     const uint32_t b1h = sAux_addr + static_cast<uint32_t>((gb & 1) * kAuxFastBytes + kAuxB1 + half * 128);
@@ -580,7 +575,6 @@ template <bool SAMPLE>
 __global__ void __launch_bounds__(18 * 32, 1) k_flow_pipe_precise(const __grid_constant__ FlowDev W, const float* __restrict__ in, int64_t n,
                                                                   float* __restrict__ out_theta, float* __restrict__ out_lq, int tpc)
 {
-    static_assert(kFlowF16, "the split-precision mode splits into FP16 pairs");
     extern __shared__ __align__(1024) uint8_t smem[];
     uint8_t* sAux = smem + 4 * kFlowW2Bytes;                      // [2][W_hi 32 KB | W_lo 32 KB] precede
     uint8_t* sOnes = sAux + 2 * kAuxPreciseBytes;

@@ -8,7 +8,7 @@ namespace glabc {
 cudaError_t launch_flow_bwd(const FlowDev& W, const float* z_final, int64_t n, float* partial, int n_slices, cudaStream_t st)
 {
     if (n <= 0 || n_slices <= 0) return cudaSuccess;
-    if (!kFlowF16 || W.w2p_lo == nullptr) return cudaErrorInvalidValue;
+    if (W.w2p_lo == nullptr) return cudaErrorInvalidValue;
     static bool configured = false;
     if (!configured) {
         cudaError_t e = cudaFuncSetAttribute(k_flow_bwd, cudaFuncAttributeMaxDynamicSharedMemorySize, kTrSmemBytes);

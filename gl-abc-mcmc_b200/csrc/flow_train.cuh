@@ -1,7 +1,7 @@
 // K4-train — the flow's training step of GLMCMC-NFs (GLMCMC_NFs.py:112-124): loss = forward_kld(x) = -mean log q(x) over the
 // resampled candidates, backward through the 32 coupling blocks, Adam(lr 5e-4, weight_decay 1e-5) (GLMCMC_NFs.py:63).
 //
-//   forward   k_flow<log_prob, PRECISE> (flow.cuh) — log q(x) and the latent z = f^-1(x)
+//   forward   k_flow_pipe_precise<false> (flow_pipe.cuh: log_prob, PRECISE) — log q(x) and the latent z = f^-1(x)
 //   backward  k_flow_bwd (this file).  The flow is invertible, so nothing is stored: starting from z the sweep walks the blocks
 //             in the order opposite to log_prob's (l = 0 .. L-1), RE-COMPUTES block l's MLP from the block's output, rebuilds the
 //             block's input (z2 = z2' e^s + shift), and back-propagates.  Per tile of 128 samples and block, three GEMMs on the

@@ -1,6 +1,7 @@
-"""Phase timeline of k_flow (CTA 0, coupling block 4) from a -DGLABC_FLOW_TRACE build:
+"""Phase timeline of the FAST pipeline k_flow_pipe (CTA 0, pipeline steps 264..279) from a -DGLABC_FLOW_TRACE build:
    python -c "import sys; sys.path.insert(0,'gl-abc-mcmc_b200'); import build; build.build(variant='trace', extra_flags=['-DGLABC_FLOW_TRACE'])"
-   GLABC_LIB=$PWD/gl-abc-mcmc_b200/csrc/libglabc.trace.so python profiles/micro/k4_trace.py [fast|precise]"""
+   GLABC_LIB=$PWD/gl-abc-mcmc_b200/csrc/libglabc.trace.so python profiles/micro/k4_trace.py [fast|precise]
+`precise` times the PRECISE pipeline only: it records no timeline."""
 import ctypes
 import sys
 import time
@@ -48,15 +49,3 @@ if hasattr(lib, "glabc_debug_pipe_trace") and mode == "fast":
         for st in range(8, 24):
             row = buf[r, st]
             print(st, [int(x - base) if x > 0 else -1 for x in row])
-elif hasattr(lib, "glabc_debug_flow_trace"):
-    buf = np.zeros((2, 2, 16, 12), dtype=np.int64)
-    rc = lib.glabc_debug_flow_trace(buf.ctypes.data_as(ctypes.c_void_p))
-    assert rc == 0, rc
-    base = buf[buf > 0].min()
-    np.set_printoptions(linewidth=250)
-    for g in range(2):
-        for w in range(2):
-            print(f"group {g} thread {'0' if w == 0 else '224'}: stamps 0..10 relative to the first, per tile")
-            for t in range(16):
-                row = buf[g, w, t, :11]
-                print(t, (row - base).tolist(), "d:", np.diff(row).tolist())

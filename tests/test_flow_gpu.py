@@ -146,7 +146,7 @@ def test_matches_fp32_torch(flow, n):
         ok = torch.isfinite(lp_r)
         assert ok.float().mean() > 0.99 and torch.equal(torch.isfinite(lp), ok)
         err = (lp[ok] - lp_r[ok]).abs() / (1 + 0.01 * lp_r[ok].abs())
-        # TF32 operand rounding (2^-11 relative) through 32 blocks: tight in the bulk, amplified by exp(-s) in the tails
+        # FP16 operand rounding (2^-11 relative) through 32 blocks: tight in the bulk, amplified by exp(-s) in the tails
         assert float(err.median()) < 3e-3 and float(err.quantile(0.99)) < 5e-2 and float(err.max()) < 5.0, float(err.max())
         if n >= 1024:
             assert float(err.quantile(0.999)) < 0.3
@@ -202,7 +202,7 @@ def test_pipeline_kernels_with_few_coupling_blocks(n_blocks):
 def test_sample_log_prob_consistency(flow):
     """the kernel's own pair: log_prob(sample(eps)) reproduces the log q returned with the sample.  sample()'s log q is the
     exact density of the map that produced theta (same s values in the transform and the log-det); log_prob() re-derives
-    each block's input to ~1e-7, which can flip the TF32 rounding of a hidden unit, hence the 1e-3-level tolerance."""
+    each block's input to ~1e-7, which can flip the FP16 rounding of a hidden unit, hence the 1e-3-level tolerance."""
     eps = torch.randn(20000, 2, device="cuda", generator=torch.Generator(device="cuda").manual_seed(3))
     th, lq = flow.fused_sample_from(eps)
     lp = flow.fused_log_prob(th)
