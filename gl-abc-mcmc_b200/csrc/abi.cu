@@ -25,6 +25,33 @@
 
 using namespace glabc;
 
+// A grow-only scratch buffer of the context, in device memory or (Pinned) in page-locked host memory.  reserve() keeps no
+// contents: it frees the old buffer and allocates the larger one, and leaves the buffer empty (cap 0) when that fails.
+template <class T, bool Pinned = false>
+struct Scratch {
+    T* p = nullptr;
+    size_t cap = 0;
+    Scratch() = default;
+    Scratch(const Scratch&) = delete;
+    Scratch& operator=(const Scratch&) = delete;
+    ~Scratch() { release(); }
+    cudaError_t reserve(size_t n)
+    {
+        if (n <= cap) return cudaSuccess;
+        release();
+        const cudaError_t e = Pinned ? cudaHostAlloc(&p, n * sizeof(T), cudaHostAllocDefault) : cudaMalloc(&p, n * sizeof(T));
+        if (e == cudaSuccess) cap = n;
+        else p = nullptr;
+        return e;
+    }
+    void release()
+    {
+        if (p) (void)(Pinned ? cudaFreeHost(p) : cudaFree(p));
+        p = nullptr;
+        cap = 0;
+    }
+};
+
 struct glabc_ctx {
     int device = 0;
     int sm_count = 0, clock_khz = 0, cc = 0;
@@ -34,21 +61,16 @@ struct glabc_ctx {
     glabc_dist_t dist[GLABC_SLOT_COUNT]{};
     bool has_dist[GLABC_SLOT_COUNT] = {false, false, false};
     // scratch of the host-buffer entry points
-    float* d_state = nullptr;  // theta | y | aux | stats
-    size_t state_cap = 0;
-    double* d_state64 = nullptr;  // GLMALA carried float64 state
-    size_t state64_cap = 0;
+    Scratch<float> d_state;       // theta | y | aux | stats
+    Scratch<double> d_state64;    // GLMALA carried float64 state
     // AGLMCMC block / KDE workspace (one allocation), KDE sampling scratch of the public entry points
     void* ag_mem = nullptr;
     size_t ag_bytes = 0, ag_used = 0;
     AgWorkspace ag{};
     int ag_dim = 0;
-    double* kde_cdf = nullptr;
-    size_t kde_cdf_cap = 0;
-    double* rs_scratch = nullptr;   // block prefixes of glabc_resample
-    size_t rs_cap = 0;
-    float* kde_part = nullptr;   // partial sums of the point-split log_prob
-    size_t kde_part_cap = 0;
+    Scratch<double> kde_cdf;
+    Scratch<double> rs_scratch;   // block prefixes of glabc_resample
+    Scratch<float> kde_part;      // partial sums of the point-split log_prob
     // RealNVP flow weights (device copies owned by the context)
     float* flow_mem = nullptr;
     size_t flow_floats = 0;
@@ -60,21 +82,17 @@ struct glabc_ctx {
     float* tr_mem = nullptr;       // m | v | grad | loss
     float* tr_partial = nullptr;
     int tr_slices = 0;
-    float* tr_fwd = nullptr;       // z [n][2] | log q [n]
-    int64_t tr_fwd_cap = 0;
+    Scratch<float> tr_fwd;         // z [n][2] | log q [n]
     int64_t tr_step = 0;
     float tr_lr = 5e-4f, tr_beta1 = 0.9f, tr_beta2 = 0.999f, tr_eps = 1e-8f, tr_wd = 1e-5f;
     bool tr_ready = false;
-    float* d_trace[2] = {nullptr, nullptr};
-    size_t trace_cap = 0;
+    Scratch<float> d_trace[2];
     cudaStream_t s_compute = nullptr, s_copy = nullptr;
     // host entry, event transport (run_global_host_hybrid): device state + event buffer of the event-encoded chains, pinned staging
     cudaStream_t s_ev = nullptr;
     cudaEvent_t ev_group[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-    float* d_ev = nullptr;
-    size_t d_ev_cap = 0;
-    float* h_ev = nullptr;
-    size_t h_ev_cap = 0;
+    Scratch<float> d_ev;
+    Scratch<float, true> h_ev;
     cudaEvent_t ev_done[2] = {nullptr, nullptr}, ev_free[2] = {nullptr, nullptr};
 };
 
@@ -145,29 +163,20 @@ int glabc_ctx_destroy(glabc_ctx* ctx)
 {
     if (!ctx) return GLABC_OK;
     cudaSetDevice(ctx->device);
-    if (ctx->d_state) cudaFree(ctx->d_state);
-    if (ctx->d_state64) cudaFree(ctx->d_state64);
     if (ctx->ag_mem) cudaFree(ctx->ag_mem);
-    if (ctx->kde_cdf) cudaFree(ctx->kde_cdf);
-    if (ctx->kde_part) cudaFree(ctx->kde_part);
-    if (ctx->rs_scratch) cudaFree(ctx->rs_scratch);
     if (ctx->flow_mem) cudaFree(ctx->flow_mem);
     if (ctx->tr_mem) cudaFree(ctx->tr_mem);
     if (ctx->tr_partial) cudaFree(ctx->tr_partial);
-    if (ctx->tr_fwd) cudaFree(ctx->tr_fwd);
     for (int b = 0; b < 2; ++b) {
-        if (ctx->d_trace[b]) cudaFree(ctx->d_trace[b]);
         if (ctx->ev_done[b]) cudaEventDestroy(ctx->ev_done[b]);
         if (ctx->ev_free[b]) cudaEventDestroy(ctx->ev_free[b]);
     }
     if (ctx->s_ev) cudaStreamDestroy(ctx->s_ev);
     for (auto& e : ctx->ev_group)
         if (e) cudaEventDestroy(e);
-    if (ctx->d_ev) cudaFree(ctx->d_ev);
-    if (ctx->h_ev) cudaFreeHost(ctx->h_ev);
     if (ctx->s_compute) cudaStreamDestroy(ctx->s_compute);
     if (ctx->s_copy) cudaStreamDestroy(ctx->s_copy);
-    delete ctx;
+    delete ctx;   // the Scratch members free their buffers (the device is current)
     return GLABC_OK;
 }
 
@@ -539,10 +548,118 @@ static int run_device(glabc_ctx* ctx, SamplerKind kind, const glabc_run_t* run)
 }
 
 // ---------------------------------------------------------------------------------------------
-// host-buffer driver: H2D state, kernels in time chunks, D2H of each chunk's trace rows on a second
-// stream overlapped with the next chunk's kernel, D2H state + stats.
+// host-buffer entry points: the argument check, the chain state on the device, the time-chunk transport
 // ---------------------------------------------------------------------------------------------
-static int ensure_host_scratch(glabc_ctx* ctx, size_t state_floats, size_t trace_floats)
+// Checks a host-buffer run before anything is allocated or launched, so that a bad argument leaves the caller's buffers
+// untouched.  With n_chains == 0 there is nothing to do: the run passes before any pointer is looked at.
+static int check_host_run(glabc_ctx* ctx, const glabc_run_t* run)
+{
+    if (!ctx) return GLABC_ERR_INVALID;
+    if (!ctx->has_model) return fail(ctx, GLABC_ERR_INVALID, "no model bound: call glabc_model_set first");
+    if (!run) return fail(ctx, GLABC_ERR_INVALID, "null run description");
+    if (run->rng_mode != GLABC_RNG_NATIVE) return fail(ctx, GLABC_ERR_INVALID, "host entry points run the native RNG only");
+    // GLABC_TRACE_EVENTS is a device-buffer layout (glabc.h): the scratch is sized for dense rows, an event writer would run
+    // past it.  The event TRANSPORT of the host entries is chosen internally (run_global_host_hybrid), never by the caller.
+    if (run->trace_layout != GLABC_TRACE_NONE && run->trace_layout != GLABC_TRACE_TIME_MAJOR &&
+        run->trace_layout != GLABC_TRACE_CHAIN_MAJOR)
+        return fail(ctx, GLABC_ERR_UNSUPPORTED, "host entry points deliver GLABC_TRACE_NONE / TIME_MAJOR / CHAIN_MAJOR traces "
+                                                "(trace_layout %d is a device-buffer layout)", run->trace_layout);
+    if (run->n_chains <= 0 || run->n_steps < 0) return run->n_chains == 0 ? GLABC_OK : fail(ctx, GLABC_ERR_INVALID, "bad sizes");
+    if (!run->theta || !run->y) return fail(ctx, GLABC_ERR_INVALID, "theta / y state pointers are required");
+    if (run->trace_layout == GLABC_TRACE_NONE) return GLABC_OK;
+    if (!run->trace) return fail(ctx, GLABC_ERR_INVALID, "trace pointer required for this trace_layout");
+    const int64_t lo = run->step_base + (run->write_row0 ? 0 : 1) - run->trace_row_base;   // first and last host row written
+    const int64_t hi = run->step_base + run->n_steps - run->trace_row_base;
+    if (lo <= hi && (lo < 0 || hi >= run->trace_rows)) return fail(ctx, GLABC_ERR_INVALID, "trace rows fall outside the host buffer");
+    if (run->trace_chain_off < 0 || run->trace_chain_off + run->n_chains > run->trace_chains)
+        return fail(ctx, GLABC_ERR_INVALID, "chains fall outside the host trace buffer");
+    return GLABC_OK;
+}
+
+// The per-chain state of a host-buffer run: theta [C][d], y [C][y_dim], aux [C][GLABC_AUX_SLOTS], stats [C][ns] and
+// state64 [C][GLABC_STATE64_SLOTS].  aux, stats and state64 are null when the run carries none.
+struct ChainState {
+    float *theta, *y, *aux, *stats;
+    double* state64;
+};
+
+static ChainState host_state(const glabc_run_t* run) { return {run->theta, run->y, run->aux, run->stats, run->state64}; }
+
+// the state from chain c0 on
+static ChainState chains_at(const glabc_ctx* ctx, const ChainState& s, int64_t c0)
+{
+    const int d = ctx->model.theta_dim;
+    auto at = [c0](auto* p, int64_t width) { return p ? p + c0 * width : p; };
+    return {at(s.theta, d), at(s.y, ctx->model.y_dim), at(s.aux, GLABC_AUX_SLOTS), at(s.stats, GLABC_NSTATS(d)),
+            at(s.state64, GLABC_STATE64_SLOTS)};
+}
+
+// floats of the device state of n chains of the run (state64 apart)
+static size_t state_floats(const glabc_ctx* ctx, const glabc_run_t* run, int64_t n)
+{
+    const int d = ctx->model.theta_dim;
+    return size_t(n) * (d + ctx->model.y_dim + (run->aux ? GLABC_AUX_SLOTS : 0) + (run->stats ? GLABC_NSTATS(d) : 0));
+}
+
+// the state of n chains of the run laid out in `f` as theta | y | aux | stats, and state64 in `f64`
+static ChainState carve_state(const glabc_ctx* ctx, const glabc_run_t* run, int64_t n, float* f, double* f64)
+{
+    ChainState s{};
+    s.theta = f;
+    s.y = s.theta + n * ctx->model.theta_dim;
+    float* next = s.y + n * ctx->model.y_dim;
+    if (run->aux) {
+        s.aux = next;
+        next += n * GLABC_AUX_SLOTS;
+    }
+    if (run->stats) s.stats = next;
+    if (run->state64) s.state64 = f64;
+    return s;
+}
+
+// Copies the state of chains [c0, c0 + n) between the run's host buffers and their device copy `dev` on stream s, in the
+// direction `dir` (cudaMemcpyHostToDevice or cudaMemcpyDeviceToHost): the arrays `dev` has.  Returns the first error.
+static cudaError_t stage_state(const glabc_ctx* ctx, const glabc_run_t* run, int64_t c0, int64_t n, const ChainState& dev,
+                               cudaMemcpyKind dir, cudaStream_t s)
+{
+    const int d = ctx->model.theta_dim;
+    const ChainState host = chains_at(ctx, host_state(run), c0);
+    cudaError_t e = cudaSuccess;
+    auto copy = [&](void* hp, void* dp, size_t chain_bytes) {
+        if (!dp || e != cudaSuccess) return;
+        const size_t bytes = size_t(n) * chain_bytes;
+        e = dir == cudaMemcpyHostToDevice ? cudaMemcpyAsync(dp, hp, bytes, dir, s) : cudaMemcpyAsync(hp, dp, bytes, dir, s);
+    };
+    copy(host.theta, dev.theta, d * sizeof(float));
+    copy(host.y, dev.y, ctx->model.y_dim * sizeof(float));
+    copy(host.aux, dev.aux, GLABC_AUX_SLOTS * sizeof(float));
+    copy(host.stats, dev.stats, GLABC_NSTATS(d) * sizeof(float));
+    copy(host.state64, dev.state64, GLABC_STATE64_SLOTS * sizeof(double));
+    return e;
+}
+
+// The run of chains [c0, c0 + n) of a host run, `s` being their state, on stream `stream`; every dump, tape and debug pointer
+// is null.  For a launch the caller points the trace at its device buffer.
+static glabc_run_t chain_slice(const glabc_run_t* run, int64_t c0, int64_t n, const ChainState& s, cudaStream_t stream)
+{
+    glabc_run_t r = *run;
+    r.n_chains = n;
+    r.chain_id_base = run->chain_id_base + c0;
+    r.theta = s.theta;
+    r.y = s.y;
+    r.aux = s.aux;
+    r.stats = s.stats;
+    r.state64 = s.state64;
+    r.stream = stream;
+    r.tape32 = r.tape_grad0 = nullptr;
+    r.tape64 = nullptr;
+    r.debug = r.tape_dump = r.tape_grad0_dump = nullptr;
+    r.debug64 = r.tape64_dump = nullptr;
+    return r;
+}
+
+// streams and events of the dense transports, the device state of n chains of the run and two trace buffers
+static int ensure_host_scratch(glabc_ctx* ctx, const glabc_run_t* run, int64_t n, size_t trace_floats, ChainState* dev)
 {
     if (!ctx->s_compute) {
         CUDA_TRY(ctx, cudaStreamCreateWithFlags(&ctx->s_compute, cudaStreamNonBlocking));
@@ -552,45 +669,20 @@ static int ensure_host_scratch(glabc_ctx* ctx, size_t state_floats, size_t trace
             CUDA_TRY(ctx, cudaEventCreateWithFlags(&ctx->ev_free[b], cudaEventDisableTiming));
         }
     }
-    if (state_floats > ctx->state_cap) {
-        if (ctx->d_state) cudaFree(ctx->d_state);
-        ctx->d_state = nullptr;
-        ctx->state_cap = 0;
-        CUDA_TRY(ctx, cudaMalloc(&ctx->d_state, state_floats * sizeof(float)));
-        ctx->state_cap = state_floats;
-    }
-    if (trace_floats > ctx->trace_cap) {
-        for (int b = 0; b < 2; ++b) {
-            if (ctx->d_trace[b]) cudaFree(ctx->d_trace[b]);
-            ctx->d_trace[b] = nullptr;
-        }
-        ctx->trace_cap = 0;
-        for (int b = 0; b < 2; ++b) CUDA_TRY(ctx, cudaMalloc(&ctx->d_trace[b], trace_floats * sizeof(float)));
-        ctx->trace_cap = trace_floats;
-    }
+    CUDA_TRY(ctx, ctx->d_state.reserve(state_floats(ctx, run, n)));
+    CUDA_TRY(ctx, ctx->d_state64.reserve(run->state64 ? size_t(n) * GLABC_STATE64_SLOTS : 0));
+    for (auto& t : ctx->d_trace) CUDA_TRY(ctx, t.reserve(trace_floats));
+    *dev = carve_state(ctx, run, n, ctx->d_state.p, ctx->d_state64.p);
     return GLABC_OK;
 }
 
+// Time-chunk transport: H2D state, kernels in time chunks, D2H of each chunk's trace rows on a second stream overlapped with
+// the next chunk's kernel, D2H state + stats.
 static int run_host(glabc_ctx* ctx, SamplerKind kind, const glabc_run_t* run, int64_t chunk_steps, const glabc_aglmcmc_t* ag = nullptr)
 {
-    if (!ctx) return GLABC_ERR_INVALID;
-    if (!ctx->has_model) return fail(ctx, GLABC_ERR_INVALID, "no model bound: call glabc_model_set first");
-    if (!run) return fail(ctx, GLABC_ERR_INVALID, "null run description");
-    if (run->rng_mode != GLABC_RNG_NATIVE) return fail(ctx, GLABC_ERR_INVALID, "host entry points run the native RNG only");
-    // GLABC_TRACE_EVENTS is a device-buffer layout (glabc.h): the scratch below is sized for dense rows, an event writer
-    // would run past it.  The event TRANSPORT of the host entries is chosen internally (run_host_hybrid), never by the caller.
-    if (run->trace_layout != GLABC_TRACE_NONE && run->trace_layout != GLABC_TRACE_TIME_MAJOR &&
-        run->trace_layout != GLABC_TRACE_CHAIN_MAJOR)
-        return fail(ctx, GLABC_ERR_UNSUPPORTED, "host entry points deliver GLABC_TRACE_NONE / TIME_MAJOR / CHAIN_MAJOR traces "
-                                                "(trace_layout %d is a device-buffer layout)", run->trace_layout);
-    if (run->n_chains <= 0 || run->n_steps < 0) return run->n_chains == 0 ? GLABC_OK : fail(ctx, GLABC_ERR_INVALID, "bad sizes");
-    if (!run->theta || !run->y) return fail(ctx, GLABC_ERR_INVALID, "theta / y state pointers are required");
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    const int d = ctx->model.theta_dim, yd = ctx->model.y_dim;
+    const int d = ctx->model.theta_dim;
     const int64_t C = run->n_chains;
-    const int ns = GLABC_NSTATS(d);
     const bool traced = run->trace_layout != GLABC_TRACE_NONE;
-    if (traced && !run->trace) return fail(ctx, GLABC_ERR_INVALID, "trace pointer required for this trace_layout");
 
     int64_t chunk = chunk_steps > 0 ? chunk_steps : (int64_t(64) << 20) / (C * d * int64_t(sizeof(float)));
     chunk = ((chunk + 31) / 32) * 32;
@@ -598,29 +690,11 @@ static int run_host(glabc_ctx* ctx, SamplerKind kind, const glabc_run_t* run, in
     if (chunk > run->n_steps) chunk = run->n_steps > 0 ? run->n_steps : 1;
     const int64_t buf_rows = chunk + 1;  // +1: the first chunk may carry row 0
 
-    const size_t n_theta = size_t(C) * d, n_y = size_t(C) * yd, n_aux = run->aux ? size_t(C) * GLABC_AUX_SLOTS : 0,
-                 n_stats = run->stats ? size_t(C) * ns : 0;
-    int st = ensure_host_scratch(ctx, n_theta + n_y + n_aux + n_stats, traced ? size_t(buf_rows) * C * d : 0);
+    ChainState state;
+    int st = ensure_host_scratch(ctx, run, C, traced ? size_t(buf_rows) * C * d : 0, &state);
     if (st) return st;
-    const size_t n_s64 = run->state64 ? size_t(C) * GLABC_STATE64_SLOTS : 0;
-    if (n_s64 > ctx->state64_cap) {
-        if (ctx->d_state64) cudaFree(ctx->d_state64);
-        ctx->d_state64 = nullptr;
-        ctx->state64_cap = 0;
-        CUDA_TRY(ctx, cudaMalloc(&ctx->d_state64, n_s64 * sizeof(double)));
-        ctx->state64_cap = n_s64;
-    }
-    float* d_theta = ctx->d_state;
-    float* d_y = d_theta + n_theta;
-    float* d_aux = n_aux ? d_y + n_y : nullptr;
-    float* d_stats = n_stats ? d_y + n_y + n_aux : nullptr;
-
     cudaStream_t sc = ctx->s_compute, sx = ctx->s_copy;
-    CUDA_TRY(ctx, cudaMemcpyAsync(d_theta, run->theta, n_theta * sizeof(float), cudaMemcpyHostToDevice, sc));
-    CUDA_TRY(ctx, cudaMemcpyAsync(d_y, run->y, n_y * sizeof(float), cudaMemcpyHostToDevice, sc));
-    if (d_aux) CUDA_TRY(ctx, cudaMemcpyAsync(d_aux, run->aux, n_aux * sizeof(float), cudaMemcpyHostToDevice, sc));
-    if (d_stats) CUDA_TRY(ctx, cudaMemcpyAsync(d_stats, run->stats, n_stats * sizeof(float), cudaMemcpyHostToDevice, sc));
-    if (n_s64) CUDA_TRY(ctx, cudaMemcpyAsync(ctx->d_state64, run->state64, n_s64 * sizeof(double), cudaMemcpyHostToDevice, sc));
+    CUDA_TRY(ctx, stage_state(ctx, run, 0, C, state, cudaMemcpyHostToDevice, sc));
 
     int64_t done = 0;
     int b = 0;
@@ -628,26 +702,15 @@ static int run_host(glabc_ctx* ctx, SamplerKind kind, const glabc_run_t* run, in
     bool first_chunk = true;
     do {
         const int64_t n = std::min<int64_t>(chunk, run->n_steps - done);
-        glabc_run_t dev = *run;
+        glabc_run_t dev = chain_slice(run, 0, C, state, sc);
         dev.n_steps = n;
         dev.step_base = run->step_base + done;
         dev.write_row0 = first_chunk && run->write_row0;
-        dev.theta = d_theta;
-        dev.y = d_y;
-        dev.aux = d_aux;
-        dev.stats = d_stats;
-        dev.state64 = n_s64 ? ctx->d_state64 : nullptr;
-        dev.stream = sc;
-        dev.tape_dump = nullptr;
-        dev.tape_grad0_dump = nullptr;
-        dev.tape64_dump = nullptr;
-        dev.debug = nullptr;
-        dev.debug64 = nullptr;
         const int64_t row_lo = dev.step_base + (dev.write_row0 ? 0 : 1);  // first absolute row this chunk writes
         const int64_t n_rows = n + (dev.write_row0 ? 1 : 0);
         if (traced) {
             if (used[b]) CUDA_TRY(ctx, cudaStreamWaitEvent(sc, ctx->ev_free[b], 0));
-            dev.trace = ctx->d_trace[b];
+            dev.trace = ctx->d_trace[b].p;
             dev.trace_rows = buf_rows;
             dev.trace_chains = C;
             dev.trace_chain_off = 0;
@@ -669,16 +732,14 @@ static int run_host(glabc_ctx* ctx, SamplerKind kind, const glabc_run_t* run, in
             CUDA_TRY(ctx, cudaEventRecord(ctx->ev_done[b], sc));
             CUDA_TRY(ctx, cudaStreamWaitEvent(sx, ctx->ev_done[b], 0));
             const int64_t host_row = row_lo - run->trace_row_base;
-            if (host_row < 0 || host_row + n_rows > run->trace_rows)
-                return fail(ctx, GLABC_ERR_INVALID, "trace rows fall outside the host buffer");
             if (run->trace_layout == GLABC_TRACE_TIME_MAJOR) {
                 float* dst = run->trace + (host_row * run->trace_chains + run->trace_chain_off) * d;
-                CUDA_TRY(ctx, cudaMemcpy2DAsync(dst, size_t(run->trace_chains) * d * sizeof(float), ctx->d_trace[b],
+                CUDA_TRY(ctx, cudaMemcpy2DAsync(dst, size_t(run->trace_chains) * d * sizeof(float), ctx->d_trace[b].p,
                                                 size_t(C) * d * sizeof(float), size_t(C) * d * sizeof(float), size_t(n_rows),
                                                 cudaMemcpyDeviceToHost, sx));
             } else {
                 float* dst = run->trace + (run->trace_chain_off * run->trace_rows + host_row) * d;
-                CUDA_TRY(ctx, cudaMemcpy2DAsync(dst, size_t(run->trace_rows) * d * sizeof(float), ctx->d_trace[b],
+                CUDA_TRY(ctx, cudaMemcpy2DAsync(dst, size_t(run->trace_rows) * d * sizeof(float), ctx->d_trace[b].p,
                                                 size_t(buf_rows) * d * sizeof(float), size_t(n_rows) * d * sizeof(float), size_t(C),
                                                 cudaMemcpyDeviceToHost, sx));
             }
@@ -690,11 +751,7 @@ static int run_host(glabc_ctx* ctx, SamplerKind kind, const glabc_run_t* run, in
         first_chunk = false;
     } while (done < run->n_steps);
 
-    CUDA_TRY(ctx, cudaMemcpyAsync(run->theta, d_theta, n_theta * sizeof(float), cudaMemcpyDeviceToHost, sc));
-    CUDA_TRY(ctx, cudaMemcpyAsync(run->y, d_y, n_y * sizeof(float), cudaMemcpyDeviceToHost, sc));
-    if (d_aux) CUDA_TRY(ctx, cudaMemcpyAsync(run->aux, d_aux, n_aux * sizeof(float), cudaMemcpyDeviceToHost, sc));
-    if (d_stats) CUDA_TRY(ctx, cudaMemcpyAsync(run->stats, d_stats, n_stats * sizeof(float), cudaMemcpyDeviceToHost, sc));
-    if (n_s64) CUDA_TRY(ctx, cudaMemcpyAsync(run->state64, ctx->d_state64, n_s64 * sizeof(double), cudaMemcpyDeviceToHost, sc));
+    CUDA_TRY(ctx, stage_state(ctx, run, 0, C, state, cudaMemcpyDeviceToHost, sc));
     CUDA_TRY(ctx, cudaStreamSynchronize(sc));
     CUDA_TRY(ctx, cudaStreamSynchronize(sx));
     return GLABC_OK;
@@ -866,19 +923,10 @@ extern "C" int glabc_kde_log_prob(glabc_ctx* ctx, const float* X, const float* w
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     KdeSets S{X, weights, bw, n, nullptr, sets, cap};
     const int ksplit = arith == GLABC_ARITH_STRICT ? 1 : kde_logprob_split(sets, m, cap);
-    if (ksplit > 1) {
-        const size_t need = size_t(ksplit) * size_t(sets) * size_t(m);
-        if (need > ctx->kde_part_cap) {
-            if (ctx->kde_part) cudaFree(ctx->kde_part);
-            ctx->kde_part = nullptr;
-            ctx->kde_part_cap = 0;
-            CUDA_TRY(ctx, cudaMalloc(&ctx->kde_part, need * sizeof(float)));
-            ctx->kde_part_cap = need;
-        }
-    }
+    if (ksplit > 1) CUDA_TRY(ctx, ctx->kde_part.reserve(size_t(ksplit) * size_t(sets) * size_t(m)));
     // (a non-null scratch pointer tells the launcher the point split is available, even when this call needs ksplit = 1)
     CUDA_TRY(ctx, launch_kde_logprob(S, nullptr, dim, x, m, out, arith == GLABC_ARITH_STRICT, static_cast<cudaStream_t>(stream), ksplit,
-                                     ksplit > 1 ? ctx->kde_part : reinterpret_cast<float*>(out)));
+                                     ksplit > 1 ? ctx->kde_part.p : reinterpret_cast<float*>(out)));
     return GLABC_OK;
 }
 
@@ -896,18 +944,11 @@ extern "C" int glabc_kde_sample(glabc_ctx* ctx, const float* X, const float* wei
     cudaStream_t cs = static_cast<cudaStream_t>(stream);
     KdeSets S{X, weights, bw, n, nullptr, sets, cap};
     if (!idx_tape) {
-        const size_t need = size_t(sets) * size_t(cap);
-        if (need > ctx->kde_cdf_cap) {
-            if (ctx->kde_cdf) cudaFree(ctx->kde_cdf);
-            ctx->kde_cdf = nullptr;
-            ctx->kde_cdf_cap = 0;
-            CUDA_TRY(ctx, cudaMalloc(&ctx->kde_cdf, need * sizeof(double)));
-            ctx->kde_cdf_cap = need;
-        }
-        CUDA_TRY(ctx, launch_kde_cdf(weights, n, nullptr, sets, cap, ctx->kde_cdf, cs));
+        CUDA_TRY(ctx, ctx->kde_cdf.reserve(size_t(sets) * size_t(cap)));
+        CUDA_TRY(ctx, launch_kde_cdf(weights, n, nullptr, sets, cap, ctx->kde_cdf.p, cs));
     }
     const RoundKeys rk = expand_key(make_uint2(static_cast<uint32_t>(seed), static_cast<uint32_t>(seed >> 32)));
-    CUDA_TRY(ctx, launch_kde_sample(S, dim, ctx->kde_cdf, m, rk, 0, nullptr, idx_tape, noise_tape, m, m * dim, 1, 0, 0, 0, out, cs));
+    CUDA_TRY(ctx, launch_kde_sample(S, dim, ctx->kde_cdf.p, m, rk, 0, nullptr, idx_tape, noise_tape, m, m * dim, 1, 0, 0, 0, out, cs));
     return GLABC_OK;
 }
 
@@ -1027,15 +1068,9 @@ extern "C" int glabc_flow_grad(glabc_ctx* ctx, const float* x, int64_t n, float*
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     cudaStream_t cs = static_cast<cudaStream_t>(stream);
     const int64_t total = FlowParamLayout(ctx->flow_blocks).total;
-    if (n > ctx->tr_fwd_cap) {
-        if (ctx->tr_fwd) cudaFree(ctx->tr_fwd);
-        ctx->tr_fwd = nullptr;
-        ctx->tr_fwd_cap = 0;
-        CUDA_TRY(ctx, cudaMalloc(&ctx->tr_fwd, size_t(n) * 3 * sizeof(float)));
-        ctx->tr_fwd_cap = n;
-    }
-    float* z = ctx->tr_fwd;
-    float* lq = ctx->tr_fwd + 2 * n;
+    CUDA_TRY(ctx, ctx->tr_fwd.reserve(size_t(n) * 3));
+    float* z = ctx->tr_fwd.p;
+    float* lq = ctx->tr_fwd.p + 2 * n;
     float* g = grad ? grad : ctx->tr_mem + 2 * total;
     float* ls = loss ? loss : ctx->tr_mem + 3 * total;
     // forward: log q(x) and the latent z = f^-1(x), split-precision mode whatever the inference mode is
@@ -1353,9 +1388,11 @@ extern "C" int glabc_run_mala_user(glabc_ctx* ctx, const glabc_run_t* run, const
 // repetition and the 5.2 GB device -> host copy of 65,536 x 1e4 rows is what bounds the call (PCIe, ~55 GB/s).  Here the
 // last `f` of the chains are run with GLABC_TRACE_EVENTS, their moves (a few hundred KB per thousand chains) are copied
 // back, and the host cores expand them into the caller's dense buffer WHILE the DMA engine brings the other chains' dense
-// rows over PCIe (the chunked, double-buffered path above).  The caller's buffer ends up bit-identical to the all-dense path.
+// rows over PCIe (dense_chain_groups below).  The caller's buffer ends up bit-identical to the all-dense path.
 // A chain with more moves than the event capacity makes the event part fall back to the dense path.
-// Tunables (environment): GLABC_HOST_EVENTS=0 disables, GLABC_HOST_EVENT_FRACTION (default 0.6), GLABC_HOST_THREADS.
+// Environment: GLABC_HOST_EVENTS=0 disables the event transport; GLABC_HOST_EVENT_FRACTION sets the share of the chains that
+// travels as events (default 1 with AVX-512 stores, else 0.6); GLABC_HOST_TIMING prints the phase times to stderr.  The
+// expansion takes the host's cores, split between the ranks of a node by LOCAL_WORLD_SIZE.
 // ---------------------------------------------------------------------------------------------
 // Run-length expansion of one chain into the caller's dense rows.  With AVX-512 and a row size that divides a cache line
 // (d in {1, 2, 4}) the whole chain is written as FULL 64-byte lines with non-temporal stores — a line that straddles a move
@@ -1447,69 +1484,72 @@ static void expand_chain(const float* ev, int64_t cap, int d, int64_t row_base, 
     }
 }
 
+// Expands chains [c0, c1) of an event buffer [chains][cap][1 + d] into the chain-major rows of `trace` [chains][trace_rows][d]
+// on n_threads host threads, the chains dealt round-robin.
+static void expand_parallel(const float* events, int64_t c0, int64_t c1, int64_t cap, int d, int64_t row_base, int64_t row_end,
+                            float* trace, int64_t trace_rows, int n_threads, bool nt512)
+{
+    std::vector<std::thread> workers;
+    for (int t = 0; t < n_threads; ++t)
+        workers.emplace_back([=]() {
+            for (int64_t c = c0 + t; c < c1; c += n_threads)
+                expand_chain(events + c * cap * (1 + d), cap, d, row_base, row_end, trace + c * trace_rows * d, nt512);
+            _mm_sfence();   // the non-temporal stores are globally visible before the thread is joined
+        });
+    for (auto& w : workers) w.join();
+}
+
 // Dense transport for a chain-major host trace: the chains are run in GROUPS over all their steps, and each group's
 // [chains][rows][d] block — contiguous on both sides — goes back in one full-rate copy while the next group's kernel runs
 // (time chunks of a chain-major trace would be 2-D copies of ~1 KB segments, which the DMA engine moves at half the rate).
 static int dense_chain_groups(glabc_ctx* ctx, SamplerKind kind, const glabc_run_t* run, int64_t Cd)
 {
-    const int d = ctx->model.theta_dim, yd = ctx->model.y_dim, ns = GLABC_NSTATS(d);
+    const int d = ctx->model.theta_dim;
     const int64_t n_rows = run->n_steps + (run->write_row0 ? 1 : 0);
     const int64_t row_lo = run->step_base + (run->write_row0 ? 0 : 1);
     int64_t Cg = (int64_t(320) << 20) / (n_rows * d * int64_t(sizeof(float))) / 32 * 32;
     if (Cg < 32) Cg = 32;
     if (Cg > Cd) Cg = Cd;
-    const size_t n_theta = size_t(Cd) * d, n_y = size_t(Cd) * yd, n_stats = run->stats ? size_t(Cd) * ns : 0;
-    const size_t n_aux = run->aux ? size_t(Cd) * GLABC_AUX_SLOTS : 0;
-    int st = ensure_host_scratch(ctx, n_theta + n_y + n_stats + n_aux, size_t(Cg) * n_rows * d);
+    ChainState state;
+    int st = ensure_host_scratch(ctx, run, Cd, size_t(Cg) * n_rows * d, &state);
     if (st) return st;
-    float* d_theta = ctx->d_state;
-    float* d_y = d_theta + n_theta;
-    float* d_stats = n_stats ? d_y + n_y : nullptr;
-    float* d_aux = n_aux ? d_y + n_y + n_stats : nullptr;
     cudaStream_t sc = ctx->s_compute, sx = ctx->s_copy;
-    CUDA_TRY(ctx, cudaMemcpyAsync(d_theta, run->theta, n_theta * sizeof(float), cudaMemcpyHostToDevice, sc));
-    CUDA_TRY(ctx, cudaMemcpyAsync(d_y, run->y, n_y * sizeof(float), cudaMemcpyHostToDevice, sc));
-    if (d_stats) CUDA_TRY(ctx, cudaMemcpyAsync(d_stats, run->stats, n_stats * sizeof(float), cudaMemcpyHostToDevice, sc));
-    if (d_aux) CUDA_TRY(ctx, cudaMemcpyAsync(d_aux, run->aux, n_aux * sizeof(float), cudaMemcpyHostToDevice, sc));
+    CUDA_TRY(ctx, stage_state(ctx, run, 0, Cd, state, cudaMemcpyHostToDevice, sc));
     bool used[2] = {false, false};
     int b = 0;
     for (int64_t g0 = 0; g0 < Cd; g0 += Cg) {
         const int64_t n = std::min<int64_t>(Cg, Cd - g0);
-        glabc_run_t dev = *run;
-        dev.n_chains = n;
-        dev.chain_id_base = run->chain_id_base + g0;
-        dev.theta = d_theta + g0 * d;
-        dev.y = d_y + g0 * yd;
-        dev.stats = d_stats ? d_stats + g0 * ns : nullptr;
-        dev.aux = d_aux ? d_aux + g0 * GLABC_AUX_SLOTS : nullptr;
-        dev.trace = ctx->d_trace[b];
-        dev.trace_layout = GLABC_TRACE_CHAIN_MAJOR;
+        glabc_run_t dev = chain_slice(run, g0, n, chains_at(ctx, state, g0), sc);
+        dev.trace = ctx->d_trace[b].p;
         dev.trace_rows = n_rows;
         dev.trace_chains = n;
         dev.trace_chain_off = 0;
         dev.trace_row_base = row_lo;
-        dev.stream = sc;
-        dev.tape_dump = nullptr;
-        dev.debug = nullptr;
         if (used[b]) CUDA_TRY(ctx, cudaStreamWaitEvent(sc, ctx->ev_free[b], 0));
         st = run_device(ctx, kind, &dev);
         if (st) return st;
         CUDA_TRY(ctx, cudaEventRecord(ctx->ev_done[b], sc));
         CUDA_TRY(ctx, cudaStreamWaitEvent(sx, ctx->ev_done[b], 0));
         float* dst = run->trace + ((run->trace_chain_off + g0) * run->trace_rows + (row_lo - run->trace_row_base)) * d;
-        CUDA_TRY(ctx, cudaMemcpy2DAsync(dst, size_t(run->trace_rows) * d * sizeof(float), ctx->d_trace[b], size_t(n_rows) * d * sizeof(float),
+        CUDA_TRY(ctx, cudaMemcpy2DAsync(dst, size_t(run->trace_rows) * d * sizeof(float), ctx->d_trace[b].p, size_t(n_rows) * d * sizeof(float),
                                         size_t(n_rows) * d * sizeof(float), size_t(n), cudaMemcpyDeviceToHost, sx));
         CUDA_TRY(ctx, cudaEventRecord(ctx->ev_free[b], sx));
         used[b] = true;
         b ^= 1;
     }
-    CUDA_TRY(ctx, cudaMemcpyAsync(run->theta, d_theta, n_theta * sizeof(float), cudaMemcpyDeviceToHost, sc));
-    CUDA_TRY(ctx, cudaMemcpyAsync(run->y, d_y, n_y * sizeof(float), cudaMemcpyDeviceToHost, sc));
-    if (d_stats) CUDA_TRY(ctx, cudaMemcpyAsync(run->stats, d_stats, n_stats * sizeof(float), cudaMemcpyDeviceToHost, sc));
-    if (d_aux) CUDA_TRY(ctx, cudaMemcpyAsync(run->aux, d_aux, n_aux * sizeof(float), cudaMemcpyDeviceToHost, sc));
+    CUDA_TRY(ctx, stage_state(ctx, run, 0, Cd, state, cudaMemcpyDeviceToHost, sc));
     CUDA_TRY(ctx, cudaStreamSynchronize(sc));
     CUDA_TRY(ctx, cudaStreamSynchronize(sx));
     return GLABC_OK;
+}
+
+// The dense transport of GlobalMCMC / GLMCMC: a chain-major trace with the default chunking (chunk_steps == 0) travels chain
+// group by chain group, anything else in time chunks.
+static int run_host_dense(glabc_ctx* ctx, SamplerKind kind, const glabc_run_t* run, int64_t chunk_steps)
+{
+    if (run->trace_layout == GLABC_TRACE_CHAIN_MAJOR && chunk_steps == 0 && run->n_steps > 0)
+        return dense_chain_groups(ctx, kind, run, run->n_chains);
+    return run_host(ctx, kind, run, chunk_steps);
 }
 
 static int run_global_host_hybrid(glabc_ctx* ctx, SamplerKind kind, const glabc_run_t* run, int64_t chunk_steps, bool* handled)
@@ -1517,33 +1557,24 @@ static int run_global_host_hybrid(glabc_ctx* ctx, SamplerKind kind, const glabc_
     *handled = false;
     const char* off = getenv("GLABC_HOST_EVENTS");
     if (off && off[0] == '0') return GLABC_OK;
-    if (!ctx->has_model || !run || run->trace_layout != GLABC_TRACE_CHAIN_MAJOR || !run->trace || run->rng_mode != GLABC_RNG_NATIVE ||
-        run->n_steps < 512 || run->n_chains < 256 || !run->theta || !run->y)
-        return GLABC_OK;
+    if (run->trace_layout != GLABC_TRACE_CHAIN_MAJOR || run->n_steps < 512 || run->n_chains < 256) return GLABC_OK;
     const int far_slot = kind == SAMPLER_ISIR ? GLABC_SLOT_IMPORTANCE : GLABC_SLOT_GLOBAL;
-    if (kind != SAMPLER_GLOBAL && kind != SAMPLER_ISIR) return GLABC_OK;
     if (!ctx->has_dist[GLABC_SLOT_LOCAL] || !ctx->has_dist[far_slot] || !all_gaussian(ctx, {GLABC_SLOT_LOCAL, far_slot})) return GLABC_OK;
     if (kind == SAMPLER_ISIR && !run->aux) return GLABC_OK;
-    const int dd = ctx->model.theta_dim;
-    const bool nt512 = (dd == 1 || dd == 2 || dd == 4) && __builtin_cpu_supports("avx512f");
+    const int d = ctx->model.theta_dim, yd = ctx->model.y_dim, ns = GLABC_NSTATS(d);
+    const bool nt512 = (d == 1 || d == 2 || d == 4) && __builtin_cpu_supports("avx512f");
     // with full-line non-temporal stores the expansion alone runs at the host's DRAM write rate, which a concurrent dense DMA
     // would only share; with ordinary stores (65 GB/s) the PCIe copy of part of the chains adds bandwidth
     double frac = nt512 ? 1.0 : 0.6;
     if (const char* f = getenv("GLABC_HOST_EVENT_FRACTION")) frac = atof(f);
     if (!(frac > 0.0)) return GLABC_OK;
     if (frac > 1.0) frac = 1.0;
-    const int d = ctx->model.theta_dim, yd = ctx->model.y_dim, ns = GLABC_NSTATS(d);
     const int64_t C = run->n_chains;
     int64_t Ce = static_cast<int64_t>(C * frac) / 32 * 32;
     if (Ce <= 0) return GLABC_OK;
     const int64_t Cd = C - Ce;
-    const int64_t row_lo = run->step_base + (run->write_row0 ? 0 : 1), row_end = run->step_base + run->n_steps;
-    if (row_lo - run->trace_row_base < 0 || row_end - run->trace_row_base >= run->trace_rows)
-        return fail(ctx, GLABC_ERR_INVALID, "trace rows fall outside the host buffer");
-    if (run->trace_chain_off < 0 || run->trace_chain_off + C > run->trace_chains)
-        return fail(ctx, GLABC_ERR_INVALID, "chains fall outside the host trace buffer");
+    const int64_t row_end = run->step_base + run->n_steps;
     *handled = true;
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     if (!ctx->s_ev) {
         CUDA_TRY(ctx, cudaStreamCreateWithFlags(&ctx->s_ev, cudaStreamNonBlocking));
         for (auto& e : ctx->ev_group) CUDA_TRY(ctx, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
@@ -1551,35 +1582,15 @@ static int run_global_host_hybrid(glabc_ctx* ctx, SamplerKind kind, const glabc_
     int64_t cap = run->n_steps / 32;
     if (cap < 64) cap = 64;
     if (cap > run->n_steps + 2) cap = run->n_steps + 2;
-    const size_t n_theta = size_t(Ce) * d, n_y = size_t(Ce) * yd, n_stats = run->stats ? size_t(Ce) * ns : 0;
-    const size_t n_aux = kind == SAMPLER_ISIR ? size_t(Ce) * GLABC_AUX_SLOTS : 0;
-    const size_t n_state = n_theta + n_y + n_stats + n_aux, n_events = size_t(Ce) * size_t(cap) * (1 + d);
-    if (n_state + n_events > ctx->d_ev_cap) {
-        if (ctx->d_ev) cudaFree(ctx->d_ev);
-        ctx->d_ev = nullptr;
-        ctx->d_ev_cap = 0;
-        CUDA_TRY(ctx, cudaMalloc(&ctx->d_ev, (n_state + n_events) * sizeof(float)));
-        ctx->d_ev_cap = n_state + n_events;
-    }
-    if (n_state + n_events > ctx->h_ev_cap) {
-        if (ctx->h_ev) cudaFreeHost(ctx->h_ev);
-        ctx->h_ev = nullptr;
-        ctx->h_ev_cap = 0;
-        CUDA_TRY(ctx, cudaHostAlloc(&ctx->h_ev, (n_state + n_events) * sizeof(float), cudaHostAllocDefault));
-        ctx->h_ev_cap = n_state + n_events;
-    }
-    float* d_theta = ctx->d_ev;
-    float* d_y = d_theta + n_theta;
-    float* d_stats = n_stats ? d_y + n_y : nullptr;
-    float* d_aux = n_aux ? d_y + n_y + n_stats : nullptr;
-    float* d_events = ctx->d_ev + n_state;
-    float* h_state = ctx->h_ev;                 // final theta | y | stats of the event chains
-    float* h_events = ctx->h_ev + n_state;
+    const size_t n_state = state_floats(ctx, run, Ce), n_events = size_t(Ce) * size_t(cap) * (1 + d);
+    CUDA_TRY(ctx, ctx->d_ev.reserve(n_state + n_events));
+    CUDA_TRY(ctx, ctx->h_ev.reserve(n_state + n_events));
+    const ChainState state = carve_state(ctx, run, Ce, ctx->d_ev.p, nullptr);   // the event chains' state, then their events
+    float* d_events = ctx->d_ev.p + n_state;
+    float* h_state = ctx->h_ev.p;                 // final state of the event chains, committed once no chain overflowed
+    float* h_events = ctx->h_ev.p + n_state;
     cudaStream_t se = ctx->s_ev;
-    CUDA_TRY(ctx, cudaMemcpyAsync(d_theta, run->theta + Cd * d, n_theta * sizeof(float), cudaMemcpyHostToDevice, se));
-    CUDA_TRY(ctx, cudaMemcpyAsync(d_y, run->y + Cd * yd, n_y * sizeof(float), cudaMemcpyHostToDevice, se));
-    if (d_stats) CUDA_TRY(ctx, cudaMemcpyAsync(d_stats, run->stats + Cd * ns, n_stats * sizeof(float), cudaMemcpyHostToDevice, se));
-    if (d_aux) CUDA_TRY(ctx, cudaMemcpyAsync(d_aux, run->aux + Cd * GLABC_AUX_SLOTS, n_aux * sizeof(float), cudaMemcpyHostToDevice, se));
+    CUDA_TRY(ctx, stage_state(ctx, run, Cd, Ce, state, cudaMemcpyHostToDevice, se));
     // the event chains in up to 8 groups: the kernel of group g + 1 and the copy of group g's events overlap the expansion of
     // group g - 1 on the host cores
     // (a group's kernel is latency-bound — a chain's steps are sequential — so it takes about as long as a full launch's warp:
@@ -1596,27 +1607,18 @@ static int run_global_host_hybrid(glabc_ctx* ctx, SamplerKind kind, const glabc_
             n_groups = g;
             break;
         }
-        glabc_run_t dev = *run;
-        dev.n_chains = gn;
-        dev.chain_id_base = run->chain_id_base + Cd + g0;
-        dev.theta = d_theta + g0 * d;
-        dev.y = d_y + g0 * yd;
-        dev.stats = d_stats ? d_stats + g0 * ns : nullptr;
-        dev.aux = d_aux ? d_aux + g0 * GLABC_AUX_SLOTS : nullptr;
+        glabc_run_t dev = chain_slice(run, Cd + g0, gn, chains_at(ctx, state, g0), se);
         dev.trace = d_events + g0 * cap * (1 + d);
         dev.trace_layout = GLABC_TRACE_EVENTS;
         dev.trace_rows = cap;
         dev.trace_chains = gn;
         dev.trace_chain_off = 0;
         dev.trace_row_base = 0;
-        dev.stream = se;
-        dev.tape_dump = nullptr;
-        dev.debug = nullptr;
         st = run_device(ctx, kind, &dev);
         if (st) return st;
         CUDA_TRY(ctx, cudaMemcpyAsync(h_events + g0 * cap * (1 + d), d_events + g0 * cap * (1 + d), size_t(gn) * cap * (1 + d) * sizeof(float),
                                       cudaMemcpyDeviceToHost, se));
-        if (g == n_groups - 1) CUDA_TRY(ctx, cudaMemcpyAsync(h_state, ctx->d_ev, n_state * sizeof(float), cudaMemcpyDeviceToHost, se));
+        if (g == n_groups - 1) CUDA_TRY(ctx, cudaMemcpyAsync(h_state, ctx->d_ev.p, n_state * sizeof(float), cudaMemcpyDeviceToHost, se));
         CUDA_TRY(ctx, cudaEventRecord(ctx->ev_group[g], se));
     }
 
@@ -1628,14 +1630,13 @@ static int run_global_host_hybrid(glabc_ctx* ctx, SamplerKind kind, const glabc_
         const int r = atoi(lws);
         if (r > 1) n_threads = (n_threads + r - 1) / r;
     }
-    if (const char* t = getenv("GLABC_HOST_THREADS")) n_threads = atoi(t);
     if (n_threads < 1) n_threads = 1;
     if (n_threads > 64) n_threads = 64;
     const int device = ctx->device;
     cudaEvent_t evg[8];
     for (int g = 0; g < 8; ++g) evg[g] = ctx->ev_group[g];
-    float* host_trace = run->trace;
-    const int64_t trace_rows = run->trace_rows, chain_off = run->trace_chain_off + Cd, row_base = run->trace_row_base;
+    const int64_t trace_rows = run->trace_rows, row_base = run->trace_row_base;
+    float* ev_trace = run->trace + (run->trace_chain_off + Cd) * trace_rows * d;   // row 0 of the first event chain
     const bool timing = getenv("GLABC_HOST_TIMING") != nullptr;
     const auto t_start = std::chrono::steady_clock::now();
     auto ms_since = [t_start]() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_start).count(); };
@@ -1657,15 +1658,7 @@ static int run_global_host_hybrid(glabc_ctx* ctx, SamplerKind kind, const glabc_
                     return;
                 }
             }
-            std::vector<std::thread> workers;
-            for (int t = 0; t < n_threads; ++t)
-                workers.emplace_back([=]() {
-                    for (int64_t j = g0 + t; j < g1; j += n_threads)
-                        expand_chain(h_events + j * cap * (1 + d), cap, d, row_base, row_end, host_trace + (chain_off + j) * trace_rows * d,
-                                     nt512);
-                    _mm_sfence();   // the non-temporal stores are globally visible before the thread is joined
-                });
-            for (auto& w : workers) w.join();
+            expand_parallel(h_events, g0, g1, cap, d, row_base, row_end, ev_trace, trace_rows, n_threads, nt512);
         }
         if (timing) fprintf(stderr, "[glabc host] first events at %.1f ms, all expanded at %.1f ms (%lld chains, %d groups, %d threads, nt512 %d)\n",
                             t_first, ms_since(), static_cast<long long>(Ce), n_groups, n_threads, static_cast<int>(nt512));
@@ -1678,72 +1671,60 @@ static int run_global_host_hybrid(glabc_ctx* ctx, SamplerKind kind, const glabc_
     if (st) return st;
     if (overflow.load() == 2) return fail(ctx, GLABC_ERR_CUDA, "event transport: waiting for the event copy failed");
     if (overflow.load() == 1) {   // redo the event chains densely from their (untouched) initial host state
-        glabc_run_t redo = *run;
-        redo.n_chains = Ce;
-        redo.chain_id_base = run->chain_id_base + Cd;
-        redo.theta = run->theta + Cd * d;
-        redo.y = run->y + Cd * yd;
-        redo.stats = run->stats ? run->stats + Cd * ns : nullptr;
-        redo.aux = run->aux ? run->aux + Cd * GLABC_AUX_SLOTS : nullptr;
+        glabc_run_t redo = chain_slice(run, Cd, Ce, chains_at(ctx, host_state(run), Cd), nullptr);
         redo.trace_chain_off = run->trace_chain_off + Cd;
-        return run_host(ctx, kind, &redo, chunk_steps);
+        return run_host_dense(ctx, kind, &redo, chunk_steps);
     }
-    memcpy(run->theta + Cd * d, h_state, n_theta * sizeof(float));
-    memcpy(run->y + Cd * yd, h_state + n_theta, n_y * sizeof(float));
-    if (n_stats) memcpy(run->stats + Cd * ns, h_state + n_theta + n_y, n_stats * sizeof(float));
-    if (n_aux) memcpy(run->aux + Cd * GLABC_AUX_SLOTS, h_state + n_theta + n_y + n_stats, n_aux * sizeof(float));
+    const ChainState staged = carve_state(ctx, run, Ce, h_state, nullptr);
+    memcpy(run->theta + Cd * d, staged.theta, size_t(Ce) * d * sizeof(float));
+    memcpy(run->y + Cd * yd, staged.y, size_t(Ce) * yd * sizeof(float));
+    if (staged.aux) memcpy(run->aux + Cd * GLABC_AUX_SLOTS, staged.aux, size_t(Ce) * GLABC_AUX_SLOTS * sizeof(float));
+    if (staged.stats) memcpy(run->stats + Cd * ns, staged.stats, size_t(Ce) * ns * sizeof(float));
     return GLABC_OK;
+}
+
+// The host-buffer entry points: the argument check, then for GlobalMCMC / GLMCMC the event transport where it applies and
+// the dense transport otherwise; GLMALA and AGLMCMC travel in time chunks.
+static int run_host_entry(glabc_ctx* ctx, SamplerKind kind, const glabc_run_t* run, int64_t chunk_steps, const glabc_aglmcmc_t* ag = nullptr)
+{
+    int st = check_host_run(ctx, run);
+    if (st || run->n_chains == 0) return st;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    if (kind == SAMPLER_MALA || kind == SAMPLER_AGLMCMC) return run_host(ctx, kind, run, chunk_steps, ag);
+    bool handled = false;
+    st = run_global_host_hybrid(ctx, kind, run, chunk_steps, &handled);
+    if (handled || st) return st;
+    return run_host_dense(ctx, kind, run, chunk_steps);
 }
 
 extern "C" {
 
 int glabc_run_global(glabc_ctx* ctx, const glabc_run_t* run) { return run_device(ctx, SAMPLER_GLOBAL, run); }
 
-// host entry of a sampler whose trace can travel as events (GlobalMCMC, GLMCMC)
-static int run_host_chain_major(glabc_ctx* ctx, SamplerKind kind, const glabc_run_t* run, int64_t chunk_steps)
-{
-    if (!ctx) return GLABC_ERR_INVALID;
-    bool handled = false;
-    const int st = run_global_host_hybrid(ctx, kind, run, chunk_steps, &handled);
-    if (handled || st) return st;
-    if (ctx->has_model && run && run->trace_layout == GLABC_TRACE_CHAIN_MAJOR && run->trace && run->theta && run->y && run->n_chains > 0 &&
-        run->n_steps > 0 && run->rng_mode == GLABC_RNG_NATIVE && chunk_steps == 0 && (kind == SAMPLER_GLOBAL || run->aux)) {
-        // chain-major host trace without the event transport: whole chains, group by group (contiguous copies)
-        const int64_t row_lo = run->step_base + (run->write_row0 ? 0 : 1), row_end = run->step_base + run->n_steps;
-        if (row_lo - run->trace_row_base < 0 || row_end - run->trace_row_base >= run->trace_rows)
-            return fail(ctx, GLABC_ERR_INVALID, "trace rows fall outside the host buffer");
-        if (run->trace_chain_off < 0 || run->trace_chain_off + run->n_chains > run->trace_chains)
-            return fail(ctx, GLABC_ERR_INVALID, "chains fall outside the host trace buffer");
-        CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-        return dense_chain_groups(ctx, kind, run, run->n_chains);
-    }
-    return run_host(ctx, kind, run, chunk_steps);
-}
-
 int glabc_run_global_host(glabc_ctx* ctx, const glabc_run_t* run, int64_t chunk_steps)
 {
-    return run_host_chain_major(ctx, SAMPLER_GLOBAL, run, chunk_steps);
+    return run_host_entry(ctx, SAMPLER_GLOBAL, run, chunk_steps);
 }
 
 int glabc_run_isir(glabc_ctx* ctx, const glabc_run_t* run) { return run_device(ctx, SAMPLER_ISIR, run); }
 
 int glabc_run_isir_host(glabc_ctx* ctx, const glabc_run_t* run, int64_t chunk_steps)
 {
-    return run_host_chain_major(ctx, SAMPLER_ISIR, run, chunk_steps);
+    return run_host_entry(ctx, SAMPLER_ISIR, run, chunk_steps);
 }
 
 int glabc_run_mala(glabc_ctx* ctx, const glabc_run_t* run) { return run_device(ctx, SAMPLER_MALA, run); }
 
 int glabc_run_mala_host(glabc_ctx* ctx, const glabc_run_t* run, int64_t chunk_steps)
 {
-    return run_host(ctx, SAMPLER_MALA, run, chunk_steps);
+    return run_host_entry(ctx, SAMPLER_MALA, run, chunk_steps);
 }
 
 int glabc_run_aglmcmc_host(glabc_ctx* ctx, const glabc_run_t* run, const glabc_aglmcmc_t* ag, int64_t chunk_steps)
 {
     if (!ctx) return GLABC_ERR_INVALID;
     if (!ag) return fail(ctx, GLABC_ERR_INVALID, "null aglmcmc description");
-    return run_host(ctx, SAMPLER_AGLMCMC, run, chunk_steps, ag);
+    return run_host_entry(ctx, SAMPLER_AGLMCMC, run, chunk_steps, ag);
 }
 
 int glabc_resample(glabc_ctx* ctx, const float* W, int64_t n, int64_t N, float u0, int64_t* idx, uint64_t* count, void* stream)
@@ -1751,15 +1732,8 @@ int glabc_resample(glabc_ctx* ctx, const float* W, int64_t n, int64_t N, float u
     if (!ctx) return GLABC_ERR_INVALID;
     if (n < 0 || N < 0 || (n > 0 && !W) || (N > 0 && !idx) || !count) return fail(ctx, GLABC_ERR_INVALID, "glabc_resample: bad sizes / null pointer");
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    const size_t need = static_cast<size_t>((n + 4095) / 4096) + 1;
-    if (need > ctx->rs_cap) {
-        if (ctx->rs_scratch) cudaFree(ctx->rs_scratch);
-        ctx->rs_scratch = nullptr;
-        ctx->rs_cap = 0;
-        CUDA_TRY(ctx, cudaMalloc(&ctx->rs_scratch, need * sizeof(double)));
-        ctx->rs_cap = need;
-    }
-    CUDA_TRY(ctx, launch_resample(W, n, N, u0, idx, reinterpret_cast<unsigned long long*>(count), ctx->rs_scratch,
+    CUDA_TRY(ctx, ctx->rs_scratch.reserve(static_cast<size_t>((n + 4095) / 4096) + 1));
+    CUDA_TRY(ctx, launch_resample(W, n, N, u0, idx, reinterpret_cast<unsigned long long*>(count), ctx->rs_scratch.p,
                                   static_cast<cudaStream_t>(stream)));
     return GLABC_OK;
 }
@@ -1802,13 +1776,7 @@ int glabc_expand_events(const float* events, int64_t chains, int64_t cap, int32_
     if (nt < 1) nt = 1;
     if (nt > 64) nt = 64;
     if (nt > chains) nt = chains > 0 ? static_cast<int>(chains) : 1;
-    std::vector<std::thread> workers;
-    for (int t = 0; t < nt; ++t)
-        workers.emplace_back([=]() {
-            for (int64_t c = t; c < chains; c += nt) expand_chain(events + c * cap * (1 + dim), cap, dim, row_base, row_end, trace + c * trace_rows * dim, nt512);
-            _mm_sfence();
-        });
-    for (auto& w : workers) w.join();
+    expand_parallel(events, 0, chains, cap, dim, row_base, row_end, trace, trace_rows, nt, nt512);
     return GLABC_OK;
 }
 
