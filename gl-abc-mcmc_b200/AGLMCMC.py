@@ -41,8 +41,9 @@ class PooledKDEProposal:
         d = pod.theta_dim
         self.y_obs = torch.tensor(list(pod.y_obs)[:pod.y_dim], device=eng.device)
         # the prior as a device distribution: its log-density of the candidates is the kernel behind glabc_dist_log_prob
-        eng.bind_proposal(_abi.SLOT_GLOBAL, DiagGaussian(d, torch.tensor(list(pod.prior_loc)[:d]),
-                                                         torch.tensor(list(pod.prior_log_scale)[:d])))
+        prior = eng.prior_pod if eng.prior_pod is not None else DiagGaussian(d, torch.tensor(list(pod.prior_loc)[:d]),
+                                                                              torch.tensor(list(pod.prior_log_scale)[:d]))
+        eng.bind_proposal(_abi.SLOT_GLOBAL, prior)
         self.floor = math.log(1e-10)
 
     def state_dict(self):

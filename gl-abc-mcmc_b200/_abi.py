@@ -140,6 +140,7 @@ _SIGNATURES = {
     "glabc_device_info": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "glabc_model_set": (C.c_int, [C.c_void_p, C.POINTER(ModelPOD), C.c_size_t]),
     "glabc_dist_set": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(DistPOD), C.c_size_t]),
+    "glabc_model_prior_set": (C.c_int, [C.c_void_p, C.POINTER(DistPOD), C.c_size_t]),
     "glabc_dist_log_prob": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
     "glabc_dist_sample": (C.c_int, [C.c_void_p, C.c_int, C.c_int64, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p]),
     "glabc_run_global": (C.c_int, [C.c_void_p, C.POINTER(RunPOD)]),

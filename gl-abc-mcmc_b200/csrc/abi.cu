@@ -57,9 +57,12 @@ struct glabc_ctx {
     int sm_count = 0, clock_khz = 0, cc = 0;
     std::string err;
     glabc_model_t model{};
+    glabc_model_t model_pod{};   // as glabc_model_set bound it: a DiagGaussian prior set later changes `model` only
     bool has_model = false;
     glabc_dist_t dist[GLABC_SLOT_COUNT]{};
     bool has_dist[GLABC_SLOT_COUNT] = {false, false, false};
+    glabc_dist_t prior{};     // a Uniform / Gamma / GaussianMixture prior of the model (glabc_model_prior_set)
+    bool has_prior = false;   // false: the DiagGaussian of `model` is the prior
     // scratch of the host-buffer entry points
     Scratch<float> d_state;       // theta | y | aux | stats
     Scratch<double> d_state64;    // GLMALA carried float64 state
@@ -205,19 +208,20 @@ int glabc_model_set(glabc_ctx* ctx, const glabc_model_t* model, size_t nbytes)
     if (!(model->eps_scale > 0.0f)) return fail(ctx, GLABC_ERR_INVALID, "epsilon must be positive");
     for (int i = 0; i < model->theta_dim; ++i)
         if (!(model->prior_scale[i] > 0.0f)) return fail(ctx, GLABC_ERR_INVALID, "prior scale must be positive");
-    ctx->model = *model;
+    ctx->model = ctx->model_pod = *model;
     ctx->has_model = true;
+    ctx->has_prior = false;
     return GLABC_OK;
 }
 
-int glabc_dist_set(glabc_ctx* ctx, int slot, const glabc_dist_t* dist, size_t nbytes)
+}  // extern "C"
+
+// the checks of a glabc_dist_t shared by glabc_dist_set and glabc_model_prior_set
+static int check_dist(glabc_ctx* ctx, const char* who, const glabc_dist_t* dist, size_t nbytes)
 {
-    if (!ctx) return GLABC_ERR_INVALID;
-    if (slot < 0 || slot >= GLABC_SLOT_COUNT) return fail(ctx, GLABC_ERR_INVALID, "bad proposal slot %d", slot);
     if (!dist || nbytes != sizeof(glabc_dist_t))
-        return fail(ctx, GLABC_ERR_INVALID, "glabc_dist_set: struct size %zu, expected %zu (ABI mismatch)", nbytes,
-                    sizeof(glabc_dist_t));
-    if (dist->dim < 1 || dist->dim > 4) return fail(ctx, GLABC_ERR_UNSUPPORTED, "proposal dim %d outside 1..4", dist->dim);
+        return fail(ctx, GLABC_ERR_INVALID, "%s: struct size %zu, expected %zu (ABI mismatch)", who, nbytes, sizeof(glabc_dist_t));
+    if (dist->dim < 1 || dist->dim > 4) return fail(ctx, GLABC_ERR_UNSUPPORTED, "%s: dim %d outside 1..4", who, dist->dim);
     switch (dist->kind) {
     case GLABC_DIST_DIAG_GAUSSIAN:
         for (int i = 0; i < dist->dim; ++i)
@@ -240,8 +244,47 @@ int glabc_dist_set(glabc_ctx* ctx, int slot, const glabc_dist_t* dist, size_t nb
     default:
         return fail(ctx, GLABC_ERR_UNSUPPORTED, "unknown distribution kind %d", dist->kind);
     }
+    return GLABC_OK;
+}
+
+extern "C" {
+
+int glabc_dist_set(glabc_ctx* ctx, int slot, const glabc_dist_t* dist, size_t nbytes)
+{
+    if (!ctx) return GLABC_ERR_INVALID;
+    if (slot < 0 || slot >= GLABC_SLOT_COUNT) return fail(ctx, GLABC_ERR_INVALID, "bad proposal slot %d", slot);
+    const int st = check_dist(ctx, "glabc_dist_set", dist, nbytes);
+    if (st) return st;
     ctx->dist[slot] = *dist;
     ctx->has_dist[slot] = true;
+    return GLABC_OK;
+}
+
+int glabc_model_prior_set(glabc_ctx* ctx, const glabc_dist_t* prior, size_t nbytes)
+{
+    if (!ctx) return GLABC_ERR_INVALID;
+    if (!ctx->has_model) return fail(ctx, GLABC_ERR_INVALID, "glabc_model_prior_set: no model bound: call glabc_model_set first");
+    glabc_model_t& m = ctx->model;
+    if (!prior) {   // back to the DiagGaussian of the glabc_model_set POD
+        m = ctx->model_pod;
+        ctx->has_prior = false;
+        return GLABC_OK;
+    }
+    if (nbytes == sizeof(glabc_dist_t) && prior->dim != m.theta_dim)
+        return fail(ctx, GLABC_ERR_INVALID, "glabc_model_prior_set: prior dim %d does not match theta_dim %d", prior->dim, m.theta_dim);
+    const int st = check_dist(ctx, "glabc_model_prior_set", prior, nbytes);
+    if (st) return st;
+    if (prior->kind == GLABC_DIST_DIAG_GAUSSIAN) {   // the tuned kernels take it from the model POD, as if given there
+        for (int i = 0; i < m.theta_dim; ++i) {
+            m.prior_loc[i] = prior->a[i];
+            m.prior_log_scale[i] = prior->b[i];
+            m.prior_scale[i] = prior->c[i];
+        }
+        ctx->has_prior = false;
+        return GLABC_OK;
+    }
+    ctx->prior = *prior;
+    ctx->has_prior = true;
     return GLABC_OK;
 }
 
@@ -325,6 +368,25 @@ static ModelConsts make_model(const glabc_model_t& m)
     k.kern_fast_m = static_cast<float>(-0.5 / (static_cast<double>(m.eps_scale) * m.eps_scale));
     k.prior = make_gauss(m.prior_loc, m.prior_log_scale, m.prior_scale, m.theta_dim);
     return k;
+}
+
+// the `prior` argument of the launchers: the bound Uniform / Gamma / GaussianMixture, or kind DiagGaussian for the model's own
+static DistConsts make_prior(const glabc_ctx* ctx)
+{
+    if (ctx->has_prior) return make_dist(ctx->prior);
+    DistConsts q{};
+    q.kind = GLABC_DIST_DIAG_GAUSSIAN;
+    return q;
+}
+
+// A Uniform / Gamma / GaussianMixture prior runs FAST arithmetic with the native RNG and records nothing: the STRICT / replay
+// kernels and the tapes and dumps are fused for the model's DiagGaussian prior.  Checked before anything is launched.
+static int check_prior_run(glabc_ctx* ctx, const char* who, const glabc_run_t* run, bool dumps)
+{
+    if (ctx->has_prior && (run->arith_mode == GLABC_ARITH_STRICT || run->rng_mode == GLABC_RNG_REPLAY || run->tape_dump || dumps))
+        return fail(ctx, GLABC_ERR_UNSUPPORTED, "%s with a Uniform / Gamma / GaussianMixture prior runs FAST arithmetic with the native RNG "
+                                                "and writes no tape or parity dump", who);
+    return GLABC_OK;
 }
 
 // native branch coin: U_b = k * 2^-16 (k < 2^16);  U_b < gf  <=>  k < ceil(gf * 2^16)  (cf. SURVEY.md B-15)
@@ -439,9 +501,9 @@ static int run_device(glabc_ctx* ctx, SamplerKind kind, const glabc_run_t* run)
         const glabc_dist_t& lp = ctx->dist[GLABC_SLOT_LOCAL];
         const glabc_dist_t& gp = ctx->dist[GLABC_SLOT_GLOBAL];
         if (lp.dim != d || gp.dim != d) return fail(ctx, GLABC_ERR_INVALID, "proposal dim does not match theta_dim %d", d);
-        const bool tuned = all_gaussian(ctx, {GLABC_SLOT_LOCAL, GLABC_SLOT_GLOBAL});
+        const bool tuned = all_gaussian(ctx, {GLABC_SLOT_LOCAL, GLABC_SLOT_GLOBAL}) && !ctx->has_prior;
         int st = make_run_params(ctx, run, d, GLABC_TAPE_GLOBAL_SLOTS(d, d), &R, &block, tuned);
-        if (st) return st;
+        if (st || (st = check_prior_run(ctx, "run_global", run, false))) return st;
         if (R.n_chains == 0) return GLABC_OK;
         if (!tuned) {
             // Uniform / Gamma / GaussianMixture proposals: the general kernel (float32; replay takes the proposal draws
@@ -453,7 +515,7 @@ static int run_device(glabc_ctx* ctx, SamplerKind kind, const glabc_run_t* run)
             G.model = make_model(ctx->model);
             G.lp = make_dist(lp);
             G.gp = make_dist(gp);
-            CUDA_TRY(ctx, launch_global_generic(G, d, R, run->trace_layout, block, run->rng_mode == GLABC_RNG_REPLAY,
+            CUDA_TRY(ctx, launch_global_generic(G, make_prior(ctx), d, R, run->trace_layout, block, run->rng_mode == GLABC_RNG_REPLAY,
                                                 static_cast<cudaStream_t>(run->stream)));
             return GLABC_OK;
         }
@@ -468,13 +530,13 @@ static int run_device(glabc_ctx* ctx, SamplerKind kind, const glabc_run_t* run)
         const glabc_dist_t& lp = ctx->dist[GLABC_SLOT_LOCAL];
         const glabc_dist_t& ip = ctx->dist[GLABC_SLOT_IMPORTANCE];
         if (lp.dim != d || ip.dim != d) return fail(ctx, GLABC_ERR_INVALID, "proposal dim does not match theta_dim %d", d);
-        const bool tuned = all_gaussian(ctx, {GLABC_SLOT_LOCAL, GLABC_SLOT_IMPORTANCE});
+        const bool tuned = all_gaussian(ctx, {GLABC_SLOT_LOCAL, GLABC_SLOT_IMPORTANCE}) && !ctx->has_prior;
         if (!run) return fail(ctx, GLABC_ERR_INVALID, "null run description");
         if (run->n_candidates < 1 || run->n_candidates > GLABC_MAX_K)
             return fail(ctx, GLABC_ERR_INVALID, "n_candidates (batch_size) must be in 1..%d", GLABC_MAX_K);
         if (!run->aux) return fail(ctx, GLABC_ERR_INVALID, "run_isir needs the aux state [C][%d] (log-weight, local flag)", GLABC_AUX_SLOTS);
         int st = make_run_params(ctx, run, d, GLABC_TAPE_ISIR_SLOTS(d, d, run->n_candidates), &R, &block, tuned);
-        if (st) return st;
+        if (st || (st = check_prior_run(ctx, "run_isir", run, false))) return st;
         if (!tuned) {
             // Uniform / Gamma / GaussianMixture in the Local / Importance slots: the general kernel (replay takes the
             // proposal draws themselves: tape64 [steps][1 + K d][C] = resampling uniform, then the draws)
@@ -487,7 +549,7 @@ static int run_device(glabc_ctx* ctx, SamplerKind kind, const glabc_run_t* run)
             G.model = make_model(ctx->model);
             G.lp = make_dist(lp);
             G.ip = make_dist(ip);
-            CUDA_TRY(ctx, launch_isir_generic(G, d, R, run->trace_layout, block, run->rng_mode == GLABC_RNG_REPLAY,
+            CUDA_TRY(ctx, launch_isir_generic(G, make_prior(ctx), d, R, run->trace_layout, block, run->rng_mode == GLABC_RNG_REPLAY,
                                               static_cast<cudaStream_t>(run->stream)));
             return GLABC_OK;
         }
@@ -517,7 +579,7 @@ static int run_device(glabc_ctx* ctx, SamplerKind kind, const glabc_run_t* run)
         if (!run->aux || !run->state64)
             return fail(ctx, GLABC_ERR_INVALID, "run_mala needs aux [C][%d] and state64 [C][%d]", GLABC_AUX_SLOTS, GLABC_STATE64_SLOTS);
         int st = make_run_params(ctx, run, d, GLABC_TAPE_MALA_SLOTS(d, d, run->n_candidates, run->num_grad), &R, &block);
-        if (st) return st;
+        if (st || (st = check_prior_run(ctx, "run_mala", run, false))) return st;
         if (run->rng_mode == GLABC_RNG_REPLAY && (!run->tape64 || !run->tape_grad0))
             return fail(ctx, GLABC_ERR_INVALID, "replay of run_mala needs tape64 and tape_grad0");
         if (run->tape_dump && !run->tape_grad0_dump)
@@ -539,7 +601,7 @@ static int run_device(glabc_ctx* ctx, SamplerKind kind, const glabc_run_t* run)
         K.tau = run->tau64 != 0.0 ? run->tau64 : static_cast<double>(run->tau);
         K.tau_f = run->tau;
         K.num_grad = run->num_grad;
-        CUDA_TRY(ctx, launch_mala(K, d, R, run->arith_mode == GLABC_ARITH_STRICT, run->rng_mode == GLABC_RNG_REPLAY, block,
+        CUDA_TRY(ctx, launch_mala(K, make_prior(ctx), d, R, run->arith_mode == GLABC_ARITH_STRICT, run->rng_mode == GLABC_RNG_REPLAY, block,
                                   static_cast<cudaStream_t>(run->stream)));
         return GLABC_OK;
     }
@@ -558,6 +620,7 @@ static int check_host_run(glabc_ctx* ctx, const glabc_run_t* run)
     if (!ctx->has_model) return fail(ctx, GLABC_ERR_INVALID, "no model bound: call glabc_model_set first");
     if (!run) return fail(ctx, GLABC_ERR_INVALID, "null run description");
     if (run->rng_mode != GLABC_RNG_NATIVE) return fail(ctx, GLABC_ERR_INVALID, "host entry points run the native RNG only");
+    if (int st = check_prior_run(ctx, "a host entry point", run, false)) return st;
     // GLABC_TRACE_EVENTS is a device-buffer layout (glabc.h): the scratch is sized for dense rows, an event writer would run
     // past it.  The event TRANSPORT of the host entries is chosen internally (run_global_host_hybrid), never by the caller.
     if (run->trace_layout != GLABC_TRACE_NONE && run->trace_layout != GLABC_TRACE_TIME_MAJOR &&
@@ -830,7 +893,7 @@ extern "C" int glabc_run_aglmcmc(glabc_ctx* ctx, const glabc_run_t* run, const g
     RunParams R;
     int block = 0;
     int st = make_run_params(ctx, run, d, GLABC_TAPE_GLOBAL_SLOTS(d, d), &R, &block);
-    if (st) return st;
+    if (st || (st = check_prior_run(ctx, "run_aglmcmc", run, ag->ad_rec || ag->ad_blk || ag->init_w))) return st;
     if (run->block_threads == 0) block = 128;
     if (block > 128) return fail(ctx, GLABC_ERR_INVALID, "run_aglmcmc: block_threads at most 128");
     const bool replay = run->rng_mode == GLABC_RNG_REPLAY;
@@ -856,7 +919,7 @@ extern "C" int glabc_run_aglmcmc(glabc_ctx* ctx, const glabc_run_t* run, const g
     K.log_prior_floor = static_cast<float>(std::log(1e-10));
     AgTapes T{ag->init_p, ag->init_s, ag->ad_noise, ag->ad_sim, ag->ad_idx, ag->ad_rec, ag->ad_blk, ag->init_w, ag->tape_rounds,
               ag->dump_rounds};
-    CUDA_TRY(ctx, launch_aglmcmc(K, ctx->ag, T, R, d, ag->init, ag->kde_rule, run->arith_mode == GLABC_ARITH_STRICT, replay,
+    CUDA_TRY(ctx, launch_aglmcmc(K, make_prior(ctx), ctx->ag, T, R, d, ag->init, ag->kde_rule, run->arith_mode == GLABC_ARITH_STRICT, replay,
                                  run->trace_layout, block, static_cast<cudaStream_t>(run->stream)));
     return GLABC_OK;
 }
@@ -1197,6 +1260,7 @@ static int block_isir_setup(glabc_ctx* ctx, const char* who, const glabc_run_t* 
     int st = make_run_params(ctx, run, d, GLABC_TAPE_GLOBAL_SLOTS(d, d), R, block);
     if (st) return st;
     if (run->rng_mode != GLABC_RNG_NATIVE) return fail(ctx, GLABC_ERR_UNSUPPORTED, "%s runs the native RNG only", who);
+    if ((st = check_prior_run(ctx, who, run, false))) return st;
     if (run->block_threads == 0) *block = 128;
     if (*block > 128) return fail(ctx, GLABC_ERR_INVALID, "%s: block_threads at most 128", who);
     *K = AgConsts{};
@@ -1226,7 +1290,7 @@ extern "C" int glabc_run_block_isir(glabc_ctx* ctx, const glabc_run_t* run, cons
     int st = block_isir_setup(ctx, "glabc_run_block_isir", run, b, true, &K, &W, &R, &block);
     if (st) return st;
     if (R.n_chains == 0) return GLABC_OK;
-    CUDA_TRY(ctx, launch_block_isir(K, W, R, ctx->model.theta_dim, run->arith_mode == GLABC_ARITH_STRICT, run->trace_layout, block,
+    CUDA_TRY(ctx, launch_block_isir(K, make_prior(ctx), W, R, ctx->model.theta_dim, run->arith_mode == GLABC_ARITH_STRICT, run->trace_layout, block,
                                     static_cast<cudaStream_t>(run->stream)));
     return GLABC_OK;
 }
@@ -1240,7 +1304,7 @@ extern "C" int glabc_block_weights(glabc_ctx* ctx, const glabc_run_t* run, const
     int st = block_isir_setup(ctx, "glabc_block_weights", run, b, false, &K, &W, &R, &block);
     if (st) return st;
     if (R.n_chains == 0) return GLABC_OK;
-    CUDA_TRY(ctx, launch_block_weights(K, W, R, ctx->model.theta_dim, round, static_cast<cudaStream_t>(run->stream)));
+    CUDA_TRY(ctx, launch_block_weights(K, make_prior(ctx), W, R, ctx->model.theta_dim, round, static_cast<cudaStream_t>(run->stream)));
     return GLABC_OK;
 }
 
@@ -1559,7 +1623,9 @@ static int run_global_host_hybrid(glabc_ctx* ctx, SamplerKind kind, const glabc_
     if (off && off[0] == '0') return GLABC_OK;
     if (run->trace_layout != GLABC_TRACE_CHAIN_MAJOR || run->n_steps < 512 || run->n_chains < 256) return GLABC_OK;
     const int far_slot = kind == SAMPLER_ISIR ? GLABC_SLOT_IMPORTANCE : GLABC_SLOT_GLOBAL;
-    if (!ctx->has_dist[GLABC_SLOT_LOCAL] || !ctx->has_dist[far_slot] || !all_gaussian(ctx, {GLABC_SLOT_LOCAL, far_slot})) return GLABC_OK;
+    // the event writer lives in the tuned kernels only: Gaussian proposals and the model's DiagGaussian prior
+    if (!ctx->has_dist[GLABC_SLOT_LOCAL] || !ctx->has_dist[far_slot] || !all_gaussian(ctx, {GLABC_SLOT_LOCAL, far_slot}) || ctx->has_prior)
+        return GLABC_OK;
     if (kind == SAMPLER_ISIR && !run->aux) return GLABC_OK;
     const int d = ctx->model.theta_dim, yd = ctx->model.y_dim, ns = GLABC_NSTATS(d);
     const bool nt512 = (d == 1 || d == 2 || d == 4) && __builtin_cpu_supports("avx512f");

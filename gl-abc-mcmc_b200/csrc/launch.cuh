@@ -13,7 +13,10 @@ cudaError_t launch_isir(const ModelConsts& model, const GaussConsts& lp, const G
                         bool strict, bool replay, int layout, int block, cudaStream_t st);
 
 struct MalaConsts;
-cudaError_t launch_mala(const MalaConsts& K, int dim, const RunParams& R, bool strict, bool replay, int block, cudaStream_t st);
+struct DistConsts;
+// `prior`: a Uniform / Gamma / GaussianMixture prior of the model (FAST, native RNG) or GLABC_DIST_DIAG_GAUSSIAN for K.model's
+cudaError_t launch_mala(const MalaConsts& K, const DistConsts& prior, int dim, const RunParams& R, bool strict, bool replay, int block,
+                        cudaStream_t st);
 
 cudaError_t launch_esjd(const float* trace, int layout, int64_t rows, int64_t chains, int dim, float* out,
                         cudaStream_t st);

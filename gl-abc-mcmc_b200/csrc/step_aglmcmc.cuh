@@ -76,7 +76,7 @@ __device__ __forceinline__ float model_discrepancy(const ModelConsts& m, const f
 // ---------------------------------------------------------------------------------------------
 template <int D, int FAMILY, bool INIT, bool REPLAY>
 __global__ void __launch_bounds__(256) k_ag_block(const __grid_constant__ AgConsts K, const __grid_constant__ RunParams R,
-                                                  AgWorkspace W, AgTapes T)
+                                                  AgWorkspace W, AgTapes T, const __grid_constant__ DistConsts prior)
 {
     const int64_t g = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
     if (g >= W.C * W.B) return;
@@ -144,7 +144,7 @@ __global__ void __launch_bounds__(256) k_ag_block(const __grid_constant__ AgCons
     model_simulate<D, true>(K.model, th, eps_s, x);
     const float dis = model_discrepancy<D>(K.model, x);
     const float like = log_kernel_dis_eps(K.model.c_kern, dis, K.model.eps_log_scale, K.model.eps_scale);
-    float w = expf(__fsub_rn(__fadd_rn(model_prior<D, true>(K.model, th), like), lq));
+    float w = expf(__fsub_rn(__fadd_rn(prior_log_prob_rt<D>(K.model, prior, th), like), lq));
     if (INIT && w != w) w = 0.0f;  // AGLMCMC.py:110-112; the regenerated blocks keep NaN weights (:248-249)
 #pragma unroll
     for (int k = 0; k < D; ++k) W.blk_x[(c * W.B + b) * D + k] = x[k];
@@ -199,7 +199,7 @@ __global__ void __launch_bounds__(256) k_ag_commit(AgWorkspace W, AgTapes T)
 // adaptation, AGLMCMC.py:174-211: one CTA per pausing chain
 // ---------------------------------------------------------------------------------------------
 template <int D>
-__global__ void __launch_bounds__(256) k_ag_adapt(const __grid_constant__ AgConsts K, AgWorkspace W)
+__global__ void __launch_bounds__(256) k_ag_adapt(const __grid_constant__ AgConsts K, AgWorkspace W, const __grid_constant__ DistConsts prior)
 {
     __shared__ float sorted[GLABC_AG_MAX_BLOCK];
     __shared__ int cnt[256];
@@ -275,7 +275,7 @@ __global__ void __launch_bounds__(256) k_ag_adapt(const __grid_constant__ AgCons
 #pragma unroll
         for (int k = 0; k < D; ++k) th[k] = W.blk_theta[(c * B + j) * D + k];
         const float like = log_kernel_dis_eps(K.model.c_kern, dis[j], ls, scale);
-        const float tw = expf(__fsub_rn(__fadd_rn(model_prior<D, true>(K.model, th), like), W.blk_lq[c * B + j]));
+        const float tw = expf(__fsub_rn(__fadd_rn(prior_log_prob_rt<D>(K.model, prior, th), like), W.blk_lq[c * B + j]));
         sorted[j] = tw;  // the sort buffer is free again
         mine += tw > 0.0f;
     }
@@ -303,9 +303,10 @@ __global__ void __launch_bounds__(256) k_ag_adapt(const __grid_constant__ AgCons
     if (tid == 0) W.kde_n[c] = total;
 }
 
-// Theta_prop0 = the first B of the 4B KDE samples whose prior log-density exceeds log(1e-10), AGLMCMC.py:220-226
+// Theta_prop0 = the first B of the 4B KDE samples whose prior log-density exceeds log(1e-10), AGLMCMC.py:220-226 (a draw
+// outside the support of a Uniform / Gamma prior has log prior -inf and never enters the block)
 template <int D>
-__global__ void __launch_bounds__(256) k_ag_filter(const __grid_constant__ AgConsts K, AgWorkspace W)
+__global__ void __launch_bounds__(256) k_ag_filter(const __grid_constant__ AgConsts K, AgWorkspace W, const __grid_constant__ DistConsts prior)
 {
     __shared__ int cnt[256];
     const int64_t c = blockIdx.x;
@@ -319,7 +320,7 @@ __global__ void __launch_bounds__(256) k_ag_filter(const __grid_constant__ AgCon
         float th[D];
 #pragma unroll
         for (int k = 0; k < D; ++k) th[k] = smp[static_cast<int64_t>(j) * D + k];
-        mine += model_prior<D, true>(K.model, th) > K.log_prior_floor;
+        mine += prior_log_prob_rt<D>(K.model, prior, th) > K.log_prior_floor;
     }
     cnt[tid] = mine;
     __syncthreads();
@@ -329,7 +330,7 @@ __global__ void __launch_bounds__(256) k_ag_filter(const __grid_constant__ AgCon
         float th[D];
 #pragma unroll
         for (int k = 0; k < D; ++k) th[k] = smp[static_cast<int64_t>(j) * D + k];
-        if (model_prior<D, true>(K.model, th) > K.log_prior_floor) {
+        if (prior_log_prob_rt<D>(K.model, prior, th) > K.log_prior_floor) {
 #pragma unroll
             for (int k = 0; k < D; ++k) W.blk_theta[(c * B + base) * D + k] = th[k];
             ++base;
@@ -343,7 +344,7 @@ __global__ void __launch_bounds__(256) k_ag_filter(const __grid_constant__ AgCon
 // k_kde_sample + k_ag_filter produce (tested through the native-mode oracle comparison).
 template <int D>
 __global__ void __launch_bounds__(256) k_ag_sample_filter(const __grid_constant__ AgConsts K, AgWorkspace W, KdeSets S, RoundKeys rk,
-                                                          uint64_t chain_id_base)
+                                                          uint64_t chain_id_base, const __grid_constant__ DistConsts prior)
 {
     __shared__ int wsum[8];
     const int64_t c = blockIdx.x;
@@ -357,7 +358,7 @@ __global__ void __launch_bounds__(256) k_ag_sample_filter(const __grid_constant_
         bool valid = false;
         if (j < M) {
             kde_draw_native<D>(S, W.cdf, c, n, round, j, rk, chain_id_base, th);
-            valid = model_prior<D, true>(K.model, th) > K.log_prior_floor;
+            valid = prior_log_prob_rt<D>(K.model, prior, th) > K.log_prior_floor;
         }
         const unsigned bal = __ballot_sync(0xffffffffu, valid);
         if (lane == 0) wsum[warp] = __popc(bal);
@@ -384,10 +385,12 @@ __global__ void __launch_bounds__(256) k_ag_sample_filter(const __grid_constant_
 // EXT = the importance proposal lives outside this kernel (GLMCMC-NFs: the shared RealNVP flow): the cached
 // proposal log-density of a state that changed is not recomputed here — the chain pauses (pending bit 1) and the
 // host refreshes it in one batched tensor-core log_prob launch (flow.cuh) before relaunching.
-template <int D, int FAMILY, bool STRICT, bool REPLAY, bool EXT = false>
+// GPRIOR: the model's prior is `prior` (FAST arithmetic, native RNG; step_generic.cuh prior_log_prob).
+template <int D, int FAMILY, bool STRICT, bool REPLAY, bool EXT, bool GPRIOR>
 __global__ void __launch_bounds__(128) k_ag_step(const __grid_constant__ AgConsts K, const __grid_constant__ RunParams R,
-                                                 AgWorkspace W, int layout)
+                                                 AgWorkspace W, int layout, const __grid_constant__ DistConsts prior)
 {
+    static_assert(!GPRIOR || (!STRICT && !REPLAY), "a general prior runs FAST arithmetic with the native RNG");
     const int lane = threadIdx.x & 31;
     const int64_t chain = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
     const bool in_range = chain < W.C;
@@ -488,7 +491,7 @@ __global__ void __launch_bounds__(128) k_ag_step(const __grid_constant__ AgConst
             bool moved = false;
             int ind = -1;
             float d1 = 0.0f, d2 = 0.0f, d3 = 0.0f;
-            const float prior_old = model_prior<D, STRICT>(K.model, theta);
+            const float prior_old = prior_log_prob<D, STRICT, GPRIOR>(K.model, prior, theta);
             const float kern_old = model_log_kernel<D, STRICT>(K.model, y);
             if (is_global) {
                 // :137-149: weight of the current state under the current importance proposal
@@ -561,7 +564,7 @@ __global__ void __launch_bounds__(128) k_ag_step(const __grid_constant__ AgConst
 #pragma unroll
                 for (int k = 0; k < D; ++k) th_l[k] = STRICT ? __fadd_rn(z[k], theta[k]) : z[k] + theta[k];
                 model_simulate<D, STRICT>(K.model, th_l, eps_s, y_l);
-                const float prior_l = model_prior<D, STRICT>(K.model, th_l);
+                const float prior_l = prior_log_prob<D, STRICT, GPRIOR>(K.model, prior, th_l);
                 const float kern_l = model_log_kernel<D, STRICT>(K.model, y_l);
                 const float log_acc = STRICT ? __fsub_rn(__fsub_rn(__fadd_rn(prior_l, kern_l), prior_old), kern_old)
                                              : (prior_l + kern_l) - (prior_old + kern_old);
@@ -636,7 +639,7 @@ __global__ void __launch_bounds__(256) k_ag_row0(RunParams R, int64_t C, int lay
 // weights exp(prior + log K - log q0) with NaN -> 0.  One thread per (chain, b); `round` keys the simulator normals.
 template <int D, int FAMILY>
 __global__ void __launch_bounds__(256) k_blk_weights(const __grid_constant__ AgConsts K, const __grid_constant__ RunParams R,
-                                                     AgWorkspace W, uint32_t round)
+                                                     AgWorkspace W, uint32_t round, const __grid_constant__ DistConsts prior)
 {
     const int64_t g = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
     if (g >= W.C * W.B) return;
@@ -655,18 +658,20 @@ __global__ void __launch_bounds__(256) k_blk_weights(const __grid_constant__ AgC
     for (int k = 0; k < D; ++k) eps_s[k] = z[k];
     model_simulate<D, true>(K.model, th, eps_s, x);
     const float like = model_log_kernel<D, true>(K.model, x);
-    float wgt = expf(__fsub_rn(__fadd_rn(model_prior<D, true>(K.model, th), like), W.blk_lq[c * W.B + b]));
+    float wgt = expf(__fsub_rn(__fadd_rn(prior_log_prob_rt<D>(K.model, prior, th), like), W.blk_lq[c * W.B + b]));
     if (wgt != wgt) wgt = 0.0f;  // GLMCMC_NFs.py:84-85 (rows with NaN proposals get weight 0 as well, :83)
 #pragma unroll
     for (int k = 0; k < D; ++k) W.blk_x[(c * W.B + b) * D + k] = x[k];
     W.blk_w[c * W.B + b] = wgt;
 }
 
-cudaError_t launch_block_isir(const AgConsts& K, const AgWorkspace& W, const RunParams& R, int dim, bool strict, int layout,
-                              int block, cudaStream_t st);
-cudaError_t launch_block_weights(const AgConsts& K, const AgWorkspace& W, const RunParams& R, int dim, uint32_t round, cudaStream_t st);
+// `prior`: a Uniform / Gamma / GaussianMixture prior of the model (FAST, native RNG only) or GLABC_DIST_DIAG_GAUSSIAN for K.model's
+cudaError_t launch_block_isir(const AgConsts& K, const DistConsts& prior, const AgWorkspace& W, const RunParams& R, int dim, bool strict,
+                              int layout, int block, cudaStream_t st);
+cudaError_t launch_block_weights(const AgConsts& K, const DistConsts& prior, const AgWorkspace& W, const RunParams& R, int dim,
+                                 uint32_t round, cudaStream_t st);
 
-cudaError_t launch_aglmcmc(const AgConsts& K, const AgWorkspace& W, const AgTapes& T, const RunParams& R, int dim, int init,
-                           int kde_rule, bool strict, bool replay, int layout, int block, cudaStream_t st);
+cudaError_t launch_aglmcmc(const AgConsts& K, const DistConsts& prior, const AgWorkspace& W, const AgTapes& T, const RunParams& R,
+                           int dim, int init, int kde_rule, bool strict, bool replay, int layout, int block, cudaStream_t st);
 
 }  // namespace glabc

@@ -122,6 +122,25 @@ __device__ __forceinline__ float dist_log_prob(const DistConsts& q, const float 
     return NAN;
 }
 
+// The model's prior.  A DiagGaussian prior lives in ModelConsts (model_prior, the tuned arithmetic of both modes); a
+// Uniform / Gamma / GaussianMixture one bound with glabc_model_prior_set arrives as a DistConsts and is evaluated by
+// dist_log_prob (FAST only): GPRIOR kernels are instantiated for that case.  The kernels that run once per adaptation
+// choose at run time (generic_prior): `prior.kind` is GLABC_DIST_DIAG_GAUSSIAN when the model's own prior applies.
+template <int D, bool STRICT, bool GPRIOR>
+__device__ __forceinline__ float prior_log_prob(const ModelConsts& m, const DistConsts& prior, const float (&theta)[D])
+{
+    if constexpr (GPRIOR) return dist_log_prob<D>(prior, theta);
+    else return model_prior<D, STRICT>(m, theta);
+}
+
+__host__ __device__ __forceinline__ bool generic_prior(const DistConsts& prior) { return prior.kind != GLABC_DIST_DIAG_GAUSSIAN; }
+
+template <int D>
+__device__ __forceinline__ float prior_log_prob_rt(const ModelConsts& m, const DistConsts& prior, const float (&theta)[D])
+{
+    return generic_prior(prior) ? dist_log_prob<D>(prior, theta) : model_prior<D, true>(m, theta);
+}
+
 // forward(): one draw and its log-density
 template <int D>
 __device__ __forceinline__ float dist_forward(const DistConsts& q, WordStream& ws, float (&z)[D])
@@ -186,10 +205,13 @@ __device__ __forceinline__ float dist_forward(const DistConsts& q, WordStream& w
 // promotion: theta becomes a float64 tensor after the first accepted float64 candidate, and `z + theta` is then a float64
 // add (GlobalMCMC.py:56) — so the float32 trace rows (Theta_Re[i] = Theta_old, :52,67) match bit for bit.  Densities are
 // evaluated in float32 from the rounded state (the reference's are float64 after promotion: agreement to 1e-6).
-template <int D, int FAMILY, bool REPLAY>
+// GPRIOR: the model's prior is `prior` (native RNG only).  Outside its support the log prior is -inf, so the first
+// candidate with a finite prior is accepted (log_acc = +inf) and one with -inf never is.
+template <int D, int FAMILY, bool REPLAY, bool GPRIOR>
 __global__ void __launch_bounds__(128) k_global_generic(const __grid_constant__ GenericConsts K, const __grid_constant__ RunParams R,
-                                                        int layout)
+                                                        int layout, const __grid_constant__ DistConsts prior)
 {
+    static_assert(!(REPLAY && GPRIOR), "replay runs the model's DiagGaussian prior");
     const int64_t c = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
     if (c >= R.n_chains) return;
     float theta[D], y[D];
@@ -211,7 +233,7 @@ __global__ void __launch_bounds__(128) k_global_generic(const __grid_constant__ 
     if (R.write_row0) put(R.first_step - 1u);
     ChainStats<D> stats;
     const Stream stream = chain_stream(R, static_cast<int32_t>(c));
-    float prior_old = model_prior<D, false>(K.model, theta), kern_old = model_log_kernel<D, false>(K.model, y);
+    float prior_old = prior_log_prob<D, false, GPRIOR>(K.model, prior, theta), kern_old = model_log_kernel<D, false>(K.model, y);
     const bool lp64 = K.lp.kind == GLABC_DIST_GAMMA || K.lp.kind == GLABC_DIST_GAUSSIAN_MIXTURE;
     const bool gp64 = K.gp.kind == GLABC_DIST_GAMMA || K.gp.kind == GLABC_DIST_GAUSSIAN_MIXTURE;
 
@@ -265,7 +287,7 @@ __global__ void __launch_bounds__(128) k_global_generic(const __grid_constant__ 
             for (int k = 0; k < D; ++k) eps_s[k] = ws.normal();
         }
         model_simulate<D, false>(K.model, th_p, eps_s, y_p);           // :41,57
-        const float prior_p = model_prior<D, false>(K.model, th_p), kern_p = model_log_kernel<D, false>(K.model, y_p);
+        const float prior_p = prior_log_prob<D, false, GPRIOR>(K.model, prior, th_p), kern_p = model_log_kernel<D, false>(K.model, y_p);
         const float log_acc = (prior_p + kern_p) + corr - (prior_old + kern_old);   // :44-46 / :60-61
         const bool accept = log_w < log_acc;                                        // :49,64 (NaN rejects)
         float prev[D];
@@ -337,10 +359,13 @@ struct IsirGenericConsts {
 // candidates' are (torch.cat promotes): their exp does not underflow near -104 as the float32 one does (B-1).
 // REPLAY: tape32 [steps][2 + K D][C] = U_b, eps_sim[K][D] (a local move: eps_sim[D] first), U_a (last slot);
 // tape64 [steps][1 + K D][C] = the numpy resampling uniform, then the proposal's own draws (theta_j; local: increment z).
-template <int D, int FAMILY, bool REPLAY>
+// GPRIOR: the model's prior is `prior` (native RNG only), as in k_global_generic; a candidate outside its support has
+// log-weight -inf, i.e. weight 0, and is never selected.
+template <int D, int FAMILY, bool REPLAY, bool GPRIOR>
 __global__ void __launch_bounds__(128) k_isir_generic(const __grid_constant__ IsirGenericConsts K, const __grid_constant__ RunParams R,
-                                                      int layout)
+                                                      int layout, const __grid_constant__ DistConsts prior)
 {
+    static_assert(!(REPLAY && GPRIOR), "replay runs the model's DiagGaussian prior");
     const int64_t c = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
     if (c >= R.n_chains) return;
     const int64_t C = R.n_chains;
@@ -396,7 +421,7 @@ __global__ void __launch_bounds__(128) k_isir_generic(const __grid_constant__ Is
 
         if (is_global) {
             if (local) {                                                     // :60-64
-                lw_old = static_cast<double>((model_prior<D, false>(K.model, theta) + model_log_kernel<D, false>(K.model, y)) -
+                lw_old = static_cast<double>((prior_log_prob<D, false, GPRIOR>(K.model, prior, theta) + model_log_kernel<D, false>(K.model, y)) -
                                              dist_log_prob<D>(K.ip, theta));
                 lw_wide = wide;
             }
@@ -422,7 +447,7 @@ __global__ void __launch_bounds__(128) k_isir_generic(const __grid_constant__ Is
                     }
                 }
                 model_simulate<D, false>(K.model, tj, es, xj);
-                lw[j + 1] = (model_prior<D, false>(K.model, tj) + model_log_kernel<D, false>(K.model, xj)) - lq;
+                lw[j + 1] = (prior_log_prob<D, false, GPRIOR>(K.model, prior, tj) + model_log_kernel<D, false>(K.model, xj)) - lq;
 #pragma unroll
                 for (int k = 0; k < D; ++k) {
                     th_c[j][k] = tj[k];
@@ -509,8 +534,9 @@ __global__ void __launch_bounds__(128) k_isir_generic(const __grid_constant__ Is
                 u_a = __uint2float_rn(step_block_ua(w0)) * 0x1p-24f;
             }
             model_simulate<D, false>(K.model, th_p, es, y_p);
-            const float pr_p = model_prior<D, false>(K.model, th_p), k_p = model_log_kernel<D, false>(K.model, y_p);
-            const float log_acc = (pr_p + k_p) - (model_prior<D, false>(K.model, theta) + model_log_kernel<D, false>(K.model, y));   // :96-97
+            const float pr_p = prior_log_prob<D, false, GPRIOR>(K.model, prior, th_p), k_p = model_log_kernel<D, false>(K.model, y_p);
+            const float log_acc = (pr_p + k_p) - (prior_log_prob<D, false, GPRIOR>(K.model, prior, theta) +
+                                                  model_log_kernel<D, false>(K.model, y));   // :96-97
             d1 = pr_p;
             d2 = k_p;
             d3 = log_acc;
@@ -577,8 +603,11 @@ __global__ void __launch_bounds__(256) k_dist_eval(const __grid_constant__ DistC
     if (logp != nullptr) logp[g] = lp;
 }
 
-cudaError_t launch_global_generic(const GenericConsts& K, int dim, const RunParams& R, int layout, int block, bool replay, cudaStream_t st);
-cudaError_t launch_isir_generic(const IsirGenericConsts& K, int dim, const RunParams& R, int layout, int block, bool replay, cudaStream_t st);
+// `prior`: the model's prior when generic_prior(prior) (native RNG only), else the DiagGaussian of K.model applies
+cudaError_t launch_global_generic(const GenericConsts& K, const DistConsts& prior, int dim, const RunParams& R, int layout, int block,
+                                  bool replay, cudaStream_t st);
+cudaError_t launch_isir_generic(const IsirGenericConsts& K, const DistConsts& prior, int dim, const RunParams& R, int layout, int block,
+                                bool replay, cudaStream_t st);
 cudaError_t launch_dist_eval(const DistConsts& q, int dim, const RoundKeys& rk, int64_t n, const float* z_in, float* z_out, float* logp,
                              cudaStream_t st);
 

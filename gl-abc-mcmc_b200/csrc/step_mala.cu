@@ -4,18 +4,19 @@
 
 namespace glabc {
 
-extern template cudaError_t launch_mala_dim<1>(const MalaConsts&, const RunParams&, bool, bool, int, cudaStream_t);
-extern template cudaError_t launch_mala_dim<2>(const MalaConsts&, const RunParams&, bool, bool, int, cudaStream_t);
-extern template cudaError_t launch_mala_dim<3>(const MalaConsts&, const RunParams&, bool, bool, int, cudaStream_t);
-extern template cudaError_t launch_mala_dim<4>(const MalaConsts&, const RunParams&, bool, bool, int, cudaStream_t);
+extern template cudaError_t launch_mala_dim<1>(const MalaConsts&, const DistConsts&, const RunParams&, bool, bool, int, cudaStream_t);
+extern template cudaError_t launch_mala_dim<2>(const MalaConsts&, const DistConsts&, const RunParams&, bool, bool, int, cudaStream_t);
+extern template cudaError_t launch_mala_dim<3>(const MalaConsts&, const DistConsts&, const RunParams&, bool, bool, int, cudaStream_t);
+extern template cudaError_t launch_mala_dim<4>(const MalaConsts&, const DistConsts&, const RunParams&, bool, bool, int, cudaStream_t);
 
-cudaError_t launch_mala(const MalaConsts& K, int dim, const RunParams& R, bool strict, bool replay, int block, cudaStream_t st)
+cudaError_t launch_mala(const MalaConsts& K, const DistConsts& prior, int dim, const RunParams& R, bool strict, bool replay, int block,
+                        cudaStream_t st)
 {
     switch (dim) {
-    case 1: return launch_mala_dim<1>(K, R, strict, replay, block, st);
-    case 2: return launch_mala_dim<2>(K, R, strict, replay, block, st);
-    case 3: return launch_mala_dim<3>(K, R, strict, replay, block, st);
-    case 4: return launch_mala_dim<4>(K, R, strict, replay, block, st);
+    case 1: return launch_mala_dim<1>(K, prior, R, strict, replay, block, st);
+    case 2: return launch_mala_dim<2>(K, prior, R, strict, replay, block, st);
+    case 3: return launch_mala_dim<3>(K, prior, R, strict, replay, block, st);
+    case 4: return launch_mala_dim<4>(K, prior, R, strict, replay, block, st);
     default: return cudaErrorInvalidValue;
     }
 }

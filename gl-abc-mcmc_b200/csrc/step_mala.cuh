@@ -893,19 +893,19 @@ static cudaError_t launch_mala_one(const MalaConsts& K, const RunParams& R, int 
 
 // the throughput path (step_mala_fast.cuh): FAST arithmetic, native Philox, no tape dump
 template <int D, int FAMILY>
-static cudaError_t launch_mala_fast(const MalaConsts& K, const RunParams& R, cudaStream_t st);
+static cudaError_t launch_mala_fast(const MalaConsts& K, const DistConsts& prior, const RunParams& R, cudaStream_t st);
 
 template <int D, int FAMILY>
-static cudaError_t launch_mala_family(const MalaConsts& K, const RunParams& R, bool strict, bool replay, int block,
-                                      cudaStream_t st)
+static cudaError_t launch_mala_family(const MalaConsts& K, const DistConsts& prior, const RunParams& R, bool strict, bool replay,
+                                      int block, cudaStream_t st)
 {
     const bool dump = R.tape_dump != nullptr;
     // block_threads == 96 keeps the warp-per-chain kernel for FAST runs too (tests compare the two layouts)
-    if (K.ip_generic) {   // host side has checked: FAST arithmetic, native RNG, no tape dump
+    if (K.ip_generic || generic_prior(prior)) {   // host side has checked: FAST arithmetic, native RNG, no tape dump
         if (strict || replay || dump) return cudaErrorInvalidValue;
-        return launch_mala_fast<D, FAMILY>(K, R, st);
+        return launch_mala_fast<D, FAMILY>(K, prior, R, st);
     }
-    if (!strict && !replay && !dump && block != 96) return launch_mala_fast<D, FAMILY>(K, R, st);
+    if (!strict && !replay && !dump && block != 96) return launch_mala_fast<D, FAMILY>(K, prior, R, st);
     if (replay)
         return strict ? launch_mala_one<D, FAMILY, true, true, false>(K, R, block, st)
                       : launch_mala_one<D, FAMILY, false, true, false>(K, R, block, st);
@@ -917,11 +917,12 @@ static cudaError_t launch_mala_family(const MalaConsts& K, const RunParams& R, b
 }
 
 template <int D>
-cudaError_t launch_mala_dim(const MalaConsts& K, const RunParams& R, bool strict, bool replay, int block, cudaStream_t st)
+cudaError_t launch_mala_dim(const MalaConsts& K, const DistConsts& prior, const RunParams& R, bool strict, bool replay, int block,
+                            cudaStream_t st)
 {
     if (K.model.family == GLABC_MODEL_ABS_NORMAL)
-        return launch_mala_family<D, GLABC_MODEL_ABS_NORMAL>(K, R, strict, replay, block, st);
-    return launch_mala_family<D, GLABC_MODEL_ID_NORMAL>(K, R, strict, replay, block, st);
+        return launch_mala_family<D, GLABC_MODEL_ABS_NORMAL>(K, prior, R, strict, replay, block, st);
+    return launch_mala_family<D, GLABC_MODEL_ID_NORMAL>(K, prior, R, strict, replay, block, st);
 }
 
 }  // namespace glabc

@@ -2,5 +2,5 @@
 #include "step_mala_fast.cuh"
 
 namespace glabc {
-template cudaError_t launch_mala_dim<1>(const MalaConsts&, const RunParams&, bool, bool, int, cudaStream_t);
+template cudaError_t launch_mala_dim<1>(const MalaConsts&, const DistConsts&, const RunParams&, bool, bool, int, cudaStream_t);
 }  // namespace glabc

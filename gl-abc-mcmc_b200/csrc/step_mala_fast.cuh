@@ -132,10 +132,11 @@ GLABC_UNROLL(GLABC_MALA_UNROLL)
     }
 }
 
-// numberical_gradient_logABC from the folded sums (GLMALA.py:84-95), per chain
-template <int D>
-__device__ __forceinline__ void gradient_from_sums(const MalaConsts& K, const float (&th)[D], const float (&sums)[D][4],
-                                                   const float (&cpm)[D][2], float (&grad)[D])
+// numberical_gradient_logABC from the folded sums (GLMALA.py:84-95), per chain.  GPRIOR: the prior's finite difference
+// straddling the edge of its support is non-finite, and so is the drift: the proposal is rejected (NaN / -inf log_acc).
+template <int D, bool GPRIOR>
+__device__ __forceinline__ void gradient_from_sums(const MalaConsts& K, const DistConsts& prior, const float (&th)[D],
+                                                   const float (&sums)[D][4], const float (&cpm)[D][2], float (&grad)[D])
 {
     const float rn = 1.0f / static_cast<float>(K.num_grad), rn1 = 1.0f / static_cast<float>(K.num_grad - 1);
     const float e2 = static_cast<float>(K.eps2);
@@ -148,7 +149,7 @@ __device__ __forceinline__ void gradient_from_sums(const MalaConsts& K, const fl
             tb[i] = i == k ? __fsub_rn(th[i], 0.00001f) : th[i];
         }
         // the float32 finite-difference prior gradient in the reference's exact operation order: its rounding IS its value (B-8)
-        const float gprior = __fdiv_rn(__fsub_rn(model_prior<D, true>(K.model, ta), model_prior<D, true>(K.model, tb)),
+        const float gprior = __fdiv_rn(__fsub_rn(prior_log_prob<D, true, GPRIOR>(K.model, prior, ta), prior_log_prob<D, true, GPRIOR>(K.model, prior, tb)),
                                        static_cast<float>(2 * 0.00001));
         const float f1p = sums[k][0], f2p = sums[k][1], f1m = sums[k][2], f2m = sums[k][3];
         const float mup = fmaf(f1p, rn, cpm[k][0]), mum = fmaf(f1m, rn, cpm[k][1]);
@@ -165,8 +166,11 @@ __device__ __forceinline__ void gradient_from_sums(const MalaConsts& K, const fl
 // same, and twice as many warps hide the latency of the Philox / MUFU chains).  The chain-major trace tile needs 32.
 // GIP: the Importance_Proposal is one of the non-Gaussian classes (K.ipg, step_generic.cuh): candidate j of a step is
 // dist_forward over the word stream of Philox slots kSlotGeneric + 64 j .., its simulator normals follow in the same stream.
-template <int D, int FAMILY, int LAYOUT, int CPW, bool GIP = false>
-__global__ void __launch_bounds__(GLABC_MALA_BLOCK) k_mala_fast(const __grid_constant__ MalaConsts K, const __grid_constant__ RunParams R)
+// GPRIOR: the model's prior is `prior` (step_generic.cuh prior_log_prob) in the iSIR weights, the MALA target and the
+// finite-difference prior gradient.
+template <int D, int FAMILY, int LAYOUT, int CPW, bool GIP, bool GPRIOR>
+__global__ void __launch_bounds__(GLABC_MALA_BLOCK) k_mala_fast(const __grid_constant__ MalaConsts K, const __grid_constant__ RunParams R,
+                                                                const __grid_constant__ DistConsts prior)
 {
     using Writer = typename WriterFor<D, LAYOUT>::type;
     static_assert(CPW == 32 || LAYOUT != GLABC_TRACE_CHAIN_MAJOR, "the chain-major tile stages 32 chains per warp");
@@ -215,7 +219,7 @@ __global__ void __launch_bounds__(GLABC_MALA_BLOCK) k_mala_fast(const __grid_con
             // ================= iSIR global move, GLMALA.py:151-180 =================
             if (local) {  // :152-156 — the only place log_weight_old is computed from the state
                 const float q_old = GIP ? dist_log_prob<D>(K.ipg, theta) : gauss_log_prob<D, false>(K.ip, theta);
-                lw_old = (model_prior<D, false>(K.model, theta) + model_log_kernel<D, false>(K.model, y)) - q_old;
+                lw_old = (prior_log_prob<D, false, GPRIOR>(K.model, prior, theta) + model_log_kernel<D, false>(K.model, y)) - q_old;
                 lw_wide = wide;
             }
             local = false;
@@ -231,7 +235,7 @@ GLABC_UNROLL(GLABC_MALA_KUNROLL)
 #pragma unroll
                     for (int k = 0; k < D; ++k) eps_s[k] = ws.normal();
                     model_simulate<D, false>(K.model, th_c, eps_s, x_c);
-                    lw_c = (model_prior<D, false>(K.model, th_c) + model_log_kernel<D, false>(K.model, x_c)) - lq;
+                    lw_c = (prior_log_prob<D, false, GPRIOR>(K.model, prior, th_c) + model_log_kernel<D, false>(K.model, x_c)) - lq;
                     if (j == 0) wfirst = stream.block(R.rk, i, kSlotNormal + 8u);
                 } else {
                     float zc[kGroups * 4];
@@ -250,7 +254,7 @@ GLABC_UNROLL(GLABC_MALA_KUNROLL)
                     }
                     const float lq = gauss_forward<D, false>(K.ip, eps_p, th_c);
                     model_simulate<D, false>(K.model, th_c, eps_s, x_c);
-                    lw_c = (model_prior<D, false>(K.model, th_c) + model_log_kernel<D, false>(K.model, x_c)) - lq;
+                    lw_c = (prior_log_prob<D, false, GPRIOR>(K.model, prior, th_c) + model_log_kernel<D, false>(K.model, x_c)) - lq;
                 }
                 lw_tab[j * blockDim.x + threadIdx.x] = lw_c;
                 m = fmaxf(m, lw_c == lw_c ? lw_c : -INFINITY);
@@ -365,7 +369,7 @@ GLABC_UNROLL(GLABC_MALA_KUNROLL)
                 const bool mine = pass == 0 ? (is_local && !have_grad) : is_local;
                 if (mine) {
                     float gout[D];
-                    gradient_from_sums<D>(K, theta_p, sums, cpm, gout);
+                    gradient_from_sums<D, GPRIOR>(K, prior, theta_p, sums, cpm, gout);
 #pragma unroll
                     for (int k = 0; k < D; ++k) {
                         if (pass == 0) grad[k] = gout[k];
@@ -379,9 +383,9 @@ GLABC_UNROLL(GLABC_MALA_KUNROLL)
                 model_simulate<D, false>(K.model, theta_p, eps_s, y_p);   // :188-189
 #pragma unroll
                 for (int k = 0; k < D; ++k) rr[k] = ((theta[k] - theta_p[k]) - grad_p[k] * half_tau2) * inv_tau;   // log_proposal, :97-116
-                const float pp = model_prior<D, false>(K.model, theta_p), kp = model_log_kernel<D, false>(K.model, y_p);
+                const float pp = prior_log_prob<D, false, GPRIOR>(K.model, prior, theta_p), kp = model_log_kernel<D, false>(K.model, y_p);
                 const float lr = gauss_log_prob<D, false>(K.unit, rr);
-                const float po = model_prior<D, false>(K.model, theta), ko = model_log_kernel<D, false>(K.model, y);
+                const float po = prior_log_prob<D, false, GPRIOR>(K.model, prior, theta), ko = model_log_kernel<D, false>(K.model, y);
                 const float log_acc = ((pp + kp) - (po + ko)) + (lr - lq_fwd);   // :190-193
                 if (log_approx(u_a) < log_acc) {   // :194-199
 #pragma unroll
@@ -421,8 +425,16 @@ GLABC_UNROLL(GLABC_MALA_KUNROLL)
     }
 }
 
+template <int D, int FAMILY, int LAYOUT, int CPW, bool GIP>
+static void launch_mala_fast_gip(const MalaConsts& K, const DistConsts& prior, const RunParams& R, int grid, int block, size_t smem,
+                                 cudaStream_t st)
+{
+    if (generic_prior(prior)) k_mala_fast<D, FAMILY, LAYOUT, CPW, GIP, true><<<grid, block, smem, st>>>(K, R, prior);
+    else k_mala_fast<D, FAMILY, LAYOUT, CPW, GIP, false><<<grid, block, smem, st>>>(K, R, prior);
+}
+
 template <int D, int FAMILY, int LAYOUT, int CPW>
-static cudaError_t launch_mala_fast_cpw(const MalaConsts& K, const RunParams& R, cudaStream_t st)
+static cudaError_t launch_mala_fast_cpw(const MalaConsts& K, const DistConsts& prior, const RunParams& R, cudaStream_t st)
 {
     using Writer = typename WriterFor<D, LAYOUT>::type;
     constexpr int block = GLABC_MALA_BLOCK;
@@ -430,13 +442,13 @@ static cudaError_t launch_mala_fast_cpw(const MalaConsts& K, const RunParams& R,
     const int grid = (R.n_chains + chains_per_block - 1) / chains_per_block;
     const size_t smem = sizeof(float) * (static_cast<size_t>(Writer::smem_floats_per_warp) * (block / 32) +
                                          static_cast<size_t>(R.n_candidates) * block);
-    if (K.ip_generic) k_mala_fast<D, FAMILY, LAYOUT, CPW, true><<<grid, block, smem, st>>>(K, R);
-    else k_mala_fast<D, FAMILY, LAYOUT, CPW, false><<<grid, block, smem, st>>>(K, R);
+    if (K.ip_generic) launch_mala_fast_gip<D, FAMILY, LAYOUT, CPW, true>(K, prior, R, grid, block, smem, st);
+    else launch_mala_fast_gip<D, FAMILY, LAYOUT, CPW, false>(K, prior, R, grid, block, smem, st);
     return cudaGetLastError();
 }
 
 template <int D, int FAMILY, int LAYOUT>
-static cudaError_t launch_mala_fast_one(const MalaConsts& K, const RunParams& R, cudaStream_t st)
+static cudaError_t launch_mala_fast_one(const MalaConsts& K, const DistConsts& prior, const RunParams& R, cudaStream_t st)
 {
     // Measured and rejected (DESIGN.md K3): pooling the 4 left-over blocks per gradient (100 blocks on 32 lanes) of all pending
     // chains into one joint round — 3 n + 1 rounds instead of 4 n — ran 11.96 ms instead of 9.78 ms at 32,768 chains and 61.5
@@ -446,18 +458,18 @@ static cudaError_t launch_mala_fast_one(const MalaConsts& K, const RunParams& R,
     // issue-active rose from 47 % to 63 % but the warp-instructions per chain-step rose from 152 to 193 — the same 9.85 ms
     // (profiles/r2_k3_mala_fast_ncu.md).  Kept behind a build flag for other shapes.
 #if defined(GLABC_MALA_FORCE_CPW) && GLABC_MALA_FORCE_CPW == 16
-    if constexpr (LAYOUT != GLABC_TRACE_CHAIN_MAJOR) return launch_mala_fast_cpw<D, FAMILY, LAYOUT, 16>(K, R, st);
+    if constexpr (LAYOUT != GLABC_TRACE_CHAIN_MAJOR) return launch_mala_fast_cpw<D, FAMILY, LAYOUT, 16>(K, prior, R, st);
 #endif
-    return launch_mala_fast_cpw<D, FAMILY, LAYOUT, 32>(K, R, st);
+    return launch_mala_fast_cpw<D, FAMILY, LAYOUT, 32>(K, prior, R, st);
 }
 
 template <int D, int FAMILY>
-static cudaError_t launch_mala_fast(const MalaConsts& K, const RunParams& R, cudaStream_t st)
+static cudaError_t launch_mala_fast(const MalaConsts& K, const DistConsts& prior, const RunParams& R, cudaStream_t st)
 {
     switch (R.trace_layout) {
-    case GLABC_TRACE_NONE: return launch_mala_fast_one<D, FAMILY, GLABC_TRACE_NONE>(K, R, st);
-    case GLABC_TRACE_TIME_MAJOR: return launch_mala_fast_one<D, FAMILY, GLABC_TRACE_TIME_MAJOR>(K, R, st);
-    case GLABC_TRACE_CHAIN_MAJOR: return launch_mala_fast_one<D, FAMILY, GLABC_TRACE_CHAIN_MAJOR>(K, R, st);
+    case GLABC_TRACE_NONE: return launch_mala_fast_one<D, FAMILY, GLABC_TRACE_NONE>(K, prior, R, st);
+    case GLABC_TRACE_TIME_MAJOR: return launch_mala_fast_one<D, FAMILY, GLABC_TRACE_TIME_MAJOR>(K, prior, R, st);
+    case GLABC_TRACE_CHAIN_MAJOR: return launch_mala_fast_one<D, FAMILY, GLABC_TRACE_CHAIN_MAJOR>(K, prior, R, st);
     }
     return cudaErrorInvalidValue;
 }

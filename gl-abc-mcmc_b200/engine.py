@@ -9,7 +9,7 @@ from dataclasses import dataclass
 import torch
 
 from . import _abi
-from .models import lower_model, lower_proposal
+from .models import fused_model, lower_proposal
 
 
 @dataclass
@@ -77,16 +77,23 @@ class Engine:
         self.ctx = _abi.Context(self.device.index if self.device.index is not None else torch.cuda.current_device())
         self.lib = self.ctx.lib
         self.dim = None
+        self.prior_pod = None   # DistPOD of the bound model's prior when it is not the DiagGaussian of its model POD
 
     # -- plugin binding -------------------------------------------------------------------------
     def bind_model(self, abc_set):
-        pod = lower_model(abc_set)
+        model = fused_model(abc_set)
+        pod = model.lower()
+        prior = model.lower_prior() if hasattr(model, "lower_prior") else None
         self.ctx.check(self.lib.glabc_model_set(self.ctx.handle, C.byref(pod), C.sizeof(pod)))
+        if prior is not None:
+            self.ctx.check(self.lib.glabc_model_prior_set(self.ctx.handle, C.byref(prior), C.sizeof(prior)))
         self.dim = pod.theta_dim
+        self.prior_pod = prior
         return pod
 
     def bind_proposal(self, slot, dist):
-        pod = lower_proposal(dist)
+        """`dist`: a distribution object, or its lowered DistPOD"""
+        pod = dist if isinstance(dist, _abi.DistPOD) else lower_proposal(dist)
         self.ctx.check(self.lib.glabc_dist_set(self.ctx.handle, slot, C.byref(pod), C.sizeof(pod)))
         return pod
 

@@ -4,21 +4,28 @@ README.md:66-104): attributes `epsilon, theta_dim, y_obs, y_dim`, methods `gener
 
 `AbsNormalModel` is the fused family the reference's `Mixture_set` belongs to:
     y | theta ~ N(link(theta) + noise_loc, diag(noise_scale^2)),  link = |.| or identity,
-    prior DiagGaussian, discrepancy = L2 distance to y_obs, Gaussian ABC kernel of width epsilon.
+    prior DiagGaussian (or any `prior=` DiagGaussian / Uniform / Gamma / GaussianMixture), discrepancy = L2
+    distance to y_obs, Gaussian ABC kernel of width epsilon.
 Its torch methods follow the reference formulas (usable on CPU or CUDA tensors, batched); its
-`lower()` gives the POD the kernels consume.  `lower_model()` also recognises a *reference*
+`lower()` gives the POD the kernels consume, `lower_prior()` the POD of a `prior=` distribution.  `lower_model()` also recognises a *reference*
 `Mixture_set` instance (duck-typed probe of its deterministic methods) so existing user scripts can
 pass their own model object unchanged.
 """
 import torch
 
 from . import _abi
-from .distribution import DiagGaussian
+from .distribution import DiagGaussian, Gamma, GaussianMixture, Uniform
+
+PRIOR_CLASSES = (DiagGaussian, Uniform, Gamma, GaussianMixture)
 
 
 class AbsNormalModel:
+    """`prior`: a DiagGaussian / Uniform / Gamma / GaussianMixture of `theta_dim` that replaces the DiagGaussian of
+    `prior_loc` / `prior_log_scale`.  The kernels run a non-Gaussian prior with FAST arithmetic and the native RNG
+    (glabc_model_prior_set)."""
+
     def __init__(self, epsilon, y_obs=(1.5, 1.5), noise_var=0.05, prior_loc=None, prior_log_scale=None,
-                 noise_loc=None, link="abs", device=None):
+                 noise_loc=None, link="abs", device=None, prior=None):
         self.epsilon = epsilon
         self.y_obs = torch.as_tensor(y_obs, dtype=torch.float32).view(1, -1)
         self.theta_dim = self.y_obs.shape[1]
@@ -32,6 +39,12 @@ class AbsNormalModel:
         if link not in ("abs", "identity"):
             raise ValueError("link must be 'abs' or 'identity'")
         self.link = link
+        if prior is not None:
+            if not isinstance(prior, PRIOR_CLASSES):
+                raise TypeError(f"prior must be one of {', '.join(c.__name__ for c in PRIOR_CLASSES)}")
+            if prior.lower().dim != d:
+                raise ValueError(f"prior dimension {prior.lower().dim} does not match theta_dim {d}")
+        self.prior = prior
         if device is not None:
             self.to(device)
 
@@ -56,6 +69,8 @@ class AbsNormalModel:
 
     def prior_log_prob(self, samples):
         samples = samples.to(self.y_obs.device).view(-1, self.theta_dim)
+        if self.prior is not None:   # the distribution's parameters stay on the CPU
+            return self.prior.log_prob(samples.cpu()).to(samples.device)
         return DiagGaussian(self.theta_dim, self.prior_loc, self.prior_log_scale).log_prob(samples)
 
     def discrepancy(self, y):
@@ -89,6 +104,10 @@ class AbsNormalModel:
         pod.eps_scale = float(torch.exp(torch.log(eps_t)))     # distribution.py:178 (0.05 -> 0.049999997)
         pod.epsilon = float(self.epsilon)                      # GLMALA.py:90 squares the Python float
         return pod
+
+    def lower_prior(self):
+        """POD of the `prior=` distribution for glabc_model_prior_set, or None for the DiagGaussian `lower()` carries"""
+        return None if self.prior is None else self.prior.lower()
 
 
 class Mixture_set(AbsNormalModel):
@@ -159,12 +178,55 @@ def mixture_user_model(epsilon=0.05):
     return UserModel(MIXTURE_USER_SOURCE, theta_dim=2, y_dim=2, n_noise=2, epsilon=epsilon, params=[1.5, 1.5, 0.05 ** 0.5])
 
 
-def lower_model(abc_set):
-    """POD for `abc_set`: our own model classes lower themselves; a foreign object is accepted only
-    if it behaves exactly like the AbsNormal family on a deterministic probe (so a reference
-    `Mixture_set` instance drops in).  Anything else raises — there is no interpreted fallback."""
+def _as_prior(dist):
+    """one of our distribution classes for `dist`: itself, or the same distribution built from a reference
+    (glabcmcmc.distribution) instance of the same class name, recognised by its attributes; None otherwise"""
+    if isinstance(dist, PRIOR_CLASSES):
+        return dist
+    name = type(dist).__name__
+    has = lambda *a: all(hasattr(dist, x) for x in a)  # noqa: E731
+    if name == "DiagGaussian" and has("loc", "log_scale", "shape", "d"):
+        return DiagGaussian(tuple(dist.shape), dist.loc, dist.log_scale)
+    if name == "Uniform" and has("shape", "low", "high"):
+        return Uniform(tuple(dist.shape), dist.low, dist.high)
+    if name == "Gamma" and has("Shape", "Rate"):
+        return Gamma(dist.Shape, dist.Rate)
+    if name == "GaussianMixture" and has("n_modes", "dim", "loc", "log_scale", "weight_scores"):
+        return GaussianMixture(int(dist.n_modes), int(dist.dim), loc=torch.as_tensor(dist.loc)[0].numpy(),
+                               scale=torch.exp(torch.as_tensor(dist.log_scale)[0]).numpy(),
+                               weights=torch.softmax(torch.as_tensor(dist.weight_scores), 1)[0].numpy())
+    return None
+
+
+def _foreign_prior(abc_set, d, th):
+    """the lowerable `prior` attribute of a foreign model, if its prior_log_prob agrees with it on the probe set and on
+    points outside the support (-inf matching -inf); None otherwise"""
+    prior = _as_prior(getattr(abc_set, "prior", None))
+    if prior is None:
+        return None
+    try:
+        if prior.lower().dim != d:
+            return None
+        pts = torch.cat([th, th * 10.0, -th.abs() - 0.5])
+        want = abc_set.prior_log_prob(pts).double().reshape(-1).cpu()
+        got = prior.log_prob(pts).double().reshape(-1).cpu()
+    except (NotImplementedError, RuntimeError, TypeError, ValueError):
+        return None
+    if want.shape != got.shape or not torch.equal(torch.isneginf(want), torch.isneginf(got)):
+        return None
+    fin = torch.isfinite(want)
+    if not torch.equal(fin, torch.isfinite(got)) or not torch.allclose(got[fin], want[fin], rtol=1e-5, atol=1e-4):
+        return None
+    return prior
+
+
+def fused_model(abc_set):
+    """our model object for `abc_set`: itself when it lowers; a foreign object is accepted only if it behaves exactly
+    like the AbsNormal family on a deterministic probe (so a reference `Mixture_set` instance drops in), with a
+    DiagGaussian prior found by the probe or the lowerable distribution in its `prior` attribute.  Anything else
+    raises — there is no interpreted fallback."""
     if hasattr(abc_set, "lower"):
-        return abc_set.lower()
+        return abc_set
     for attr in ("epsilon", "theta_dim", "y_obs", "prior_log_prob", "discrepancy", "calculate_log_kernel", "generate_samples"):
         if not hasattr(abc_set, attr):
             raise NotImplementedError(f"ABC model lacks `{attr}`; cannot lower it to a fused family")
@@ -175,11 +237,12 @@ def lower_model(abc_set):
     # probe: recover prior loc/scale, noise scale and link from the object's own methods
     g = torch.Generator().manual_seed(1234)
     th = torch.randn(64, d, generator=g) * 2.0
-    # prior: fit a diagonal Gaussian through 2d+1 evaluations, then verify on the probe set
+    prior = _foreign_prior(abc_set, d, th)
+    # otherwise the prior: fit a diagonal Gaussian through 2d+1 evaluations, then verify on the probe set
     zero = torch.zeros(1, d)
     p0 = abc_set.prior_log_prob(zero).float().reshape(-1)[0]
     loc, ls = torch.zeros(d), torch.zeros(d)
-    for i in range(d):
+    for i in range(d if prior is None else 0):
         e = torch.zeros(1, d)
         e[0, i] = 1.0
         pp = abc_set.prior_log_prob(e).float().reshape(-1)[0]
@@ -210,14 +273,19 @@ def lower_model(abc_set):
     if link is None:
         raise NotImplementedError("simulator is not y = link(theta) + scale*eps; no fused lowering")
     model = AbsNormalModel(abc_set.epsilon, y_obs=y_obs.tolist(), noise_var=(noise_scale ** 2).tolist(),
-                           prior_loc=loc.tolist(), prior_log_scale=ls.tolist(), link=link)
+                           prior_loc=loc.tolist(), prior_log_scale=ls.tolist(), link=link, prior=prior)
     # verify the deterministic plugin methods agree before trusting the lowering
-    ok = (torch.allclose(model.prior_log_prob(th), abc_set.prior_log_prob(th).float(), rtol=1e-5, atol=1e-5)
+    ok = (torch.allclose(model.prior_log_prob(th).float(), abc_set.prior_log_prob(th).float(), rtol=1e-5, atol=1e-5)
           and torch.allclose(model.discrepancy(y), abc_set.discrepancy(y).float(), rtol=1e-5, atol=1e-6)
           and torch.allclose(model.calculate_log_kernel(y), abc_set.calculate_log_kernel(y).float(), rtol=1e-5, atol=1e-4))
     if not ok:
         raise NotImplementedError("model does not match the AbsNormal family on the probe set; no fused lowering")
-    return model.lower()
+    return model
+
+
+def lower_model(abc_set):
+    """the model POD of `abc_set` (fused_model); its prior's POD is `fused_model(abc_set).lower_prior()`"""
+    return fused_model(abc_set).lower()
 
 
 def lower_proposal(dist):

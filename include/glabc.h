@@ -348,6 +348,14 @@ GLABC_API int glabc_model_set(glabc_ctx* ctx, const glabc_model_t* model, size_t
 /* replaces Local_Proposal / Global_Proposal / Importance_Proposal (GlobalMCMC.py:6-7,
  * GLMCMC.py:24-25)                                                                               */
 GLABC_API int glabc_dist_set(glabc_ctx* ctx, int slot, const glabc_dist_t* dist, size_t nbytes);
+/* Prior of the bound model (replaces the DiagGaussian in glabc_model_t's prior_* fields): any glabc_dist_t kind,
+ * dim == theta_dim.  NULL restores the model's DiagGaussian.  glabc_model_set clears a bound prior.
+ * A DiagGaussian is written into the model's prior_* fields (the same run as giving it in the model POD).  With a Uniform /
+ * Gamma / GaussianMixture prior every sampler runs FAST arithmetic with the native RNG: GLABC_ARITH_STRICT, GLABC_RNG_REPLAY,
+ * tape_dump and the AGLMCMC parity dumps are refused with GLABC_ERR_UNSUPPORTED.  Outside the prior's support the log prior
+ * is -inf: from such a state the first proposal with a finite prior is accepted, a candidate with -inf is never selected.
+ * GLABC_ERR_INVALID: no model bound, dim != theta_dim, invalid parameters (the checks of glabc_dist_set).               */
+GLABC_API int glabc_model_prior_set(glabc_ctx* ctx, const glabc_dist_t* prior, size_t nbytes);
 
 /* device-side forward() / log_prob() of the distribution bound to `slot` (distribution.py:73-86, 106-137, 166-181,
  * 242-293): z[n][dim] -> log_p[n], and n fresh draws z[n][dim] (+ their log-densities, log_p may be NULL)            */
@@ -359,7 +367,8 @@ GLABC_API int glabc_dist_sample(glabc_ctx* ctx, int slot, int64_t n, uint64_t se
  * in both slots run the tuned kernel (replay + strict arithmetic available); any Uniform / Gamma / GaussianMixture
  * proposal selects the general kernel (float32).  Its replay mode takes the reference's proposal draws themselves:
  * tape32 [n_steps][2 + d][C] = U_b, eps_sim[d], U_a and tape64 [n_steps][d][C] = the draw in float64 (theta' of a global
- * move, the increment of a local one); debug slots 0..3 as for the tuned kernel.                                    */
+ * move, the increment of a local one); debug slots 0..3 as for the tuned kernel.
+ * A non-Gaussian model prior (glabc_model_prior_set) also selects the general kernel: FAST arithmetic, native RNG.    */
 GLABC_API int glabc_run_global(glabc_ctx* ctx, const glabc_run_t* run);
 
 /* GLMCMC loop body, GLMCMC.py:58-104, incl. weight_sampling GLMCMC.py:7-22: iSIR global move with
@@ -370,7 +379,7 @@ GLABC_API int glabc_run_global(glabc_ctx* ctx, const glabc_run_t* run);
  * Its replay mode takes the proposal draws themselves: tape32 [n_steps][2 + K y_dim][C] = U_b, eps_sim[K][y_dim] (a local
  * move: eps_sim[y_dim] first), U_a (last slot); tape64 [n_steps][1 + K d][C] = the float64 resampling uniform, then the draws
  * theta_j (a local move: the increment z in the first d); debug slots as for the tuned kernel, + bit 16 of slot 0 = float64
- * weights.                                                                                                             */
+ * weights.  A non-Gaussian model prior (glabc_model_prior_set) also selects the general kernel: FAST, native RNG.       */
 GLABC_API int glabc_run_isir(glabc_ctx* ctx, const glabc_run_t* run);
 
 /* GLMALA loop body, GLMALA.py:150-200: the iSIR global move of run_isir (GLMALA.py:151-180) and a MALA
@@ -379,7 +388,8 @@ GLABC_API int glabc_run_isir(glabc_ctx* ctx, const glabc_run_t* run);
  * common random numbers.  run->tau, run->num_grad, run->n_candidates; needs aux and state64.
  * A Uniform / Gamma / GaussianMixture Importance_Proposal runs in the throughput kernel (GLABC_ARITH_FAST, native RNG, no
  * tape dump; candidates drawn as in glabc_run_isir's general kernel); with GLABC_ARITH_STRICT / GLABC_RNG_REPLAY it is refused
- * with GLABC_ERR_UNSUPPORTED — the replay kernel is fused for a DiagGaussian importance proposal.     */
+ * with GLABC_ERR_UNSUPPORTED — the replay kernel is fused for a DiagGaussian importance proposal.  The same holds for a
+ * non-Gaussian model prior (glabc_model_prior_set), whatever block_threads is.                                          */
 GLABC_API int glabc_run_mala(glabc_ctx* ctx, const glabc_run_t* run);
 
 /* AGLMCMC loop body, AGLMCMC.py:124-272.  LOCAL slot = Local_Proposal, IMPORTANCE slot = Initial_ISIR_prop;
@@ -389,7 +399,9 @@ GLABC_API int glabc_run_mala(glabc_ctx* ctx, const glabc_run_t* run);
  * K+1 weights; local move: as run_global.
  * A Uniform / Gamma / GaussianMixture Initial_ISIR_prop (the initial candidate block, AGLMCMC.py:84-112, and the weight
  * of the current state before the first adaptation, :137-149) is taken with GLABC_ARITH_FAST and the native RNG; STRICT /
- * replay / recording runs and a non-Gaussian Local_Proposal are refused with GLABC_ERR_UNSUPPORTED.           */
+ * replay / recording runs and a non-Gaussian Local_Proposal are refused with GLABC_ERR_UNSUPPORTED.  A non-Gaussian model
+ * prior (glabc_model_prior_set) runs FAST with the native RNG as well; KDE draws with log prior <= log(1e-10) (outside a
+ * Uniform box, say) never enter a block.                                                                                */
 GLABC_API int glabc_run_aglmcmc(glabc_ctx* ctx, const glabc_run_t* run, const glabc_aglmcmc_t* ag);
 
 /* GlobalMCMC loop body (GlobalMCMC.py:37-68) for a user-supplied model: LOCAL / GLOBAL slots must hold DiagGaussian
@@ -432,6 +444,7 @@ GLABC_API int glabc_kde_sample(glabc_ctx* ctx, const float* X, const float* weig
  * log-density of a changed state (pending bit 1).  The caller refreshes lq_cur with glabc_flow_log_prob, refills the
  * block with glabc_flow_sample + glabc_block_weights, and calls again.  LOCAL slot = Local_Proposal.             */
 GLABC_API int glabc_run_block_isir(glabc_ctx* ctx, const glabc_run_t* run, const glabc_block_isir_t* blk);
+/* (a non-Gaussian model prior: FAST arithmetic only, as glabc_run_aglmcmc)                                               */
 /* GLMCMC_NFs.py:73-85,129-140: blk_x = simulate(blk_theta), blk_w = exp(prior + log K - blk_lq), NaN -> 0;
  * `round` keys the simulator's Philox normals (run->seed, run->chain_id_base as usual)                           */
 GLABC_API int glabc_block_weights(glabc_ctx* ctx, const glabc_run_t* run, const glabc_block_isir_t* blk, uint32_t round);
