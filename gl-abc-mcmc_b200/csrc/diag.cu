@@ -87,12 +87,10 @@ static cudaError_t esjd_dim(const float* trace, int layout, int64_t rows, int64_
 
 cudaError_t launch_esjd(const float* trace, int layout, int64_t rows, int64_t chains, int dim, float* out, cudaStream_t st)
 {
-    switch (dim) {
-    case 1: return esjd_dim<1>(trace, layout, rows, chains, out, st);
-    case 2: return esjd_dim<2>(trace, layout, rows, chains, out, st);
-    case 3: return esjd_dim<3>(trace, layout, rows, chains, out, st);
-    default: return cudaErrorInvalidValue;
-    }
+    return with_dim(dim, [&](auto d) {
+        if constexpr (d == 4) return cudaErrorInvalidValue;   // esjd_from_gram: D <= 3
+        else return esjd_dim<d>(trace, layout, rows, chains, out, st);
+    });
 }
 
 // Summary of a shard's per-chain statistics in ONE launch (sharding.summarize): out[6 + 2d] float64 +=
@@ -164,14 +162,10 @@ cudaError_t launch_summarize(const float* stats, int64_t chains, int dim, double
     int64_t blocks = (chains + 255) / 256;
     if (blocks > 296) blocks = 296;
     const unsigned g = static_cast<unsigned>(blocks);
-    switch (dim) {
-    case 1: k_summarize<1><<<g, 256, 0, st>>>(stats, chains, out); break;
-    case 2: k_summarize<2><<<g, 256, 0, st>>>(stats, chains, out); break;
-    case 3: k_summarize<3><<<g, 256, 0, st>>>(stats, chains, out); break;
-    case 4: k_summarize<4><<<g, 256, 0, st>>>(stats, chains, out); break;
-    default: return cudaErrorInvalidValue;
-    }
-    return cudaGetLastError();
+    return with_dim(dim, [&](auto d) {
+        k_summarize<d><<<g, 256, 0, st>>>(stats, chains, out);
+        return cudaGetLastError();
+    });
 }
 
 __global__ void k_philox_kat(const uint32_t* __restrict__ ctr, const uint32_t* __restrict__ key, int64_t n,

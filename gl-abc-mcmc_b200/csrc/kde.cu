@@ -1,5 +1,6 @@
 // Host launchers of the KernelDensity kernels (kde.cuh), dispatched over the feature dimension.
 #include "kde.cuh"
+#include "launch.cuh"
 
 namespace glabc {
 
@@ -8,14 +9,10 @@ cudaError_t launch_kde_fit(const float* X, const float* w, const int32_t* n, con
 {
     if (sets <= 0) return cudaSuccess;
     const unsigned grid = static_cast<unsigned>(sets);
-    switch (dim) {
-    case 1: k_kde_fit<1><<<grid, 256, 0, st>>>(X, w, n, active, cap, rule, weights_out, lw_out, bw_out); break;
-    case 2: k_kde_fit<2><<<grid, 256, 0, st>>>(X, w, n, active, cap, rule, weights_out, lw_out, bw_out); break;
-    case 3: k_kde_fit<3><<<grid, 256, 0, st>>>(X, w, n, active, cap, rule, weights_out, lw_out, bw_out); break;
-    case 4: k_kde_fit<4><<<grid, 256, 0, st>>>(X, w, n, active, cap, rule, weights_out, lw_out, bw_out); break;
-    default: return cudaErrorInvalidValue;
-    }
-    return cudaGetLastError();
+    return with_dim(dim, [&](auto d) {
+        k_kde_fit<d><<<grid, 256, 0, st>>>(X, w, n, active, cap, rule, weights_out, lw_out, bw_out);
+        return cudaGetLastError();
+    });
 }
 
 // Queries per thread for (sets, m): more queries per thread amortise the shared-memory broadcast of a point pair
@@ -74,13 +71,7 @@ static cudaError_t logprob_dim(const KdeSets& S, const float* lw, const float* x
 cudaError_t launch_kde_logprob(const KdeSets& S, const float* lw, int dim, const float* x, int64_t m, float* out, bool strict,
                                cudaStream_t st, int ksplit, float* partial)
 {
-    switch (dim) {
-    case 1: return logprob_dim<1>(S, lw, x, m, out, strict, st, ksplit, partial);
-    case 2: return logprob_dim<2>(S, lw, x, m, out, strict, st, ksplit, partial);
-    case 3: return logprob_dim<3>(S, lw, x, m, out, strict, st, ksplit, partial);
-    case 4: return logprob_dim<4>(S, lw, x, m, out, strict, st, ksplit, partial);
-    default: return cudaErrorInvalidValue;
-    }
+    return with_dim(dim, [&](auto d) { return logprob_dim<d>(S, lw, x, m, out, strict, st, ksplit, partial); });
 }
 
 cudaError_t launch_kde_cdf(const float* weights, const int32_t* n, const int32_t* active, int64_t sets, int64_t cap, double* cdf,
@@ -101,18 +92,11 @@ cudaError_t launch_kde_sample(const KdeSets& S, int dim, const double* cdf, int6
     const int64_t grid = (total + 255) / 256;
     if (grid > 0x7fffffffll) return cudaErrorInvalidValue;
     const unsigned g = static_cast<unsigned>(grid);
-#define GLABC_SAMPLE(DD)                                                                                                       \
-    k_kde_sample<DD><<<g, 256, 0, st>>>(S, cdf, m, rk, chain_id_base, round_dev, idx_tape, noise_tape, tape_set_stride,          \
-                                        tape_set_stride_noise, tape_q_stride, tape_round_stride_idx, tape_round_stride_noise, max_round, out)
-    switch (dim) {
-    case 1: GLABC_SAMPLE(1); break;
-    case 2: GLABC_SAMPLE(2); break;
-    case 3: GLABC_SAMPLE(3); break;
-    case 4: GLABC_SAMPLE(4); break;
-    default: return cudaErrorInvalidValue;
-    }
-#undef GLABC_SAMPLE
-    return cudaGetLastError();
+    return with_dim(dim, [&](auto d) {
+        k_kde_sample<d><<<g, 256, 0, st>>>(S, cdf, m, rk, chain_id_base, round_dev, idx_tape, noise_tape, tape_set_stride,
+                                           tape_set_stride_noise, tape_q_stride, tape_round_stride_idx, tape_round_stride_noise, max_round, out);
+        return cudaGetLastError();
+    });
 }
 
 }  // namespace glabc

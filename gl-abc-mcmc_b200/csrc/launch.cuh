@@ -2,9 +2,35 @@
 #pragma once
 #include <cuda_runtime.h>
 
+#include <type_traits>
+
 #include "sampler_common.cuh"
 
 namespace glabc {
+
+// The theta dimensions the kernels are instantiated for: f(std::integral_constant<int, D>{}) for D in 1..4.
+template <class F>
+cudaError_t with_dim(int dim, F&& f)
+{
+    switch (dim) {
+    case 1: return f(std::integral_constant<int, 1>{});
+    case 2: return f(std::integral_constant<int, 2>{});
+    case 3: return f(std::integral_constant<int, 3>{});
+    case 4: return f(std::integral_constant<int, 4>{});
+    }
+    return cudaErrorInvalidValue;
+}
+
+// The link of the fused model family as a compile-time constant, for the tuned kernels that read it at compile time.
+template <class F>
+cudaError_t with_family(int family, F&& f)
+{
+    switch (family) {
+    case GLABC_MODEL_ABS_NORMAL: return f(std::integral_constant<int, GLABC_MODEL_ABS_NORMAL>{});
+    case GLABC_MODEL_ID_NORMAL: return f(std::integral_constant<int, GLABC_MODEL_ID_NORMAL>{});
+    }
+    return cudaErrorInvalidValue;
+}
 
 cudaError_t launch_global_mcmc(const ModelConsts& model, const GaussConsts& lp, const GaussConsts& gp, int dim,
                                const RunParams& R, bool strict, bool replay, int layout, int block, cudaStream_t st);

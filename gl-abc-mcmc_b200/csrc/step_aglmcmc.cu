@@ -1,11 +1,11 @@
-// Orchestration of K6 (AGLMCMC): step / adapt rounds on one stream, dispatched over theta_dim and model family.
+// Orchestration of K6 (AGLMCMC): step / adapt rounds on one stream, dispatched over theta_dim.
 #include "step_aglmcmc.cuh"
 
 namespace glabc {
 
-template <int D, int FAMILY>
-static cudaError_t run_family(const AgConsts& K, const DistConsts& prior, const AgWorkspace& W, const AgTapes& T, const RunParams& R,
-                              int init, int kde_rule, bool strict, bool replay, int layout, int block, cudaStream_t st)
+template <int D>
+static cudaError_t run_aglmcmc(const AgConsts& K, const DistConsts& prior, const AgWorkspace& W, const AgTapes& T, const RunParams& R,
+                               int init, int kde_rule, bool strict, bool replay, int layout, int block, cudaStream_t st)
 {
     const bool gprior = generic_prior(prior);
     if (gprior && (strict || replay)) return cudaErrorInvalidValue;
@@ -18,8 +18,8 @@ static cudaError_t run_family(const AgConsts& K, const DistConsts& prior, const 
     cudaError_t e;
     if (init) {
         k_ag_reset<<<g_chain, 256, 0, st>>>(W, R.first_step);
-        if (replay) k_ag_block<D, FAMILY, true, true><<<g_cb, 256, 0, st>>>(K, R, W, T, prior);
-        else k_ag_block<D, FAMILY, true, false><<<g_cb, 256, 0, st>>>(K, R, W, T, prior);
+        if (replay) k_ag_block<D, true, true><<<g_cb, 256, 0, st>>>(K, R, W, T, prior);
+        else k_ag_block<D, true, false><<<g_cb, 256, 0, st>>>(K, R, W, T, prior);
         if ((e = cudaGetLastError()) != cudaSuccess) return e;
     }
     if (R.write_row0 && layout != GLABC_TRACE_NONE) k_ag_row0<D><<<g_chain, 256, 0, st>>>(R, C, layout);
@@ -28,13 +28,13 @@ static cudaError_t run_family(const AgConsts& K, const DistConsts& prior, const 
     KdeSets S{W.kde_X, W.kde_wn, W.kde_bw, W.kde_n, W.pending, C, B};
     for (int64_t r = 0; r < rounds; ++r) {
         if (gprior) {
-            k_ag_step<D, FAMILY, false, false, false, true><<<g_step, block, 0, st>>>(K, R, W, layout, prior);
+            k_ag_step<D, false, false, false, true><<<g_step, block, 0, st>>>(K, R, W, layout, prior);
         } else if (strict) {
-            if (replay) k_ag_step<D, FAMILY, true, true, false, false><<<g_step, block, 0, st>>>(K, R, W, layout, prior);
-            else k_ag_step<D, FAMILY, true, false, false, false><<<g_step, block, 0, st>>>(K, R, W, layout, prior);
+            if (replay) k_ag_step<D, true, true, false, false><<<g_step, block, 0, st>>>(K, R, W, layout, prior);
+            else k_ag_step<D, true, false, false, false><<<g_step, block, 0, st>>>(K, R, W, layout, prior);
         } else {
-            if (replay) k_ag_step<D, FAMILY, false, true, false, false><<<g_step, block, 0, st>>>(K, R, W, layout, prior);
-            else k_ag_step<D, FAMILY, false, false, false, false><<<g_step, block, 0, st>>>(K, R, W, layout, prior);
+            if (replay) k_ag_step<D, false, true, false, false><<<g_step, block, 0, st>>>(K, R, W, layout, prior);
+            else k_ag_step<D, false, false, false, false><<<g_step, block, 0, st>>>(K, R, W, layout, prior);
         }
         if ((e = cudaGetLastError()) != cudaSuccess) return e;
         if (r == rounds - 1) break;
@@ -53,52 +53,27 @@ static cudaError_t run_family(const AgConsts& K, const DistConsts& prior, const 
             k_ag_sample_filter<D><<<static_cast<unsigned>(C), 256, 0, st>>>(K, W, S, R.rk, base, prior);
         }
         if ((e = launch_kde_logprob(S, W.kde_lw, D, W.blk_theta, B, W.blk_lq, strict, st)) != cudaSuccess) return e;
-        if (replay) k_ag_block<D, FAMILY, false, true><<<g_cb, 256, 0, st>>>(K, R, W, T, prior);
-        else k_ag_block<D, FAMILY, false, false><<<g_cb, 256, 0, st>>>(K, R, W, T, prior);
+        if (replay) k_ag_block<D, false, true><<<g_cb, 256, 0, st>>>(K, R, W, T, prior);
+        else k_ag_block<D, false, false><<<g_cb, 256, 0, st>>>(K, R, W, T, prior);
         k_ag_commit<D><<<g_chain, 256, 0, st>>>(W, T);
         if ((e = cudaGetLastError()) != cudaSuccess) return e;
     }
     return cudaSuccess;
 }
 
-template <int D>
-static cudaError_t run_dim(const AgConsts& K, const DistConsts& prior, const AgWorkspace& W, const AgTapes& T, const RunParams& R,
-                           int init, int kde_rule, bool strict, bool replay, int layout, int block, cudaStream_t st)
-{
-    if (K.model.family == GLABC_MODEL_ABS_NORMAL)
-        return run_family<D, GLABC_MODEL_ABS_NORMAL>(K, prior, W, T, R, init, kde_rule, strict, replay, layout, block, st);
-    return run_family<D, GLABC_MODEL_ID_NORMAL>(K, prior, W, T, R, init, kde_rule, strict, replay, layout, block, st);
-}
-
-template <int D, int FAMILY>
-static cudaError_t block_isir_family(const AgConsts& K, const DistConsts& prior, const AgWorkspace& W, const RunParams& R, bool strict,
-                                     int layout, int block, cudaStream_t st)
-{
-    const bool gprior = generic_prior(prior);
-    if (gprior && strict) return cudaErrorInvalidValue;
-    const unsigned g_step = static_cast<unsigned>((W.C + block - 1) / block);
-    if (R.write_row0 && layout != GLABC_TRACE_NONE) k_ag_row0<D><<<static_cast<unsigned>((W.C + 255) / 256), 256, 0, st>>>(R, W.C, layout);
-    if (gprior) k_ag_step<D, FAMILY, false, false, true, true><<<g_step, block, 0, st>>>(K, R, W, layout, prior);
-    else if (strict) k_ag_step<D, FAMILY, true, false, true, false><<<g_step, block, 0, st>>>(K, R, W, layout, prior);
-    else k_ag_step<D, FAMILY, false, false, true, false><<<g_step, block, 0, st>>>(K, R, W, layout, prior);
-    return cudaGetLastError();
-}
-
 cudaError_t launch_block_isir(const AgConsts& K, const DistConsts& prior, const AgWorkspace& W, const RunParams& R, int dim, bool strict,
                               int layout, int block, cudaStream_t st)
 {
-    const bool ab = K.model.family == GLABC_MODEL_ABS_NORMAL;
-    switch (dim) {
-    case 1: return ab ? block_isir_family<1, GLABC_MODEL_ABS_NORMAL>(K, prior, W, R, strict, layout, block, st)
-                      : block_isir_family<1, GLABC_MODEL_ID_NORMAL>(K, prior, W, R, strict, layout, block, st);
-    case 2: return ab ? block_isir_family<2, GLABC_MODEL_ABS_NORMAL>(K, prior, W, R, strict, layout, block, st)
-                      : block_isir_family<2, GLABC_MODEL_ID_NORMAL>(K, prior, W, R, strict, layout, block, st);
-    case 3: return ab ? block_isir_family<3, GLABC_MODEL_ABS_NORMAL>(K, prior, W, R, strict, layout, block, st)
-                      : block_isir_family<3, GLABC_MODEL_ID_NORMAL>(K, prior, W, R, strict, layout, block, st);
-    case 4: return ab ? block_isir_family<4, GLABC_MODEL_ABS_NORMAL>(K, prior, W, R, strict, layout, block, st)
-                      : block_isir_family<4, GLABC_MODEL_ID_NORMAL>(K, prior, W, R, strict, layout, block, st);
-    default: return cudaErrorInvalidValue;
-    }
+    return with_dim(dim, [&](auto d) {
+        const bool gprior = generic_prior(prior);
+        if (gprior && strict) return cudaErrorInvalidValue;
+        const unsigned g_step = static_cast<unsigned>((W.C + block - 1) / block);
+        if (R.write_row0 && layout != GLABC_TRACE_NONE) k_ag_row0<d><<<static_cast<unsigned>((W.C + 255) / 256), 256, 0, st>>>(R, W.C, layout);
+        if (gprior) k_ag_step<d, false, false, true, true><<<g_step, block, 0, st>>>(K, R, W, layout, prior);
+        else if (strict) k_ag_step<d, true, false, true, false><<<g_step, block, 0, st>>>(K, R, W, layout, prior);
+        else k_ag_step<d, false, false, true, false><<<g_step, block, 0, st>>>(K, R, W, layout, prior);
+        return cudaGetLastError();
+    });
 }
 
 cudaError_t launch_block_weights(const AgConsts& K, const DistConsts& prior, const AgWorkspace& W, const RunParams& R, int dim,
@@ -107,31 +82,16 @@ cudaError_t launch_block_weights(const AgConsts& K, const DistConsts& prior, con
     const int64_t cb = (W.C * W.B + 255) / 256;
     if (cb > 0x7fffffffll) return cudaErrorInvalidValue;
     const unsigned g = static_cast<unsigned>(cb);
-    const bool ab = K.model.family == GLABC_MODEL_ABS_NORMAL;
-#define GLABC_BW(DD)                                                                                          \
-    if (ab) k_blk_weights<DD, GLABC_MODEL_ABS_NORMAL><<<g, 256, 0, st>>>(K, R, W, round, prior);              \
-    else k_blk_weights<DD, GLABC_MODEL_ID_NORMAL><<<g, 256, 0, st>>>(K, R, W, round, prior)
-    switch (dim) {
-    case 1: GLABC_BW(1); break;
-    case 2: GLABC_BW(2); break;
-    case 3: GLABC_BW(3); break;
-    case 4: GLABC_BW(4); break;
-    default: return cudaErrorInvalidValue;
-    }
-#undef GLABC_BW
-    return cudaGetLastError();
+    return with_dim(dim, [&](auto d) {
+        k_blk_weights<d><<<g, 256, 0, st>>>(K, R, W, round, prior);
+        return cudaGetLastError();
+    });
 }
 
 cudaError_t launch_aglmcmc(const AgConsts& K, const DistConsts& prior, const AgWorkspace& W, const AgTapes& T, const RunParams& R,
                            int dim, int init, int kde_rule, bool strict, bool replay, int layout, int block, cudaStream_t st)
 {
-    switch (dim) {
-    case 1: return run_dim<1>(K, prior, W, T, R, init, kde_rule, strict, replay, layout, block, st);
-    case 2: return run_dim<2>(K, prior, W, T, R, init, kde_rule, strict, replay, layout, block, st);
-    case 3: return run_dim<3>(K, prior, W, T, R, init, kde_rule, strict, replay, layout, block, st);
-    case 4: return run_dim<4>(K, prior, W, T, R, init, kde_rule, strict, replay, layout, block, st);
-    default: return cudaErrorInvalidValue;
-    }
+    return with_dim(dim, [&](auto d) { return run_aglmcmc<d>(K, prior, W, T, R, init, kde_rule, strict, replay, layout, block, st); });
 }
 
 }  // namespace glabc

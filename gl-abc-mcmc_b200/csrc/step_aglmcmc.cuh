@@ -74,7 +74,7 @@ __device__ __forceinline__ float model_discrepancy(const ModelConsts& m, const f
 // block construction: INIT draws theta0 / log q0 from Initial_ISIR_prop (AGLMCMC.py:84-91); both variants
 // simulate, take the discrepancy and form the weights (:94-112 / :232-249).  One thread per (chain, b).
 // ---------------------------------------------------------------------------------------------
-template <int D, int FAMILY, bool INIT, bool REPLAY>
+template <int D, bool INIT, bool REPLAY>
 __global__ void __launch_bounds__(256) k_ag_block(const __grid_constant__ AgConsts K, const __grid_constant__ RunParams R,
                                                   AgWorkspace W, AgTapes T, const __grid_constant__ DistConsts prior)
 {
@@ -386,7 +386,7 @@ __global__ void __launch_bounds__(256) k_ag_sample_filter(const __grid_constant_
 // proposal log-density of a state that changed is not recomputed here — the chain pauses (pending bit 1) and the
 // host refreshes it in one batched tensor-core log_prob launch (flow.cuh) before relaunching.
 // GPRIOR: the model's prior is `prior` (FAST arithmetic, native RNG; step_generic.cuh prior_log_prob).
-template <int D, int FAMILY, bool STRICT, bool REPLAY, bool EXT, bool GPRIOR>
+template <int D, bool STRICT, bool REPLAY, bool EXT, bool GPRIOR>
 __global__ void __launch_bounds__(128) k_ag_step(const __grid_constant__ AgConsts K, const __grid_constant__ RunParams R,
                                                  AgWorkspace W, int layout, const __grid_constant__ DistConsts prior)
 {
@@ -637,7 +637,7 @@ __global__ void __launch_bounds__(256) k_ag_row0(RunParams R, int64_t C, int lay
 
 // GLMCMC-NFs block refresh (GLMCMC_NFs.py:73-85,129-140): theta0 / log q0 come from the flow; simulate, log-kernel,
 // weights exp(prior + log K - log q0) with NaN -> 0.  One thread per (chain, b); `round` keys the simulator normals.
-template <int D, int FAMILY>
+template <int D>
 __global__ void __launch_bounds__(256) k_blk_weights(const __grid_constant__ AgConsts K, const __grid_constant__ RunParams R,
                                                      AgWorkspace W, uint32_t round, const __grid_constant__ DistConsts prior)
 {

@@ -207,7 +207,7 @@ __device__ __forceinline__ float dist_forward(const DistConsts& q, WordStream& w
 // evaluated in float32 from the rounded state (the reference's are float64 after promotion: agreement to 1e-6).
 // GPRIOR: the model's prior is `prior` (native RNG only).  Outside its support the log prior is -inf, so the first
 // candidate with a finite prior is accepted (log_acc = +inf) and one with -inf never is.
-template <int D, int FAMILY, bool REPLAY, bool GPRIOR>
+template <int D, bool REPLAY, bool GPRIOR>
 __global__ void __launch_bounds__(128) k_global_generic(const __grid_constant__ GenericConsts K, const __grid_constant__ RunParams R,
                                                         int layout, const __grid_constant__ DistConsts prior)
 {
@@ -361,7 +361,7 @@ struct IsirGenericConsts {
 // tape64 [steps][1 + K D][C] = the numpy resampling uniform, then the proposal's own draws (theta_j; local: increment z).
 // GPRIOR: the model's prior is `prior` (native RNG only), as in k_global_generic; a candidate outside its support has
 // log-weight -inf, i.e. weight 0, and is never selected.
-template <int D, int FAMILY, bool REPLAY, bool GPRIOR>
+template <int D, bool REPLAY, bool GPRIOR>
 __global__ void __launch_bounds__(128) k_isir_generic(const __grid_constant__ IsirGenericConsts K, const __grid_constant__ RunParams R,
                                                       int layout, const __grid_constant__ DistConsts prior)
 {

@@ -12,13 +12,7 @@ extern template cudaError_t launch_global_mcmc_dim<4>(const ModelConsts&, const 
 cudaError_t launch_global_mcmc(const ModelConsts& model, const GaussConsts& lp, const GaussConsts& gp, int dim,
                                const RunParams& R, bool strict, bool replay, int layout, int block, cudaStream_t st)
 {
-    switch (dim) {
-    case 1: return launch_global_mcmc_dim<1>(model, lp, gp, R, strict, replay, layout, block, st);
-    case 2: return launch_global_mcmc_dim<2>(model, lp, gp, R, strict, replay, layout, block, st);
-    case 3: return launch_global_mcmc_dim<3>(model, lp, gp, R, strict, replay, layout, block, st);
-    case 4: return launch_global_mcmc_dim<4>(model, lp, gp, R, strict, replay, layout, block, st);
-    default: return cudaErrorInvalidValue;
-    }
+    return with_dim(dim, [&](auto d) { return launch_global_mcmc_dim<d>(model, lp, gp, R, strict, replay, layout, block, st); });
 }
 
 }  // namespace glabc

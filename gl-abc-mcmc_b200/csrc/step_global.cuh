@@ -375,12 +375,10 @@ cudaError_t launch_global_mcmc_dim(const ModelConsts& model, const GaussConsts& 
                                    const RunParams& R, bool strict, bool replay, int layout, int block, cudaStream_t st)
 {
     GlobalConsts K{model, lp, gp};
-    if (model.family == GLABC_MODEL_ABS_NORMAL) {
-        return strict ? launch_mode<D, GLABC_MODEL_ABS_NORMAL, true>(K, R, replay, layout, block, st)
-                      : launch_mode<D, GLABC_MODEL_ABS_NORMAL, false>(K, R, replay, layout, block, st);
-    }
-    return strict ? launch_mode<D, GLABC_MODEL_ID_NORMAL, true>(K, R, replay, layout, block, st)
-                  : launch_mode<D, GLABC_MODEL_ID_NORMAL, false>(K, R, replay, layout, block, st);
+    return with_family(model.family, [&](auto f) {
+        return strict ? launch_mode<D, f, true>(K, R, replay, layout, block, st)
+                      : launch_mode<D, f, false>(K, R, replay, layout, block, st);
+    });
 }
 
 }  // namespace glabc

@@ -12,13 +12,7 @@ extern template cudaError_t launch_isir_dim<4>(const ModelConsts&, const GaussCo
 cudaError_t launch_isir(const ModelConsts& model, const GaussConsts& lp, const GaussConsts& ip, int dim, const RunParams& R,
                         bool strict, bool replay, int layout, int block, cudaStream_t st)
 {
-    switch (dim) {
-    case 1: return launch_isir_dim<1>(model, lp, ip, R, strict, replay, layout, block, st);
-    case 2: return launch_isir_dim<2>(model, lp, ip, R, strict, replay, layout, block, st);
-    case 3: return launch_isir_dim<3>(model, lp, ip, R, strict, replay, layout, block, st);
-    case 4: return launch_isir_dim<4>(model, lp, ip, R, strict, replay, layout, block, st);
-    default: return cudaErrorInvalidValue;
-    }
+    return with_dim(dim, [&](auto d) { return launch_isir_dim<d>(model, lp, ip, R, strict, replay, layout, block, st); });
 }
 
 }  // namespace glabc

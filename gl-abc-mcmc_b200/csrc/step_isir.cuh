@@ -620,12 +620,10 @@ cudaError_t launch_isir_dim(const ModelConsts& model, const GaussConsts& lp, con
                             bool strict, bool replay, int layout, int block, cudaStream_t st)
 {
     IsirConsts K{model, lp, ip};
-    if (model.family == GLABC_MODEL_ABS_NORMAL) {
-        return strict ? launch_isir_mode<D, GLABC_MODEL_ABS_NORMAL, true>(K, R, replay, layout, block, st)
-                      : launch_isir_mode<D, GLABC_MODEL_ABS_NORMAL, false>(K, R, replay, layout, block, st);
-    }
-    return strict ? launch_isir_mode<D, GLABC_MODEL_ID_NORMAL, true>(K, R, replay, layout, block, st)
-                  : launch_isir_mode<D, GLABC_MODEL_ID_NORMAL, false>(K, R, replay, layout, block, st);
+    return with_family(model.family, [&](auto f) {
+        return strict ? launch_isir_mode<D, f, true>(K, R, replay, layout, block, st)
+                      : launch_isir_mode<D, f, false>(K, R, replay, layout, block, st);
+    });
 }
 
 }  // namespace glabc

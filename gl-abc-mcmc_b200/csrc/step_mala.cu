@@ -12,13 +12,7 @@ extern template cudaError_t launch_mala_dim<4>(const MalaConsts&, const DistCons
 cudaError_t launch_mala(const MalaConsts& K, const DistConsts& prior, int dim, const RunParams& R, bool strict, bool replay, int block,
                         cudaStream_t st)
 {
-    switch (dim) {
-    case 1: return launch_mala_dim<1>(K, prior, R, strict, replay, block, st);
-    case 2: return launch_mala_dim<2>(K, prior, R, strict, replay, block, st);
-    case 3: return launch_mala_dim<3>(K, prior, R, strict, replay, block, st);
-    case 4: return launch_mala_dim<4>(K, prior, R, strict, replay, block, st);
-    default: return cudaErrorInvalidValue;
-    }
+    return with_dim(dim, [&](auto d) { return launch_mala_dim<d>(K, prior, R, strict, replay, block, st); });
 }
 
 }  // namespace glabc

@@ -920,9 +920,7 @@ template <int D>
 cudaError_t launch_mala_dim(const MalaConsts& K, const DistConsts& prior, const RunParams& R, bool strict, bool replay, int block,
                             cudaStream_t st)
 {
-    if (K.model.family == GLABC_MODEL_ABS_NORMAL)
-        return launch_mala_family<D, GLABC_MODEL_ABS_NORMAL>(K, prior, R, strict, replay, block, st);
-    return launch_mala_family<D, GLABC_MODEL_ID_NORMAL>(K, prior, R, strict, replay, block, st);
+    return with_family(K.model.family, [&](auto f) { return launch_mala_family<D, f>(K, prior, R, strict, replay, block, st); });
 }
 
 }  // namespace glabc

@@ -161,24 +161,20 @@ __device__ __forceinline__ void gradient_from_sums(const MalaConsts& K, const Di
     }
 }
 
-// CPW = chains per warp: 32, or 16 when there are too few chains to occupy the schedulers (lanes 16..31 then only help with
-// the gradients: the thread-per-chain phases cost twice the issue slots per chain, the gradients — 80 % of the work — the
-// same, and twice as many warps hide the latency of the Philox / MUFU chains).  The chain-major trace tile needs 32.
 // GIP: the Importance_Proposal is one of the non-Gaussian classes (K.ipg, step_generic.cuh): candidate j of a step is
 // dist_forward over the word stream of Philox slots kSlotGeneric + 64 j .., its simulator normals follow in the same stream.
 // GPRIOR: the model's prior is `prior` (step_generic.cuh prior_log_prob) in the iSIR weights, the MALA target and the
 // finite-difference prior gradient.
-template <int D, int FAMILY, int LAYOUT, int CPW, bool GIP, bool GPRIOR>
+template <int D, int FAMILY, int LAYOUT, bool GIP, bool GPRIOR>
 __global__ void __launch_bounds__(GLABC_MALA_BLOCK) k_mala_fast(const __grid_constant__ MalaConsts K, const __grid_constant__ RunParams R,
                                                                 const __grid_constant__ DistConsts prior)
 {
     using Writer = typename WriterFor<D, LAYOUT>::type;
-    static_assert(CPW == 32 || LAYOUT != GLABC_TRACE_CHAIN_MAJOR, "the chain-major tile stages 32 chains per warp");
     extern __shared__ float smem[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int32_t warp_chain0 = static_cast<int32_t>((blockIdx.x * blockDim.x + threadIdx.x) >> 5) * CPW;
+    const int32_t warp_chain0 = static_cast<int32_t>((blockIdx.x * blockDim.x + threadIdx.x) >> 5) * 32;
     const int32_t chain = warp_chain0 + lane;
-    const bool active = lane < CPW && chain < R.n_chains;
+    const bool active = chain < R.n_chains;
     const int32_t cidx = active ? chain : R.n_chains - 1;   // tail lanes read a valid chain and never write
     const int NK = R.n_candidates;
     constexpr int kGroups = (2 * D + 3) / 4;
@@ -425,42 +421,25 @@ GLABC_UNROLL(GLABC_MALA_KUNROLL)
     }
 }
 
-template <int D, int FAMILY, int LAYOUT, int CPW, bool GIP>
+template <int D, int FAMILY, int LAYOUT, bool GIP>
 static void launch_mala_fast_gip(const MalaConsts& K, const DistConsts& prior, const RunParams& R, int grid, int block, size_t smem,
                                  cudaStream_t st)
 {
-    if (generic_prior(prior)) k_mala_fast<D, FAMILY, LAYOUT, CPW, GIP, true><<<grid, block, smem, st>>>(K, R, prior);
-    else k_mala_fast<D, FAMILY, LAYOUT, CPW, GIP, false><<<grid, block, smem, st>>>(K, R, prior);
-}
-
-template <int D, int FAMILY, int LAYOUT, int CPW>
-static cudaError_t launch_mala_fast_cpw(const MalaConsts& K, const DistConsts& prior, const RunParams& R, cudaStream_t st)
-{
-    using Writer = typename WriterFor<D, LAYOUT>::type;
-    constexpr int block = GLABC_MALA_BLOCK;
-    constexpr int chains_per_block = block / 32 * CPW;
-    const int grid = (R.n_chains + chains_per_block - 1) / chains_per_block;
-    const size_t smem = sizeof(float) * (static_cast<size_t>(Writer::smem_floats_per_warp) * (block / 32) +
-                                         static_cast<size_t>(R.n_candidates) * block);
-    if (K.ip_generic) launch_mala_fast_gip<D, FAMILY, LAYOUT, CPW, true>(K, prior, R, grid, block, smem, st);
-    else launch_mala_fast_gip<D, FAMILY, LAYOUT, CPW, false>(K, prior, R, grid, block, smem, st);
-    return cudaGetLastError();
+    if (generic_prior(prior)) k_mala_fast<D, FAMILY, LAYOUT, GIP, true><<<grid, block, smem, st>>>(K, R, prior);
+    else k_mala_fast<D, FAMILY, LAYOUT, GIP, false><<<grid, block, smem, st>>>(K, R, prior);
 }
 
 template <int D, int FAMILY, int LAYOUT>
 static cudaError_t launch_mala_fast_one(const MalaConsts& K, const DistConsts& prior, const RunParams& R, cudaStream_t st)
 {
-    // Measured and rejected (DESIGN.md K3): pooling the 4 left-over blocks per gradient (100 blocks on 32 lanes) of all pending
-    // chains into one joint round — 3 n + 1 rounds instead of 4 n — ran 11.96 ms instead of 9.78 ms at 32,768 chains and 61.5
-    // instead of 50.5 ms at 262,144: the second code path (per-lane owner lookup, hand-over shuffles) costs more instruction
-    // fetch and issue than the nearly empty fourth round it removes.
-    // CPW = 16 (twice the warps for the same chains) was measured at 32,768 chains, where only 1.7 warps sit on a scheduler:
-    // issue-active rose from 47 % to 63 % but the warp-instructions per chain-step rose from 152 to 193 — the same 9.85 ms
-    // (profiles/r2_k3_mala_fast_ncu.md).  Kept behind a build flag for other shapes.
-#if defined(GLABC_MALA_FORCE_CPW) && GLABC_MALA_FORCE_CPW == 16
-    if constexpr (LAYOUT != GLABC_TRACE_CHAIN_MAJOR) return launch_mala_fast_cpw<D, FAMILY, LAYOUT, 16>(K, prior, R, st);
-#endif
-    return launch_mala_fast_cpw<D, FAMILY, LAYOUT, 32>(K, prior, R, st);
+    using Writer = typename WriterFor<D, LAYOUT>::type;
+    constexpr int block = GLABC_MALA_BLOCK;   // one chain per thread
+    const int grid = (R.n_chains + block - 1) / block;
+    const size_t smem = sizeof(float) * (static_cast<size_t>(Writer::smem_floats_per_warp) * (block / 32) +
+                                         static_cast<size_t>(R.n_candidates) * block);
+    if (K.ip_generic) launch_mala_fast_gip<D, FAMILY, LAYOUT, true>(K, prior, R, grid, block, smem, st);
+    else launch_mala_fast_gip<D, FAMILY, LAYOUT, false>(K, prior, R, grid, block, smem, st);
+    return cudaGetLastError();
 }
 
 template <int D, int FAMILY>

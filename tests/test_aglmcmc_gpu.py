@@ -150,16 +150,14 @@ def test_aglmcmc_replay_golden(eng, ci):
         assert rel_max(rec_f[:n, 0], case["ad_rec"][:n, 0]) < 1e-4
 
 
-def readme_setup(eng):
+def readme_setup(eng, family=abi.MODEL_ABS_NORMAL):
     case = load_cases("aglmcmc.npz")[0]
-    bind(eng, model_pod(case), gauss_pod(case, "lp"), gauss_pod(case, "ip"))
+    bind(eng, model_pod(case, family), gauss_pod(case, "lp"), gauss_pod(case, "ip"))
     return case
 
 
-def test_aglmcmc_native_matches_oracle(eng):
-    """native Philox mode, strict arithmetic, gf < 1 (chains pause at different iterations): the kernels and the
-    oracle draw the same streams; decisions agree except where MUFU-vs-libm normals differ in the last bits"""
-    case = readme_setup(eng)
+def check_native_matches_oracle(eng, family):
+    case = readme_setup(eng, family)
     Cn, T, d, K, S = 64, 300, 2, 4, 20
     theta0 = np.zeros((Cn, d), np.float32)
     y0 = (np.random.default_rng(1).standard_normal((Cn, d)) * 0.2236).astype(np.float32)
@@ -170,12 +168,23 @@ def test_aglmcmc_native_matches_oracle(eng):
                   trace_layout=abi.TRACE_TIME_MAJOR, K=K, ag=ag, stats=st).cpu().numpy()
     th_o, y_o = theta0.copy(), y0.copy()
     st_o = np.zeros((Cn, abi.nstats(d)), np.float32)
-    want = oracle.run("aglmcmc", model_pod(case), gauss_pod(case, "lp"), gauss_pod(case, "ip"), theta=th_o, y=y_o, n_steps=T,
+    want = oracle.run("aglmcmc", model_pod(case, family), gauss_pod(case, "lp"), gauss_pod(case, "ip"), theta=th_o, y=y_o, n_steps=T,
                       gf=0.8, seed=9, chain_id_base=5, K=K, stats=st_o, ag=oracle.aglmcmc_params(S=S, alpha=0.8, hat_eps_T=0.2))
     assert np.array_equal(st.cpu().numpy()[:, abi.STAT_GLOBAL_STEPS], st_o[:, abi.STAT_GLOBAL_STEPS])   # same branch coins
     close = np.isclose(got, want, rtol=1e-4, atol=1e-4).all(-1)
     assert close[:40].mean() > 0.99          # identical until approximate-vs-libm normals flip a decision somewhere
     assert close.mean() > 0.7
+
+
+def test_aglmcmc_native_matches_oracle(eng):
+    """native Philox mode, strict arithmetic, gf < 1 (chains pause at different iterations): the kernels and the
+    oracle draw the same streams; decisions agree except where MUFU-vs-libm normals differ in the last bits"""
+    check_native_matches_oracle(eng, abi.MODEL_ABS_NORMAL)
+
+
+def test_aglmcmc_native_matches_oracle_identity_link(eng):
+    """the same with the identity link, which the AGLMCMC kernels choose at run time (model_simulate)"""
+    check_native_matches_oracle(eng, abi.MODEL_ID_NORMAL)
 
 
 def test_aglmcmc_invariances(eng):
