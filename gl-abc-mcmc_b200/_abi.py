@@ -148,6 +148,7 @@ _SIGNATURES = {
     "glabc_run_isir_user": (C.c_int, [C.c_void_p, C.POINTER(RunPOD), C.POINTER(UserModelPOD)]),
     "glabc_run_mala_user": (C.c_int, [C.c_void_p, C.POINTER(RunPOD), C.POINTER(UserModelPOD)]),
     "glabc_user_model_check": (C.c_int, [C.POINTER(UserModelPOD), C.c_int32, C.c_char_p, C.c_size_t]),
+    "glabc_user_model_check_proposals": (C.c_int, [C.POINTER(UserModelPOD), C.c_int32, C.c_int32, C.c_int32, C.c_char_p, C.c_size_t]),
     "glabc_run_global_host": (C.c_int, [C.c_void_p, C.POINTER(RunPOD), C.c_int64]),
     "glabc_run_isir": (C.c_int, [C.c_void_p, C.POINTER(RunPOD)]),
     "glabc_run_isir_host": (C.c_int, [C.c_void_p, C.POINTER(RunPOD), C.c_int64]),

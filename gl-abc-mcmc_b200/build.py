@@ -34,6 +34,20 @@ def _deps():
            [os.path.join(ROOT, "include", "glabc.h")]
 
 
+def _embed_dist_device():
+    """csrc/dist_device_src.inc: the text of dist_device.cuh as a C++ raw string literal.  user_model.cu hands it to
+    NVRTC as a named header, so the user-model kernels compile the same distribution code as the built-in ones and the
+    library needs no file of the tree at run time."""
+    with open(os.path.join(CSRC, "dist_device.cuh")) as f:
+        text = f.read()
+    assert ')GLABC_DIST"' not in text
+    out = os.path.join(CSRC, "dist_device_src.inc")
+    body = 'R"GLABC_DIST(' + text + ')GLABC_DIST"\n'
+    if not os.path.exists(out) or open(out).read() != body:
+        with open(out, "w") as f:
+            f.write(body)
+
+
 def build(force=False, verbose=False, variant=None, extra_flags=()):
     """`variant` builds csrc/libglabc.<variant>.so with `extra_flags` (kernel experiments; select it
     at run time with GLABC_LIB=<path>)."""
@@ -42,6 +56,7 @@ def build(force=False, verbose=False, variant=None, extra_flags=()):
     if not force and os.path.exists(lib_path) and os.path.getmtime(lib_path) >= newest:
         return lib_path
     nvcc = _nvcc()
+    _embed_dist_device()
     logs = {}
     tag = "" if variant is None else "." + variant
 

@@ -221,7 +221,7 @@ static int check_dist(glabc_ctx* ctx, const char* who, const glabc_dist_t* dist,
 {
     if (!dist || nbytes != sizeof(glabc_dist_t))
         return fail(ctx, GLABC_ERR_INVALID, "%s: struct size %zu, expected %zu (ABI mismatch)", who, nbytes, sizeof(glabc_dist_t));
-    if (dist->dim < 1 || dist->dim > 4) return fail(ctx, GLABC_ERR_UNSUPPORTED, "%s: dim %d outside 1..4", who, dist->dim);
+    if (dist->dim < 1 || dist->dim > GLABC_MAX_DIM) return fail(ctx, GLABC_ERR_UNSUPPORTED, "%s: dim %d outside 1..%d", who, dist->dim, GLABC_MAX_DIM);
     switch (dist->kind) {
     case GLABC_DIST_DIAG_GAUSSIAN:
         for (int i = 0; i < dist->dim; ++i)
@@ -244,6 +244,15 @@ static int check_dist(glabc_ctx* ctx, const char* who, const glabc_dist_t* dist,
     default:
         return fail(ctx, GLABC_ERR_UNSUPPORTED, "unknown distribution kind %d", dist->kind);
     }
+    return GLABC_OK;
+}
+
+// The built-in kernels take distributions of dim <= kGenMaxDim (DistConsts); only the user-model kernels take wider ones
+static int check_builtin_dim(glabc_ctx* ctx, const char* who, const glabc_dist_t& dist)
+{
+    if (dist.dim > kGenMaxDim)
+        return fail(ctx, GLABC_ERR_UNSUPPORTED, "%s: a distribution of dim %d; the built-in kernels take dim 1..%d (user models up to %d)", who,
+                    dist.dim, kGenMaxDim, GLABC_MAX_DIM);
     return GLABC_OK;
 }
 
@@ -270,6 +279,7 @@ int glabc_model_prior_set(glabc_ctx* ctx, const glabc_dist_t* prior, size_t nbyt
         ctx->has_prior = false;
         return GLABC_OK;
     }
+    if (nbytes == sizeof(glabc_dist_t) && check_builtin_dim(ctx, "glabc_model_prior_set", *prior)) return GLABC_ERR_UNSUPPORTED;
     if (nbytes == sizeof(glabc_dist_t) && prior->dim != m.theta_dim)
         return fail(ctx, GLABC_ERR_INVALID, "glabc_model_prior_set: prior dim %d does not match theta_dim %d", prior->dim, m.theta_dim);
     const int st = check_dist(ctx, "glabc_model_prior_set", prior, nbytes);
@@ -312,15 +322,17 @@ static GaussConsts make_gauss(const float* loc, const float* log_scale, const fl
     return g;
 }
 
-// glabc_dist_t -> constants of the general-proposal kernel (step_generic.cuh)
-static DistConsts make_dist(const glabc_dist_t& p)
+// glabc_dist_t -> constants of a kernel that takes distributions of dim <= MAXD (dist_device.cuh): DistConsts for the
+// built-in kernels, DistConstsT<GLABC_MAX_DIM> for the user-model kernels
+template <int MAXD = kGenMaxDim>
+static DistConstsT<MAXD> make_dist(const glabc_dist_t& p)
 {
-    DistConsts q{};
+    DistConstsT<MAXD> q{};
     q.kind = p.kind;
     q.dim = p.dim;
     q.n_modes = p.n_modes;
     q.half_log_2pi = half_log_2pi(p.dim);
-    for (int i = 0; i < p.dim && i < kGenMaxDim; ++i) {
+    for (int i = 0; i < p.dim && i < MAXD; ++i) {
         q.a[i] = p.a[i];
         q.b[i] = p.b[i];
         q.c[i] = p.c[i];
@@ -331,7 +343,7 @@ static DistConsts make_dist(const glabc_dist_t& p)
         double run = 0.0;
         for (int m = 0; m < p.n_modes; ++m) {
             double sls = 0.0;
-            for (int i = 0; i < p.dim && i < kGenMaxDim; ++i) {
+            for (int i = 0; i < p.dim && i < MAXD; ++i) {
                 q.mix_loc[m][i] = p.mix_loc[m][i];
                 q.mix_scale[m][i] = p.mix_scale[m][i];
                 q.mix_inv_scale[m][i] = 1.0f / p.mix_scale[m][i];
@@ -1316,6 +1328,7 @@ extern "C" int glabc_dist_log_prob(glabc_ctx* ctx, int slot, const float* z, int
 {
     if (!ctx) return GLABC_ERR_INVALID;
     if (slot < 0 || slot >= GLABC_SLOT_COUNT || !ctx->has_dist[slot]) return fail(ctx, GLABC_ERR_INVALID, "glabc_dist_log_prob: slot %d is not bound", slot);
+    if (check_builtin_dim(ctx, "glabc_dist_log_prob", ctx->dist[slot])) return GLABC_ERR_UNSUPPORTED;
     if (!z || !log_p || n < 0) return fail(ctx, GLABC_ERR_INVALID, "glabc_dist_log_prob: null pointer / bad n");
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     const RoundKeys rk = expand_key(make_uint2(0u, 0u));
@@ -1327,6 +1340,7 @@ extern "C" int glabc_dist_sample(glabc_ctx* ctx, int slot, int64_t n, uint64_t s
 {
     if (!ctx) return GLABC_ERR_INVALID;
     if (slot < 0 || slot >= GLABC_SLOT_COUNT || !ctx->has_dist[slot]) return fail(ctx, GLABC_ERR_INVALID, "glabc_dist_sample: slot %d is not bound", slot);
+    if (check_builtin_dim(ctx, "glabc_dist_sample", ctx->dist[slot])) return GLABC_ERR_UNSUPPORTED;
     if (!z || n < 0) return fail(ctx, GLABC_ERR_INVALID, "glabc_dist_sample: null pointer / bad n");
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     const RoundKeys rk = expand_key(make_uint2(static_cast<uint32_t>(seed), static_cast<uint32_t>(seed >> 32)));
@@ -1337,20 +1351,28 @@ extern "C" int glabc_dist_sample(glabc_ctx* ctx, int slot, int64_t n, uint64_t s
 // ---------------------------------------------------------------------------------------------
 // GlobalMCMC with a user-supplied model compiled at run time (user_model.cu)
 // ---------------------------------------------------------------------------------------------
-extern "C" int glabc_user_model_check(const glabc_user_model_t* um, int32_t cc, char* log, size_t log_cap)
+static bool valid_dist_kind(int kind) { return kind >= GLABC_DIST_DIAG_GAUSSIAN && kind <= GLABC_DIST_GAUSSIAN_MIXTURE; }
+
+extern "C" int glabc_user_model_check_proposals(const glabc_user_model_t* um, int32_t local_kind, int32_t far_kind, int32_t cc, char* log,
+                                                size_t log_cap)
 {
     if (log && log_cap) log[0] = '\0';
     if (!um || !um->source) return GLABC_ERR_INVALID;
     if (um->theta_dim < 1 || um->theta_dim > GLABC_MAX_DIM || um->y_dim < 1 || um->y_dim > 2 * GLABC_MAX_DIM || um->n_noise < 0 ||
-        um->n_noise > GLABC_USER_MAX_NOISE)
+        um->n_noise > GLABC_USER_MAX_NOISE || !valid_dist_kind(local_kind) || !valid_dist_kind(far_kind))
         return GLABC_ERR_INVALID;
     std::string err;
-    const int st = user_model_check(cc, *um, err);
+    const int st = user_model_check(cc, *um, local_kind, far_kind, err);
     if (log && log_cap) {
         strncpy(log, err.c_str(), log_cap - 1);
         log[log_cap - 1] = '\0';
     }
     return st;
+}
+
+extern "C" int glabc_user_model_check(const glabc_user_model_t* um, int32_t cc, char* log, size_t log_cap)
+{
+    return glabc_user_model_check_proposals(um, GLABC_DIST_DIAG_GAUSSIAN, GLABC_DIST_DIAG_GAUSSIAN, cc, log, log_cap);
 }
 
 static int run_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_user_model_t* um, int kind)
@@ -1369,8 +1391,6 @@ static int run_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_user_mod
         if (!ctx->has_dist[slot])
             return fail(ctx, GLABC_ERR_INVALID, "%s needs the %s%s proposal slot(s) bound", mala ? "glabc_run_mala_user" : isir ? "glabc_run_isir_user" : "glabc_run_global_user",
                         mala ? "" : "LOCAL and ", isir ? "IMPORTANCE" : "GLOBAL");
-        if (ctx->dist[slot].kind != GLABC_DIST_DIAG_GAUSSIAN)
-            return fail(ctx, GLABC_ERR_UNSUPPORTED, "the user-model kernels are fused for DiagGaussian proposals");
         if (ctx->dist[slot].dim != d) return fail(ctx, GLABC_ERR_INVALID, "proposal dim does not match the user model's theta_dim %d", d);
     }
     if (isir) {
@@ -1393,7 +1413,11 @@ static int run_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_user_mod
     CUDA_TRY(ctx, cudaFree(nullptr));   // make sure the primary context exists and is current for the driver calls
     void* fn = nullptr;
     std::string err;
-    st = user_model_compile(ctx->device, ctx->cc, *um, kind, &fn, err);
+    const glabc_dist_t& lp = ctx->dist[mala ? far_slot : GLABC_SLOT_LOCAL];   // GLMALA has no Local_Proposal
+    const glabc_dist_t& gp = ctx->dist[far_slot];
+    // the kinds are compiled in; GLMALA reads only the IMPORTANCE slot, so its module takes the Gaussian local path
+    const int lp_kind = mala ? GLABC_DIST_DIAG_GAUSSIAN : lp.kind;
+    st = user_model_compile(ctx->device, ctx->cc, *um, lp_kind, gp.kind, kind, &fn, err);
     if (st) return fail(ctx, st, "%s", err.c_str());
     UserRun U{};
     U.n_chains = R.n_chains;
@@ -1416,8 +1440,6 @@ static int run_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_user_mod
     U.y = R.y;
     U.trace = R.trace;
     U.stats = R.stats;
-    const glabc_dist_t& lp = ctx->dist[mala ? far_slot : GLABC_SLOT_LOCAL];   // GLMALA has no Local_Proposal
-    const glabc_dist_t& gp = ctx->dist[far_slot];
     if (mala) {
         U.tau = run->tau;
         U.eps2 = static_cast<float>(um->epsilon * um->epsilon);
@@ -1426,12 +1448,18 @@ static int run_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_user_mod
     U.aux = isir ? run->aux : nullptr;
     U.n_candidates = isir ? run->n_candidates : 0;
     for (int k = 0; k < d; ++k) {   // glabc_dist_t DiagGaussian: a = loc, b = log_scale, c = exp(log_scale) in float32
-        U.lp_loc[k] = lp.a[k];
-        U.lp_scale[k] = lp.c[k];
-        U.gp_loc[k] = gp.a[k];
-        U.gp_scale[k] = gp.c[k];
-        U.gp_inv_scale[k] = 1.0f / gp.c[k];
+        if (lp.kind == GLABC_DIST_DIAG_GAUSSIAN) {
+            U.lp_loc[k] = lp.a[k];
+            U.lp_scale[k] = lp.c[k];
+        }
+        if (gp.kind == GLABC_DIST_DIAG_GAUSSIAN) {
+            U.gp_loc[k] = gp.a[k];
+            U.gp_scale[k] = gp.c[k];
+            U.gp_inv_scale[k] = 1.0f / gp.c[k];
+        }
     }
+    U.lq = make_dist<GLABC_MAX_DIM>(lp);   // read by the kernels compiled for a Uniform / Gamma / GaussianMixture slot
+    U.gq = make_dist<GLABC_MAX_DIM>(gp);
     const float eps = static_cast<float>(um->epsilon);
     U.kern_c = static_cast<float>(-0.5 * std::log(2.0 * M_PI)) - std::log(eps);
     U.kern_m = -0.5f / (eps * eps);

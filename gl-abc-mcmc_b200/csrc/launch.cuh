@@ -39,7 +39,9 @@ cudaError_t launch_isir(const ModelConsts& model, const GaussConsts& lp, const G
                         bool strict, bool replay, int layout, int block, cudaStream_t st);
 
 struct MalaConsts;
-struct DistConsts;
+template <int MAXD>
+struct DistConstsT;
+using DistConsts = DistConstsT<4>;   // dist_device.cuh; the built-in kernels take distributions of dim <= 4
 // `prior`: a Uniform / Gamma / GaussianMixture prior of the model (FAST, native RNG) or GLABC_DIST_DIAG_GAUSSIAN for K.model's
 cudaError_t launch_mala(const MalaConsts& K, const DistConsts& prior, int dim, const RunParams& R, bool strict, bool replay, int block,
                         cudaStream_t st);

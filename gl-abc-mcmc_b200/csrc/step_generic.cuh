@@ -1,29 +1,17 @@
-// Device versions of the reference's proposal distributions (distribution.py: Uniform :50-86, Gamma :90-137,
-// DiagGaussian :143-181, GaussianMixture :206-293) and the GlobalMCMC step (GlobalMCMC.py:37-68) for ANY of them in the
+// The GlobalMCMC step (GlobalMCMC.py:37-68) for ANY of the reference's proposal distributions (dist_device.cuh) in the
 // Local_Proposal / Global_Proposal slots.  K1 (step_global.cuh) is the tuned kernel for the all-Gaussian case; this is
 // the general one: one thread = one chain, native Philox RNG, float32 (the reference evaluates Gamma / GaussianMixture
 // in float64 — agreement is to float32 rounding, checked against the reference's recorded log-densities).
-//   Uniform          z = low + (high - low) * U                         log p = -log prod(high - low), -inf outside
-//   Gamma            Marsaglia-Tsang squeeze per coordinate (+ the U^(1/a) boost for shape < 1)
-//                                                                        log p = sum a log b - lgamma(a) + (a-1) log z - b z
-//   GaussianMixture  mode by inverse CDF of the soft-maxed weights, then a diagonal Gaussian; log p = logsumexp over modes
 #pragma once
 #include "launch.cuh"
 #include "sampler_common.cuh"
+#include "dist_device.cuh"
 
 namespace glabc {
 
 constexpr int kGenMaxDim = 4;
 
-struct DistConsts {
-    int32_t kind, dim, n_modes;
-    float a[kGenMaxDim], b[kGenMaxDim], c[kGenMaxDim];  // Gauss: loc, log_scale, scale; Uniform: low, high, c[0] = log p;
-                                                        // Gamma: shape, rate, c = a log b - lgamma(a)
-    float half_log_2pi;                                 // float32(-0.5 d log 2 pi)
-    float mix_loc[GLABC_MAX_MODES][kGenMaxDim], mix_inv_scale[GLABC_MAX_MODES][kGenMaxDim], mix_scale[GLABC_MAX_MODES][kGenMaxDim];
-    float mix_c[GLABC_MAX_MODES];    // -0.5 d log 2 pi + log w_m - sum log_scale_m
-    float mix_cdf[GLABC_MAX_MODES];  // inclusive prefix sums of the weights
-};
+using DistConsts = DistConstsT<kGenMaxDim>;
 
 struct GenericConsts {
     ModelConsts model;
@@ -70,58 +58,6 @@ struct WordStream {
     }
 };
 
-template <int D>
-__device__ __forceinline__ float dist_log_prob(const DistConsts& q, const float (&z)[D])
-{
-    switch (q.kind) {
-    case GLABC_DIST_DIAG_GAUSSIAN: {
-        float s = 0.0f;
-#pragma unroll
-        for (int i = 0; i < D; ++i) {
-            const float r = (z[i] - q.a[i]) / q.c[i];
-            s += q.b[i] + 0.5f * (r * r);
-        }
-        return q.half_log_2pi - s;
-    }
-    case GLABC_DIST_UNIFORM: {
-        bool out = false;
-#pragma unroll
-        for (int i = 0; i < D; ++i) out |= (z[i] < q.a[i]) || (z[i] > q.b[i]);  // distribution.py:82-85
-        return out ? -INFINITY : q.c[0];
-    }
-    case GLABC_DIST_GAMMA: {
-        float s = 0.0f;
-#pragma unroll
-        for (int i = 0; i < D; ++i) {
-            float lp;
-            if (z[i] > 0.0f) lp = q.c[i] + (q.a[i] - 1.0f) * logf(z[i]) - q.b[i] * z[i];
-            else if (z[i] == 0.0f && q.a[i] == 1.0f) lp = q.c[i];   // pdf(0) = b for shape 1
-            else lp = -INFINITY;                                     // pdf == 0 -> -inf, distribution.py:133-136
-            s += lp;
-        }
-        return s;
-    }
-    case GLABC_DIST_GAUSSIAN_MIXTURE: {
-        float t[GLABC_MAX_MODES], mx = -INFINITY;
-        for (int m = 0; m < q.n_modes; ++m) {
-            float s = 0.0f;
-#pragma unroll
-            for (int i = 0; i < D; ++i) {
-                const float r = (z[i] - q.mix_loc[m][i]) * q.mix_inv_scale[m][i];
-                s = fmaf(r, r, s);
-            }
-            t[m] = fmaf(-0.5f, s, q.mix_c[m]);  // distribution.py:283-288
-            mx = fmaxf(mx, t[m]);
-        }
-        if (mx == -INFINITY) return -INFINITY;
-        float acc = 0.0f;
-        for (int m = 0; m < q.n_modes; ++m) acc += expf(t[m] - mx);
-        return mx + logf(acc);
-    }
-    }
-    return NAN;
-}
-
 // The model's prior.  A DiagGaussian prior lives in ModelConsts (model_prior, the tuned arithmetic of both modes); a
 // Uniform / Gamma / GaussianMixture one bound with glabc_model_prior_set arrives as a DistConsts and is evaluated by
 // dist_log_prob (FAST only): GPRIOR kernels are instantiated for that case.  The kernels that run once per adaptation
@@ -139,63 +75,6 @@ template <int D>
 __device__ __forceinline__ float prior_log_prob_rt(const ModelConsts& m, const DistConsts& prior, const float (&theta)[D])
 {
     return generic_prior(prior) ? dist_log_prob<D>(prior, theta) : model_prior<D, true>(m, theta);
-}
-
-// forward(): one draw and its log-density
-template <int D>
-__device__ __forceinline__ float dist_forward(const DistConsts& q, WordStream& ws, float (&z)[D])
-{
-    switch (q.kind) {
-    case GLABC_DIST_DIAG_GAUSSIAN: {
-        float s = 0.0f;
-#pragma unroll
-        for (int i = 0; i < D; ++i) {
-            const float e = ws.normal();
-            z[i] = fmaf(q.c[i], e, q.a[i]);
-            s += q.b[i] + 0.5f * (e * e);  // log p from eps, distribution.py:171-173
-        }
-        return q.half_log_2pi - s;
-    }
-    case GLABC_DIST_UNIFORM: {
-#pragma unroll
-        for (int i = 0; i < D; ++i) z[i] = fmaf(q.b[i] - q.a[i], ws.uniform(), q.a[i]);  // distribution.py:73-77
-        return q.c[0];
-    }
-    case GLABC_DIST_GAMMA: {
-#pragma unroll
-        for (int i = 0; i < D; ++i) {
-            // Marsaglia & Tsang (2000): Gamma(a >= 1) by squeeze-rejection from a cubed normal; shape < 1 via Gamma(a + 1) * U^(1/a)
-            const float a0 = q.a[i];
-            const float a = a0 < 1.0f ? a0 + 1.0f : a0;
-            const float dd = a - (1.0f / 3.0f), cc = rsqrtf(9.0f * dd);
-            float g = dd;
-            for (int it = 0; it < 64; ++it) {
-                const float x = ws.normal();
-                const float t = fmaf(cc, x, 1.0f);
-                if (t <= 0.0f) continue;
-                const float v = t * t * t;
-                const float u = ws.uniform_open();
-                if (logf(u) < 0.5f * x * x + dd - dd * v + dd * logf(v)) {
-                    g = dd * v;
-                    break;
-                }
-            }
-            if (a0 < 1.0f) g *= powf(ws.uniform_open(), 1.0f / a0);
-            z[i] = g / q.b[i];  // scale = 1 / rate, distribution.py:118
-        }
-        return dist_log_prob<D>(q, z);
-    }
-    case GLABC_DIST_GAUSSIAN_MIXTURE: {
-        const float u = ws.uniform();
-        int m = q.n_modes - 1;
-        for (int j = q.n_modes - 2; j >= 0; --j)
-            if (u < q.mix_cdf[j]) m = j;  // torch.multinomial(weights, 1): first mode whose cumulative weight exceeds u
-#pragma unroll
-        for (int i = 0; i < D; ++i) z[i] = fmaf(ws.normal(), q.mix_scale[m][i], q.mix_loc[m][i]);  // distribution.py:258-260
-        return dist_log_prob<D>(q, z);
-    }
-    }
-    return NAN;
 }
 
 // GlobalMCMC.py:37-68 with arbitrary proposal kinds.

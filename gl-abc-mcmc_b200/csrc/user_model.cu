@@ -28,7 +28,12 @@ namespace glabc {
 
 namespace {
 
-// ---- the kernel's source: prelude + (user source) + step kernel.  D, YD, NN arrive as -D macros. ----
+// ---- the kernel's source: prelude + (user source) + step kernel.  D, YD, NN and the two proposal kinds GLABC_LP_KIND,
+// GLABC_GP_KIND arrive as -D macros; the prelude includes dist_device.cuh, whose text build.py embeds here. ----
+const char kDistDevice[] =
+#include "dist_device_src.inc"
+    ;
+
 const char* kPrelude = R"GLABC(
 typedef unsigned int u32;
 typedef unsigned long long u64;
@@ -42,21 +47,8 @@ typedef unsigned long long u64;
 #ifndef M_PI
 #define M_PI 3.14159265358979323846
 #endif
-struct UserRun {
-    int n_chains;
-    u32 first_step, last_step, chain_lo0, chain_hi0, key0, key1, gf_thr;
-    int gf_all_global, write_row0, trace_layout, pad;
-    long long trace_rows, trace_chains, trace_chain_off, trace_row_base;
-    float *theta, *y, *trace, *stats;
-    float lp_loc[8], lp_scale[8], gp_loc[8], gp_scale[8], gp_inv_scale[8];
-    float kern_c, kern_m;     // log K(dis) = kern_c + kern_m * dis^2   (Mixture.py:38-53)
-    float params[64];
-    float* aux;               // iSIR: [C][8] carried state (slot 0 cached log-weight, slot 1 `local` flag;
-                              // GLMALA adds slot 2 = gradient cached, slots 3.. = the cached gradient)
-    int n_candidates, pad2;
-    float tau, eps2;          // GLMALA: step size, ABCset.epsilon ** 2
-    int num_grad, pad3;
-};
+#include "dist_device.cuh"
+using glabc::UserRun;
 // A prior may return exactly this value to say "outside the support: draw the local proposal again" — the reference's
 // `while prior_log_prob(theta') == 7 * np.log(1e-10)` (GLMCMC.py:92-93; the float32 tensor is compared with the float64
 // scalar cast down to float32)
@@ -83,6 +75,55 @@ __device__ __forceinline__ void glabc_box_muller(u32 w0, u32 w1, float& n0, floa
     n0 = r * c;
     n1 = r * s;
 }
+// dist_forward's word source: successive 32-bit words of the Philox blocks (chain, step, slot0), (.., slot0 + 1), ..
+struct GlabcWords {
+    u32 g0, g1, step, slot, k0, k1;
+    uint4 cur;
+    int used;
+    float spare;
+    bool has_spare;
+    __device__ __forceinline__ GlabcWords(u32 c0, u32 c1, u32 i, u32 slot0, u32 key0, u32 key1)
+        : g0(c0), g1(c1), step(i), slot(slot0), k0(key0), k1(key1), cur(make_uint4(0, 0, 0, 0)), used(4), spare(0.f), has_spare(false) {}
+    __device__ __forceinline__ u32 next()
+    {
+        if (used == 4) {
+            cur = glabc_philox(g0, g1, step, slot++, k0, k1);
+            used = 0;
+        }
+        const u32 w = used == 0 ? cur.x : used == 1 ? cur.y : used == 2 ? cur.z : cur.w;
+        ++used;
+        return w;
+    }
+    __device__ __forceinline__ float uniform() { return __uint2float_rn(next() >> 8) * 0x1p-24f; }                 // [0, 1)
+    __device__ __forceinline__ float uniform_open() { return fmaf(__uint2float_rn(next() >> 8), 0x1p-24f, 0x1p-25f); }  // (0, 1)
+    __device__ __forceinline__ float normal()
+    {
+        if (has_spare) {
+            has_spare = false;
+            return spare;
+        }
+        const u32 w0 = next(), w1 = next();
+        float n0;
+        glabc_box_muller(w0, w1, n0, spare);
+        has_spare = true;
+        return n0;
+    }
+};
+// Philox slots (the counter's last word) the user kernels draw from, per (chain, step):
+//   1                        the step's coin and MH uniform
+//   2 ..                     NB blocks of normals: a DiagGaussian proposal's D, then the simulator's NN
+//   0x100 + j NB ..          the same for iSIR candidate j < GLABC_MAX_K
+//   0x10000 .., 0x20000 ..   GLMALA's gradient draws
+//   0x40000000 + r ..        redraw r < 64 of a DiagGaussian local proposal the prior answered with GLABC_PRIOR_SENTINEL
+//   0x80000000               the iSIR resampling uniform
+//   GLABC_SLOT_PROP ..       a Uniform / Gamma / GaussianMixture local or global draw; sentinel redraws continue its stream
+//   GLABC_SLOT_CAND + j GLABC_CAND_BLOCKS ..   iSIR candidate j from a Uniform / Gamma / GaussianMixture importance proposal
+// A non-Gaussian proposal only moves the proposal's draws: the simulator keeps its blocks.  One dist_forward takes at most
+// 386 blocks at D = 8 (Gamma: 8 x (64 squeeze iterations x 3 words + 1) words, dist_device.cuh), so a candidate's range
+// of 0x200 blocks holds it, and the 65 draws of a local move with every redraw (25090 blocks) fit under GLABC_SLOT_CAND.
+#define GLABC_SLOT_PROP 0x60000000u
+#define GLABC_SLOT_CAND 0x60010000u
+#define GLABC_CAND_BLOCKS 0x200u
 )GLABC";
 
 const char* kKernel = R"GLABC(
@@ -136,6 +177,7 @@ extern "C" __global__ void __launch_bounds__(128) glabc_k_global_user(const __gr
         }
         float thp[D], yp[YD], corr = 0.f;
         if (is_global) {                       // independence proposal q = Global_Proposal, :40-46
+#if GLABC_GP_KIND == GLABC_DIST_DIAG_GAUSSIAN
             float qn = 0.f, qo = 0.f;
 #pragma unroll
             for (int k = 0; k < D; ++k) {
@@ -145,9 +187,22 @@ extern "C" __global__ void __launch_bounds__(128) glabc_k_global_user(const __gr
                 qo = fmaf(r, r, qo);
             }
             corr = 0.5f * (qn - qo);           // log q(theta) - log q(theta'): the constants cancel
-        } else {                               // symmetric random walk, :56-60
+#else
+            GlabcWords ws(g0, g1, i, GLABC_SLOT_PROP, R.key0, R.key1);
+            const float lq_p = glabc::dist_forward<D>(R.gq, ws, thp);
+            corr = glabc::dist_log_prob<D>(R.gq, th) - lq_p;
+#endif
+        } else {                               // random walk theta + z, z ~ Local_Proposal, :56-60 (no q term)
+#if GLABC_LP_KIND == GLABC_DIST_DIAG_GAUSSIAN
 #pragma unroll
             for (int k = 0; k < D; ++k) thp[k] = th[k] + fmaf(R.lp_scale[k], z[k], R.lp_loc[k]);
+#else
+            GlabcWords ws(g0, g1, i, GLABC_SLOT_PROP, R.key0, R.key1);
+            float zl[D];
+            (void)glabc::dist_forward<D>(R.lq, ws, zl);
+#pragma unroll
+            for (int k = 0; k < D; ++k) thp[k] = th[k] + zl[k];
+#endif
         }
         glabc_user_simulate(thp, z + D, R.params, yp);
         const float tgt_p = glabc_target(R, thp, yp);
@@ -200,7 +255,7 @@ extern "C" __global__ void __launch_bounds__(128) glabc_k_global_user(const __gr
 }
 
 // ---- GLMCMC (iSIR) step for a user model: GLMCMC.py:58-104 with weight_sampling :7-22 --------------------------------
-// gp_* hold the Importance_Proposal here.  Candidate j of step i is a pure function of (chain, i, j) through Philox, so
+// gp_* (gq when it is not a DiagGaussian) hold the Importance_Proposal here.  Candidate j of step i is a pure function of (chain, i, j) through Philox, so
 // the K weights are computed first and only the selected candidate is rebuilt — no per-candidate storage.
 __device__ __forceinline__ float glabc_candidate(const UserRun& R, u32 g0, u32 g1, u32 i, int j, float* th, float* y, float& pk)
 {
@@ -212,6 +267,7 @@ __device__ __forceinline__ float glabc_candidate(const UserRun& R, u32 g0, u32 g
         glabc_box_muller(w.x, w.y, z[4 * b], z[4 * b + 1]);
         glabc_box_muller(w.z, w.w, z[4 * b + 2], z[4 * b + 3]);
     }
+#if GLABC_GP_KIND == GLABC_DIST_DIAG_GAUSSIAN
     float q = 0.f;
 #pragma unroll
     for (int k = 0; k < D; ++k) {
@@ -221,7 +277,26 @@ __device__ __forceinline__ float glabc_candidate(const UserRun& R, u32 g0, u32 g
     glabc_user_simulate(th, z + D, R.params, y);            // :71
     pk = glabc_target(R, th, y);                            // log prior + log kernel
     return pk + 0.5f * q;                                   // log-weight up to the proposal's constant (it cancels in the ratio)
+#else
+    GlabcWords ws(g0, g1, i, GLABC_SLOT_CAND + (u32)j * GLABC_CAND_BLOCKS, R.key0, R.key1);
+    float tj[D];
+    const float lq = glabc::dist_forward<D>(R.gq, ws, tj);
+#pragma unroll
+    for (int k = 0; k < D; ++k) th[k] = tj[k];
+    glabc_user_simulate(th, z + D, R.params, y);
+    pk = glabc_target(R, th, y);
+    return pk - lq;                                         // log prior + log K - log q, GLMCMC.py:66-74
+#endif
 }
+#if GLABC_GP_KIND != GLABC_DIST_DIAG_GAUSSIAN
+// log-weight of the current state, GLMCMC.py:60-64: +inf outside the support of q, so that global move selects nothing
+// (the reference's resample after inf / inf); a NaN weight counts as 0, as the candidates'
+__device__ __forceinline__ float glabc_state_logw(const UserRun& R, const float (&th)[D], float pk)
+{
+    const float lw = pk - glabc::dist_log_prob<D>(R.gq, th);
+    return lw == lw ? lw : -INFINITY;
+}
+#endif
 extern "C" __global__ void __launch_bounds__(128) glabc_k_isir_user(const __grid_constant__ UserRun R)
 {
     const int chain = blockIdx.x * blockDim.x + threadIdx.x;
@@ -263,6 +338,7 @@ extern "C" __global__ void __launch_bounds__(128) glabc_k_isir_user(const __grid
         bool moved = false;
         if (is_global) {
             if (local) {                                                          // :60-64: log-weight of the current state
+#if GLABC_GP_KIND == GLABC_DIST_DIAG_GAUSSIAN
                 float qo = 0.f;
 #pragma unroll
                 for (int k = 0; k < D; ++k) {
@@ -270,6 +346,9 @@ extern "C" __global__ void __launch_bounds__(128) glabc_k_isir_user(const __grid
                     qo = fmaf(r, r, qo);
                 }
                 lw_old = pk + 0.5f * qo;
+#else
+                lw_old = glabc_state_logw(R, th, pk);
+#endif
             }
             local = false;
             // shifted weights (the reference exponentiates un-shifted in float32, :78; the shift only removes underflow)
@@ -315,6 +394,7 @@ extern "C" __global__ void __launch_bounds__(128) glabc_k_isir_user(const __grid
                 glabc_box_muller(w.x, w.y, z[4 * b], z[4 * b + 1]);
                 glabc_box_muller(w.z, w.w, z[4 * b + 2], z[4 * b + 3]);
             }
+#if GLABC_LP_KIND == GLABC_DIST_DIAG_GAUSSIAN
 #pragma unroll
             for (int k = 0; k < D; ++k) thp[k] = th[k] + fmaf(R.lp_scale[k], z[k], R.lp_loc[k]);
             // GLMCMC.py:92-93: while the prior answers with the sentinel, draw the local proposal again (fresh normals from
@@ -330,6 +410,18 @@ extern "C" __global__ void __launch_bounds__(128) glabc_k_isir_user(const __grid
 #pragma unroll
                 for (int k = 0; k < D; ++k) thp[k] = th[k] + fmaf(R.lp_scale[k], zr[k], R.lp_loc[k]);
             }
+#else
+            GlabcWords ws(g0, g1, i, GLABC_SLOT_PROP, R.key0, R.key1);
+            float zl[D];
+            (void)glabc::dist_forward<D>(R.lq, ws, zl);
+#pragma unroll
+            for (int k = 0; k < D; ++k) thp[k] = th[k] + zl[k];
+            for (u32 redraw = 0; redraw < 64u && glabc_user_prior_log_prob(thp, R.params) == GLABC_PRIOR_SENTINEL; ++redraw) {
+                (void)glabc::dist_forward<D>(R.lq, ws, zl);   // GLMCMC.py:92-93, from the stream's next words
+#pragma unroll
+                for (int k = 0; k < D; ++k) thp[k] = th[k] + zl[k];
+            }
+#endif
             glabc_user_simulate(thp, z + D, R.params, yp);
             const float pkp = glabc_target(R, thp, yp);
             const float log_u = __logf(__uint2float_rn(w0.y >> 8) * 0x1p-24f);
@@ -503,6 +595,7 @@ extern "C" __global__ void __launch_bounds__(64) glabc_k_mala_user(const __grid_
         bool moved = false;
         if (is_global) {                                                          // :151-180, as glabc_k_isir_user
             if (local) {
+#if GLABC_GP_KIND == GLABC_DIST_DIAG_GAUSSIAN
                 float qo = 0.f;
 #pragma unroll
                 for (int k = 0; k < D; ++k) {
@@ -510,6 +603,9 @@ extern "C" __global__ void __launch_bounds__(64) glabc_k_mala_user(const __grid_
                     qo = fmaf(r, r, qo);
                 }
                 lw_old = pk + 0.5f * qo;
+#else
+                lw_old = glabc_state_logw(R, th, pk);
+#endif
             }
             local = false;
             float lw[17], thc[D], yc[YD], pkc, mx = lw_old;
@@ -735,7 +831,7 @@ struct Compiled {
     CUfunction fn_mala = nullptr;   // glabc_k_mala_user (models with theta_dim <= 5: the gradient is cached in the aux slots)
 };
 std::mutex g_cache_mu;
-std::map<std::string, Compiled> g_cache;   // key: device | arch | dims | source
+std::map<std::string, Compiled> g_cache;   // key: device | arch | dims | proposal kinds | source
 
 std::string cu_err(Dyn& d, CUresult r)
 {
@@ -746,22 +842,37 @@ std::string cu_err(Dyn& d, CUresult r)
 
 }  // namespace
 
-// NVRTC: prelude + user source + step kernel -> cubin for sm_<cc>
-static int compile_to_cubin(Dyn& d, int cc, const glabc_user_model_t& um, std::vector<char>& cubin, std::string& err)
+// NVRTC: prelude + user source + step kernel -> cubin for sm_<cc>, the Local / Global-or-Importance proposal kinds fixed
+static int compile_to_cubin(Dyn& d, int cc, const glabc_user_model_t& um, int lp_kind, int gp_kind, std::vector<char>& cubin,
+                            std::string& err)
 {
     const std::string src = std::string(kPrelude) + "\n// ---- user model ----\n" + um.source + "\n// ---- step kernel ----\n" + kKernel;
     nvrtcProgram prog = nullptr;
-    nvrtcResult r = d.createProgram(&prog, src.c_str(), "glabc_user_model.cu", 0, nullptr, nullptr);
+    const char* hdr_src[] = {kDistDevice};
+    const char* hdr_name[] = {"dist_device.cuh"};
+    nvrtcResult r = d.createProgram(&prog, src.c_str(), "glabc_user_model.cu", 1, hdr_src, hdr_name);
     if (r != NVRTC_SUCCESS) {
         err = std::string("nvrtcCreateProgram: ") + d.errString(r);
         return GLABC_ERR_CUDA;
     }
-    char arch[48], dD[24], dY[24], dN[24];
+    char arch[48], dD[24], dY[24], dN[24], dLP[32], dGP[32];
     snprintf(arch, sizeof(arch), "--gpu-architecture=sm_%d%s", cc, cc >= 90 ? "a" : "");
     snprintf(dD, sizeof(dD), "-DD=%d", um.theta_dim);
     snprintf(dY, sizeof(dY), "-DYD=%d", um.y_dim);
     snprintf(dN, sizeof(dN), "-DNN=%d", um.n_noise);
-    const char* opts[] = {arch, dD, dY, dN, "--std=c++17", "--use_fast_math", "-lineinfo"};
+    snprintf(dLP, sizeof(dLP), "-DGLABC_LP_KIND=%d", lp_kind);
+    snprintf(dGP, sizeof(dGP), "-DGLABC_GP_KIND=%d", gp_kind);
+    // dist_device.cuh's constants, from include/glabc.h
+    char kinds[4][48], sizes[3][40];
+    snprintf(kinds[0], sizeof(kinds[0]), "-DGLABC_DIST_DIAG_GAUSSIAN=%d", GLABC_DIST_DIAG_GAUSSIAN);
+    snprintf(kinds[1], sizeof(kinds[1]), "-DGLABC_DIST_UNIFORM=%d", GLABC_DIST_UNIFORM);
+    snprintf(kinds[2], sizeof(kinds[2]), "-DGLABC_DIST_GAMMA=%d", GLABC_DIST_GAMMA);
+    snprintf(kinds[3], sizeof(kinds[3]), "-DGLABC_DIST_GAUSSIAN_MIXTURE=%d", GLABC_DIST_GAUSSIAN_MIXTURE);
+    snprintf(sizes[0], sizeof(sizes[0]), "-DGLABC_MAX_DIM=%d", GLABC_MAX_DIM);
+    snprintf(sizes[1], sizeof(sizes[1]), "-DGLABC_MAX_MODES=%d", GLABC_MAX_MODES);
+    snprintf(sizes[2], sizeof(sizes[2]), "-DGLABC_USER_MAX_PARAMS=%d", GLABC_USER_MAX_PARAMS);
+    const char* opts[] = {arch, dD, dY, dN, dLP, dGP, kinds[0], kinds[1], kinds[2], kinds[3], sizes[0], sizes[1], sizes[2],
+                          "--std=c++17", "--use_fast_math", "-lineinfo"};
     r = d.compileProgram(prog, static_cast<int>(sizeof(opts) / sizeof(opts[0])), opts);
     if (r != NVRTC_SUCCESS) {
         size_t n = 0;
@@ -780,7 +891,7 @@ static int compile_to_cubin(Dyn& d, int cc, const glabc_user_model_t& um, std::v
     return GLABC_OK;
 }
 
-int user_model_check(int cc, const glabc_user_model_t& um, std::string& err)
+int user_model_check(int cc, const glabc_user_model_t& um, int lp_kind, int gp_kind, std::string& err)
 {
     Dyn& d = dyn();
     if (!d.rt_ok) {
@@ -788,10 +899,11 @@ int user_model_check(int cc, const glabc_user_model_t& um, std::string& err)
         return GLABC_ERR_UNSUPPORTED;
     }
     std::vector<char> cubin;
-    return compile_to_cubin(d, cc, um, cubin, err);
+    return compile_to_cubin(d, cc, um, lp_kind, gp_kind, cubin, err);
 }
 
-int user_model_compile(int device, int cc, const glabc_user_model_t& um, int kind, void** fn_out, std::string& err)
+int user_model_compile(int device, int cc, const glabc_user_model_t& um, int lp_kind, int gp_kind, int kind, void** fn_out,
+                       std::string& err)
 {
     Dyn& d = dyn();
     if (!d.ok) {
@@ -799,7 +911,7 @@ int user_model_compile(int device, int cc, const glabc_user_model_t& um, int kin
         return GLABC_ERR_UNSUPPORTED;
     }
     char head[160];
-    snprintf(head, sizeof(head), "%d|%d|%d|%d|%d|", device, cc, um.theta_dim, um.y_dim, um.n_noise);
+    snprintf(head, sizeof(head), "%d|%d|%d|%d|%d|%d|%d|", device, cc, um.theta_dim, um.y_dim, um.n_noise, lp_kind, gp_kind);
     const std::string key = std::string(head) + um.source;
     std::lock_guard<std::mutex> lock(g_cache_mu);
     auto it = g_cache.find(key);
@@ -808,7 +920,7 @@ int user_model_compile(int device, int cc, const glabc_user_model_t& um, int kin
         return GLABC_OK;
     }
     std::vector<char> cubin;
-    int st = compile_to_cubin(d, cc, um, cubin, err);
+    int st = compile_to_cubin(d, cc, um, lp_kind, gp_kind, cubin, err);
     if (st) return st;
     Compiled c;
     CUresult cr = d.moduleLoadData(&c.mod, cubin.data());

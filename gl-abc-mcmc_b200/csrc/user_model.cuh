@@ -6,31 +6,16 @@
 #include <cuda_runtime.h>
 
 #include "../../include/glabc.h"
+#include "dist_device.cuh"
 
 namespace glabc {
 
-// kernel parameter of glabc_k_global_user — field for field the `UserRun` of the NVRTC prelude in user_model.cu
-struct UserRun {
-    int32_t n_chains;
-    uint32_t first_step, last_step, chain_lo0, chain_hi0, key0, key1, gf_thr;
-    int32_t gf_all_global, write_row0, trace_layout, pad;
-    long long trace_rows, trace_chains, trace_chain_off, trace_row_base;
-    float *theta, *y, *trace, *stats;
-    float lp_loc[8], lp_scale[8], gp_loc[8], gp_scale[8], gp_inv_scale[8];
-    float kern_c, kern_m;
-    float params[GLABC_USER_MAX_PARAMS];
-    float* aux;
-    int32_t n_candidates, pad2;
-    float tau, eps2;
-    int32_t num_grad, pad3;
-};
-static_assert(GLABC_USER_MAX_PARAMS == 64 && GLABC_MAX_DIM == 8, "the NVRTC prelude hard-codes these sizes");
-
-// compile (or fetch from the process-wide cache) the step kernel specialised for `um`; *fn is a CUfunction
+// compile (or fetch from the process-wide cache) the step kernels specialised for `um` and the glabc_dist_kind of the
+// Local (lp_kind) and Global / Importance (gp_kind) proposals; *fn is a CUfunction
 // kind: 0 = GlobalMCMC step, 1 = GLMCMC (iSIR) step, 2 = GLMALA step
-int user_model_compile(int device, int cc, const glabc_user_model_t& um, int kind, void** fn, std::string& err);
+int user_model_compile(int device, int cc, const glabc_user_model_t& um, int lp_kind, int gp_kind, int kind, void** fn, std::string& err);
 // compile only (needs NVRTC, no driver / GPU): validates a model's source; err receives the NVRTC log
-int user_model_check(int cc, const glabc_user_model_t& um, std::string& err);
+int user_model_check(int cc, const glabc_user_model_t& um, int lp_kind, int gp_kind, std::string& err);
 int user_model_launch(void* fn, const UserRun& R, int block, cudaStream_t st, std::string& err);
 
 }  // namespace glabc

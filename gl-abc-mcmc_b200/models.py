@@ -143,12 +143,16 @@ class UserModel:
         _abi.fill(pod.params, self.params)
         return pod
 
-    def check(self, cc=100):
-        """compile-only validation (NVRTC, no GPU needed); raises ValueError with the compiler log"""
+    def check(self, cc=100, proposals=None):
+        """compile-only validation (NVRTC, no GPU needed); raises ValueError with the compiler log.
+        `proposals`: the (Local_Proposal, Global_Proposal or Importance_Proposal) pair a run will bind, to compile the
+        kernels for their kinds; None in either place (GLMALA has no Local_Proposal) or for the pair means DiagGaussian."""
         import ctypes as C
         log = C.create_string_buffer(8192)
         pod = self.user_pod()
-        st = _abi.load().glabc_user_model_check(C.byref(pod), int(cc), log, len(log))
+        local, far = proposals if proposals is not None else (None, None)
+        kinds = [_abi.DIST_DIAG_GAUSSIAN if d is None else lower_proposal(d).kind for d in (local, far)]
+        st = _abi.load().glabc_user_model_check_proposals(C.byref(pod), kinds[0], kinds[1], int(cc), log, len(log))
         if st != _abi.OK:
             raise ValueError(f"user model rejected (status {st}): {log.value.decode(errors='replace')}")
         return True

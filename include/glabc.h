@@ -346,7 +346,7 @@ GLABC_API int glabc_device_info(const glabc_ctx* ctx, int32_t* sm_count, int32_t
 /* replaces the `ABCset` argument of every sampler (GlobalMCMC.py:6, GLMCMC.py:24, ...)           */
 GLABC_API int glabc_model_set(glabc_ctx* ctx, const glabc_model_t* model, size_t nbytes);
 /* replaces Local_Proposal / Global_Proposal / Importance_Proposal (GlobalMCMC.py:6-7,
- * GLMCMC.py:24-25)                                                                               */
+ * GLMCMC.py:24-25).  dim 1..GLABC_MAX_DIM: the built-in model family runs dim <= 4 (its theta_dim), a user model up to 8. */
 GLABC_API int glabc_dist_set(glabc_ctx* ctx, int slot, const glabc_dist_t* dist, size_t nbytes);
 /* Prior of the bound model (replaces the DiagGaussian in glabc_model_t's prior_* fields): any glabc_dist_t kind,
  * dim == theta_dim.  NULL restores the model's DiagGaussian.  glabc_model_set clears a bound prior.
@@ -354,11 +354,13 @@ GLABC_API int glabc_dist_set(glabc_ctx* ctx, int slot, const glabc_dist_t* dist,
  * Gamma / GaussianMixture prior every sampler runs FAST arithmetic with the native RNG: GLABC_ARITH_STRICT, GLABC_RNG_REPLAY,
  * tape_dump and the AGLMCMC parity dumps are refused with GLABC_ERR_UNSUPPORTED.  Outside the prior's support the log prior
  * is -inf: from such a state the first proposal with a finite prior is accepted, a candidate with -inf is never selected.
- * GLABC_ERR_INVALID: no model bound, dim != theta_dim, invalid parameters (the checks of glabc_dist_set).               */
+ * GLABC_ERR_INVALID: no model bound, dim != theta_dim, invalid parameters (the checks of glabc_dist_set);
+ * GLABC_ERR_UNSUPPORTED: dim > 4.                                                                                        */
 GLABC_API int glabc_model_prior_set(glabc_ctx* ctx, const glabc_dist_t* prior, size_t nbytes);
 
 /* device-side forward() / log_prob() of the distribution bound to `slot` (distribution.py:73-86, 106-137, 166-181,
- * 242-293): z[n][dim] -> log_p[n], and n fresh draws z[n][dim] (+ their log-densities, log_p may be NULL)            */
+ * 242-293): z[n][dim] -> log_p[n], and n fresh draws z[n][dim] (+ their log-densities, log_p may be NULL).
+ * dim <= 4; a wider distribution (for a user model) is refused with GLABC_ERR_UNSUPPORTED.                            */
 GLABC_API int glabc_dist_log_prob(glabc_ctx* ctx, int slot, const float* z, int64_t n, float* log_p, void* stream);
 GLABC_API int glabc_dist_sample(glabc_ctx* ctx, int slot, int64_t n, uint64_t seed, float* z, float* log_p, void* stream);
 
@@ -404,23 +406,36 @@ GLABC_API int glabc_run_mala(glabc_ctx* ctx, const glabc_run_t* run);
  * Uniform box, say) never enter a block.                                                                                */
 GLABC_API int glabc_run_aglmcmc(glabc_ctx* ctx, const glabc_run_t* run, const glabc_aglmcmc_t* ag);
 
-/* GlobalMCMC loop body (GlobalMCMC.py:37-68) for a user-supplied model: LOCAL / GLOBAL slots must hold DiagGaussian
- * proposals of the model's theta_dim; native RNG; run->theta [C][theta_dim], run->y [C][y_dim]; trace / stats as
- * glabc_run_global.  The first call for a given source compiles it (about a second); the module is cached for the
- * life of the process.  A compile error is returned as GLABC_ERR_INVALID with the NVRTC log in glabc_last_error.     */
+/* GlobalMCMC loop body (GlobalMCMC.py:37-68) for a user-supplied model: LOCAL / GLOBAL slots hold proposals of any
+ * glabc_dist_kind and of the model's theta_dim (1..GLABC_MAX_DIM); native RNG, FAST arithmetic; run->theta [C][theta_dim],
+ * run->y [C][y_dim]; trace / stats as glabc_run_global.  The first call for a given source and pair of proposal kinds
+ * compiles it (about a second); the module is cached for the life of the process.  A compile error is returned as
+ * GLABC_ERR_INVALID with the NVRTC log in glabc_last_error.
+ * Semantics of the proposals as glabc_run_global's general kernel: a local move is theta + z, z ~ Local_Proposal, with no
+ * proposal term in the MH ratio (so an asymmetric Gamma local proposal gives the reference's biased chain); a global move
+ * adds log q(theta) - log q(theta').  Two DiagGaussian slots run the fused Gaussian arithmetic; the simulator's noise is
+ * drawn from the same random numbers whatever the proposal kinds.                                                     */
 GLABC_API int glabc_run_global_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_user_model_t* model);
 /* GLMCMC loop body (GLMCMC.py:58-104, weight_sampling :7-22) for a user-supplied model: LOCAL = Local_Proposal, IMPORTANCE =
- * Importance_Proposal (DiagGaussian), run->n_candidates = batch_size, run->aux as glabc_run_isir.  The importance weights are
- * exponentiated max-shifted (the reference's un-shifted float32 exp can underflow a whole row to `None`; the shift removes
- * that artefact and nothing else).                                                                                        */
+ * Importance_Proposal (any glabc_dist_kind, as glabc_run_global_user), run->n_candidates = batch_size, run->aux as
+ * glabc_run_isir.  The importance weights are exponentiated max-shifted (the reference's un-shifted float32 exp can underflow a
+ * whole row to `None`; the shift removes that artefact and nothing else).  log-weight = log prior + log K - log q; a NaN
+ * weight counts as 0, a -inf candidate is never selected, and a current state outside the importance proposal's support has
+ * log-weight +inf: that global move selects nothing and the chain stays.                                                  */
 GLABC_API int glabc_run_isir_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_user_model_t* model);
-/* GLMALA (GLMALA.py:150-200) for a user model: IMPORTANCE slot, run->n_candidates, run->tau, run->num_grad; aux [C][8] carries
+/* GLMALA (GLMALA.py:150-200) for a user model: IMPORTANCE slot (any glabc_dist_kind, its global move as
+ * glabc_run_isir_user), run->n_candidates, run->tau, run->num_grad; aux [C][8] carries
  * the cached log-weight (slot 0), the `local` flag (1), "gradient cached" (2) and the cached gradient (3 ..): theta_dim <= 5.
  * A thread per chain; the finite-difference gradient's draws (GLMALA.py:46-95) are dealt over the warp.                    */
 GLABC_API int glabc_run_mala_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_user_model_t* model);
 /* Compile-only check of a user model for compute capability `cc` (100 = sm_100a): needs NVRTC but neither a GPU nor a
- * context.  The NVRTC log (or "" on success) is copied to log[log_cap].                                              */
+ * context.  The NVRTC log (or "" on success) is copied to log[log_cap].  Compiles the kernels for DiagGaussian proposals. */
 GLABC_API int glabc_user_model_check(const glabc_user_model_t* model, int32_t cc, char* log, size_t log_cap);
+/* The same for the proposal kinds (glabc_dist_kind) a run will bind: local_kind for the LOCAL slot, far_kind for the
+ * GLOBAL (glabc_run_global_user) or IMPORTANCE (glabc_run_isir_user, glabc_run_mala_user) slot.  An unknown kind is
+ * GLABC_ERR_INVALID.                                                                                                  */
+GLABC_API int glabc_user_model_check_proposals(const glabc_user_model_t* model, int32_t local_kind, int32_t far_kind, int32_t cc,
+                                               char* log, size_t log_cap);
 
 /* ---- KernelDensity (kernel_density.py:4-177), batched over `sets` independent point sets ------------------
  * Set s holds n[s] points X[s][cap][dim] (n == NULL: every set holds `cap` points).                          */
