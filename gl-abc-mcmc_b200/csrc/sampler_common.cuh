@@ -22,6 +22,7 @@ struct RunParams {
                             // branch uniform and gf_thr_hi = ceil(gf * 2^16) << 16   (cf. B-15/B-16)
     int32_t gf_all_global;  // gf >= 1: every step is global (the threshold would not fit 32 bits)
     int32_t write_row0;
+    int32_t trace_runs_16b;  // chain-major d = 2: every chain's 32-row run starts 16-byte aligned (chain_major_runs_16b)
     int64_t trace_rows, trace_chains, trace_chain_off, trace_row_base;
     float* theta;
     float* y;
@@ -153,39 +154,68 @@ struct ChainMajorWriter {
     {
         if (count > 0) flush(r);
     }
+
+    // full-tile entry points of K1's steady loop: the row's slot is the loop position, and the tile
+    // [first_row, first_row + 32) ends with one flush
+    __device__ __forceinline__ void put_slot(uint32_t slot, const float (&v)[D])
+    {
+#pragma unroll
+        for (int k = 0; k < D; ++k) tile[k * kPlane + slot * kPitch + lane] = v[k];
+    }
+    __device__ __forceinline__ void flush_tile(const RunParams& r, uint32_t first_row)
+    {
+        row0 = first_row;
+        count = 32;
+        flush(r);
+    }
 };
 
-// D in {1, 2, 4}: a row is one 4/8/16-byte vector, so the tile is [32 rows][33] vectors — a lane
-// stores its chain's row with one STS (consecutive lanes, conflict-free), and a flush reads column c
-// with one LDS per lane (lane = row; pitch 33 keeps the 64/128-bit phases conflict-free) and writes
-// chain c's 32 rows as ONE coalesced store instruction of 32 vectors (128/256/512 contiguous bytes).
-template <int D>
+// D in {1, 2, 4}: a row is one 4/8/16-byte vector.  The tile is chain-major, [32 chains][kPitch]
+// vectors, so a lane stores its chain's row with one STS into its own line of the tile, and a flush
+// writes chain c's rows as one coalesced run (128/256/512 contiguous bytes for a full tile).
+//  - full tile of a full warp, WIDE (D = 2 only) and runs 16-byte aligned (RunParams::trace_runs_16b):
+//    a lane moves two rows of one chain as one LDS.128 / STG.128, lanes 0-15 chain c and 16-31 chain
+//    c+1, so the tile is 16 STG.128 instead of 32 STG.64;
+//  - full tile of a full warp otherwise: one STG per chain, lane = row;
+//  - partial tile or tail warp: the same, predicated on lane < count.
+// Banks (32 x 4 bytes): pitch 33 vectors is conflict-free both ways.  The 16-byte reads of WIDE need
+// an even pitch: 34 float2 = 17 16-byte units.  The STS.64 of a step then runs in two half-warp phases
+// in which lanes l and l + 8 meet in 8-byte bank pair 34 l mod 16 (2-way); each quarter-warp phase of
+// the LDS.128 reads 8 consecutive 16-byte units of one chain (conflict-free), and the lane = row
+// reads are consecutive (conflict-free).  WIDE pays where the trace writer is a large share of the
+// issue budget (K1's steady loop); the samplers with heavier steps keep the conflict-free pitch.
+template <int D, bool WIDE = false>
 struct ChainMajorVecWriter {
+    static_assert(!WIDE || D == 2, "the 16-byte flush moves two float2 rows per lane");
     using V = typename VecOf<D>::type;
-    static constexpr int kPitch = 33;
+    static constexpr int kPitch = WIDE ? 34 : 33;
     static constexpr int smem_floats_per_warp = 32 * kPitch * D;
-    V* tile;
-    V* out;            // &trace[chain0_of_warp][0] in vector units
+    V* line;           // this lane's chain in the warp's tile (the tile is line - lane * kPitch)
+    V* out;            // &trace[chain0_of_warp][0] - trace_row_base, in vector units: indexed by absolute row
     int64_t chain_stride;  // vectors per chain
     uint32_t row0;
     int32_t count, lane, chains_in_warp;
 
     __device__ __forceinline__ ChainMajorVecWriter(const RunParams& r, int32_t, bool, float* smem_warp)
-        : tile(reinterpret_cast<V*>(smem_warp)), chain_stride(r.trace_rows), row0(0), count(0), lane(threadIdx.x & 31)
+        : chain_stride(r.trace_rows), row0(0), count(0), lane(threadIdx.x & 31)
     {
         const int32_t chain0 = blockIdx.x * blockDim.x + (threadIdx.x & ~31u);
-        out = reinterpret_cast<V*>(r.trace) + (r.trace_chain_off + chain0) * chain_stride;
+        line = reinterpret_cast<V*>(smem_warp) + lane * kPitch;
+        out = reinterpret_cast<V*>(r.trace) + ((r.trace_chain_off + chain0) * chain_stride - r.trace_row_base);
         chains_in_warp = min(32, r.n_chains - chain0);
+    }
+
+    static __device__ __forceinline__ V pack(const float (&v)[D])
+    {
+        if constexpr (D == 1) return v[0];
+        else if constexpr (D == 2) return make_float2(v[0], v[1]);
+        else return make_float4(v[0], v[1], v[2], v[3]);
     }
 
     __device__ __forceinline__ void put(const RunParams&, uint32_t row, const float (&v)[D])
     {
         if (count == 0) row0 = row;
-        V x;
-        if constexpr (D == 1) x = v[0];
-        else if constexpr (D == 2) x = make_float2(v[0], v[1]);
-        else x = make_float4(v[0], v[1], v[2], v[3]);
-        tile[count * kPitch + lane] = x;
+        line[count] = pack(v);
         ++count;
     }
 
@@ -196,17 +226,7 @@ struct ChainMajorVecWriter {
 
     __device__ __forceinline__ void flush(const RunParams& r)
     {
-        __syncwarp();
-        V* dst = out + (static_cast<int64_t>(row0) - r.trace_row_base) + lane;
-        const V* src = tile + lane * kPitch;
-        if (count == 32 && chains_in_warp == 32) {
-#pragma unroll 8
-            for (int32_t c = 0; c < 32; ++c) dst[c * chain_stride] = src[c];
-        } else {
-            for (int32_t c = 0; c < chains_in_warp; ++c)
-                if (lane < count) dst[c * chain_stride] = src[c];
-        }
-        __syncwarp();
+        flush_rows(r, row0, count);
         count = 0;
     }
 
@@ -214,7 +234,46 @@ struct ChainMajorVecWriter {
     {
         if (count > 0) flush(r);
     }
+
+    // full-tile entry points of K1's steady loop: the row's slot is the loop position, and the tile
+    // [first_row, first_row + 32) ends with one flush
+    __device__ __forceinline__ void put_slot(uint32_t slot, const float (&v)[D]) { line[slot] = pack(v); }
+    __device__ __forceinline__ void flush_tile(const RunParams& r, uint32_t first_row) { flush_rows(r, first_row, 32); }
+
+    // rows [first_row, first_row + n) of the warp's chains; the tile holds them in slots [0, n)
+    __device__ __forceinline__ void flush_rows(const RunParams& r, uint32_t first_row, int32_t n)
+    {
+        __syncwarp();
+        const V* tile = line - lane * kPitch;
+        if (n == 32 && chains_in_warp == 32) {
+            if (WIDE && r.trace_runs_16b) {
+                const int32_t h = lane >> 4, j = 2 * (lane & 15);
+                const V* src = tile + h * kPitch + j;
+                V* dst = out + h * chain_stride + first_row + j;
+#pragma unroll
+                for (int32_t c = 0; c < 32; c += 2)
+                    *reinterpret_cast<float4*>(dst + c * chain_stride) = *reinterpret_cast<const float4*>(src + c * kPitch);
+            } else {
+                V* dst = out + first_row + lane;
+#pragma unroll 8
+                for (int32_t c = 0; c < 32; ++c) dst[c * chain_stride] = tile[c * kPitch + lane];
+            }
+        } else {
+            V* dst = out + first_row + lane;
+            for (int32_t c = 0; c < chains_in_warp; ++c)
+                if (lane < n) dst[c * chain_stride] = tile[c * kPitch + lane];
+        }
+        __syncwarp();
+    }
 };
+
+// RunParams::trace_runs_16b of a launch with a WIDE writer: a 32-row run of chain c starts at float2
+// (trace_chain_off + c) * trace_rows + row - trace_row_base with row % 32 == 0, so every run is
+// 16-byte aligned when the buffer is and trace_rows and trace_row_base are even.
+inline bool chain_major_runs_16b(const RunParams& r)
+{
+    return (reinterpret_cast<uintptr_t>(r.trace) & 15u) == 0 && (r.trace_rows & 1) == 0 && (r.trace_row_base & 1) == 0;
+}
 
 // EVENTS: the chain as its moves (glabc.h GLABC_TRACE_EVENTS).  One scattered store per move instead of one row per step.
 template <int D>
@@ -264,12 +323,13 @@ struct NoTraceWriter {
     static constexpr int smem_floats_per_warp = 0;
 };
 
-template <int D, int LAYOUT> struct WriterFor;
-template <int D> struct WriterFor<D, GLABC_TRACE_NONE> { using type = NoTraceWriter; };
-template <int D> struct WriterFor<D, GLABC_TRACE_TIME_MAJOR> { using type = TimeMajorWriter<D>; };
-template <int D> struct WriterFor<D, GLABC_TRACE_CHAIN_MAJOR> { using type = ChainMajorVecWriter<D>; };
-template <> struct WriterFor<3, GLABC_TRACE_CHAIN_MAJOR> { using type = ChainMajorWriter<3>; };
-template <int D> struct WriterFor<D, GLABC_TRACE_EVENTS> { using type = EventWriter<D>; };
+// WIDE: the chain-major d = 2 writer with the 16-byte full-tile flush (ChainMajorVecWriter)
+template <int D, int LAYOUT, bool WIDE = false> struct WriterFor;
+template <int D, bool W> struct WriterFor<D, GLABC_TRACE_NONE, W> { using type = NoTraceWriter; };
+template <int D, bool W> struct WriterFor<D, GLABC_TRACE_TIME_MAJOR, W> { using type = TimeMajorWriter<D>; };
+template <int D, bool W> struct WriterFor<D, GLABC_TRACE_CHAIN_MAJOR, W> { using type = ChainMajorVecWriter<D, W && D == 2>; };
+template <bool W> struct WriterFor<3, GLABC_TRACE_CHAIN_MAJOR, W> { using type = ChainMajorWriter<3>; };
+template <int D, bool W> struct WriterFor<D, GLABC_TRACE_EVENTS, W> { using type = EventWriter<D>; };
 
 // ---------------------------------------------------------------------------------------------
 // Per-chain statistics (layout: GLABC_STAT_* in glabc.h)

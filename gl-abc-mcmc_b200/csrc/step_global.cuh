@@ -219,7 +219,7 @@ template <int D, int FAMILY, bool STRICT, bool REPLAY, int LAYOUT, bool DUMP>
 __global__ void __launch_bounds__(256) k_global_mcmc(const __grid_constant__ GlobalConsts K,
                                                      const __grid_constant__ RunParams R)
 {
-    using Writer = typename WriterFor<D, LAYOUT>::type;
+    using Writer = typename WriterFor<D, LAYOUT, true>::type;
     extern __shared__ float smem[];
     const int32_t chain = blockIdx.x * blockDim.x + threadIdx.x;
     const bool active = chain < R.n_chains;
@@ -279,43 +279,45 @@ __global__ void __launch_bounds__(256) k_global_mcmc(const __grid_constant__ Glo
 #pragma unroll
             for (int k = 0; k < 4; ++k) b[k] = inputs_native<D, STRICT, DUMP>(K, R, R.rk, stream, i + k);
         };
-        auto advance4 = [&](uint32_t i, const StepInputs<D> (&b)[4]) {
+        // The steady loop runs whole trace tiles: 32 rows for the chain-major writers, whose tiles end on
+        // absolute rows i % 32 == 31, one 8-step body for the others.  Inside a tile a row's slot is
+        // the loop position, so the chain-major put is one shared-memory store at a fixed offset from
+        // the body's base, with no row bookkeeping, and the tile ends in one unconditional flush.
+        constexpr bool kTiled = LAYOUT == GLABC_TRACE_CHAIN_MAJOR;
+        constexpr uint32_t kTile = kTiled ? 32u : 8u;
+        auto advance4 = [&](uint32_t i, uint32_t slot, const StepInputs<D> (&b)[4]) {
 #pragma unroll
             for (int k = 0; k < 4; ++k) {
                 advance<D, FAMILY, STRICT>(K, st, stats, b[k]);
-                writer.put(R, i + k, st.theta);
+                if constexpr (kTiled) writer.put_slot(slot + k, st.theta);
+                else writer.put(R, i + k, st.theta);
                 dump(i + k, b[k]);
             }
-            writer.maybe_flush(R, i + 3u);  // 32-row tile boundaries only fall on i % 4 == 3
         };
 
         if (R.last_step >= R.first_step) {
             uint32_t i = R.first_step;
-            while (i <= R.last_step && (i & 3u)) single(i++);
-            if (i + 3u <= R.last_step) {
+            while (i <= R.last_step && (i % kTile)) single(i++);  // head, up to the first tile boundary
+            if (i + (kTile - 1u) <= R.last_step) {
                 // ping-pong between two input buffers so no registers are copied between batches:
                 // prepare() of the next batch is independent of the chain state and overlaps with the
-                // dependent advance() chain of the current one.
+                // dependent advance() chain of the current one, across tile edges too (the last
+                // tile's look-ahead batch is computed and dropped)
                 StepInputs<D> a[4], b[4];
                 prepare4(i, a);
-                while (i + 11u <= R.last_step) {
-                    prepare4(i + 4u, b);
-                    advance4(i, a);
-                    prepare4(i + 8u, a);
-                    advance4(i + 4u, b);
-                    i += 8u;
-                }
-                if (i + 7u <= R.last_step) {
-                    prepare4(i + 4u, b);
-                    advance4(i, a);
-                    advance4(i + 4u, b);
-                    i += 8u;
-                } else {
-                    advance4(i, a);
-                    i += 4u;
-                }
+                do {
+#pragma unroll 1
+                    for (uint32_t s = 0; s < kTile; s += 8u) {
+                        prepare4(i + s + 4u, b);
+                        advance4(i + s, s, a);
+                        prepare4(i + s + 8u, a);
+                        advance4(i + s + 4u, s + 4u, b);
+                    }
+                    if constexpr (kTiled) writer.flush_tile(R, i);
+                    i += kTile;
+                } while (i + (kTile - 1u) <= R.last_step);
             }
-            while (i <= R.last_step) single(i++);
+            while (i <= R.last_step) single(i++);  // tail, < kTile steps
         }
     }
     writer.finish(R);
@@ -334,7 +336,7 @@ __global__ void __launch_bounds__(256) k_global_mcmc(const __grid_constant__ Glo
 template <int D, int FAMILY, bool STRICT, bool REPLAY, int LAYOUT, bool DUMP>
 static cudaError_t launch_one(const GlobalConsts& K, const RunParams& R, int block, cudaStream_t st)
 {
-    using Writer = typename WriterFor<D, LAYOUT>::type;
+    using Writer = typename WriterFor<D, LAYOUT, true>::type;
     const int grid = (R.n_chains + block - 1) / block;
     const size_t smem = sizeof(float) * Writer::smem_floats_per_warp * (block / 32);
     auto kern = k_global_mcmc<D, FAMILY, STRICT, REPLAY, LAYOUT, DUMP>;
@@ -342,7 +344,9 @@ static cudaError_t launch_one(const GlobalConsts& K, const RunParams& R, int blo
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
         if (e != cudaSuccess) return e;
     }
-    kern<<<grid, block, smem, st>>>(K, R);
+    RunParams P = R;
+    P.trace_runs_16b = LAYOUT == GLABC_TRACE_CHAIN_MAJOR && D == 2 && chain_major_runs_16b(R);
+    kern<<<grid, block, smem, st>>>(K, P);
     return cudaGetLastError();
 }
 
