@@ -28,7 +28,7 @@ def GLMALA(ABCset, num_ite, Initial_theta, Initial_y, tau, num_grad, filelocatio
         eng.bind_proposal(_abi.SLOT_IMPORTANCE, Importance_Proposal)
         return run_user_model(eng, ABCset, "mala", num_ite, Initial_theta, Initial_y, None, filelocation, global_frequency, num_chains,
                               seed, chain_id_base, trace, return_stats, verbose, block_threads, K=int(batch_size), num_grad=int(num_grad),
-                              tau=float(tau))
+                              tau=float(tau), checkpoint=checkpoint, resume=resume)
     pod = eng.bind_model(ABCset)
     eng.bind_proposal(_abi.SLOT_IMPORTANCE, Importance_Proposal)
     state64 = None      # resume: the carried float64 state comes from the checkpoint (Initial_theta / Initial_y are not read)

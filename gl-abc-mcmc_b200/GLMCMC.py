@@ -23,7 +23,8 @@ def GLMCMC(ABCset, num_ite, Initial_theta, Initial_y, Local_Proposal, filelocati
     if isinstance(ABCset, UserModel):       # run-time compiled model (csrc/user_model.cu)
         eng.bind_proposal(_abi.SLOT_IMPORTANCE, Importance_Proposal)
         return run_user_model(eng, ABCset, "isir", num_ite, Initial_theta, Initial_y, Local_Proposal, filelocation, global_frequency,
-                              num_chains, seed, chain_id_base, trace, return_stats, verbose, block_threads, K=int(batch_size))
+                              num_chains, seed, chain_id_base, trace, return_stats, verbose, block_threads, K=int(batch_size),
+                              checkpoint=checkpoint, resume=resume)
     pod = eng.bind_model(ABCset)
     eng.bind_proposal(_abi.SLOT_LOCAL, Local_Proposal)
     eng.bind_proposal(_abi.SLOT_IMPORTANCE, Importance_Proposal)

@@ -8,7 +8,8 @@ import torch
 from . import _abi
 from .engine import RunStats, get_engine
 from .models import UserModel
-from .samplers import _LAYOUT, default_seed, print_summary, run_chains, write_csv
+from .samplers import (_LAYOUT, continuation, default_seed, load_checkpoint, print_summary, run_chains, save_checkpoint,
+                       write_csv)
 
 
 def GlobalMCMC(ABCset, num_ite, Initial_theta, Initial_y, Global_Proposal, filelocation, global_frequency,
@@ -30,7 +31,8 @@ def GlobalMCMC(ABCset, num_ite, Initial_theta, Initial_y, Global_Proposal, filel
     if isinstance(ABCset, UserModel):
         eng.bind_proposal(_abi.SLOT_GLOBAL, Global_Proposal)
         return run_user_model(eng, ABCset, "global", num_ite, Initial_theta, Initial_y, Local_Proposal, filelocation,
-                              global_frequency, num_chains, seed, chain_id_base, trace, return_stats, verbose, block_threads)
+                              global_frequency, num_chains, seed, chain_id_base, trace, return_stats, verbose, block_threads,
+                              checkpoint=checkpoint, resume=resume)
     pod = eng.bind_model(ABCset)
     eng.bind_proposal(_abi.SLOT_LOCAL, Local_Proposal)
     eng.bind_proposal(_abi.SLOT_GLOBAL, Global_Proposal)
@@ -41,34 +43,57 @@ def GlobalMCMC(ABCset, num_ite, Initial_theta, Initial_y, Global_Proposal, filel
 
 
 def run_user_model(eng, model, sampler, num_ite, Initial_theta, Initial_y, Local_Proposal, filelocation, gf, num_chains,
-                   seed, chain_id_base, trace, return_stats, verbose, block_threads, K=0, num_grad=0, tau=0.0):
-    """GlobalMCMC / GLMCMC for a run-time compiled `UserModel` (glabc_run_global_user / glabc_run_isir_user); the caller has
-    bound the sampler's state-independent proposal (GLOBAL / IMPORTANCE slot)."""
+                   seed, chain_id_base, trace, return_stats, verbose, block_threads, K=0, num_grad=0, tau=0.0, checkpoint=None,
+                   resume=None):
+    """GlobalMCMC / GLMCMC / GLMALA for a run-time compiled `UserModel` (glabc_run_{global,isir,mala}_user); the caller has
+    bound the sampler's state-independent proposal (GLOBAL / IMPORTANCE slot).  `Initial_y=None` draws y0 of chain c with the
+    model's simulator (glabc_user_simulate, Philox id chain_id_base + c at step 0), so y0 does not depend on the sharding.
+    `checkpoint=` / `resume=` as in samplers.run_chains; the checkpoint also names the model (UserModel.fingerprint), and a
+    resume refuses one written for another model or by another sampler (a built-in run's included)."""
     if num_ite < 1:
         raise ValueError("num_ite must be at least 1")
-    if Initial_y is None:
-        raise ValueError("a UserModel run needs Initial_y (the library cannot call the simulator outside the kernel)")
+    if trace not in _LAYOUT:
+        raise ValueError(f"trace must be one of {sorted(_LAYOUT)}")
     if sampler != "mala":
         eng.bind_proposal(_abi.SLOT_LOCAL, Local_Proposal)
     d, yd = model.theta_dim, model.y_dim
-    seed = default_seed() if seed is None else int(seed)
-    theta = torch.as_tensor(Initial_theta, dtype=torch.float32).reshape(-1, d)
-    c = num_chains if num_chains is not None else theta.shape[0]
-    y = torch.as_tensor(Initial_y, dtype=torch.float32).reshape(-1, yd)
-    if theta.shape[0] not in (1, c) or y.shape[0] not in (1, c):
-        raise ValueError(f"Initial_theta / Initial_y must have 1 or {c} rows")
-    theta = theta.to(eng.device).expand(c, d).contiguous().clone()
-    y = y.to(eng.device).expand(c, yd).contiguous().clone()
-    single = num_chains is None and c == 1
+    name = sampler + "_user"
     layout = _LAYOUT[trace]
-    stats = torch.zeros(c, _abi.nstats(d), dtype=torch.float32, device=eng.device)
-    aux = None
-    if sampler in ("isir", "mala"):
-        aux = torch.zeros(c, _abi.AUX_SLOTS, dtype=torch.float32, device=eng.device)
-        aux[:, _abi.AUX_LOCAL] = 1.0                        # `local` starts True, GLMCMC.py:49-55
-    out = eng.run_user(model, theta=theta, y=y, n_steps=num_ite - 1, gf=gf, seed=seed, chain_id_base=chain_id_base,
+    resumed = {}
+    if resume is not None:
+        ck = load_checkpoint(resume, name, eng.device)
+        if ck.get("model") != model.fingerprint():
+            raise ValueError("the checkpoint was written for another user model (source, dims, params or epsilon differ)")
+        theta, y, stats, aux = ck["theta"], ck["y"], ck["stats"], ck["aux"]
+        seed, chain_id_base, c = ck["seed"], ck["chain_id_base"], theta.shape[0]
+        resumed, layout = continuation(ck["step_base"], num_ite, layout)
+    else:
+        seed = default_seed() if seed is None else int(seed)
+        theta = torch.as_tensor(Initial_theta, dtype=torch.float32).reshape(-1, d)
+        c = num_chains if num_chains is not None else theta.shape[0]
+        if theta.shape[0] not in (1, c):
+            raise ValueError(f"Initial_theta must have 1 or {c} rows")
+        theta = theta.to(eng.device).expand(c, d).contiguous().clone()
+        if Initial_y is None:
+            y = eng.user_simulate(model, theta, seed, row_base=chain_id_base)
+        else:
+            y = torch.as_tensor(Initial_y, dtype=torch.float32).reshape(-1, yd)
+            if y.shape[0] not in (1, c):
+                raise ValueError(f"Initial_y must have 1 or {c} rows")
+            y = y.to(eng.device).expand(c, yd).contiguous().clone()
+        stats = torch.zeros(c, _abi.nstats(d), dtype=torch.float32, device=eng.device)
+        aux = None
+        if sampler in ("isir", "mala"):
+            aux = torch.zeros(c, _abi.AUX_SLOTS, dtype=torch.float32, device=eng.device)
+            aux[:, _abi.AUX_LOCAL] = 1.0                        # `local` starts True, GLMCMC.py:49-55
+    single = num_chains is None and c == 1
+    step_base = resumed.get("step_base", 0)
+    out = eng.run_user(model, theta=theta, y=y, n_steps=num_ite - 1 - step_base, gf=gf, seed=seed, chain_id_base=chain_id_base,
                        trace_layout=layout, stats=stats, block_threads=block_threads, sampler=sampler, K=K, aux=aux,
-                       num_grad=num_grad, tau=tau)
+                       num_grad=num_grad, tau=tau, **resumed)
+    if checkpoint is not None:
+        save_checkpoint(checkpoint, sampler=name, step_base=num_ite - 1, seed=seed, chain_id_base=chain_id_base, theta=theta, y=y,
+                        stats=stats, aux=aux, model=model.fingerprint())
     rs = RunStats(stats, d)
     if single:
         result = (out[0] if layout == _abi.TRACE_CHAIN_MAJOR else out[:, 0]).cpu() if out is not None else None

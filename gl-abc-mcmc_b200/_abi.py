@@ -105,6 +105,7 @@ class BlockIsirPOD(C.Structure):
 
 
 USER_MAX_PARAMS, USER_MAX_NOISE = 64, 32
+USER_SIMULATE, USER_PRIOR, USER_DISCREPANCY, USER_LOG_KERNEL = range(4)
 
 
 class UserModelPOD(C.Structure):
@@ -149,6 +150,10 @@ _SIGNATURES = {
     "glabc_run_mala_user": (C.c_int, [C.c_void_p, C.POINTER(RunPOD), C.POINTER(UserModelPOD)]),
     "glabc_user_model_check": (C.c_int, [C.POINTER(UserModelPOD), C.c_int32, C.c_char_p, C.c_size_t]),
     "glabc_user_model_check_proposals": (C.c_int, [C.POINTER(UserModelPOD), C.c_int32, C.c_int32, C.c_int32, C.c_char_p, C.c_size_t]),
+    "glabc_user_simulate": (C.c_int, [C.c_void_p, C.POINTER(UserModelPOD), C.c_void_p, C.c_int64, C.c_uint64, C.c_uint64,
+                                      C.c_void_p, C.c_void_p]),
+    "glabc_user_evaluate": (C.c_int, [C.c_void_p, C.POINTER(UserModelPOD), C.c_int32, C.c_void_p, C.c_int64, C.c_void_p,
+                                      C.c_void_p]),
     "glabc_run_global_host": (C.c_int, [C.c_void_p, C.POINTER(RunPOD), C.c_int64]),
     "glabc_run_isir": (C.c_int, [C.c_void_p, C.POINTER(RunPOD)]),
     "glabc_run_isir_host": (C.c_int, [C.c_void_p, C.POINTER(RunPOD), C.c_int64]),

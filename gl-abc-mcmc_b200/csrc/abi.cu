@@ -1375,16 +1375,31 @@ extern "C" int glabc_user_model_check(const glabc_user_model_t* um, int32_t cc, 
     return glabc_user_model_check_proposals(um, GLABC_DIST_DIAG_GAUSSIAN, GLABC_DIST_DIAG_GAUSSIAN, cc, log, log_cap);
 }
 
-static int run_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_user_model_t* um, int kind)
+// the checks of a user model every entry that launches one of its kernels makes first
+static int check_user_model(glabc_ctx* ctx, const glabc_user_model_t* um, const char* who)
 {
-    const bool isir = kind >= 1, mala = kind == 2;   // 0 GlobalMCMC, 1 GLMCMC (iSIR), 2 GLMALA
-    if (!ctx) return GLABC_ERR_INVALID;
-    if (!um || !um->source) return fail(ctx, GLABC_ERR_INVALID, "glabc_run_*_user: null model / source");
+    if (!um || !um->source) return fail(ctx, GLABC_ERR_INVALID, "%s: null model / source", who);
     if (um->theta_dim < 1 || um->theta_dim > GLABC_MAX_DIM || um->y_dim < 1 || um->y_dim > 2 * GLABC_MAX_DIM)
         return fail(ctx, GLABC_ERR_INVALID, "user model: theta_dim in 1..%d, y_dim in 1..%d", GLABC_MAX_DIM, 2 * GLABC_MAX_DIM);
     if (um->n_noise < 0 || um->n_noise > GLABC_USER_MAX_NOISE || um->n_params < 0 || um->n_params > GLABC_USER_MAX_PARAMS)
         return fail(ctx, GLABC_ERR_INVALID, "user model: n_noise in 0..%d, n_params in 0..%d", GLABC_USER_MAX_NOISE, GLABC_USER_MAX_PARAMS);
     if (!(um->epsilon > 0.0)) return fail(ctx, GLABC_ERR_INVALID, "user model: epsilon must be positive");
+    return GLABC_OK;
+}
+
+// log K(dis) = kern_c + kern_m * dis^2, the Gaussian ABC kernel of width epsilon (Mixture.py:38-53)
+static void user_kernel_consts(const glabc_user_model_t& um, float* kern_c, float* kern_m)
+{
+    const float eps = static_cast<float>(um.epsilon);
+    *kern_c = static_cast<float>(-0.5 * std::log(2.0 * M_PI)) - std::log(eps);
+    *kern_m = -0.5f / (eps * eps);
+}
+
+static int run_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_user_model_t* um, int kind)
+{
+    const bool isir = kind >= 1, mala = kind == 2;   // 0 GlobalMCMC, 1 GLMCMC (iSIR), 2 GLMALA
+    if (!ctx) return GLABC_ERR_INVALID;
+    if (int st = check_user_model(ctx, um, "glabc_run_*_user")) return st;
     const int d = um->theta_dim;
     const int far_slot = isir ? GLABC_SLOT_IMPORTANCE : GLABC_SLOT_GLOBAL;   // the state-independent proposal of the sampler
     for (int slot : {mala ? far_slot : static_cast<int>(GLABC_SLOT_LOCAL), far_slot}) {
@@ -1460,9 +1475,7 @@ static int run_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_user_mod
     }
     U.lq = make_dist<GLABC_MAX_DIM>(lp);   // read by the kernels compiled for a Uniform / Gamma / GaussianMixture slot
     U.gq = make_dist<GLABC_MAX_DIM>(gp);
-    const float eps = static_cast<float>(um->epsilon);
-    U.kern_c = static_cast<float>(-0.5 * std::log(2.0 * M_PI)) - std::log(eps);
-    U.kern_m = -0.5f / (eps * eps);
+    user_kernel_consts(*um, &U.kern_c, &U.kern_m);
     for (int k = 0; k < um->n_params; ++k) U.params[k] = um->params[k];
     st = user_model_launch(fn, U, mala ? 64 : (block > 128 ? 128 : block), static_cast<cudaStream_t>(run->stream), err);
     if (st) return fail(ctx, st, "%s", err.c_str());
@@ -1472,6 +1485,53 @@ static int run_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_user_mod
 extern "C" int glabc_run_global_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_user_model_t* um) { return run_user(ctx, run, um, 0); }
 extern "C" int glabc_run_isir_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_user_model_t* um) { return run_user(ctx, run, um, 1); }
 extern "C" int glabc_run_mala_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_user_model_t* um) { return run_user(ctx, run, um, 2); }
+
+// glabc_k_eval_user on n rows; the caller has checked ctx, the model, n and the buffers
+static int eval_user(glabc_ctx* ctx, const glabc_user_model_t* um, int op, const float* in, int64_t n, uint64_t seed,
+                     uint64_t row_base, float* out, void* stream)
+{
+    if (n == 0) return GLABC_OK;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    CUDA_TRY(ctx, cudaFree(nullptr));   // the primary context, current for the driver calls
+    void* fn = nullptr;
+    std::string err;
+    int st = user_model_eval_fn(ctx->device, ctx->cc, *um, &fn, err);
+    if (st) return fail(ctx, st, "%s", err.c_str());
+    UserEval E{};
+    E.n = n;
+    E.op = op;
+    E.row_lo = static_cast<uint32_t>(row_base);
+    E.row_hi = static_cast<uint32_t>(row_base >> 32);
+    E.key0 = static_cast<uint32_t>(seed);
+    E.key1 = static_cast<uint32_t>(seed >> 32);
+    E.in = in;
+    E.out = out;
+    user_kernel_consts(*um, &E.kern_c, &E.kern_m);
+    for (int k = 0; k < um->n_params; ++k) E.params[k] = um->params[k];
+    st = user_model_eval_launch(fn, E, ctx->sm_count, static_cast<cudaStream_t>(stream), err);
+    if (st) return fail(ctx, st, "%s", err.c_str());
+    return GLABC_OK;
+}
+
+extern "C" int glabc_user_simulate(glabc_ctx* ctx, const glabc_user_model_t* um, const float* theta, int64_t n, uint64_t seed,
+                                   uint64_t row_base, float* y, void* stream)
+{
+    if (!ctx) return GLABC_ERR_INVALID;
+    if (int st = check_user_model(ctx, um, "glabc_user_simulate")) return st;
+    if (n < 0 || (n > 0 && (!theta || !y))) return fail(ctx, GLABC_ERR_INVALID, "glabc_user_simulate: null buffer / n < 0");
+    return eval_user(ctx, um, GLABC_USER_SIMULATE, theta, n, seed, row_base, y, stream);
+}
+
+extern "C" int glabc_user_evaluate(glabc_ctx* ctx, const glabc_user_model_t* um, int32_t op, const float* x, int64_t n, float* out,
+                                   void* stream)
+{
+    if (!ctx) return GLABC_ERR_INVALID;
+    if (int st = check_user_model(ctx, um, "glabc_user_evaluate")) return st;
+    if (op != GLABC_USER_PRIOR && op != GLABC_USER_DISCREPANCY && op != GLABC_USER_LOG_KERNEL)
+        return fail(ctx, GLABC_ERR_INVALID, "glabc_user_evaluate: unknown op %d", op);
+    if (n < 0 || (n > 0 && (!x || !out))) return fail(ctx, GLABC_ERR_INVALID, "glabc_user_evaluate: null buffer / n < 0");
+    return eval_user(ctx, um, op, x, n, 0, 0, out, stream);
+}
 
 
 // ---------------------------------------------------------------------------------------------

@@ -161,4 +161,17 @@ struct UserRun {
     DistConstsT<GLABC_MAX_DIM> lq, gq;   // Local_Proposal; Global_Proposal (GlobalMCMC) or Importance_Proposal
 };
 
+// kernel parameter of the user-model evaluation kernel glabc_k_eval_user (user_model.cu): one row per thread,
+// op = glabc_user_op (include/glabc.h)
+struct UserEval {
+    long long n;              // rows
+    int op, pad;
+    unsigned row_lo, row_hi;  // SIMULATE: Philox chain id of row 0 (row r draws from row_base + r)
+    unsigned key0, key1;      // SIMULATE: the seed
+    const float* in;          // theta [n][D] (SIMULATE, PRIOR) or y [n][YD] (DISCREPANCY, LOG_KERNEL)
+    float* out;               // y [n][YD] (SIMULATE) or [n]
+    float kern_c, kern_m;     // LOG_KERNEL: as UserRun
+    float params[GLABC_USER_MAX_PARAMS];
+};
+
 }  // namespace glabc

@@ -49,6 +49,7 @@ typedef unsigned long long u64;
 #endif
 #include "dist_device.cuh"
 using glabc::UserRun;
+using glabc::UserEval;
 // A prior may return exactly this value to say "outside the support: draw the local proposal again" — the reference's
 // `while prior_log_prob(theta') == 7 * np.log(1e-10)` (GLMCMC.py:92-93; the float32 tensor is compared with the float64
 // scalar cast down to float32)
@@ -110,6 +111,9 @@ struct GlabcWords {
     }
 };
 // Philox slots (the counter's last word) the user kernels draw from, per (chain, step):
+//   step 0, 2 ..             glabc_k_eval_user's SIMULATE: ceil(NN / 4) blocks of the simulator's normals for row
+//                            row_base + r.  The step kernels draw only at steps step_base + 1 .. (the loop index i >= 1),
+//                            so step 0 is never used by a run, and y0 of chain c is the SIMULATE row chain_id_base + c.
 //   1                        the step's coin and MH uniform
 //   2 ..                     NB blocks of normals: a DiagGaussian proposal's D, then the simulator's NN
 //   0x100 + j NB ..          the same for iSIR candidate j < GLABC_MAX_K
@@ -758,6 +762,50 @@ extern "C" __global__ void __launch_bounds__(64) glabc_k_mala_user(const __grid_
         for (int k = 0; k < D * (D + 1) / 2; ++k) st[4 + 2 * D + k] += gram[k];
     }
 }
+
+// ---- the model's functions outside a run: generate_samples / prior_log_prob / discrepancy / calculate_log_kernel ------
+// One row per thread, grid-stride.  SIMULATE row r draws its NN normals as a step kernel draws its simulator noise, from the
+// Philox blocks (row_base + r, step 0, slot 2 + b): step 0 is no step's, see the slot table.
+extern "C" __global__ void __launch_bounds__(256) glabc_k_eval_user(const __grid_constant__ UserEval E)
+{
+    const u64 row0 = (u64)E.row_hi << 32 | E.row_lo;
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    const long long first = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (E.op == GLABC_USER_SIMULATE) {
+        constexpr int NB = (NN + 3) / 4;
+        for (long long r = first; r < E.n; r += stride) {
+            float th[D], y[YD], z[NB > 0 ? NB * 4 : 4];
+#pragma unroll
+            for (int k = 0; k < D; ++k) th[k] = E.in[r * D + k];
+            const u64 gid = row0 + (u64)r;
+#pragma unroll
+            for (int b = 0; b < NB; ++b) {
+                const uint4 w = glabc_philox((u32)gid, (u32)(gid >> 32), 0u, 2u + b, E.key0, E.key1);
+                glabc_box_muller(w.x, w.y, z[4 * b], z[4 * b + 1]);
+                glabc_box_muller(w.z, w.w, z[4 * b + 2], z[4 * b + 3]);
+            }
+            glabc_user_simulate(th, z, E.params, y);
+#pragma unroll
+            for (int k = 0; k < YD; ++k) E.out[r * YD + k] = y[k];
+        }
+    } else if (E.op == GLABC_USER_PRIOR) {
+        for (long long r = first; r < E.n; r += stride) {
+            float th[D];
+#pragma unroll
+            for (int k = 0; k < D; ++k) th[k] = E.in[r * D + k];
+            E.out[r] = glabc_user_prior_log_prob(th, E.params);
+        }
+    } else {                                   // DISCREPANCY, LOG_KERNEL (the kernel term of glabc_target)
+        const bool log_kernel = E.op == GLABC_USER_LOG_KERNEL;
+        for (long long r = first; r < E.n; r += stride) {
+            float y[YD];
+#pragma unroll
+            for (int k = 0; k < YD; ++k) y[k] = E.in[r * YD + k];
+            const float dis = glabc_user_discrepancy(y, E.params);
+            E.out[r] = log_kernel ? fmaf(E.kern_m, dis * dis, E.kern_c) : dis;
+        }
+    }
+}
 )GLABC";
 
 // ---- lazily bound NVRTC / driver entry points --------------------------------------------------------------------
@@ -829,9 +877,20 @@ struct Compiled {
     CUfunction fn = nullptr;        // glabc_k_global_user
     CUfunction fn_isir = nullptr;   // glabc_k_isir_user
     CUfunction fn_mala = nullptr;   // glabc_k_mala_user (models with theta_dim <= 5: the gradient is cached in the aux slots)
+    CUfunction fn_eval = nullptr;   // glabc_k_eval_user
 };
 std::mutex g_cache_mu;
-std::map<std::string, Compiled> g_cache;   // key: device | arch | dims | proposal kinds | source
+// key: model_key() + proposal kinds, so the modules of one model are adjacent in the map
+std::map<std::string, Compiled> g_cache;
+
+// device | arch | dims | n_noise | source length | source: names a model, whatever the proposal kinds it was compiled for
+std::string model_key(int device, int cc, const glabc_user_model_t& um)
+{
+    const size_t len = strlen(um.source);
+    char head[160];
+    snprintf(head, sizeof(head), "%d|%d|%d|%d|%d|%zu|", device, cc, um.theta_dim, um.y_dim, um.n_noise, len);
+    return std::string(head) + std::string(um.source, len);
+}
 
 std::string cu_err(Dyn& d, CUresult r)
 {
@@ -871,8 +930,13 @@ static int compile_to_cubin(Dyn& d, int cc, const glabc_user_model_t& um, int lp
     snprintf(sizes[0], sizeof(sizes[0]), "-DGLABC_MAX_DIM=%d", GLABC_MAX_DIM);
     snprintf(sizes[1], sizeof(sizes[1]), "-DGLABC_MAX_MODES=%d", GLABC_MAX_MODES);
     snprintf(sizes[2], sizeof(sizes[2]), "-DGLABC_USER_MAX_PARAMS=%d", GLABC_USER_MAX_PARAMS);
+    char ops[4][40];   // glabc_k_eval_user's operations
+    snprintf(ops[0], sizeof(ops[0]), "-DGLABC_USER_SIMULATE=%d", GLABC_USER_SIMULATE);
+    snprintf(ops[1], sizeof(ops[1]), "-DGLABC_USER_PRIOR=%d", GLABC_USER_PRIOR);
+    snprintf(ops[2], sizeof(ops[2]), "-DGLABC_USER_DISCREPANCY=%d", GLABC_USER_DISCREPANCY);
+    snprintf(ops[3], sizeof(ops[3]), "-DGLABC_USER_LOG_KERNEL=%d", GLABC_USER_LOG_KERNEL);
     const char* opts[] = {arch, dD, dY, dN, dLP, dGP, kinds[0], kinds[1], kinds[2], kinds[3], sizes[0], sizes[1], sizes[2],
-                          "--std=c++17", "--use_fast_math", "-lineinfo"};
+                          ops[0], ops[1], ops[2], ops[3], "--std=c++17", "--use_fast_math", "-lineinfo"};
     r = d.compileProgram(prog, static_cast<int>(sizeof(opts) / sizeof(opts[0])), opts);
     if (r != NVRTC_SUCCESS) {
         size_t n = 0;
@@ -902,21 +966,16 @@ int user_model_check(int cc, const glabc_user_model_t& um, int lp_kind, int gp_k
     return compile_to_cubin(d, cc, um, lp_kind, gp_kind, cubin, err);
 }
 
-int user_model_compile(int device, int cc, const glabc_user_model_t& um, int lp_kind, int gp_kind, int kind, void** fn_out,
+// the module of (model, proposal kinds): from the cache, or compiled and loaded.  Called with g_cache_mu held.
+static int load_module(Dyn& d, int device, int cc, const glabc_user_model_t& um, int lp_kind, int gp_kind, const Compiled** out,
                        std::string& err)
 {
-    Dyn& d = dyn();
-    if (!d.ok) {
-        err = d.why;
-        return GLABC_ERR_UNSUPPORTED;
-    }
-    char head[160];
-    snprintf(head, sizeof(head), "%d|%d|%d|%d|%d|%d|%d|", device, cc, um.theta_dim, um.y_dim, um.n_noise, lp_kind, gp_kind);
-    const std::string key = std::string(head) + um.source;
-    std::lock_guard<std::mutex> lock(g_cache_mu);
+    char kinds[32];
+    snprintf(kinds, sizeof(kinds), "|%d|%d", lp_kind, gp_kind);
+    const std::string key = model_key(device, cc, um) + kinds;
     auto it = g_cache.find(key);
     if (it != g_cache.end()) {
-        *fn_out = kind == 2 ? it->second.fn_mala : kind == 1 ? it->second.fn_isir : it->second.fn;
+        *out = &it->second;
         return GLABC_OK;
     }
     std::vector<char> cubin;
@@ -928,37 +987,64 @@ int user_model_compile(int device, int cc, const glabc_user_model_t& um, int lp_
         err = "cuModuleLoadData: " + cu_err(d, cr);
         return GLABC_ERR_CUDA;
     }
-    cr = d.moduleGetFunction(&c.fn, c.mod, "glabc_k_global_user");
-    if (cr != CUDA_SUCCESS) {
-        err = "cuModuleGetFunction: " + cu_err(d, cr);
-        return GLABC_ERR_CUDA;
+    const std::pair<CUfunction*, const char*> fns[] = {{&c.fn, "glabc_k_global_user"}, {&c.fn_isir, "glabc_k_isir_user"},
+                                                       {&c.fn_mala, "glabc_k_mala_user"}, {&c.fn_eval, "glabc_k_eval_user"}};
+    for (const auto& f : fns) {
+        cr = d.moduleGetFunction(f.first, c.mod, f.second);
+        if (cr != CUDA_SUCCESS) {
+            err = "cuModuleGetFunction: " + cu_err(d, cr);
+            return GLABC_ERR_CUDA;
+        }
     }
-    cr = d.moduleGetFunction(&c.fn_isir, c.mod, "glabc_k_isir_user");
-    if (cr != CUDA_SUCCESS) {
-        err = "cuModuleGetFunction: " + cu_err(d, cr);
-        return GLABC_ERR_CUDA;
-    }
-    cr = d.moduleGetFunction(&c.fn_mala, c.mod, "glabc_k_mala_user");
-    if (cr != CUDA_SUCCESS) {
-        err = "cuModuleGetFunction: " + cu_err(d, cr);
-        return GLABC_ERR_CUDA;
-    }
-    g_cache[key] = c;
-    *fn_out = kind == 2 ? c.fn_mala : kind == 1 ? c.fn_isir : c.fn;
+    *out = &(g_cache[key] = c);
     return GLABC_OK;
 }
 
-int user_model_launch(void* fn, const UserRun& R, int block, cudaStream_t st, std::string& err)
+int user_model_compile(int device, int cc, const glabc_user_model_t& um, int lp_kind, int gp_kind, int kind, void** fn_out,
+                       std::string& err)
 {
     Dyn& d = dyn();
     if (!d.ok) {
         err = d.why;
         return GLABC_ERR_UNSUPPORTED;
     }
-    if (R.n_chains <= 0) return GLABC_OK;
-    UserRun copy = R;
-    void* args[] = {&copy};
-    const unsigned grid = static_cast<unsigned>((R.n_chains + block - 1) / block);
+    std::lock_guard<std::mutex> lock(g_cache_mu);
+    const Compiled* c = nullptr;
+    const int st = load_module(d, device, cc, um, lp_kind, gp_kind, &c, err);
+    if (st) return st;
+    *fn_out = kind == 2 ? c->fn_mala : kind == 1 ? c->fn_isir : c->fn;
+    return GLABC_OK;
+}
+
+int user_model_eval_fn(int device, int cc, const glabc_user_model_t& um, void** fn_out, std::string& err)
+{
+    Dyn& d = dyn();
+    if (!d.ok) {
+        err = d.why;
+        return GLABC_ERR_UNSUPPORTED;
+    }
+    std::lock_guard<std::mutex> lock(g_cache_mu);
+    const std::string prefix = model_key(device, cc, um) + "|";   // then only the proposal kinds follow
+    auto it = g_cache.lower_bound(prefix);
+    if (it != g_cache.end() && it->first.compare(0, prefix.size(), prefix) == 0) {
+        *fn_out = it->second.fn_eval;
+        return GLABC_OK;
+    }
+    const Compiled* c = nullptr;
+    const int st = load_module(d, device, cc, um, GLABC_DIST_DIAG_GAUSSIAN, GLABC_DIST_DIAG_GAUSSIAN, &c, err);
+    if (st) return st;
+    *fn_out = c->fn_eval;
+    return GLABC_OK;
+}
+
+static int launch(void* fn, void* param, unsigned grid, int block, cudaStream_t st, std::string& err)
+{
+    Dyn& d = dyn();
+    if (!d.ok) {
+        err = d.why;
+        return GLABC_ERR_UNSUPPORTED;
+    }
+    void* args[] = {param};
     const CUresult cr = d.launchKernel(static_cast<CUfunction>(fn), grid, 1, 1, static_cast<unsigned>(block), 1, 1, 0,
                                        reinterpret_cast<CUstream>(st), args, nullptr);
     if (cr != CUDA_SUCCESS) {
@@ -966,6 +1052,23 @@ int user_model_launch(void* fn, const UserRun& R, int block, cudaStream_t st, st
         return GLABC_ERR_CUDA;
     }
     return GLABC_OK;
+}
+
+int user_model_launch(void* fn, const UserRun& R, int block, cudaStream_t st, std::string& err)
+{
+    if (R.n_chains <= 0) return GLABC_OK;
+    UserRun copy = R;
+    return launch(fn, &copy, static_cast<unsigned>((R.n_chains + block - 1) / block), block, st, err);
+}
+
+int user_model_eval_launch(void* fn, const UserEval& E, int sm_count, cudaStream_t st, std::string& err)
+{
+    if (E.n <= 0) return GLABC_OK;
+    constexpr int block = 256;   // glabc_k_eval_user's __launch_bounds__
+    // a grid-stride loop: enough blocks to fill every SM several times over, fewer for a small n
+    const long long want = (E.n + block - 1) / block, cap = 32LL * (sm_count > 0 ? sm_count : 1);
+    UserEval copy = E;
+    return launch(fn, &copy, static_cast<unsigned>(want < cap ? want : cap), block, st, err);
 }
 
 }  // namespace glabc

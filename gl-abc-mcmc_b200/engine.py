@@ -154,25 +154,47 @@ class Engine:
         return trace
 
     def run_user(self, model, *, theta, y, n_steps, gf, step_base=0, chain_id_base=0, seed=0, trace_layout=_abi.TRACE_CHAIN_MAJOR,
-                 trace=None, trace_rows=None, write_row0=True, stats=None, block_threads=0, sampler="global", K=0, aux=None,
-                 num_grad=0, tau=0.0):
+                 trace=None, trace_rows=None, trace_row_base=0, write_row0=True, stats=None, block_threads=0, sampler="global", K=0,
+                 aux=None, num_grad=0, tau=0.0):
         """GlobalMCMC (`sampler="global"`, LOCAL / GLOBAL slots), GLMCMC (`"isir"`, LOCAL / IMPORTANCE slots, K candidates, aux) or
         GLMALA (`"mala"`, IMPORTANCE slot, K, tau, num_grad, aux) transitions for a `models.UserModel` (compiled on first use)"""
         cn, d = theta.shape
-        rows = trace_rows if trace_rows is not None else step_base + n_steps + 1
+        rows = trace_rows if trace_rows is not None else step_base + n_steps + 1 - trace_row_base
         if trace is None and trace_layout != _abi.TRACE_NONE:
             shape = (rows, cn, d) if trace_layout == _abi.TRACE_TIME_MAJOR else (cn, rows, d)
             trace = torch.empty(shape, dtype=torch.float32, device=self.device)
         r = _abi.RunPOD(n_chains=cn, n_steps=n_steps, step_base=step_base, chain_id_base=chain_id_base,
                         seed=int(seed) & 0xFFFFFFFFFFFFFFFF, global_frequency=float(gf), rng_mode=_abi.RNG_NATIVE,
                         arith_mode=_abi.ARITH_FAST, trace_layout=trace_layout, write_row0=int(write_row0),
-                        block_threads=block_threads, n_candidates=int(K), trace_rows=rows, trace_chains=cn, theta=self._ptr(theta),
-                        y=self._ptr(y), aux=self._ptr(aux), trace=self._ptr(trace), stats=self._ptr(stats), stream=self._stream(),
-                        num_grad=int(num_grad), tau=float(tau), tau64=float(tau))
+                        block_threads=block_threads, n_candidates=int(K), trace_rows=rows, trace_chains=cn,
+                        trace_row_base=trace_row_base, theta=self._ptr(theta), y=self._ptr(y), aux=self._ptr(aux),
+                        trace=self._ptr(trace), stats=self._ptr(stats), stream=self._stream(), num_grad=int(num_grad), tau=float(tau),
+                        tau64=float(tau))
         pod = model.user_pod()
         fn = {"isir": self.lib.glabc_run_isir_user, "mala": self.lib.glabc_run_mala_user}.get(sampler, self.lib.glabc_run_global_user)
         self.ctx.check(fn(self.ctx.handle, C.byref(r), C.byref(pod)))
         return trace
+
+    def user_simulate(self, model, theta, seed, row_base=0):
+        """y [n, y_dim]: one draw of a `models.UserModel`'s simulator per row of theta [n, theta_dim] (glabc_user_simulate;
+        row r draws from the Philox stream of id row_base + r at step 0)"""
+        theta = self._f32(theta).reshape(-1, model.theta_dim)
+        y = torch.empty(theta.shape[0], model.y_dim, dtype=torch.float32, device=self.device)
+        pod = model.user_pod()
+        self.ctx.check(self.lib.glabc_user_simulate(self.ctx.handle, C.byref(pod), self._ptr(theta), theta.shape[0],
+                                                    int(seed) & 0xFFFFFFFFFFFFFFFF, int(row_base) & 0xFFFFFFFFFFFFFFFF,
+                                                    self._ptr(y), self._stream()))
+        return y
+
+    def user_evaluate(self, model, op, x):
+        """out [n]: the prior (op USER_PRIOR, x = theta rows), discrepancy (USER_DISCREPANCY, x = y rows) or log ABC kernel
+        (USER_LOG_KERNEL) of a `models.UserModel` (glabc_user_evaluate)"""
+        x = self._f32(x).reshape(-1, model.theta_dim if op == _abi.USER_PRIOR else model.y_dim)
+        out = torch.empty(x.shape[0], dtype=torch.float32, device=self.device)
+        pod = model.user_pod()
+        self.ctx.check(self.lib.glabc_user_evaluate(self.ctx.handle, C.byref(pod), int(op), self._ptr(x), x.shape[0], self._ptr(out),
+                                                    self._stream()))
+        return out
 
     def aglmcmc_params(self, *, step_size, alpha, hat_eps_T, rule=_abi.BW_SILVERMAN, init=True, init_p=None, init_s=None,
                        ad_idx=None, ad_noise=None, ad_sim=None, ad_rec=None, ad_blk=None, init_w=None):

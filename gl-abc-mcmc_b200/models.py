@@ -11,6 +11,9 @@ Its torch methods follow the reference formulas (usable on CPU or CUDA tensors, 
 `Mixture_set` instance (duck-typed probe of its deterministic methods) so existing user scripts can
 pass their own model object unchanged.
 """
+import hashlib
+import struct
+
 import torch
 
 from . import _abi
@@ -128,7 +131,11 @@ class UserModel:
         __device__ float glabc_user_discrepancy(const float* y, const float* params);
 
     `noise` holds `n_noise` independent N(0,1) draws per simulator call, `params` the model's constants.  The Gaussian
-    ABC kernel of width `epsilon` (Mixture.py:38-53) stays the library's.  `check()` compiles the source without a GPU."""
+    ABC kernel of width `epsilon` (Mixture.py:38-53) stays the library's.  `check()` compiles the source without a GPU.
+
+    The plugin methods (`generate_samples`, `prior_log_prob`, `discrepancy`, `calculate_log_kernel`) run the compiled
+    functions on the GPU (glabc_user_simulate / glabc_user_evaluate): inputs on any device, float32 outputs on the engine's
+    device.  There is no `y_obs`: the observation lives in `params`, and the fused-family samplers refuse the object."""
 
     def __init__(self, source, theta_dim, y_dim, n_noise, epsilon, params=()):
         self.source, self.theta_dim, self.y_dim, self.n_noise = str(source), int(theta_dim), int(y_dim), int(n_noise)
@@ -136,6 +143,63 @@ class UserModel:
         self.params = [float(p) for p in params]
         if len(self.params) > _abi.USER_MAX_PARAMS:
             raise ValueError(f"at most {_abi.USER_MAX_PARAMS} params")
+
+    # -- plugin methods (reference Mixture.py:13-53), compiled -----------------------------------
+    def generate_samples(self, theta, num_samples=1, *, seed=None, row_base=0):
+        """Simulator draws, shaped as AbsNormalModel.generate_samples: theta [d] or [1, d] -> [m, y_dim]; [n, d] -> [n, y_dim]
+        for m = 1 and [n, m, y_dim] for m > 1.  Row i * m + j (repeat j of theta row i) draws its noise from the Philox stream
+        of id row_base + i * m + j at step 0 under key `seed` (default: samplers.default_seed()), so
+        `generate_samples(theta0, seed=s, row_base=chain_id_base)` is the initial y a run with seed s draws for Initial_y=None."""
+        from .engine import get_engine
+        from .samplers import default_seed
+        eng = get_engine()
+        theta = torch.as_tensor(theta, dtype=torch.float32)
+        if theta.dim() not in (1, 2) or theta.shape[-1] != self.theta_dim:
+            raise ValueError(f"theta must be [{self.theta_dim}] or [n, {self.theta_dim}], got {tuple(theta.shape)}")
+        m = int(num_samples)
+        if m < 1:
+            raise ValueError("num_samples must be at least 1")
+        rows = theta.reshape(-1, self.theta_dim)
+        n = rows.shape[0]
+        seed = default_seed() if seed is None else int(seed)
+        rows = rows.to(eng.device)
+        y = eng.user_simulate(self, rows if m == 1 else rows.repeat_interleave(m, dim=0), seed, row_base)
+        return y if n == 1 or m == 1 else y.view(n, m, self.y_dim)
+
+    def prior_log_prob(self, samples):
+        from .engine import get_engine
+        return get_engine().user_evaluate(self, _abi.USER_PRIOR, torch.as_tensor(samples).reshape(-1, self.theta_dim))
+
+    def discrepancy(self, y):
+        from .engine import get_engine
+        return get_engine().user_evaluate(self, _abi.USER_DISCREPANCY, torch.as_tensor(y).reshape(-1, self.y_dim))
+
+    def calculate_log_kernel_dis(self, dis, epsilon=None):
+        """log N(dis; 0, eps^2), the torch formula of AbsNormalModel.calculate_log_kernel_dis"""
+        from .engine import get_engine
+        dev = get_engine().device
+        eps = self.epsilon if epsilon is None else epsilon
+        eps_t = torch.as_tensor([float(eps)], dtype=torch.float32, device=dev)
+        dis = torch.as_tensor(dis, dtype=torch.float32).to(dev)
+        return DiagGaussian(1, torch.zeros(1, device=dev), torch.log(eps_t)).log_prob(dis.view(-1, 1))
+
+    def calculate_log_kernel(self, y, epsilon=None):
+        """the step kernels' kernel term of the model's epsilon, on the device; another epsilon goes through
+        calculate_log_kernel_dis"""
+        if epsilon is not None and float(epsilon) != self.epsilon:
+            return self.calculate_log_kernel_dis(self.discrepancy(y), epsilon)
+        from .engine import get_engine
+        return get_engine().user_evaluate(self, _abi.USER_LOG_KERNEL, torch.as_tensor(y).reshape(-1, self.y_dim))
+
+    def fingerprint(self):
+        """sha256 of what a run computes with: source, dims, n_noise, params (as the float32 the kernels read) and epsilon.
+        A user-model checkpoint carries it, and a resume refuses a checkpoint of another model."""
+        h = hashlib.sha256()
+        h.update(struct.pack("<4i", self.theta_dim, self.y_dim, self.n_noise, len(self.params)))
+        h.update(torch.tensor(self.params, dtype=torch.float32).numpy().tobytes())
+        h.update(struct.pack("<d", self.epsilon))
+        h.update(self.source.encode())
+        return h.hexdigest()
 
     def user_pod(self):
         pod = _abi.UserModelPOD(theta_dim=self.theta_dim, y_dim=self.y_dim, n_noise=self.n_noise, n_params=len(self.params),

@@ -77,14 +77,17 @@ def print_summary(chain):
 CHECKPOINT_VERSION = 1
 
 
-def save_checkpoint(path, *, sampler, step_base, seed, chain_id_base, theta, y, stats, aux=None, state64=None, ag_state=None):
+def save_checkpoint(path, *, sampler, step_base, seed, chain_id_base, theta, y, stats, aux=None, state64=None, ag_state=None,
+                    model=None):
     """Everything a run needs to continue bit-identically (SURVEY.md 8(f) n4): the chain state, the carried iSIR / MALA
     state, the statistics accumulators and the Philox coordinates (seed, global chain id base, next step index) — the
-    generator itself is stateless, so no RNG state exists beyond these three integers."""
+    generator itself is stateless, so no RNG state exists beyond these three integers.  `model`: a user model's
+    fingerprint (models.UserModel.fingerprint)."""
     cpu = lambda t: None if t is None else t.detach().cpu()  # noqa: E731
+    extra = {} if model is None else dict(model=model)
     torch.save(dict(version=CHECKPOINT_VERSION, sampler=sampler, step_base=int(step_base), seed=int(seed),
                     chain_id_base=int(chain_id_base), theta=cpu(theta), y=cpu(y), stats=cpu(stats), aux=cpu(aux),
-                    state64=cpu(state64), ag_state=cpu(ag_state)), path)
+                    state64=cpu(state64), ag_state=cpu(ag_state), **extra), path)
 
 
 def load_checkpoint(path_or_dict, sampler, device):
@@ -98,6 +101,15 @@ def load_checkpoint(path_or_dict, sampler, device):
                 ag_state=dev(ck.get("ag_state")))
 
 
+def continuation(step_base, num_ite, layout):
+    """(launch arguments, trace layout) of a run resumed at iteration `step_base` up to iteration num_ite - 1: the launch
+    continues the Philox steps and writes only the new rows step_base + 1 .. num_ite - 1; no trace when none is left."""
+    if num_ite - 1 < step_base:
+        raise ValueError(f"the checkpoint is already at iteration {step_base}")
+    kw = dict(step_base=step_base, trace_row_base=step_base + 1, write_row0=False, trace_rows=num_ite - 1 - step_base)
+    return kw, (_abi.TRACE_NONE if num_ite - 1 == step_base else layout)
+
+
 def run_chains(sampler, eng, model_pod, *, num_ite, Initial_theta, Initial_y, global_frequency, filelocation,
                num_chains, seed, chain_id_base, arith, trace, return_stats, verbose, K=0, aux_init=None,
                block_threads=0, checkpoint=None, resume=None, **sampler_kw):
@@ -109,15 +121,15 @@ def run_chains(sampler, eng, model_pod, *, num_ite, Initial_theta, Initial_y, gl
     if trace not in _LAYOUT:
         raise ValueError(f"trace must be one of {sorted(_LAYOUT)}")
     d = model_pod.theta_dim
-    step_base = 0
+    layout = _LAYOUT[trace]
+    resumed = {}
     if resume is not None:
         ck = load_checkpoint(resume, sampler, eng.device)
-        theta, y, stats, aux, step_base = ck["theta"], ck["y"], ck["stats"], ck["aux"], ck["step_base"]
+        theta, y, stats, aux = ck["theta"], ck["y"], ck["stats"], ck["aux"]
         seed, chain_id_base, c = ck["seed"], ck["chain_id_base"], ck["theta"].shape[0]
         if theta.shape[1] != d:
             raise ValueError("checkpoint theta_dim does not match the model")
-        if num_ite - 1 < step_base:
-            raise ValueError(f"the checkpoint is already at iteration {step_base}")
+        resumed, layout = continuation(ck["step_base"], num_ite, layout)
         if "state64" in sampler_kw:
             sampler_kw["state64"] = ck["state64"]
         if sampler == "aglmcmc":     # the chains' candidate blocks, KDEs, counters and eps-hat live in the context's workspace
@@ -136,11 +148,7 @@ def run_chains(sampler, eng, model_pod, *, num_ite, Initial_theta, Initial_y, gl
             for slot, val in aux_init.items():
                 aux[:, slot] = val
     single = num_chains is None and c == 1
-    layout = _LAYOUT[trace]
-    resumed = dict(step_base=step_base, trace_row_base=step_base + 1, write_row0=False,
-                   trace_rows=num_ite - 1 - step_base) if resume is not None else {}
-    if resume is not None and num_ite - 1 == step_base:
-        layout = _abi.TRACE_NONE
+    step_base = resumed.get("step_base", 0)
     out = eng.run(sampler, theta=theta, y=y, n_steps=num_ite - 1 - step_base, gf=global_frequency, seed=seed,
                   chain_id_base=chain_id_base, arith=_ARITH[arith], trace_layout=layout, stats=stats, aux=aux, K=K,
                   block_threads=block_threads, **resumed, **sampler_kw)

@@ -437,6 +437,29 @@ GLABC_API int glabc_user_model_check(const glabc_user_model_t* model, int32_t cc
 GLABC_API int glabc_user_model_check_proposals(const glabc_user_model_t* model, int32_t local_kind, int32_t far_kind, int32_t cc,
                                                char* log, size_t log_cap);
 
+/* The model's functions outside a run (generate_samples / prior_log_prob / discrepancy / calculate_log_kernel of the plugin
+ * surface, Mixture.py:13-53), one row per thread in the kernel glabc_k_eval_user of the same NVRTC module as the step kernels:
+ * a module already loaded for the model (any proposal kinds) serves them, otherwise the DiagGaussian one is compiled.
+ * DEVICE buffers, asynchronous on `stream`.  n == 0 launches nothing; n < 0, a NULL buffer with n > 0, an invalid model or
+ * (glabc_user_evaluate) an unknown op are GLABC_ERR_INVALID, refused before anything is launched.                          */
+typedef enum {
+    GLABC_USER_SIMULATE = 0,      /* theta[n][theta_dim] -> y[n][y_dim]: the entry glabc_user_simulate below           */
+    GLABC_USER_PRIOR = 1,         /* x = theta[n][theta_dim] -> out[n] = glabc_user_prior_log_prob                     */
+    GLABC_USER_DISCREPANCY = 2,   /* x = y[n][y_dim]         -> out[n] = glabc_user_discrepancy                         */
+    GLABC_USER_LOG_KERNEL = 3     /* x = y[n][y_dim]         -> out[n] = log K(dis) = -0.5 log(2 pi) - log eps - dis^2 / (2 eps^2),
+                                     evaluated as the step kernels' kernel term (model->epsilon)                            */
+} glabc_user_op;
+/* y[n][y_dim] = one simulator draw per row of theta[n][theta_dim].  Row r takes its n_noise N(0,1) draws from the Philox4x32-10
+ * blocks with counter (row_base + r, step 0, slot 2 + b), b < ceil(n_noise / 4), key = seed, as Box-Muller pairs -- the
+ * numbers a step kernel would draw for its simulator at step 0.  No run draws at step 0 (a launch draws at steps
+ * step_base + 1 ..), so with row_base = run->chain_id_base and the run's seed, row c is a simulated initial y of chain c that
+ * depends on the chain's global id only, not on the shard that runs it.                                                     */
+GLABC_API int glabc_user_simulate(glabc_ctx* ctx, const glabc_user_model_t* model, const float* theta, int64_t n, uint64_t seed,
+                                  uint64_t row_base, float* y, void* stream);
+/* op = GLABC_USER_PRIOR, GLABC_USER_DISCREPANCY or GLABC_USER_LOG_KERNEL on the n rows of x, out[n] float32.                  */
+GLABC_API int glabc_user_evaluate(glabc_ctx* ctx, const glabc_user_model_t* model, int32_t op, const float* x, int64_t n, float* out,
+                                  void* stream);
+
 /* ---- KernelDensity (kernel_density.py:4-177), batched over `sets` independent point sets ------------------
  * Set s holds n[s] points X[s][cap][dim] (n == NULL: every set holds `cap` points).                          */
 /* fit, kernel_density.py:22-94: weights_out[s][j] = w / sum(w) (uniform when w == NULL),
