@@ -20,6 +20,8 @@ from . import _abi
 from .block_isir import run_block_isir
 from .engine import get_engine
 from .flows import RealNVP
+from .GlobalMCMC import user_initial_state
+from .models import UserModel
 from .pooled import average_flat, average_gradients
 from .samplers import default_seed, initial_state
 
@@ -141,19 +143,26 @@ def GLMCMC_NF(ABCset, num_ite, Initial_theta, Initial_y, Local_Proposal, fileloc
     either way because sample() returns the density of the map it applied); `flow_train`: "native" (the training step as
     kernels of the extension, the default) or "torch" (the fp32 autograd restatement, kept as the tests' checker);
     `checkpoint=` / `resume=`: the end-of-run state incl. the candidate blocks, the flow's weights and its Adam moments — a
-    resumed run continues bit-identically (block_isir.run_block_isir)."""
+    resumed run continues bit-identically (block_isir.run_block_isir).
+    `ABCset` may be a `models.UserModel` of theta_dim 2: its simulator, prior and discrepancy run in the block-iSIR kernels
+    compiled with it (FAST arithmetic, `arith` ignored); `Initial_y=None` then draws y0 with the model's simulator, as
+    `GlobalMCMC` does for a user model."""
     if num_ite < 1:
         raise ValueError("num_ite must be at least 1")
     K, S = int(batch_size), int(step_size)
     if not 1 <= K <= _abi.MAX_K or S < 1 or K * S > _abi.AG_MAX_BLOCK:
         raise ValueError(f"batch_size in 1..{_abi.MAX_K} and batch_size * step_size <= {_abi.AG_MAX_BLOCK}")
     eng = get_engine(device)
-    pod = eng.bind_model(ABCset)
+    user = isinstance(ABCset, UserModel)      # run-time compiled model (csrc/user_model.cu: glabc_k_block_isir_user)
+    pod = ABCset if user else eng.bind_model(ABCset)
     if pod.theta_dim != 2:
         raise NotImplementedError("the reference's flow is MLP([1,128,128,2]) couplings: theta_dim must be 2 (GLMCMC_NFs.py:56)")
     eng.bind_proposal(_abi.SLOT_LOCAL, Local_Proposal)
     seed = default_seed() if seed is None else int(seed)
-    theta, y, c = initial_state(eng, pod, Initial_theta, Initial_y, num_chains, seed)
+    if user:
+        theta, y, c = user_initial_state(eng, ABCset, Initial_theta, Initial_y, num_chains, seed, chain_id_base)
+    else:
+        theta, y, c = initial_state(eng, pod, Initial_theta, Initial_y, num_chains, seed)
     single = num_chains is None and c == 1
     dev = eng.device
     if flow is None:

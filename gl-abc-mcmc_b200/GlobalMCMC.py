@@ -42,6 +42,25 @@ def GlobalMCMC(ABCset, num_ite, Initial_theta, Initial_y, Global_Proposal, filel
                       block_threads=block_threads, checkpoint=checkpoint, resume=resume)
 
 
+def user_initial_state(eng, model, Initial_theta, Initial_y, num_chains, seed, chain_id_base):
+    """(theta [C, theta_dim], y [C, y_dim], C) of a user-model run: Initial_theta / Initial_y of 1 or C rows; Initial_y=None
+    draws y0 of chain c with the model's simulator (glabc_user_simulate, Philox id chain_id_base + c at step 0)"""
+    d, yd = model.theta_dim, model.y_dim
+    theta = torch.as_tensor(Initial_theta, dtype=torch.float32).reshape(-1, d)
+    c = num_chains if num_chains is not None else theta.shape[0]
+    if theta.shape[0] not in (1, c):
+        raise ValueError(f"Initial_theta must have 1 or {c} rows")
+    theta = theta.to(eng.device).expand(c, d).contiguous().clone()
+    if Initial_y is None:
+        y = eng.user_simulate(model, theta, seed, row_base=chain_id_base)
+    else:
+        y = torch.as_tensor(Initial_y, dtype=torch.float32).reshape(-1, yd)
+        if y.shape[0] not in (1, c):
+            raise ValueError(f"Initial_y must have 1 or {c} rows")
+        y = y.to(eng.device).expand(c, yd).contiguous().clone()
+    return theta, y, c
+
+
 def run_user_model(eng, model, sampler, num_ite, Initial_theta, Initial_y, Local_Proposal, filelocation, gf, num_chains,
                    seed, chain_id_base, trace, return_stats, verbose, block_threads, K=0, num_grad=0, tau=0.0, checkpoint=None,
                    resume=None):
@@ -69,18 +88,7 @@ def run_user_model(eng, model, sampler, num_ite, Initial_theta, Initial_y, Local
         resumed, layout = continuation(ck["step_base"], num_ite, layout)
     else:
         seed = default_seed() if seed is None else int(seed)
-        theta = torch.as_tensor(Initial_theta, dtype=torch.float32).reshape(-1, d)
-        c = num_chains if num_chains is not None else theta.shape[0]
-        if theta.shape[0] not in (1, c):
-            raise ValueError(f"Initial_theta must have 1 or {c} rows")
-        theta = theta.to(eng.device).expand(c, d).contiguous().clone()
-        if Initial_y is None:
-            y = eng.user_simulate(model, theta, seed, row_base=chain_id_base)
-        else:
-            y = torch.as_tensor(Initial_y, dtype=torch.float32).reshape(-1, yd)
-            if y.shape[0] not in (1, c):
-                raise ValueError(f"Initial_y must have 1 or {c} rows")
-            y = y.to(eng.device).expand(c, yd).contiguous().clone()
+        theta, y, c = user_initial_state(eng, model, Initial_theta, Initial_y, num_chains, seed, chain_id_base)
         stats = torch.zeros(c, _abi.nstats(d), dtype=torch.float32, device=eng.device)
         aux = None
         if sampler in ("isir", "mala"):

@@ -168,6 +168,9 @@ _SIGNATURES = {
                                    C.c_int32, C.c_int64, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "glabc_run_block_isir": (C.c_int, [C.c_void_p, C.POINTER(RunPOD), C.POINTER(BlockIsirPOD)]),
     "glabc_block_weights": (C.c_int, [C.c_void_p, C.POINTER(RunPOD), C.POINTER(BlockIsirPOD), C.c_uint32]),
+    "glabc_run_block_isir_user": (C.c_int, [C.c_void_p, C.POINTER(RunPOD), C.POINTER(BlockIsirPOD), C.POINTER(UserModelPOD)]),
+    "glabc_block_weights_user": (C.c_int, [C.c_void_p, C.POINTER(RunPOD), C.POINTER(BlockIsirPOD), C.c_uint32,
+                                           C.POINTER(UserModelPOD)]),
     "glabc_flow_set": (C.c_int, [C.c_void_p, C.POINTER(FlowPOD), C.c_size_t, C.c_void_p]),
     "glabc_flow_sample": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
     "glabc_flow_log_prob": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),

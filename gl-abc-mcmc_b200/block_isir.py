@@ -1,7 +1,9 @@
 """Host driver of the block-iSIR samplers whose importance proposal is SHARED by all chains: GLMCMC-NFs (one RealNVP,
 GLMCMC_NFs.py:90-152) and pooled AGLMCMC (one KernelDensity over the pooled training draws, AGLMCMC.py:124-272).
 
-The chain step is the fused kernel `k_ag_step<EXT>` (csrc/step_aglmcmc.cuh) behind `glabc_run_block_isir`: a chain pauses
+The chain step is the fused kernel `k_ag_step<EXT>` (csrc/step_aglmcmc.cuh) behind `glabc_run_block_isir` — for a run-time
+compiled `models.UserModel` its NVRTC twin `glabc_k_block_isir_user` (csrc/user_model.cu) behind `glabc_run_block_isir_user`,
+with the block weights from `glabc_block_weights_user`: a chain pauses
 when its block of batch_size * step_size candidates is consumed or when the proposal log-density of a changed state is
 needed.  This loop refreshes those log-densities in one batched launch of the proposal's kernel and, when every chain of
 the rank has consumed its block, lets the proposal adapt (train / refit — the only place ranks exchange data) and refills.
@@ -15,6 +17,7 @@ import torch
 
 from . import _abi
 from .engine import RunStats
+from .models import UserModel
 from .pooled import RoundSync, _world
 from .samplers import _ARITH, _LAYOUT, print_summary, write_csv
 
@@ -44,9 +47,12 @@ BLOCK_CHECKPOINT_VERSION = 1
 _BLOCK_TENSORS = ("theta", "x", "w", "lq", "kk", "pending", "lq_valid", "next_step", "lq_cur")
 
 
-def run_block_isir(eng, pod, proposal, *, num_ite, theta, y, K, S, gf, seed, chain_id_base, arith, trace, single,
+def run_block_isir(eng, model, proposal, *, num_ite, theta, y, K, S, gf, seed, chain_id_base, arith, trace, single,
                    filelocation, verbose, max_adapt=None, checkpoint=None, resume=None):
     """Advance every chain to iteration num_ite - 1.  Returns (result, RunStats, rounds).
+    `model`: the bound built-in model's POD (Engine.bind_model), or a `models.UserModel`, whose kernels run FAST arithmetic
+    (`arith` is ignored) and whose checkpoints carry its fingerprint: a resume refuses another model's checkpoint and one written
+    by a built-in run, and a built-in run refuses a user model's.
     `checkpoint=path` writes the end-of-run state: chain state, statistics, every chain's candidate block and counters, the
     round / adaptation counters, the proposal's own state (`proposal.state_dict()`: flow weights + Adam moments, or the pooled
     KDE) and the host generators the adaptation draws from; `resume=path` continues from exactly that state (the returned trace
@@ -55,13 +61,17 @@ def run_block_isir(eng, pod, proposal, *, num_ite, theta, y, K, S, gf, seed, cha
     consume their blocks in step (global_frequency = 1; tested), and is a deterministic function of the checkpoint otherwise."""
     c, d = theta.shape
     dev = eng.device
-    blk = Block(c, K, S, d, pod.y_dim, dev)
+    user = isinstance(model, UserModel)
+    blk = Block(c, K, S, d, model.y_dim, dev)
     done0, rnd, n_adapt = 0, 0, 0
     stats = torch.zeros(c, _abi.nstats(d), device=dev)
     if resume is not None:
         ck = resume if isinstance(resume, dict) else torch.load(resume, map_location="cpu", weights_only=False)
         if ck.get("version") != BLOCK_CHECKPOINT_VERSION or ck.get("kind") != type(proposal).__name__:
             raise ValueError("not a block-iSIR checkpoint of this sampler")
+        if ck.get("model") != (model.fingerprint() if user else None):
+            raise ValueError("the checkpoint was written for another model (a user model's source, dims, params or epsilon differ, "
+                             "or one of the two runs used the built-in family)")
         if ck["theta"].shape != theta.shape or (ck["K"], ck["S"]) != (K, S):
             raise ValueError("the checkpoint was written for another number of chains / block shape")
         theta.copy_(ck["theta"])
@@ -78,7 +88,10 @@ def run_block_isir(eng, pod, proposal, *, num_ite, theta, y, K, S, gf, seed, cha
 
     def refill(rnd):    # GLMCMC_NFs.py:70-85,125-140 / AGLMCMC.py:84-112,219-249
         proposal.fill(blk.theta, blk.lq, rnd)
-        eng.run("block_weights", n_steps=0, step_base=rnd, trace_layout=_abi.TRACE_NONE, **common)
+        if user:
+            eng.run_user(model, sampler="block_weights", n_steps=0, round=rnd, trace_layout=_abi.TRACE_NONE, **common)
+        else:
+            eng.run("block_weights", n_steps=0, step_base=rnd, trace_layout=_abi.TRACE_NONE, **common)
 
     def refresh_lq(idx=None):   # proposal.log_prob(Theta_old), GLMCMC_NFs.py:96-98 / AGLMCMC.py:137-140, where the state changed
         if idx is None:
@@ -104,8 +117,12 @@ def run_block_isir(eng, pod, proposal, *, num_ite, theta, y, K, S, gf, seed, cha
     first = resume is None
     window = dict(step_base=done0, trace_row_base=0 if resume is None else done0 + 1, trace_rows=rows)
     while True:
-        eng.run("block_isir", n_steps=n_steps - done0, arith=_ARITH[arith], trace_layout=layout, trace=out,
-                write_row0=first, stats=stats, **window, **common)
+        if user:
+            eng.run_user(model, sampler="block_isir", n_steps=n_steps - done0, trace_layout=layout, trace=out, write_row0=first,
+                         stats=stats, **window, **common)
+        else:
+            eng.run("block_isir", n_steps=n_steps - done0, arith=_ARITH[arith], trace_layout=layout, trace=out,
+                    write_row0=first, stats=stats, **window, **common)
         first = False
         need = (blk.pending & 2) != 0
         settled = (blk.next_step > n_steps) | ((blk.pending & 1) != 0)
@@ -128,10 +145,11 @@ def run_block_isir(eng, pod, proposal, *, num_ite, theta, y, K, S, gf, seed, cha
                 blk.pending.zero_()
     if checkpoint is not None:
         cpu = lambda t: t.detach().cpu()  # noqa: E731
+        extra = dict(model=model.fingerprint()) if user else {}
         torch.save(dict(version=BLOCK_CHECKPOINT_VERSION, kind=type(proposal).__name__, K=K, S=S, done=n_steps, rnd=rnd, n_adapt=n_adapt,
                         seed=int(seed), chain_id_base=int(chain_id_base), theta=cpu(theta), y=cpu(y), stats=cpu(stats),
                         blk={name: cpu(getattr(blk, name)) for name in _BLOCK_TENSORS}, proposal=proposal.state_dict(),
-                        torch_rng=torch.get_rng_state()), checkpoint)
+                        torch_rng=torch.get_rng_state(), **extra), checkpoint)
     rs = RunStats(stats, d)
     if single:
         chain = (out[0] if layout == _abi.TRACE_CHAIN_MAJOR else out[:, 0]).cpu() if out is not None else None

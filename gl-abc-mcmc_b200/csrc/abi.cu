@@ -1255,6 +1255,17 @@ extern "C" int glabc_flow_log_prob(glabc_ctx* ctx, const float* theta, int64_t n
 // ---------------------------------------------------------------------------------------------
 // block iSIR with an external importance proposal (GLMCMC-NFs)
 // ---------------------------------------------------------------------------------------------
+// the block description of glabc_run_block_isir / glabc_block_weights and their user-model twins
+static int check_block(glabc_ctx* ctx, const char* who, const glabc_run_t* run, const glabc_block_isir_t* b)
+{
+    if (run->n_candidates < 1 || run->n_candidates > GLABC_MAX_K) return fail(ctx, GLABC_ERR_INVALID, "n_candidates must be in 1..%d", GLABC_MAX_K);
+    if (b->step_size < 1 || int64_t(b->step_size) * run->n_candidates != b->block || b->block > GLABC_AG_MAX_BLOCK)
+        return fail(ctx, GLABC_ERR_INVALID, "%s: block must equal batch_size * step_size and be at most %d", who, GLABC_AG_MAX_BLOCK);
+    if (!b->blk_theta || !b->blk_x || !b->blk_w || !b->blk_lq || !b->kk || !b->pending || !b->next_step || !b->lq_cur || !b->lq_valid)
+        return fail(ctx, GLABC_ERR_INVALID, "%s: null block / state buffer", who);
+    return GLABC_OK;
+}
+
 static int block_isir_setup(glabc_ctx* ctx, const char* who, const glabc_run_t* run, const glabc_block_isir_t* b, bool need_local,
                             AgConsts* K, AgWorkspace* W, RunParams* R, int* block)
 {
@@ -1263,11 +1274,7 @@ static int block_isir_setup(glabc_ctx* ctx, const char* who, const glabc_run_t* 
     if (!run || !b) return fail(ctx, GLABC_ERR_INVALID, "%s: null run / block description", who);
     if (need_local && !ctx->has_dist[GLABC_SLOT_LOCAL]) return fail(ctx, GLABC_ERR_INVALID, "%s needs the LOCAL proposal slot bound", who);
     const int d = ctx->model.theta_dim;
-    if (run->n_candidates < 1 || run->n_candidates > GLABC_MAX_K) return fail(ctx, GLABC_ERR_INVALID, "n_candidates must be in 1..%d", GLABC_MAX_K);
-    if (b->step_size < 1 || int64_t(b->step_size) * run->n_candidates != b->block || b->block > GLABC_AG_MAX_BLOCK)
-        return fail(ctx, GLABC_ERR_INVALID, "%s: block must equal batch_size * step_size and be at most %d", who, GLABC_AG_MAX_BLOCK);
-    if (!b->blk_theta || !b->blk_x || !b->blk_w || !b->blk_lq || !b->kk || !b->pending || !b->next_step || !b->lq_cur || !b->lq_valid)
-        return fail(ctx, GLABC_ERR_INVALID, "%s: null block / state buffer", who);
+    if (int st = check_block(ctx, who, run, b)) return st;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     int st = make_run_params(ctx, run, d, GLABC_TAPE_GLOBAL_SLOTS(d, d), R, block);
     if (st) return st;
@@ -1485,6 +1492,91 @@ static int run_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_user_mod
 extern "C" int glabc_run_global_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_user_model_t* um) { return run_user(ctx, run, um, 0); }
 extern "C" int glabc_run_isir_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_user_model_t* um) { return run_user(ctx, run, um, 1); }
 extern "C" int glabc_run_mala_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_user_model_t* um) { return run_user(ctx, run, um, 2); }
+
+// glabc_k_block_isir_user (weights = false) / glabc_k_block_weights_user: the block-iSIR step and the block weights of
+// glabc_run_block_isir / glabc_block_weights for a user model
+static int run_block_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_block_isir_t* b, uint32_t round,
+                          const glabc_user_model_t* um, bool weights)
+{
+    const char* who = weights ? "glabc_block_weights_user" : "glabc_run_block_isir_user";
+    if (!ctx) return GLABC_ERR_INVALID;
+    if (int st = check_user_model(ctx, um, who)) return st;
+    if (!run || !b) return fail(ctx, GLABC_ERR_INVALID, "%s: null run / block description", who);
+    const int d = um->theta_dim;
+    if (!ctx->has_dist[GLABC_SLOT_LOCAL]) return fail(ctx, GLABC_ERR_INVALID, "%s needs the LOCAL proposal slot bound", who);
+    const glabc_dist_t& lp = ctx->dist[GLABC_SLOT_LOCAL];
+    if (lp.dim != d) return fail(ctx, GLABC_ERR_INVALID, "proposal dim does not match the user model's theta_dim %d", d);
+    if (int st = check_block(ctx, who, run, b)) return st;
+    if (run->arith_mode == GLABC_ARITH_STRICT || run->rng_mode == GLABC_RNG_REPLAY)
+        return fail(ctx, GLABC_ERR_UNSUPPORTED, "%s: the user-model kernels run FAST arithmetic with the native RNG only", who);
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    RunParams R;
+    int block = 0;
+    int st = make_run_params(ctx, run, d, 0, &R, &block);
+    if (st) return st;
+    if (R.n_chains == 0) return GLABC_OK;
+    CUDA_TRY(ctx, cudaFree(nullptr));   // the primary context, current for the driver calls
+    void* fn = nullptr;
+    std::string err;
+    st = user_model_block_fn(ctx->device, ctx->cc, *um, lp.kind, weights, &fn, err);
+    if (st) return fail(ctx, st, "%s", err.c_str());
+    UserBlockRun U{};
+    U.n_chains = R.n_chains;
+    U.block = b->block;
+    U.step_size = b->step_size;
+    U.n_candidates = run->n_candidates;
+    U.first_step = R.first_step;
+    U.last_step = R.last_step;
+    U.chain_lo0 = R.chain_lo0;
+    U.chain_hi0 = R.chain_hi0;
+    U.key0 = static_cast<uint32_t>(run->seed);
+    U.key1 = static_cast<uint32_t>(run->seed >> 32);
+    const double gf = static_cast<double>(run->global_frequency);
+    U.gf_all_global = gf >= 1.0;
+    U.gf_thr = gf <= 0.0 ? 0u : (gf >= 1.0 ? 0xFFFFFFFFu : static_cast<uint32_t>(gf * 4294967296.0));
+    U.round = round;
+    U.write_row0 = R.write_row0;
+    U.trace_layout = run->trace_layout;
+    U.trace_rows = R.trace_rows;
+    U.trace_chains = R.trace_chains;
+    U.trace_chain_off = R.trace_chain_off;
+    U.trace_row_base = R.trace_row_base;
+    U.theta = R.theta;
+    U.y = R.y;
+    U.trace = R.trace;
+    U.stats = R.stats;
+    U.blk_theta = b->blk_theta;
+    U.blk_x = b->blk_x;
+    U.blk_w = b->blk_w;
+    U.blk_lq = b->blk_lq;
+    U.kk = b->kk;
+    U.pending = b->pending;
+    U.next_step = b->next_step;
+    U.lq_cur = b->lq_cur;
+    U.lq_valid = b->lq_valid;
+    if (lp.kind == GLABC_DIST_DIAG_GAUSSIAN)
+        for (int k = 0; k < d; ++k) {
+            U.lp_loc[k] = lp.a[k];
+            U.lp_scale[k] = lp.c[k];
+        }
+    U.lq = make_dist<GLABC_MAX_DIM>(lp);
+    user_kernel_consts(*um, &U.kern_c, &U.kern_m);
+    for (int k = 0; k < um->n_params; ++k) U.params[k] = um->params[k];
+    st = user_model_block_launch(fn, U, weights, static_cast<cudaStream_t>(run->stream), err);
+    if (st) return fail(ctx, st, "%s", err.c_str());
+    return GLABC_OK;
+}
+
+extern "C" int glabc_run_block_isir_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_block_isir_t* blk, const glabc_user_model_t* model)
+{
+    return run_block_user(ctx, run, blk, 0u, model, false);
+}
+
+extern "C" int glabc_block_weights_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_block_isir_t* blk, uint32_t round,
+                                        const glabc_user_model_t* model)
+{
+    return run_block_user(ctx, run, blk, round, model, true);
+}
 
 // glabc_k_eval_user on n rows; the caller has checked ctx, the model, n and the buffers
 static int eval_user(glabc_ctx* ctx, const glabc_user_model_t* um, int op, const float* in, int64_t n, uint64_t seed,

@@ -174,4 +174,23 @@ struct UserEval {
     float params[GLABC_USER_MAX_PARAMS];
 };
 
+// kernel parameter of the user-model block-iSIR kernels glabc_k_block_isir_user / glabc_k_block_weights_user (user_model.cu):
+// the UserRun fields they read, the glabc_block_isir_t buffers (include/glabc.h) and the block shape
+struct UserBlockRun {
+    int n_chains, block, step_size, n_candidates;   // C, B = K S, S, K
+    unsigned first_step, last_step, chain_lo0, chain_hi0, key0, key1, gf_thr, round;   // round: block_weights' refill round
+    int gf_all_global, write_row0, trace_layout, pad;
+    long long trace_rows, trace_chains, trace_chain_off, trace_row_base;
+    float *theta, *y, *trace, *stats;
+    float *blk_theta, *blk_x, *blk_w, *blk_lq;       // [C][B][D], [C][B][YD], [C][B], [C][B]
+    int *kk, *pending;
+    unsigned* next_step;
+    float* lq_cur;
+    int* lq_valid;
+    float lp_loc[GLABC_MAX_DIM], lp_scale[GLABC_MAX_DIM];
+    float kern_c, kern_m;
+    float params[GLABC_USER_MAX_PARAMS];
+    DistConstsT<GLABC_MAX_DIM> lq;                   // a Uniform / Gamma / GaussianMixture Local_Proposal
+};
+
 }  // namespace glabc

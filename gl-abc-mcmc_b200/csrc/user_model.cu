@@ -122,12 +122,18 @@ struct GlabcWords {
 //   0x80000000               the iSIR resampling uniform
 //   GLABC_SLOT_PROP ..       a Uniform / Gamma / GaussianMixture local or global draw; sentinel redraws continue its stream
 //   GLABC_SLOT_CAND + j GLABC_CAND_BLOCKS ..   iSIR candidate j from a Uniform / Gamma / GaussianMixture importance proposal
+//   GLABC_SLOT_BLOCK + b ceil(NN / 4) ..      glabc_k_block_weights_user: the simulator's normals of block candidate b, with
+//                            the refill round r < 2^32 in the step coordinate (round 0 shares step 0 with SIMULATE)
 // A non-Gaussian proposal only moves the proposal's draws: the simulator keeps its blocks.  One dist_forward takes at most
 // 386 blocks at D = 8 (Gamma: 8 x (64 squeeze iterations x 3 words + 1) words, dist_device.cuh), so a candidate's range
 // of 0x200 blocks holds it, and the 65 draws of a local move with every redraw (25090 blocks) fit under GLABC_SLOT_CAND.
+// The block range ends below GLABC_SLOT_BLOCK + GLABC_AG_MAX_BLOCK x ceil(GLABC_USER_MAX_NOISE / 4) = 0xA0008000; every
+// other range lies below 0x80000001 (the highest, GLABC_SLOT_CAND + 16 x 0x200 = 0x60012000), so none meets it, step 0's
+// SIMULATE slots 2 .. 9 included.
 #define GLABC_SLOT_PROP 0x60000000u
 #define GLABC_SLOT_CAND 0x60010000u
 #define GLABC_CAND_BLOCKS 0x200u
+#define GLABC_SLOT_BLOCK 0xA0000000u
 )GLABC";
 
 const char* kKernel = R"GLABC(
@@ -806,6 +812,208 @@ extern "C" __global__ void __launch_bounds__(256) glabc_k_eval_user(const __grid
         }
     }
 }
+
+// ---- block iSIR against an importance proposal shared by all chains (GLMCMC-NFs: the RealNVP; pooled AGLMCMC: the pooled
+// KernelDensity), GLMCMC_NFs.py:90-152 / AGLMCMC.py:124-168,251-271.  The proposal lives outside the module: the host fills
+// blk_theta / blk_lq with its candidates and their log-densities, glabc_k_block_weights_user simulates them and weighs them,
+// and glabc_k_block_isir_user steps the chains against the block, as k_ag_step<EXT = true> (step_aglmcmc.cuh) does for the
+// built-in family.  A chain pauses when its block is consumed (pending bit 0) or when a global move needs the proposal
+// log-density of a state a local move changed (bit 1): the host refreshes it in one batched launch and calls again.
+__device__ __forceinline__ float glabc_block_target(const glabc::UserBlockRun& R, const float* th, const float* y)
+{
+    const float dis = glabc_user_discrepancy(y, R.params);
+    return glabc_user_prior_log_prob(th, R.params) + fmaf(R.kern_m, dis * dis, R.kern_c);
+}
+// exp to a few ulp: --use_fast_math makes expf ex2.approx(x log2 e), whose relative error grows as |x| 2^-24 (1e-5 at the
+// |x| ~ 100 of a far candidate's weight).  Reduced to |r| <= ln2 / 2 first (Cody-Waite), then scaled by 2^k in two exact steps.
+__device__ __forceinline__ float glabc_exp(float x)
+{
+    if (x < -104.0f) return 0.0f;              // below the smallest subnormal (and -inf)
+    if (x > 88.8f) return INFINITY;
+    const float k = rintf(x * 1.44269504088896341f);
+    float r = fmaf(k, -0.693145751953125f, x); // ln 2 = 0.693145751953125 + 1.428606765330187e-06
+    r = fmaf(k, -1.428606765330187e-06f, r);
+    const int ki = (int)k, k1 = ki / 2, k2 = ki - k1;
+    return exp2f(r * 1.44269504088896341f) * __int_as_float((k1 + 127) << 23) * __int_as_float((k2 + 127) << 23);
+}
+extern "C" __global__ void __launch_bounds__(128) glabc_k_block_isir_user(const __grid_constant__ glabc::UserBlockRun R)
+{
+    const int chain = blockIdx.x * blockDim.x + threadIdx.x;
+    if (chain >= R.n_chains) return;
+    const u64 gid = ((u64)R.chain_hi0 << 32 | R.chain_lo0) + (u64)chain;
+    const u32 g0 = (u32)gid, g1 = (u32)(gid >> 32);
+    const int B = R.block, NK = R.n_candidates;
+    float th[D], y[YD];
+#pragma unroll
+    for (int k = 0; k < D; ++k) th[k] = R.theta[(long long)chain * D + k];
+#pragma unroll
+    for (int k = 0; k < YD; ++k) y[k] = R.y[(long long)chain * YD + k];
+    int kk = R.kk[chain];
+    u32 i = R.next_step[chain];
+    float lq_cur = R.lq_cur[chain];
+    bool lq_valid = R.lq_valid[chain] != 0, pend_lq = false;
+    float pk = glabc_block_target(R, th, y);
+    float n_glob = 0.f, acc_l = 0.f, acc_g = 0.f, sum[D], sumsq[D], gram[D * (D + 1) / 2];
+#pragma unroll
+    for (int k = 0; k < D; ++k) sum[k] = sumsq[k] = 0.f;
+#pragma unroll
+    for (int k = 0; k < D * (D + 1) / 2; ++k) gram[k] = 0.f;
+    auto row_ptr = [&](long long row) {       // trace row = loop index i (k_ag_step's layout)
+        return R.trace_layout == 2 ? R.trace + ((R.trace_chain_off + chain) * R.trace_rows + row) * D
+                                   : R.trace + (row * R.trace_chains + R.trace_chain_off + chain) * D;
+    };
+    if (R.trace_layout != 0 && R.write_row0) {   // row 0 = the initial theta, as k_ag_row0
+        float* row = row_ptr((long long)R.first_step - 1 - R.trace_row_base);
+#pragma unroll
+        for (int k = 0; k < D; ++k) row[k] = th[k];
+    }
+    u32 done = 0;
+    constexpr int NZ = D + NN, NB = (NZ + 3) / 4;
+    for (; R.last_step >= R.first_step && i <= R.last_step && kk < R.step_size; ++i) {
+        const uint4 w0 = glabc_philox(g0, g1, i, 1u, R.key0, R.key1);
+        const bool is_global = R.gf_all_global || (w0.x < R.gf_thr);
+        if (is_global && !lq_valid) {         // pause before the move: its draws are counter-based, so it replays
+            pend_lq = true;
+            break;
+        }
+        float dl[D];
+#pragma unroll
+        for (int k = 0; k < D; ++k) dl[k] = 0.f;
+        bool moved = false;
+        if (is_global) {                      // AGLMCMC.py:137-166 / GLMCMC_NFs.py:96-110
+            const float w_old = glabc_exp(pk - lq_cur);
+            const long long o0 = (long long)chain * B + (long long)kk * NK;
+            const float* bw = R.blk_w + o0;
+            double S = (double)w_old;
+            for (int j = 0; j < NK; ++j) S += (double)bw[j];
+            const uint4 wu = glabc_philox(g0, g1, i, 0x80000000u, R.key0, R.key1);
+            const double thr = (double)(((u64)wu.x << 21) | (u64)(wu.y >> 11)) * 0x1p-53 * S;   // weight_sampling, float64
+            double run = (double)w_old;
+            int ind = thr < run ? 0 : -1;
+            for (int j = 0; j < NK; ++j) {
+                run += (double)bw[j];
+                if (ind < 0 && thr < run) ind = j + 1;
+            }
+            if (ind > 0) {
+                const long long o = o0 + ind - 1;
+#pragma unroll
+                for (int k = 0; k < D; ++k) {
+                    const float t = R.blk_theta[o * D + k];
+                    dl[k] = t - th[k];
+                    moved |= t != th[k];
+                    th[k] = t;
+                }
+#pragma unroll
+                for (int k = 0; k < YD; ++k) y[k] = R.blk_x[o * YD + k];
+                lq_cur = R.blk_lq[o];
+                pk = glabc_block_target(R, th, y);
+            }
+            ++kk;
+        } else {                              // local random walk theta + z, z ~ Local_Proposal (no q term), :251-271
+            float z[NB * 4], thp[D], yp[YD];
+#pragma unroll
+            for (int b = 0; b < NB; ++b) {
+                const uint4 w = glabc_philox(g0, g1, i, 2u + b, R.key0, R.key1);
+                glabc_box_muller(w.x, w.y, z[4 * b], z[4 * b + 1]);
+                glabc_box_muller(w.z, w.w, z[4 * b + 2], z[4 * b + 3]);
+            }
+#if GLABC_LP_KIND == GLABC_DIST_DIAG_GAUSSIAN
+#pragma unroll
+            for (int k = 0; k < D; ++k) thp[k] = th[k] + fmaf(R.lp_scale[k], z[k], R.lp_loc[k]);
+#else
+            GlabcWords ws(g0, g1, i, GLABC_SLOT_PROP, R.key0, R.key1);
+            float zl[D];
+            (void)glabc::dist_forward<D>(R.lq, ws, zl);
+#pragma unroll
+            for (int k = 0; k < D; ++k) thp[k] = th[k] + zl[k];
+#endif
+            glabc_user_simulate(thp, z + D, R.params, yp);
+            const float pkp = glabc_block_target(R, thp, yp);
+            const float log_u = __logf(__uint2float_rn(w0.y >> 8) * 0x1p-24f);
+            if (log_u < pkp - pk) {
+#pragma unroll
+                for (int k = 0; k < D; ++k) {
+                    dl[k] = thp[k] - th[k];
+                    th[k] = thp[k];
+                }
+#pragma unroll
+                for (int k = 0; k < YD; ++k) y[k] = yp[k];
+                pk = pkp;
+                moved = true;
+                lq_valid = false;             // the proposal log-density of the new state is the host's to refresh
+            }
+        }
+#pragma unroll
+        for (int k = 0; k < D; ++k) {
+            sum[k] += th[k];
+            sumsq[k] = fmaf(th[k], th[k], sumsq[k]);
+        }
+        int t = 0;
+#pragma unroll
+        for (int a = 0; a < D; ++a)
+#pragma unroll
+            for (int b = a; b < D; ++b, ++t) gram[t] = fmaf(dl[a], dl[b], gram[t]);
+        n_glob += is_global ? 1.f : 0.f;
+        acc_g += (moved && is_global) ? 1.f : 0.f;
+        acc_l += (moved && !is_global) ? 1.f : 0.f;
+        ++done;
+        if (R.trace_layout != 0) {
+            float* row = row_ptr((long long)i - R.trace_row_base);
+#pragma unroll
+            for (int k = 0; k < D; ++k) row[k] = th[k];
+        }
+    }
+#pragma unroll
+    for (int k = 0; k < D; ++k) R.theta[(long long)chain * D + k] = th[k];
+#pragma unroll
+    for (int k = 0; k < YD; ++k) R.y[(long long)chain * YD + k] = y[k];
+    R.kk[chain] = kk;
+    R.next_step[chain] = i;
+    R.lq_cur[chain] = lq_cur;
+    R.lq_valid[chain] = lq_valid ? 1 : 0;
+    R.pending[chain] = (kk >= R.step_size ? 1 : 0) | (pend_lq ? 2 : 0);
+    if (R.stats != nullptr && done > 0) {
+        float* st = R.stats + (long long)chain * (4 + 2 * D + D * (D + 1) / 2);
+        st[0] += (float)done;
+        st[1] += n_glob;
+        st[2] += acc_l;
+        st[3] += acc_g;
+#pragma unroll
+        for (int k = 0; k < D; ++k) {
+            st[4 + k] += sum[k];
+            st[4 + D + k] += sumsq[k];
+        }
+#pragma unroll
+        for (int k = 0; k < D * (D + 1) / 2; ++k) st[4 + 2 * D + k] += gram[k];
+    }
+}
+// GLMCMC_NFs.py:73-85,129-140 / AGLMCMC.py:219-249: blk_x = simulate(blk_theta), blk_w = exp(prior + log K - blk_lq), NaN -> 0.
+// One thread per (chain, b); candidate b of refill round r draws its simulator normals from the Philox blocks
+// (chain, step r, GLABC_SLOT_BLOCK + b ceil(NN / 4) ..), see the slot table.
+extern "C" __global__ void __launch_bounds__(256) glabc_k_block_weights_user(const __grid_constant__ glabc::UserBlockRun R)
+{
+    const long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (g >= (long long)R.n_chains * R.block) return;
+    const long long c = g / R.block;
+    const int b = (int)(g - c * R.block);
+    const u64 gid = ((u64)R.chain_hi0 << 32 | R.chain_lo0) + (u64)c;
+    constexpr int NBS = (NN + 3) / 4;
+    float th[D], x[YD], z[NBS > 0 ? NBS * 4 : 4];
+#pragma unroll
+    for (int k = 0; k < D; ++k) th[k] = R.blk_theta[g * D + k];
+#pragma unroll
+    for (int q = 0; q < NBS; ++q) {
+        const uint4 w = glabc_philox((u32)gid, (u32)(gid >> 32), R.round, GLABC_SLOT_BLOCK + (u32)(b * NBS + q), R.key0, R.key1);
+        glabc_box_muller(w.x, w.y, z[4 * q], z[4 * q + 1]);
+        glabc_box_muller(w.z, w.w, z[4 * q + 2], z[4 * q + 3]);
+    }
+    glabc_user_simulate(th, z, R.params, x);
+    float wgt = glabc_exp(glabc_block_target(R, th, x) - R.blk_lq[g]);
+    if (wgt != wgt) wgt = 0.0f;
+#pragma unroll
+    for (int k = 0; k < YD; ++k) R.blk_x[g * YD + k] = x[k];
+    R.blk_w[g] = wgt;
+}
 )GLABC";
 
 // ---- lazily bound NVRTC / driver entry points --------------------------------------------------------------------
@@ -878,6 +1086,8 @@ struct Compiled {
     CUfunction fn_isir = nullptr;   // glabc_k_isir_user
     CUfunction fn_mala = nullptr;   // glabc_k_mala_user (models with theta_dim <= 5: the gradient is cached in the aux slots)
     CUfunction fn_eval = nullptr;   // glabc_k_eval_user
+    CUfunction fn_block = nullptr;  // glabc_k_block_isir_user
+    CUfunction fn_blk_w = nullptr;  // glabc_k_block_weights_user
 };
 std::mutex g_cache_mu;
 // key: model_key() + proposal kinds, so the modules of one model are adjacent in the map
@@ -988,7 +1198,9 @@ static int load_module(Dyn& d, int device, int cc, const glabc_user_model_t& um,
         return GLABC_ERR_CUDA;
     }
     const std::pair<CUfunction*, const char*> fns[] = {{&c.fn, "glabc_k_global_user"}, {&c.fn_isir, "glabc_k_isir_user"},
-                                                       {&c.fn_mala, "glabc_k_mala_user"}, {&c.fn_eval, "glabc_k_eval_user"}};
+                                                       {&c.fn_mala, "glabc_k_mala_user"}, {&c.fn_eval, "glabc_k_eval_user"},
+                                                       {&c.fn_block, "glabc_k_block_isir_user"},
+                                                       {&c.fn_blk_w, "glabc_k_block_weights_user"}};
     for (const auto& f : fns) {
         cr = d.moduleGetFunction(f.first, c.mod, f.second);
         if (cr != CUDA_SUCCESS) {
@@ -1037,6 +1249,29 @@ int user_model_eval_fn(int device, int cc, const glabc_user_model_t& um, void** 
     return GLABC_OK;
 }
 
+int user_model_block_fn(int device, int cc, const glabc_user_model_t& um, int lp_kind, bool weights, void** fn_out, std::string& err)
+{
+    Dyn& d = dyn();
+    if (!d.ok) {
+        err = d.why;
+        return GLABC_ERR_UNSUPPORTED;
+    }
+    std::lock_guard<std::mutex> lock(g_cache_mu);
+    char lp[16];
+    snprintf(lp, sizeof(lp), "|%d|", lp_kind);
+    const std::string prefix = model_key(device, cc, um) + lp;   // then only the Global / Importance kind follows
+    const Compiled* c = nullptr;
+    auto it = g_cache.lower_bound(prefix);
+    if (it != g_cache.end() && it->first.compare(0, prefix.size(), prefix) == 0) {
+        c = &it->second;
+    } else {
+        const int st = load_module(d, device, cc, um, lp_kind, GLABC_DIST_DIAG_GAUSSIAN, &c, err);
+        if (st) return st;
+    }
+    *fn_out = weights ? c->fn_blk_w : c->fn_block;
+    return GLABC_OK;
+}
+
 static int launch(void* fn, void* param, unsigned grid, int block, cudaStream_t st, std::string& err)
 {
     Dyn& d = dyn();
@@ -1059,6 +1294,20 @@ int user_model_launch(void* fn, const UserRun& R, int block, cudaStream_t st, st
     if (R.n_chains <= 0) return GLABC_OK;
     UserRun copy = R;
     return launch(fn, &copy, static_cast<unsigned>((R.n_chains + block - 1) / block), block, st, err);
+}
+
+int user_model_block_launch(void* fn, const UserBlockRun& R, bool weights, cudaStream_t st, std::string& err)
+{
+    const int block = weights ? 256 : 128;   // the kernels' __launch_bounds__
+    const long long n = weights ? (long long)R.n_chains * R.block : R.n_chains;
+    if (n <= 0) return GLABC_OK;
+    const long long grid = (n + block - 1) / block;
+    if (grid > 0x7fffffffLL) {
+        err = "too many block candidates for one launch";
+        return GLABC_ERR_INVALID;
+    }
+    UserBlockRun copy = R;
+    return launch(fn, &copy, static_cast<unsigned>(grid), block, st, err);
 }
 
 int user_model_eval_launch(void* fn, const UserEval& E, int sm_count, cudaStream_t st, std::string& err)

@@ -21,5 +21,10 @@ int user_model_launch(void* fn, const UserRun& R, int block, cudaStream_t st, st
 // (DiagGaussian, DiagGaussian) module, compiled here
 int user_model_eval_fn(int device, int cc, const glabc_user_model_t& um, void** fn, std::string& err);
 int user_model_eval_launch(void* fn, const UserEval& E, int sm_count, cudaStream_t st, std::string& err);
+// glabc_k_block_isir_user (weights = false) or glabc_k_block_weights_user (true) of `um`: they read only the LOCAL kind, so any
+// module loaded for the model with that local kind serves them, otherwise the (lp_kind, DiagGaussian) module is compiled here
+int user_model_block_fn(int device, int cc, const glabc_user_model_t& um, int lp_kind, bool weights, void** fn, std::string& err);
+// one thread per chain (the step) or per block candidate (the weights)
+int user_model_block_launch(void* fn, const UserBlockRun& R, bool weights, cudaStream_t st, std::string& err);
 
 }  // namespace glabc

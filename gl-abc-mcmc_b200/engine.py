@@ -155,9 +155,11 @@ class Engine:
 
     def run_user(self, model, *, theta, y, n_steps, gf, step_base=0, chain_id_base=0, seed=0, trace_layout=_abi.TRACE_CHAIN_MAJOR,
                  trace=None, trace_rows=None, trace_row_base=0, write_row0=True, stats=None, block_threads=0, sampler="global", K=0,
-                 aux=None, num_grad=0, tau=0.0):
+                 aux=None, num_grad=0, tau=0.0, blk=None, round=0):
         """GlobalMCMC (`sampler="global"`, LOCAL / GLOBAL slots), GLMCMC (`"isir"`, LOCAL / IMPORTANCE slots, K candidates, aux) or
-        GLMALA (`"mala"`, IMPORTANCE slot, K, tau, num_grad, aux) transitions for a `models.UserModel` (compiled on first use)"""
+        GLMALA (`"mala"`, IMPORTANCE slot, K, tau, num_grad, aux) transitions for a `models.UserModel` (compiled on first use).
+        `"block_isir"` / `"block_weights"`: the block-iSIR step against the candidate block `blk` (a BlockIsirPOD, LOCAL slot,
+        K candidates per global move) and the weights of refill `round` (glabc_run_block_isir_user / glabc_block_weights_user)."""
         cn, d = theta.shape
         rows = trace_rows if trace_rows is not None else step_base + n_steps + 1 - trace_row_base
         if trace is None and trace_layout != _abi.TRACE_NONE:
@@ -171,6 +173,13 @@ class Engine:
                         trace=self._ptr(trace), stats=self._ptr(stats), stream=self._stream(), num_grad=int(num_grad), tau=float(tau),
                         tau64=float(tau))
         pod = model.user_pod()
+        if sampler == "block_isir":
+            self.ctx.check(self.lib.glabc_run_block_isir_user(self.ctx.handle, C.byref(r), C.byref(blk), C.byref(pod)))
+            return trace
+        if sampler == "block_weights":
+            self.ctx.check(self.lib.glabc_block_weights_user(self.ctx.handle, C.byref(r), C.byref(blk), int(round) & 0xFFFFFFFF,
+                                                             C.byref(pod)))
+            return None
         fn = {"isir": self.lib.glabc_run_isir_user, "mala": self.lib.glabc_run_mala_user}.get(sampler, self.lib.glabc_run_global_user)
         self.ctx.check(fn(self.ctx.handle, C.byref(r), C.byref(pod)))
         return trace

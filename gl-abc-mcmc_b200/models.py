@@ -135,7 +135,11 @@ class UserModel:
 
     The plugin methods (`generate_samples`, `prior_log_prob`, `discrepancy`, `calculate_log_kernel`) run the compiled
     functions on the GPU (glabc_user_simulate / glabc_user_evaluate): inputs on any device, float32 outputs on the engine's
-    device.  There is no `y_obs`: the observation lives in `params`, and the fused-family samplers refuse the object."""
+    device.  There is no `y_obs`: the observation lives in `params`.
+
+    Samplers that take it: GlobalMCMC, GLMCMC, GLMALA (theta_dim <= 5), GLMCMC_NF (theta_dim 2: the flow) and
+    AGLMCMC(..., pooled=True) (theta_dim <= 4: the KernelDensity kernels), the last two through the block-iSIR kernels compiled
+    with the model.  Per-chain AGLMCMC (pooled=False) refuses it: its adaptation kernels are built for the fused family."""
 
     def __init__(self, source, theta_dim, y_dim, n_noise, epsilon, params=()):
         self.source, self.theta_dim, self.y_dim, self.n_noise = str(source), int(theta_dim), int(y_dim), int(n_noise)

@@ -486,6 +486,20 @@ GLABC_API int glabc_run_block_isir(glabc_ctx* ctx, const glabc_run_t* run, const
 /* GLMCMC_NFs.py:73-85,129-140: blk_x = simulate(blk_theta), blk_w = exp(prior + log K - blk_lq), NaN -> 0;
  * `round` keys the simulator's Philox normals (run->seed, run->chain_id_base as usual)                           */
 GLABC_API int glabc_block_weights(glabc_ctx* ctx, const glabc_run_t* run, const glabc_block_isir_t* blk, uint32_t round);
+/* The same two entries for a user-supplied model (glabc_user_model_t, compiled at run time with the model's other kernels):
+ * run->theta [C][theta_dim], run->y [C][y_dim], blk_x [C][B][y_dim]; the LOCAL slot holds a Local_Proposal of any
+ * glabc_dist_kind and of the model's theta_dim.  Semantics of glabc_run_block_isir with the model's prior, simulator and
+ * discrepancy: a local move is theta + z, z ~ Local_Proposal, with no proposal term in the MH ratio (as glabc_run_global_user);
+ * a global move selects among the current state and the next K candidates by a float64 running sum of the weights against a
+ * 53-bit uniform.  glabc_block_weights_user: candidate b of refill `round` draws its simulator normals from Philox blocks of
+ * its own (chain id, step = round, a slot range no step kernel or glabc_user_simulate uses).  Native RNG, FAST arithmetic.
+ * GLABC_ERR_INVALID: an invalid model, a null block buffer, block != K * step_size, K outside 1..GLABC_MAX_K, an unbound LOCAL
+ * slot or one whose dim != theta_dim; GLABC_ERR_UNSUPPORTED: GLABC_ARITH_STRICT or GLABC_RNG_REPLAY.  Both are refused before
+ * anything is launched; n_chains == 0 launches nothing.                                                                    */
+GLABC_API int glabc_run_block_isir_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_block_isir_t* blk,
+                                        const glabc_user_model_t* model);
+GLABC_API int glabc_block_weights_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_block_isir_t* blk, uint32_t round,
+                                       const glabc_user_model_t* model);
 
 /* ---- RealNVP flow on the tensor cores (tcgen05 kind::f16, FP32 accumulate in TMEM) --------------------------
  * NormalizingFlow.sample(n) (GLMCMC_NFs.py:72,127): eps[n][2] standard normals in -> theta[n][2], log_q[n];
