@@ -134,6 +134,9 @@ def AGLMCMC(ABCset, num_ite, Initial_theta, Initial_y, Local_Proposal, Initial_I
     if user and not pooled:
         raise NotImplementedError("AGLMCMC runs a UserModel with pooled=True (one KernelDensity shared by all chains); the "
                                   "per-chain mode's adaptation kernels are built for the fused model family only")
+    if user and ABCset.batched:
+        raise ValueError("pooled AGLMCMC pools one KernelDensity over all chains, which is meaningless across the datasets of "
+                         "a batched UserModel: run each model.dataset(g) on its own")
     if user and ABCset.theta_dim > 4:
         raise NotImplementedError("pooled AGLMCMC with a UserModel needs theta_dim <= 4 (the KernelDensity and proposal-sampling "
                                   "kernels are built for 1..4 dimensions)")

@@ -7,16 +7,17 @@ import torch
 
 from . import _abi
 from .engine import get_engine
-from .GlobalMCMC import run_user_model
+from .GlobalMCMC import refuse_chains_per_dataset, run_user_model
 from .models import UserModel
 from .samplers import run_chains
 
 
 def GLMALA(ABCset, num_ite, Initial_theta, Initial_y, tau, num_grad, filelocation, global_frequency=0,
            Importance_Proposal=None, batch_size=None, *, num_chains=None, seed=None, chain_id_base=0, arith="fast",
-           trace="chain", return_stats=False, verbose=None, device=None, block_threads=0, checkpoint=None, resume=None):
+           trace="chain", return_stats=False, verbose=None, device=None, block_threads=0, checkpoint=None, resume=None,
+           chains_per_dataset=None):
     """Same positional signature and return value as the reference for one chain; keyword extensions as in
-    `GlobalMCMC` (num_chains, seed, chain_id_base, arith, trace, return_stats)."""
+    `GlobalMCMC` (num_chains, seed, chain_id_base, arith, trace, return_stats, chains_per_dataset)."""
     if Importance_Proposal is None or batch_size is None:
         raise ValueError("Importance_Proposal and batch_size are required (GLMALA.py:155,158 dereference them)")
     if not 1 <= int(batch_size) <= _abi.MAX_K:
@@ -28,7 +29,8 @@ def GLMALA(ABCset, num_ite, Initial_theta, Initial_y, tau, num_grad, filelocatio
         eng.bind_proposal(_abi.SLOT_IMPORTANCE, Importance_Proposal)
         return run_user_model(eng, ABCset, "mala", num_ite, Initial_theta, Initial_y, None, filelocation, global_frequency, num_chains,
                               seed, chain_id_base, trace, return_stats, verbose, block_threads, K=int(batch_size), num_grad=int(num_grad),
-                              tau=float(tau), checkpoint=checkpoint, resume=resume)
+                              tau=float(tau), checkpoint=checkpoint, resume=resume, chains_per_dataset=chains_per_dataset)
+    refuse_chains_per_dataset(chains_per_dataset)
     pod = eng.bind_model(ABCset)
     eng.bind_proposal(_abi.SLOT_IMPORTANCE, Importance_Proposal)
     state64 = None      # resume: the carried float64 state comes from the checkpoint (Initial_theta / Initial_y are not read)

@@ -154,6 +154,9 @@ def GLMCMC_NF(ABCset, num_ite, Initial_theta, Initial_y, Local_Proposal, fileloc
         raise ValueError(f"batch_size in 1..{_abi.MAX_K} and batch_size * step_size <= {_abi.AG_MAX_BLOCK}")
     eng = get_engine(device)
     user = isinstance(ABCset, UserModel)      # run-time compiled model (csrc/user_model.cu: glabc_k_block_isir_user)
+    if user and ABCset.batched:
+        raise ValueError("GLMCMC_NF trains one flow on all chains, which is meaningless across the datasets of a batched "
+                         "UserModel: run each model.dataset(g) on its own")
     pod = ABCset if user else eng.bind_model(ABCset)
     if pod.theta_dim != 2:
         raise NotImplementedError("the reference's flow is MLP([1,128,128,2]) couplings: theta_dim must be 2 (GLMCMC_NFs.py:56)")

@@ -109,9 +109,10 @@ USER_SIMULATE, USER_PRIOR, USER_DISCREPANCY, USER_LOG_KERNEL = range(4)
 
 
 class UserModelPOD(C.Structure):
-    """glabc_user_model_t"""
+    """glabc_user_model_t (dataset_params / n_datasets / chains_per_dataset: a batched model, zero otherwise)"""
     _fields_ = [("theta_dim", C.c_int32), ("y_dim", C.c_int32), ("n_noise", C.c_int32), ("n_params", C.c_int32),
-                ("source", C.c_char_p), ("params", C.c_float * USER_MAX_PARAMS), ("epsilon", C.c_double)]
+                ("source", C.c_char_p), ("params", C.c_float * USER_MAX_PARAMS), ("epsilon", C.c_double),
+                ("dataset_params", C.c_void_p), ("n_datasets", C.c_int64), ("chains_per_dataset", C.c_int64)]
 
 
 BW_SILVERMAN, BW_SCOTT = 0, 1

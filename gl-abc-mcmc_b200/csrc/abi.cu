@@ -1366,7 +1366,7 @@ extern "C" int glabc_user_model_check_proposals(const glabc_user_model_t* um, in
     if (log && log_cap) log[0] = '\0';
     if (!um || !um->source) return GLABC_ERR_INVALID;
     if (um->theta_dim < 1 || um->theta_dim > GLABC_MAX_DIM || um->y_dim < 1 || um->y_dim > 2 * GLABC_MAX_DIM || um->n_noise < 0 ||
-        um->n_noise > GLABC_USER_MAX_NOISE || !valid_dist_kind(local_kind) || !valid_dist_kind(far_kind))
+        um->n_noise > GLABC_USER_MAX_NOISE || um->n_datasets < 0 || !valid_dist_kind(local_kind) || !valid_dist_kind(far_kind))
         return GLABC_ERR_INVALID;
     std::string err;
     const int st = user_model_check(cc, *um, local_kind, far_kind, err);
@@ -1391,7 +1391,39 @@ static int check_user_model(glabc_ctx* ctx, const glabc_user_model_t* um, const 
     if (um->n_noise < 0 || um->n_noise > GLABC_USER_MAX_NOISE || um->n_params < 0 || um->n_params > GLABC_USER_MAX_PARAMS)
         return fail(ctx, GLABC_ERR_INVALID, "user model: n_noise in 0..%d, n_params in 0..%d", GLABC_USER_MAX_NOISE, GLABC_USER_MAX_PARAMS);
     if (!(um->epsilon > 0.0)) return fail(ctx, GLABC_ERR_INVALID, "user model: epsilon must be positive");
+    if (um->n_datasets < 0) return fail(ctx, GLABC_ERR_INVALID, "user model: n_datasets must be >= 0");
+    if (um->n_datasets == 0) {
+        if (um->dataset_params || um->chains_per_dataset != 0)
+            return fail(ctx, GLABC_ERR_INVALID, "user model: dataset_params / chains_per_dataset given without n_datasets");
+        return GLABC_OK;
+    }
+    if (!um->dataset_params) return fail(ctx, GLABC_ERR_INVALID, "batched user model: dataset_params is NULL with n_datasets %lld",
+                                         static_cast<long long>(um->n_datasets));
+    if (um->chains_per_dataset < 1) return fail(ctx, GLABC_ERR_INVALID, "batched user model: chains_per_dataset must be >= 1");
+    if (um->chains_per_dataset > INT64_MAX / um->n_datasets)
+        return fail(ctx, GLABC_ERR_INVALID, "batched user model: n_datasets * chains_per_dataset overflows int64");
     return GLABC_OK;
+}
+
+// a batched model's rows (chains or evaluation rows) first .. first + n - 1 must name datasets of its table
+static int check_dataset_rows(glabc_ctx* ctx, const glabc_user_model_t* um, uint64_t first, int64_t n, const char* who)
+{
+    if (um->n_datasets == 0 || n <= 0) return GLABC_OK;
+    const uint64_t total = static_cast<uint64_t>(um->n_datasets) * static_cast<uint64_t>(um->chains_per_dataset);
+    if (first >= total || static_cast<uint64_t>(n) > total - first)
+        return fail(ctx, GLABC_ERR_INVALID, "%s: ids %llu .. %llu reach beyond n_datasets x chains_per_dataset = %llu", who,
+                    static_cast<unsigned long long>(first), static_cast<unsigned long long>(first + n - 1),
+                    static_cast<unsigned long long>(total));
+    return GLABC_OK;
+}
+
+// the batched-model fields of UserRun / UserEval (read by the kernels compiled with -DGLABC_BATCHED only)
+template <class P>
+static void set_dataset_table(const glabc_user_model_t& um, P* p)
+{
+    p->ds_params = um.dataset_params;
+    p->ds_m = um.chains_per_dataset;
+    p->ds_np = um.n_params;
 }
 
 // log K(dis) = kern_c + kern_m * dis^2, the Gaussian ABC kernel of width epsilon (Mixture.py:38-53)
@@ -1407,6 +1439,9 @@ static int run_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_user_mod
     const bool isir = kind >= 1, mala = kind == 2;   // 0 GlobalMCMC, 1 GLMCMC (iSIR), 2 GLMALA
     if (!ctx) return GLABC_ERR_INVALID;
     if (int st = check_user_model(ctx, um, "glabc_run_*_user")) return st;
+    if (run) {   // a batched model's chain ids (a negative chain_id_base reads as one beyond any table)
+        if (int st = check_dataset_rows(ctx, um, static_cast<uint64_t>(run->chain_id_base), run->n_chains, "glabc_run_*_user")) return st;
+    }
     const int d = um->theta_dim;
     const int far_slot = isir ? GLABC_SLOT_IMPORTANCE : GLABC_SLOT_GLOBAL;   // the state-independent proposal of the sampler
     for (int slot : {mala ? far_slot : static_cast<int>(GLABC_SLOT_LOCAL), far_slot}) {
@@ -1484,6 +1519,7 @@ static int run_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_user_mod
     U.gq = make_dist<GLABC_MAX_DIM>(gp);
     user_kernel_consts(*um, &U.kern_c, &U.kern_m);
     for (int k = 0; k < um->n_params; ++k) U.params[k] = um->params[k];
+    set_dataset_table(*um, &U);
     st = user_model_launch(fn, U, mala ? 64 : (block > 128 ? 128 : block), static_cast<cudaStream_t>(run->stream), err);
     if (st) return fail(ctx, st, "%s", err.c_str());
     return GLABC_OK;
@@ -1501,6 +1537,8 @@ static int run_block_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_bl
     const char* who = weights ? "glabc_block_weights_user" : "glabc_run_block_isir_user";
     if (!ctx) return GLABC_ERR_INVALID;
     if (int st = check_user_model(ctx, um, who)) return st;
+    if (um->n_datasets > 0)   // a block-iSIR proposal is trained on, or pooled over, all chains: meaningless across datasets
+        return fail(ctx, GLABC_ERR_UNSUPPORTED, "%s: a batched user model (n_datasets > 0) is not supported", who);
     if (!run || !b) return fail(ctx, GLABC_ERR_INVALID, "%s: null run / block description", who);
     const int d = um->theta_dim;
     if (!ctx->has_dist[GLABC_SLOT_LOCAL]) return fail(ctx, GLABC_ERR_INVALID, "%s needs the LOCAL proposal slot bound", who);
@@ -1600,6 +1638,7 @@ static int eval_user(glabc_ctx* ctx, const glabc_user_model_t* um, int op, const
     E.out = out;
     user_kernel_consts(*um, &E.kern_c, &E.kern_m);
     for (int k = 0; k < um->n_params; ++k) E.params[k] = um->params[k];
+    set_dataset_table(*um, &E);
     st = user_model_eval_launch(fn, E, ctx->sm_count, static_cast<cudaStream_t>(stream), err);
     if (st) return fail(ctx, st, "%s", err.c_str());
     return GLABC_OK;
@@ -1611,6 +1650,7 @@ extern "C" int glabc_user_simulate(glabc_ctx* ctx, const glabc_user_model_t* um,
     if (!ctx) return GLABC_ERR_INVALID;
     if (int st = check_user_model(ctx, um, "glabc_user_simulate")) return st;
     if (n < 0 || (n > 0 && (!theta || !y))) return fail(ctx, GLABC_ERR_INVALID, "glabc_user_simulate: null buffer / n < 0");
+    if (int st = check_dataset_rows(ctx, um, row_base, n, "glabc_user_simulate")) return st;
     return eval_user(ctx, um, GLABC_USER_SIMULATE, theta, n, seed, row_base, y, stream);
 }
 
@@ -1622,6 +1662,7 @@ extern "C" int glabc_user_evaluate(glabc_ctx* ctx, const glabc_user_model_t* um,
     if (op != GLABC_USER_PRIOR && op != GLABC_USER_DISCREPANCY && op != GLABC_USER_LOG_KERNEL)
         return fail(ctx, GLABC_ERR_INVALID, "glabc_user_evaluate: unknown op %d", op);
     if (n < 0 || (n > 0 && (!x || !out))) return fail(ctx, GLABC_ERR_INVALID, "glabc_user_evaluate: null buffer / n < 0");
+    if (int st = check_dataset_rows(ctx, um, 0, n, "glabc_user_evaluate")) return st;
     return eval_user(ctx, um, op, x, n, 0, 0, out, stream);
 }
 

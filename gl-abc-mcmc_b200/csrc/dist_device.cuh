@@ -159,6 +159,11 @@ struct UserRun {
     int num_grad, pad3;
     // appended after the fields above so none of them moves: a Uniform / Gamma / GaussianMixture slot
     DistConstsT<GLABC_MAX_DIM> lq, gq;   // Local_Proposal; Global_Proposal (GlobalMCMC) or Importance_Proposal
+    // appended likewise, read by the batched kernels (-DGLABC_BATCHED) only: chain id g reads row g / ds_m of
+    // ds_params [G][ds_np] in place of params
+    const float* ds_params;
+    long long ds_m;
+    int ds_np, pad4;
 };
 
 // kernel parameter of the user-model evaluation kernel glabc_k_eval_user (user_model.cu): one row per thread,
@@ -172,6 +177,9 @@ struct UserEval {
     float* out;               // y [n][YD] (SIMULATE) or [n]
     float kern_c, kern_m;     // LOG_KERNEL: as UserRun
     float params[GLABC_USER_MAX_PARAMS];
+    const float* ds_params;   // batched (-DGLABC_BATCHED): row r reads row (row_base + r) / ds_m of ds_params [G][ds_np]
+    long long ds_m;
+    int ds_np, pad2;
 };
 
 // kernel parameter of the user-model block-iSIR kernels glabc_k_block_isir_user / glabc_k_block_weights_user (user_model.cu):

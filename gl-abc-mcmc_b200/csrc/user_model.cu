@@ -137,10 +137,17 @@ struct GlabcWords {
 )GLABC";
 
 const char* kKernel = R"GLABC(
-__device__ __forceinline__ float glabc_target(const UserRun& R, const float* th, const float* y)
+// GLABC_PARAMS(S, gid): the params the model functions of chain (or row) `gid` get.  A batched model (-DGLABC_BATCHED)
+// reads row gid / ds_m of the device table ds_params [G][ds_np]; otherwise the kernel parameter's params.
+#ifdef GLABC_BATCHED
+#define GLABC_PARAMS(S, gid) ((S).ds_params + (long long)((u64)(gid) / (u64)(S).ds_m) * (S).ds_np)
+#else
+#define GLABC_PARAMS(S, gid) ((S).params)
+#endif
+__device__ __forceinline__ float glabc_target(const UserRun& R, const float* P, const float* th, const float* y)
 {
-    const float dis = glabc_user_discrepancy(y, R.params);
-    return glabc_user_prior_log_prob(th, R.params) + fmaf(R.kern_m, dis * dis, R.kern_c);
+    const float dis = glabc_user_discrepancy(y, P);
+    return glabc_user_prior_log_prob(th, P) + fmaf(R.kern_m, dis * dis, R.kern_c);
 }
 extern "C" __global__ void __launch_bounds__(128) glabc_k_global_user(const __grid_constant__ UserRun R)
 {
@@ -148,12 +155,13 @@ extern "C" __global__ void __launch_bounds__(128) glabc_k_global_user(const __gr
     if (chain >= R.n_chains) return;
     const u64 gid = ((u64)R.chain_hi0 << 32 | R.chain_lo0) + (u64)chain;
     const u32 g0 = (u32)gid, g1 = (u32)(gid >> 32);
+    const float* P = GLABC_PARAMS(R, gid);   // the chain's dataset row (batched) or R.params
     float th[D], y[YD];
 #pragma unroll
     for (int k = 0; k < D; ++k) th[k] = R.theta[(long long)chain * D + k];
 #pragma unroll
     for (int k = 0; k < YD; ++k) y[k] = R.y[(long long)chain * YD + k];
-    float tgt = glabc_target(R, th, y);
+    float tgt = glabc_target(R, P, th, y);
     float n_glob = 0.f, acc_l = 0.f, acc_g = 0.f, sum[D], sumsq[D], gram[D * (D + 1) / 2];
 #pragma unroll
     for (int k = 0; k < D; ++k) sum[k] = sumsq[k] = 0.f;
@@ -214,8 +222,8 @@ extern "C" __global__ void __launch_bounds__(128) glabc_k_global_user(const __gr
             for (int k = 0; k < D; ++k) thp[k] = th[k] + zl[k];
 #endif
         }
-        glabc_user_simulate(thp, z + D, R.params, yp);
-        const float tgt_p = glabc_target(R, thp, yp);
+        glabc_user_simulate(thp, z + D, P, yp);
+        const float tgt_p = glabc_target(R, P, thp, yp);
         const bool acc = log_u < (tgt_p - tgt) + corr;
         float dl[D];
 #pragma unroll
@@ -267,7 +275,7 @@ extern "C" __global__ void __launch_bounds__(128) glabc_k_global_user(const __gr
 // ---- GLMCMC (iSIR) step for a user model: GLMCMC.py:58-104 with weight_sampling :7-22 --------------------------------
 // gp_* (gq when it is not a DiagGaussian) hold the Importance_Proposal here.  Candidate j of step i is a pure function of (chain, i, j) through Philox, so
 // the K weights are computed first and only the selected candidate is rebuilt — no per-candidate storage.
-__device__ __forceinline__ float glabc_candidate(const UserRun& R, u32 g0, u32 g1, u32 i, int j, float* th, float* y, float& pk)
+__device__ __forceinline__ float glabc_candidate(const UserRun& R, const float* P, u32 g0, u32 g1, u32 i, int j, float* th, float* y, float& pk)
 {
     constexpr int NZ = D + NN, NB = (NZ + 3) / 4;
     float z[NB * 4];
@@ -284,8 +292,8 @@ __device__ __forceinline__ float glabc_candidate(const UserRun& R, u32 g0, u32 g
         th[k] = fmaf(R.gp_scale[k], z[k], R.gp_loc[k]);     // Importance_Proposal.forward, GLMCMC.py:66
         q = fmaf(z[k], z[k], q);
     }
-    glabc_user_simulate(th, z + D, R.params, y);            // :71
-    pk = glabc_target(R, th, y);                            // log prior + log kernel
+    glabc_user_simulate(th, z + D, P, y);                   // :71
+    pk = glabc_target(R, P, th, y);                         // log prior + log kernel
     return pk + 0.5f * q;                                   // log-weight up to the proposal's constant (it cancels in the ratio)
 #else
     GlabcWords ws(g0, g1, i, GLABC_SLOT_CAND + (u32)j * GLABC_CAND_BLOCKS, R.key0, R.key1);
@@ -293,8 +301,8 @@ __device__ __forceinline__ float glabc_candidate(const UserRun& R, u32 g0, u32 g
     const float lq = glabc::dist_forward<D>(R.gq, ws, tj);
 #pragma unroll
     for (int k = 0; k < D; ++k) th[k] = tj[k];
-    glabc_user_simulate(th, z + D, R.params, y);
-    pk = glabc_target(R, th, y);
+    glabc_user_simulate(th, z + D, P, y);
+    pk = glabc_target(R, P, th, y);
     return pk - lq;                                         // log prior + log K - log q, GLMCMC.py:66-74
 #endif
 }
@@ -313,13 +321,14 @@ extern "C" __global__ void __launch_bounds__(128) glabc_k_isir_user(const __grid
     if (chain >= R.n_chains) return;
     const u64 gid = ((u64)R.chain_hi0 << 32 | R.chain_lo0) + (u64)chain;
     const u32 g0 = (u32)gid, g1 = (u32)(gid >> 32);
+    const float* P = GLABC_PARAMS(R, gid);   // the chain's dataset row (batched) or R.params
     const int NK = R.n_candidates;
     float th[D], y[YD];
 #pragma unroll
     for (int k = 0; k < D; ++k) th[k] = R.theta[(long long)chain * D + k];
 #pragma unroll
     for (int k = 0; k < YD; ++k) y[k] = R.y[(long long)chain * YD + k];
-    float pk = glabc_target(R, th, y);
+    float pk = glabc_target(R, P, th, y);
     float lw_old = R.aux[(long long)chain * 8 + 0];
     bool local = R.aux[(long long)chain * 8 + 1] != 0.f;
     float n_glob = 0.f, acc_l = 0.f, acc_g = 0.f, sum[D], sumsq[D], gram[D * (D + 1) / 2];
@@ -365,7 +374,7 @@ extern "C" __global__ void __launch_bounds__(128) glabc_k_isir_user(const __grid
             float lw[17], thc[D], yc[YD], pkc, mx = lw_old;
             lw[0] = lw_old;
             for (int j = 0; j < NK; ++j) {
-                lw[j + 1] = glabc_candidate(R, g0, g1, i, j, thc, yc, pkc);
+                lw[j + 1] = glabc_candidate(R, P, g0, g1, i, j, thc, yc, pkc);
                 if (!(lw[j + 1] == lw[j + 1])) lw[j + 1] = -INFINITY;             // :80-81 NaN weight -> 0
                 mx = fmaxf(mx, lw[j + 1]);
             }
@@ -382,7 +391,7 @@ extern "C" __global__ void __launch_bounds__(128) glabc_k_isir_user(const __grid
                     if (ind < 0 && thr < run) ind = j;
                 }
                 if (ind > 0) {                                                    // :84-88
-                    const float lwn = glabc_candidate(R, g0, g1, i, ind - 1, thc, yc, pkc);
+                    const float lwn = glabc_candidate(R, P, g0, g1, i, ind - 1, thc, yc, pkc);
 #pragma unroll
                     for (int k = 0; k < D; ++k) {
                         dl[k] = thc[k] - th[k];
@@ -409,7 +418,7 @@ extern "C" __global__ void __launch_bounds__(128) glabc_k_isir_user(const __grid
             for (int k = 0; k < D; ++k) thp[k] = th[k] + fmaf(R.lp_scale[k], z[k], R.lp_loc[k]);
             // GLMCMC.py:92-93: while the prior answers with the sentinel, draw the local proposal again (fresh normals from
             // further Philox blocks of the same step; 64 redraws at most, then the proposal stands and is rejected)
-            for (u32 redraw = 0; redraw < 64u && glabc_user_prior_log_prob(thp, R.params) == GLABC_PRIOR_SENTINEL; ++redraw) {
+            for (u32 redraw = 0; redraw < 64u && glabc_user_prior_log_prob(thp, P) == GLABC_PRIOR_SENTINEL; ++redraw) {
                 float zr[((D + 3) / 4) * 4];
 #pragma unroll
                 for (int b = 0; b < (D + 3) / 4; ++b) {
@@ -426,14 +435,14 @@ extern "C" __global__ void __launch_bounds__(128) glabc_k_isir_user(const __grid
             (void)glabc::dist_forward<D>(R.lq, ws, zl);
 #pragma unroll
             for (int k = 0; k < D; ++k) thp[k] = th[k] + zl[k];
-            for (u32 redraw = 0; redraw < 64u && glabc_user_prior_log_prob(thp, R.params) == GLABC_PRIOR_SENTINEL; ++redraw) {
+            for (u32 redraw = 0; redraw < 64u && glabc_user_prior_log_prob(thp, P) == GLABC_PRIOR_SENTINEL; ++redraw) {
                 (void)glabc::dist_forward<D>(R.lq, ws, zl);   // GLMCMC.py:92-93, from the stream's next words
 #pragma unroll
                 for (int k = 0; k < D; ++k) thp[k] = th[k] + zl[k];
             }
 #endif
-            glabc_user_simulate(thp, z + D, R.params, yp);
-            const float pkp = glabc_target(R, thp, yp);
+            glabc_user_simulate(thp, z + D, P, yp);
+            const float pkp = glabc_target(R, P, thp, yp);
             const float log_u = __logf(__uint2float_rn(w0.y >> 8) * 0x1p-24f);
             if (log_u < pkp - pk) {
 #pragma unroll
@@ -493,7 +502,7 @@ extern "C" __global__ void __launch_bounds__(128) glabc_k_isir_user(const __grid
 // A thread per chain for the iSIR global move and the tail of the MALA move; the WARP for the gradient
 // (numberical_gradient_logABC): the chains of a warp that drew a local move are served one after the other, the num_grad
 // common-random-number draws of a dimension dealt over the 32 lanes.  gp_* hold the Importance_Proposal.
-__device__ __forceinline__ void glabc_grad_sums(const UserRun& R, u32 g0, u32 g1, u32 i, u32 slot0, const float* th, int lane,
+__device__ __forceinline__ void glabc_grad_sums(const UserRun& R, const float* P, u32 g0, u32 g1, u32 i, u32 slot0, const float* th, int lane,
                                                 bool mine, float (*sums)[4], float (*cpm)[2])
 {
     constexpr int NB = (NN + 3) / 4 > 0 ? (NN + 3) / 4 : 1;
@@ -506,10 +515,10 @@ __device__ __forceinline__ void glabc_grad_sums(const UserRun& R, u32 g0, u32 g1
         }
 #pragma unroll
         for (int q = 0; q < NB * 4; ++q) zero[q] = 0.f;
-        glabc_user_simulate(tp, zero, R.params, yy);
-        const float cp = glabc_user_discrepancy(yy, R.params);
-        glabc_user_simulate(tm, zero, R.params, yy);
-        const float cm = glabc_user_discrepancy(yy, R.params);
+        glabc_user_simulate(tp, zero, P, yy);
+        const float cp = glabc_user_discrepancy(yy, P);
+        glabc_user_simulate(tm, zero, P, yy);
+        const float cm = glabc_user_discrepancy(yy, P);
         float f1p = 0.f, f2p = 0.f, f1m = 0.f, f2m = 0.f;
         for (int j = lane; j < R.num_grad; j += 32) {
             float z[NB * 4];
@@ -519,10 +528,10 @@ __device__ __forceinline__ void glabc_grad_sums(const UserRun& R, u32 g0, u32 g1
                 glabc_box_muller(w.x, w.y, z[4 * b], z[4 * b + 1]);
                 glabc_box_muller(w.z, w.w, z[4 * b + 2], z[4 * b + 3]);
             }
-            glabc_user_simulate(tp, z, R.params, yy);        // :78-79
-            const float xp = glabc_user_discrepancy(yy, R.params) - cp;
-            glabc_user_simulate(tm, z, R.params, yy);        // :80-83: the same draws (common random numbers)
-            const float xm = glabc_user_discrepancy(yy, R.params) - cm;
+            glabc_user_simulate(tp, z, P, yy);        // :78-79
+            const float xp = glabc_user_discrepancy(yy, P) - cp;
+            glabc_user_simulate(tm, z, P, yy);        // :80-83: the same draws (common random numbers)
+            const float xm = glabc_user_discrepancy(yy, P) - cm;
             f1p += xp; f2p = fmaf(xp, xp, f2p);
             f1m += xm; f2m = fmaf(xm, xm, f2m);
         }
@@ -547,6 +556,7 @@ extern "C" __global__ void __launch_bounds__(64) glabc_k_mala_user(const __grid_
     const int cidx = active ? chain : R.n_chains - 1;
     const u64 gid = ((u64)R.chain_hi0 << 32 | R.chain_lo0) + (u64)cidx;
     const u32 g0 = (u32)gid, g1 = (u32)(gid >> 32);
+    const float* P = GLABC_PARAMS(R, gid);
     const u64 gid0 = ((u64)R.chain_hi0 << 32 | R.chain_lo0) + (u64)(chain - lane);   // the warp's first chain, the same on every lane (tail lanes included)
     const int NK = R.n_candidates;
     float th[D], y[YD], grad[D];
@@ -554,7 +564,7 @@ extern "C" __global__ void __launch_bounds__(64) glabc_k_mala_user(const __grid_
     for (int k = 0; k < D; ++k) th[k] = R.theta[(long long)cidx * D + k];
 #pragma unroll
     for (int k = 0; k < YD; ++k) y[k] = R.y[(long long)cidx * YD + k];
-    float pk = glabc_target(R, th, y);
+    float pk = glabc_target(R, P, th, y);
     float lw_old = R.aux[(long long)cidx * 8 + 0];
     bool local = R.aux[(long long)cidx * 8 + 1] != 0.f, have_grad = R.aux[(long long)cidx * 8 + 2] != 0.f;
 #pragma unroll
@@ -587,7 +597,7 @@ extern "C" __global__ void __launch_bounds__(64) glabc_k_mala_user(const __grid_
                 ta[q] = q == k ? __fadd_rn(tt[q], 0.00001f) : tt[q];      // GLMALA.py:84-85, float32 finite difference
                 tb[q] = q == k ? __fsub_rn(tt[q], 0.00001f) : tt[q];
             }
-            const float gprior = __fdiv_rn(__fsub_rn(glabc_user_prior_log_prob(ta, R.params), glabc_user_prior_log_prob(tb, R.params)), 2e-5f);
+            const float gprior = __fdiv_rn(__fsub_rn(glabc_user_prior_log_prob(ta, P), glabc_user_prior_log_prob(tb, P)), 2e-5f);
             const float mup = fmaf(sums[k][0], rn, cpm[k][0]), mum = fmaf(sums[k][2], rn, cpm[k][1]);
             const float vp = fmaf(fmaf(-sums[k][0] * rn, sums[k][0], sums[k][1]), rn1, R.eps2);
             const float vm = fmaf(fmaf(-sums[k][2] * rn, sums[k][2], sums[k][3]), rn1, R.eps2);
@@ -621,7 +631,7 @@ extern "C" __global__ void __launch_bounds__(64) glabc_k_mala_user(const __grid_
             float lw[17], thc[D], yc[YD], pkc, mx = lw_old;
             lw[0] = lw_old;
             for (int j = 0; j < NK; ++j) {
-                lw[j + 1] = glabc_candidate(R, g0, g1, i, j, thc, yc, pkc);
+                lw[j + 1] = glabc_candidate(R, P, g0, g1, i, j, thc, yc, pkc);
                 if (!(lw[j + 1] == lw[j + 1])) lw[j + 1] = -INFINITY;
                 mx = fmaxf(mx, lw[j + 1]);
             }
@@ -638,7 +648,7 @@ extern "C" __global__ void __launch_bounds__(64) glabc_k_mala_user(const __grid_
                     if (ind < 0 && thr < run) ind = j;
                 }
                 if (ind > 0) {                                                    // :175-179: the cached gradient is NOT refreshed (B-6)
-                    const float lwn = glabc_candidate(R, g0, g1, i, ind - 1, thc, yc, pkc);
+                    const float lwn = glabc_candidate(R, P, g0, g1, i, ind - 1, thc, yc, pkc);
 #pragma unroll
                     for (int k = 0; k < D; ++k) {
                         dl[k] = thc[k] - th[k];
@@ -686,7 +696,13 @@ extern "C" __global__ void __launch_bounds__(64) glabc_k_mala_user(const __grid_
 #pragma unroll
                     for (int k = 0; k < D; ++k) ts[k] = __shfl_sync(0xffffffffu, thp[k], src);
                     const u64 gs = gid0 + (u64)src;
-                    glabc_grad_sums(R, (u32)gs, (u32)(gs >> 32), i, pass == 0 ? 0x20000u : 0x10000u, ts, lane, lane == src, sums, cpm);
+#ifdef GLABC_BATCHED
+                    // the whole warp works for chain src, so it reads src's row: a warp may span several datasets
+                    const float* Ps = reinterpret_cast<const float*>(__shfl_sync(0xffffffffu, reinterpret_cast<u64>(P), src));
+#else
+                    const float* Ps = P;
+#endif
+                    glabc_grad_sums(R, Ps, (u32)gs, (u32)(gs >> 32), i, pass == 0 ? 0x20000u : 0x10000u, ts, lane, lane == src, sums, cpm);
                 }
                 if (pass == 0 ? (is_local && !have_grad) : is_local) {
                     float gout[D];
@@ -701,8 +717,8 @@ extern "C" __global__ void __launch_bounds__(64) glabc_k_mala_user(const __grid_
             }
             if (is_local) {
                 float yp[YD], lr = 0.f;
-                glabc_user_simulate(thp, z + D, R.params, yp);                    // :188-189
-                const float pkp = glabc_target(R, thp, yp);
+                glabc_user_simulate(thp, z + D, P, yp);                    // :188-189
+                const float pkp = glabc_target(R, P, thp, yp);
 #pragma unroll
                 for (int k = 0; k < D; ++k) {
                     const float r = ((th[k] - thp[k]) - gp[k] * half_tau2) * inv_tau;   // log_proposal, :97-116
@@ -771,7 +787,8 @@ extern "C" __global__ void __launch_bounds__(64) glabc_k_mala_user(const __grid_
 
 // ---- the model's functions outside a run: generate_samples / prior_log_prob / discrepancy / calculate_log_kernel ------
 // One row per thread, grid-stride.  SIMULATE row r draws its NN normals as a step kernel draws its simulator noise, from the
-// Philox blocks (row_base + r, step 0, slot 2 + b): step 0 is no step's, see the slot table.
+// Philox blocks (row_base + r, step 0, slot 2 + b): step 0 is no step's, see the slot table.  A batched model evaluates row r
+// with dataset (row_base + r) / ds_m, so the SIMULATE row chain_id_base + c is chain c's initial y with its own dataset.
 extern "C" __global__ void __launch_bounds__(256) glabc_k_eval_user(const __grid_constant__ UserEval E)
 {
     const u64 row0 = (u64)E.row_hi << 32 | E.row_lo;
@@ -784,13 +801,14 @@ extern "C" __global__ void __launch_bounds__(256) glabc_k_eval_user(const __grid
 #pragma unroll
             for (int k = 0; k < D; ++k) th[k] = E.in[r * D + k];
             const u64 gid = row0 + (u64)r;
+            const float* P = GLABC_PARAMS(E, gid);
 #pragma unroll
             for (int b = 0; b < NB; ++b) {
                 const uint4 w = glabc_philox((u32)gid, (u32)(gid >> 32), 0u, 2u + b, E.key0, E.key1);
                 glabc_box_muller(w.x, w.y, z[4 * b], z[4 * b + 1]);
                 glabc_box_muller(w.z, w.w, z[4 * b + 2], z[4 * b + 3]);
             }
-            glabc_user_simulate(th, z, E.params, y);
+            glabc_user_simulate(th, z, P, y);
 #pragma unroll
             for (int k = 0; k < YD; ++k) E.out[r * YD + k] = y[k];
         }
@@ -799,7 +817,8 @@ extern "C" __global__ void __launch_bounds__(256) glabc_k_eval_user(const __grid
             float th[D];
 #pragma unroll
             for (int k = 0; k < D; ++k) th[k] = E.in[r * D + k];
-            E.out[r] = glabc_user_prior_log_prob(th, E.params);
+            const float* P = GLABC_PARAMS(E, row0 + (u64)r);
+            E.out[r] = glabc_user_prior_log_prob(th, P);
         }
     } else {                                   // DISCREPANCY, LOG_KERNEL (the kernel term of glabc_target)
         const bool log_kernel = E.op == GLABC_USER_LOG_KERNEL;
@@ -807,7 +826,8 @@ extern "C" __global__ void __launch_bounds__(256) glabc_k_eval_user(const __grid
             float y[YD];
 #pragma unroll
             for (int k = 0; k < YD; ++k) y[k] = E.in[r * YD + k];
-            const float dis = glabc_user_discrepancy(y, E.params);
+            const float* P = GLABC_PARAMS(E, row0 + (u64)r);
+            const float dis = glabc_user_discrepancy(y, P);
             E.out[r] = log_kernel ? fmaf(E.kern_m, dis * dis, E.kern_c) : dis;
         }
     }
@@ -1093,12 +1113,14 @@ std::mutex g_cache_mu;
 // key: model_key() + proposal kinds, so the modules of one model are adjacent in the map
 std::map<std::string, Compiled> g_cache;
 
-// device | arch | dims | n_noise | source length | source: names a model, whatever the proposal kinds it was compiled for
+// device | arch | dims | n_noise | batched | source length | source: names a model, whatever the proposal kinds it was
+// compiled for.  Neither the params nor a batched model's table or chains_per_dataset: they are launch arguments.
 std::string model_key(int device, int cc, const glabc_user_model_t& um)
 {
     const size_t len = strlen(um.source);
     char head[160];
-    snprintf(head, sizeof(head), "%d|%d|%d|%d|%d|%zu|", device, cc, um.theta_dim, um.y_dim, um.n_noise, len);
+    snprintf(head, sizeof(head), "%d|%d|%d|%d|%d|%d|%zu|", device, cc, um.theta_dim, um.y_dim, um.n_noise, um.n_datasets > 0 ? 1 : 0,
+             len);
     return std::string(head) + std::string(um.source, len);
 }
 
@@ -1111,7 +1133,8 @@ std::string cu_err(Dyn& d, CUresult r)
 
 }  // namespace
 
-// NVRTC: prelude + user source + step kernel -> cubin for sm_<cc>, the Local / Global-or-Importance proposal kinds fixed
+// NVRTC: prelude + user source + step kernel -> cubin for sm_<cc>, the Local / Global-or-Importance proposal kinds fixed;
+// a batched model (n_datasets > 0) compiles with -DGLABC_BATCHED
 static int compile_to_cubin(Dyn& d, int cc, const glabc_user_model_t& um, int lp_kind, int gp_kind, std::vector<char>& cubin,
                             std::string& err)
 {
@@ -1146,8 +1169,9 @@ static int compile_to_cubin(Dyn& d, int cc, const glabc_user_model_t& um, int lp
     snprintf(ops[2], sizeof(ops[2]), "-DGLABC_USER_DISCREPANCY=%d", GLABC_USER_DISCREPANCY);
     snprintf(ops[3], sizeof(ops[3]), "-DGLABC_USER_LOG_KERNEL=%d", GLABC_USER_LOG_KERNEL);
     const char* opts[] = {arch, dD, dY, dN, dLP, dGP, kinds[0], kinds[1], kinds[2], kinds[3], sizes[0], sizes[1], sizes[2],
-                          ops[0], ops[1], ops[2], ops[3], "--std=c++17", "--use_fast_math", "-lineinfo"};
-    r = d.compileProgram(prog, static_cast<int>(sizeof(opts) / sizeof(opts[0])), opts);
+                          ops[0], ops[1], ops[2], ops[3], "--std=c++17", "--use_fast_math", "-lineinfo", "-DGLABC_BATCHED"};
+    const int n_opts = static_cast<int>(sizeof(opts) / sizeof(opts[0])) - (um.n_datasets > 0 ? 0 : 1);
+    r = d.compileProgram(prog, n_opts, opts);
     if (r != NVRTC_SUCCESS) {
         size_t n = 0;
         d.getLogSize(prog, &n);

@@ -155,11 +155,12 @@ class Engine:
 
     def run_user(self, model, *, theta, y, n_steps, gf, step_base=0, chain_id_base=0, seed=0, trace_layout=_abi.TRACE_CHAIN_MAJOR,
                  trace=None, trace_rows=None, trace_row_base=0, write_row0=True, stats=None, block_threads=0, sampler="global", K=0,
-                 aux=None, num_grad=0, tau=0.0, blk=None, round=0):
+                 aux=None, num_grad=0, tau=0.0, blk=None, round=0, chains_per_dataset=0):
         """GlobalMCMC (`sampler="global"`, LOCAL / GLOBAL slots), GLMCMC (`"isir"`, LOCAL / IMPORTANCE slots, K candidates, aux) or
         GLMALA (`"mala"`, IMPORTANCE slot, K, tau, num_grad, aux) transitions for a `models.UserModel` (compiled on first use).
         `"block_isir"` / `"block_weights"`: the block-iSIR step against the candidate block `blk` (a BlockIsirPOD, LOCAL slot,
-        K candidates per global move) and the weights of refill `round` (glabc_run_block_isir_user / glabc_block_weights_user)."""
+        K candidates per global move) and the weights of refill `round` (glabc_run_block_isir_user / glabc_block_weights_user).
+        A batched model runs chain id g against dataset g // chains_per_dataset."""
         cn, d = theta.shape
         rows = trace_rows if trace_rows is not None else step_base + n_steps + 1 - trace_row_base
         if trace is None and trace_layout != _abi.TRACE_NONE:
@@ -172,7 +173,7 @@ class Engine:
                         trace_row_base=trace_row_base, theta=self._ptr(theta), y=self._ptr(y), aux=self._ptr(aux),
                         trace=self._ptr(trace), stats=self._ptr(stats), stream=self._stream(), num_grad=int(num_grad), tau=float(tau),
                         tau64=float(tau))
-        pod = model.user_pod()
+        pod = model.user_pod(self.device, chains_per_dataset)
         if sampler == "block_isir":
             self.ctx.check(self.lib.glabc_run_block_isir_user(self.ctx.handle, C.byref(r), C.byref(blk), C.byref(pod)))
             return trace
@@ -184,12 +185,13 @@ class Engine:
         self.ctx.check(fn(self.ctx.handle, C.byref(r), C.byref(pod)))
         return trace
 
-    def user_simulate(self, model, theta, seed, row_base=0):
+    def user_simulate(self, model, theta, seed, row_base=0, chains_per_dataset=0):
         """y [n, y_dim]: one draw of a `models.UserModel`'s simulator per row of theta [n, theta_dim] (glabc_user_simulate;
-        row r draws from the Philox stream of id row_base + r at step 0)"""
+        row r draws from the Philox stream of id row_base + r at step 0, a batched model's with dataset
+        (row_base + r) // chains_per_dataset)"""
         theta = self._f32(theta).reshape(-1, model.theta_dim)
         y = torch.empty(theta.shape[0], model.y_dim, dtype=torch.float32, device=self.device)
-        pod = model.user_pod()
+        pod = model.user_pod(self.device, chains_per_dataset)
         self.ctx.check(self.lib.glabc_user_simulate(self.ctx.handle, C.byref(pod), self._ptr(theta), theta.shape[0],
                                                     int(seed) & 0xFFFFFFFFFFFFFFFF, int(row_base) & 0xFFFFFFFFFFFFFFFF,
                                                     self._ptr(y), self._stream()))

@@ -139,14 +139,61 @@ class UserModel:
 
     Samplers that take it: GlobalMCMC, GLMCMC, GLMALA (theta_dim <= 5), GLMCMC_NF (theta_dim 2: the flow) and
     AGLMCMC(..., pooled=True) (theta_dim <= 4: the KernelDensity kernels), the last two through the block-iSIR kernels compiled
-    with the model.  Per-chain AGLMCMC (pooled=False) refuses it: its adaptation kernels are built for the fused family."""
+    with the model.  Per-chain AGLMCMC (pooled=False) refuses it: its adaptation kernels are built for the fused family.
+
+    A 2-D `params` of shape [G, n_params] makes a *batched* model: G observed datasets fitted in one run (simulation-based
+    calibration, coverage studies, many subjects with one simulator).  GlobalMCMC, GLMCMC and GLMALA then take
+    `chains_per_dataset=m`: the chain with global id `chain_id_base + c` belongs to dataset `(chain_id_base + c) // m` and
+    its model functions read that dataset's row, so a chain-major trace [G m, rows, d] views as [G, m, rows, d].  Chain g of
+    a batched run equals chain g of a run of `dataset(g // m)` (same seed, same global id), bit for bit.  The plugin methods
+    of a batched model refuse to run (use `dataset(g)`), and GLMCMC_NF / pooled AGLMCMC refuse it: they train one proposal
+    on all chains."""
 
     def __init__(self, source, theta_dim, y_dim, n_noise, epsilon, params=()):
         self.source, self.theta_dim, self.y_dim, self.n_noise = str(source), int(theta_dim), int(y_dim), int(n_noise)
         self.epsilon = float(epsilon)
+        self.table = None                         # batched: float32 [G, n_params] on the CPU
+        self._dev_table = {}                      # its device copies, by device
+        if getattr(params, "ndim", None) == 2 or (isinstance(params, (list, tuple)) and len(params) > 0
+                                                   and all(isinstance(r, (list, tuple)) for r in params)):
+            table = torch.as_tensor(params, dtype=torch.float32).detach().cpu().contiguous()
+            if table.shape[0] < 1:
+                raise ValueError("a batched UserModel needs at least one dataset (params of shape [G, n_params], G >= 1)")
+            if table.shape[1] > _abi.USER_MAX_PARAMS:
+                raise ValueError(f"at most {_abi.USER_MAX_PARAMS} params")
+            self.table = table
+            self.params = None
+            return
         self.params = [float(p) for p in params]
         if len(self.params) > _abi.USER_MAX_PARAMS:
             raise ValueError(f"at most {_abi.USER_MAX_PARAMS} params")
+
+    @property
+    def batched(self):
+        return self.table is not None
+
+    @property
+    def n_datasets(self):
+        """G of a batched model, 1 otherwise"""
+        return self.table.shape[0] if self.batched else 1
+
+    @property
+    def n_params(self):
+        return self.table.shape[1] if self.batched else len(self.params)
+
+    def dataset(self, g):
+        """the ordinary single-dataset UserModel of row g (itself for g == 0 of an unbatched model)"""
+        g = int(g)
+        if not 0 <= g < self.n_datasets:
+            raise IndexError(f"dataset {g} of {self.n_datasets}")
+        if not self.batched:
+            return self
+        return UserModel(self.source, self.theta_dim, self.y_dim, self.n_noise, self.epsilon, params=self.table[g].tolist())
+
+    def _single(self, what):
+        if self.batched:
+            raise ValueError(f"{what} of a batched UserModel ({self.n_datasets} datasets) is ambiguous: call it on "
+                             "model.dataset(g), the single-dataset model of row g")
 
     # -- plugin methods (reference Mixture.py:13-53), compiled -----------------------------------
     def generate_samples(self, theta, num_samples=1, *, seed=None, row_base=0):
@@ -154,6 +201,7 @@ class UserModel:
         for m = 1 and [n, m, y_dim] for m > 1.  Row i * m + j (repeat j of theta row i) draws its noise from the Philox stream
         of id row_base + i * m + j at step 0 under key `seed` (default: samplers.default_seed()), so
         `generate_samples(theta0, seed=s, row_base=chain_id_base)` is the initial y a run with seed s draws for Initial_y=None."""
+        self._single("generate_samples")
         from .engine import get_engine
         from .samplers import default_seed
         eng = get_engine()
@@ -171,10 +219,12 @@ class UserModel:
         return y if n == 1 or m == 1 else y.view(n, m, self.y_dim)
 
     def prior_log_prob(self, samples):
+        self._single("prior_log_prob")
         from .engine import get_engine
         return get_engine().user_evaluate(self, _abi.USER_PRIOR, torch.as_tensor(samples).reshape(-1, self.theta_dim))
 
     def discrepancy(self, y):
+        self._single("discrepancy")
         from .engine import get_engine
         return get_engine().user_evaluate(self, _abi.USER_DISCREPANCY, torch.as_tensor(y).reshape(-1, self.y_dim))
 
@@ -190,6 +240,7 @@ class UserModel:
     def calculate_log_kernel(self, y, epsilon=None):
         """the step kernels' kernel term of the model's epsilon, on the device; another epsilon goes through
         calculate_log_kernel_dis"""
+        self._single("calculate_log_kernel")
         if epsilon is not None and float(epsilon) != self.epsilon:
             return self.calculate_log_kernel_dis(self.discrepancy(y), epsilon)
         from .engine import get_engine
@@ -197,24 +248,41 @@ class UserModel:
 
     def fingerprint(self):
         """sha256 of what a run computes with: source, dims, n_noise, params (as the float32 the kernels read) and epsilon.
-        A user-model checkpoint carries it, and a resume refuses a checkpoint of another model."""
+        A user-model checkpoint carries it, and a resume refuses a checkpoint of another model.  A batched model's covers its
+        whole table (G, n_params and every row)."""
         h = hashlib.sha256()
-        h.update(struct.pack("<4i", self.theta_dim, self.y_dim, self.n_noise, len(self.params)))
-        h.update(torch.tensor(self.params, dtype=torch.float32).numpy().tobytes())
+        h.update(struct.pack("<4i", self.theta_dim, self.y_dim, self.n_noise, self.n_params))
+        if self.batched:
+            h.update(struct.pack("<q", self.n_datasets))
+            h.update(self.table.numpy().tobytes())
+        else:
+            h.update(torch.tensor(self.params, dtype=torch.float32).numpy().tobytes())
         h.update(struct.pack("<d", self.epsilon))
         h.update(self.source.encode())
         return h.hexdigest()
 
-    def user_pod(self):
-        pod = _abi.UserModelPOD(theta_dim=self.theta_dim, y_dim=self.y_dim, n_noise=self.n_noise, n_params=len(self.params),
+    def user_pod(self, device=None, chains_per_dataset=0):
+        """glabc_user_model_t.  A batched model's table is copied to `device` (once; the copy lives as long as the model), or
+        left NULL without a device (a compile check needs none)."""
+        pod = _abi.UserModelPOD(theta_dim=self.theta_dim, y_dim=self.y_dim, n_noise=self.n_noise, n_params=self.n_params,
                                 source=self.source.encode(), epsilon=self.epsilon)
-        _abi.fill(pod.params, self.params)
+        if not self.batched:
+            _abi.fill(pod.params, self.params)
+            return pod
+        pod.n_datasets = self.n_datasets
+        pod.chains_per_dataset = int(chains_per_dataset)
+        if device is not None:
+            key = str(torch.device(device))
+            if key not in self._dev_table:
+                self._dev_table[key] = self.table.to(device)
+            pod.dataset_params = self._dev_table[key].data_ptr()
         return pod
 
     def check(self, cc=100, proposals=None):
         """compile-only validation (NVRTC, no GPU needed); raises ValueError with the compiler log.
         `proposals`: the (Local_Proposal, Global_Proposal or Importance_Proposal) pair a run will bind, to compile the
-        kernels for their kinds; None in either place (GLMALA has no Local_Proposal) or for the pair means DiagGaussian."""
+        kernels for their kinds; None in either place (GLMALA has no Local_Proposal) or for the pair means DiagGaussian.
+        A batched model compiles the batched kernels."""
         import ctypes as C
         log = C.create_string_buffer(8192)
         pod = self.user_pod()

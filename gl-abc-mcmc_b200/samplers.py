@@ -78,13 +78,15 @@ CHECKPOINT_VERSION = 1
 
 
 def save_checkpoint(path, *, sampler, step_base, seed, chain_id_base, theta, y, stats, aux=None, state64=None, ag_state=None,
-                    model=None):
+                    model=None, chains_per_dataset=None):
     """Everything a run needs to continue bit-identically (SURVEY.md 8(f) n4): the chain state, the carried iSIR / MALA
     state, the statistics accumulators and the Philox coordinates (seed, global chain id base, next step index) — the
     generator itself is stateless, so no RNG state exists beyond these three integers.  `model`: a user model's
-    fingerprint (models.UserModel.fingerprint)."""
+    fingerprint (models.UserModel.fingerprint); `chains_per_dataset`: a batched user model's m."""
     cpu = lambda t: None if t is None else t.detach().cpu()  # noqa: E731
     extra = {} if model is None else dict(model=model)
+    if chains_per_dataset is not None:
+        extra["chains_per_dataset"] = int(chains_per_dataset)
     torch.save(dict(version=CHECKPOINT_VERSION, sampler=sampler, step_base=int(step_base), seed=int(seed),
                     chain_id_base=int(chain_id_base), theta=cpu(theta), y=cpu(y), stats=cpu(stats), aux=cpu(aux),
                     state64=cpu(state64), ag_state=cpu(ag_state), **extra), path)

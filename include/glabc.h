@@ -311,7 +311,17 @@ typedef struct {
  *   __device__ float glabc_user_prior_log_prob(const float* theta, const float* params);      (Mixture.py:28-31)
  *   __device__ float glabc_user_discrepancy(const float* y, const float* params);             (Mixture.py:33-36)
  *
- * `params` (<= GLABC_USER_MAX_PARAMS floats) carries the model's constants (y_obs, noise scales, ...).            */
+ * `params` (<= GLABC_USER_MAX_PARAMS floats) carries the model's constants (y_obs, noise scales, ...).
+ *
+ * Batched model: many observed datasets in one run.  The three trailing fields (appended, so no earlier field moves)
+ * describe a DEVICE table dataset_params[n_datasets][n_params], read-only while a launch runs; `params` is then unused.
+ * The chain with global id g = chain_id_base + c belongs to dataset g / chains_per_dataset, and every model function
+ * that chain calls gets that dataset's row; chain ids must stay below n_datasets * chains_per_dataset.  The kernels are
+ * a separate compile of the same program (-DGLABC_BATCHED) and draw exactly the random numbers of the one-dataset
+ * kernels, so chain g of a batched run equals chain g of a one-dataset run with params = row g / chains_per_dataset.
+ * All three zero (NULL) is the one-dataset model.  GLABC_ERR_INVALID, before any launch: n_datasets < 0, a NULL table
+ * with n_datasets > 0, a table without n_datasets, chains_per_dataset < 1 for a batched model (or != 0 for another),
+ * n_datasets * chains_per_dataset beyond int64.                                                                     */
 #define GLABC_USER_MAX_PARAMS 64
 #define GLABC_USER_MAX_NOISE 32
 typedef struct {
@@ -322,6 +332,9 @@ typedef struct {
     const char* source;       /* NUL-terminated CUDA C++ defining the three functions above                  */
     float params[GLABC_USER_MAX_PARAMS];
     double epsilon;           /* width of the Gaussian ABC kernel (Mixture.py:7,43)                          */
+    const float* dataset_params;   /* batched: DEVICE [n_datasets][n_params], row g = the params of dataset g; NULL otherwise */
+    int64_t n_datasets;            /* batched: G >= 1; 0 otherwise                                               */
+    int64_t chains_per_dataset;    /* batched: m >= 1, chain id g -> dataset g / m; 0 otherwise                  */
 } glabc_user_model_t;
 
 typedef struct glabc_ctx glabc_ctx;
@@ -414,7 +427,11 @@ GLABC_API int glabc_run_aglmcmc(glabc_ctx* ctx, const glabc_run_t* run, const gl
  * Semantics of the proposals as glabc_run_global's general kernel: a local move is theta + z, z ~ Local_Proposal, with no
  * proposal term in the MH ratio (so an asymmetric Gamma local proposal gives the reference's biased chain); a global move
  * adds log q(theta) - log q(theta').  Two DiagGaussian slots run the fused Gaussian arithmetic; the simulator's noise is
- * drawn from the same random numbers whatever the proposal kinds.                                                     */
+ * drawn from the same random numbers whatever the proposal kinds.
+ * A batched model (glabc_user_model_t.n_datasets > 0) runs chain id chain_id_base + c against dataset
+ * (chain_id_base + c) / chains_per_dataset with the same draws; ids at or beyond n_datasets * chains_per_dataset are
+ * GLABC_ERR_INVALID, as is an invalid table description (see glabc_user_model_t), before anything is launched.  The same
+ * holds for glabc_run_isir_user and glabc_run_mala_user.                                                                */
 GLABC_API int glabc_run_global_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_user_model_t* model);
 /* GLMCMC loop body (GLMCMC.py:58-104, weight_sampling :7-22) for a user-supplied model: LOCAL = Local_Proposal, IMPORTANCE =
  * Importance_Proposal (any glabc_dist_kind, as glabc_run_global_user), run->n_candidates = batch_size, run->aux as
@@ -426,7 +443,8 @@ GLABC_API int glabc_run_isir_user(glabc_ctx* ctx, const glabc_run_t* run, const 
 /* GLMALA (GLMALA.py:150-200) for a user model: IMPORTANCE slot (any glabc_dist_kind, its global move as
  * glabc_run_isir_user), run->n_candidates, run->tau, run->num_grad; aux [C][8] carries
  * the cached log-weight (slot 0), the `local` flag (1), "gradient cached" (2) and the cached gradient (3 ..): theta_dim <= 5.
- * A thread per chain; the finite-difference gradient's draws (GLMALA.py:46-95) are dealt over the warp.                    */
+ * A thread per chain; the finite-difference gradient's draws (GLMALA.py:46-95) are dealt over the warp, which evaluates
+ * them with the served chain's dataset row when the model is batched.                                                      */
 GLABC_API int glabc_run_mala_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_user_model_t* model);
 /* Compile-only check of a user model for compute capability `cc` (100 = sm_100a): needs NVRTC but neither a GPU nor a
  * context.  The NVRTC log (or "" on success) is copied to log[log_cap].  Compiles the kernels for DiagGaussian proposals. */
@@ -456,7 +474,10 @@ typedef enum {
  * depends on the chain's global id only, not on the shard that runs it.                                                     */
 GLABC_API int glabc_user_simulate(glabc_ctx* ctx, const glabc_user_model_t* model, const float* theta, int64_t n, uint64_t seed,
                                   uint64_t row_base, float* y, void* stream);
-/* op = GLABC_USER_PRIOR, GLABC_USER_DISCREPANCY or GLABC_USER_LOG_KERNEL on the n rows of x, out[n] float32.                  */
+/* A batched model: row r of glabc_user_simulate uses dataset (row_base + r) / chains_per_dataset, so row chain_id_base + c is
+ * chain c's initial y with its own dataset; row r of glabc_user_evaluate uses dataset r / chains_per_dataset.  Rows at or beyond
+ * n_datasets * chains_per_dataset are GLABC_ERR_INVALID.
+ * op = GLABC_USER_PRIOR, GLABC_USER_DISCREPANCY or GLABC_USER_LOG_KERNEL on the n rows of x, out[n] float32.                  */
 GLABC_API int glabc_user_evaluate(glabc_ctx* ctx, const glabc_user_model_t* model, int32_t op, const float* x, int64_t n, float* out,
                                   void* stream);
 
@@ -494,7 +515,8 @@ GLABC_API int glabc_block_weights(glabc_ctx* ctx, const glabc_run_t* run, const 
  * 53-bit uniform.  glabc_block_weights_user: candidate b of refill `round` draws its simulator normals from Philox blocks of
  * its own (chain id, step = round, a slot range no step kernel or glabc_user_simulate uses).  Native RNG, FAST arithmetic.
  * GLABC_ERR_INVALID: an invalid model, a null block buffer, block != K * step_size, K outside 1..GLABC_MAX_K, an unbound LOCAL
- * slot or one whose dim != theta_dim; GLABC_ERR_UNSUPPORTED: GLABC_ARITH_STRICT or GLABC_RNG_REPLAY.  Both are refused before
+ * slot or one whose dim != theta_dim; GLABC_ERR_UNSUPPORTED: GLABC_ARITH_STRICT, GLABC_RNG_REPLAY or a batched model (one
+ * proposal trained on or pooled over all chains means nothing across datasets).  Both are refused before
  * anything is launched; n_chains == 0 launches nothing.                                                                    */
 GLABC_API int glabc_run_block_isir_user(glabc_ctx* ctx, const glabc_run_t* run, const glabc_block_isir_t* blk,
                                         const glabc_user_model_t* model);
